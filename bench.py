@@ -514,6 +514,8 @@ def run_ours(a):
     ms = D.max_over_ranks(ms_local, dev)
     kernel_ms = sum(x.elapsed_time(y) for x, y in kernel_events) / len(kernel_events)
     value = npix * spp * world * a.steps / (ms * 1e-3)
+    if a.dump_outputs and rank == 0:  # the last timed step's images, before the legs below render into the same buffers
+        dump_outputs(a.dump_outputs, {"hdr": r.hdr_image(), "ldr": r.ldr_image()})
     cell_used = grid_cell(r)  # before other scenes are loaded into the renderer
     base_volume, base_camera, base_lights = r.volume, r.camera, list(r.lights)  # the PODs of the benched scene (copies are taken by the oracle)
     gather = gather_ceilings(r) if rank == 0 else None
@@ -1226,6 +1228,28 @@ def run_reference(a):
         print("mapped:", libs, file=sys.stderr)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, images):
+    """Writes each (H, W, C) image as out_dir/<name>.npy in float32.  Above DUMP_LIMIT_BYTES in all, the same fixed,
+    seeded sample of pixels is written for every image, with its flat pixel indices as pixel_index.npy (float64), so that
+    two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {name: img.float().cpu().numpy() for name, img in images.items()}
+    total = sum(v.size * 4 for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        H, W = next(iter(arrays.values())).shape[:2]
+        keep = int(H * W * (DUMP_LIMIT_BYTES - 4096) // (total + 8 * H * W))  # 4 KiB for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(H * W, size=keep, replace=False))
+        arrays = {name: v.reshape(H * W, -1)[idx] for name, v in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v)
+
+
 _REAL_STDOUT = None
 
 
@@ -1265,7 +1289,11 @@ def main():
     ap.add_argument("--c5", action="store_true", help="run the C5 line at any N > 1")
     ap.add_argument("--ref-device", default="cuda", choices=["cuda", "cpu"])
     ap.add_argument("--ref-r32", action="store_true", help="reference built with the shipped -maxrregcount=32")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the HDR and tone-mapped images of the last timed step as DIR/<name>.npy (float32)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the product's timed path (--impl ours)")
     a.warmup = max(a.warmup, 0)
     world = env_int("WORLD_SIZE", 1)
     if a.impl == "ours" and world != a.gpus and world == 1 and a.gpus > 1:

@@ -144,6 +144,28 @@ def ref(width, height, r32=False, f32=False, env=False):
     return lib
 
 
+GOLDEN_KERNELS = os.path.join(os.path.dirname(_HERE), "tests", "golden", "reference_kernels.npz")
+
+
+def load_golden_scene(r, g, name):
+    """Loads scene `name` of tests/golden/reference_kernels.npz (what the reference's own kernels rendered, stored by
+    tests/golden/make_golden.py) into the product renderer r; returns (step size, trace depth, frames)."""
+    from sunvolumerender_b200 import scene as S
+
+    n, fmt, W, H, depth, frames, nl = [int(v) for v in g[f"{name}_meta"]]
+    r.load_volume(g[f"{name}_vox"], fmt, (n, n, n))
+    stored = L.Volume.from_buffer_copy(bytes(g[f"{name}_volume"]))
+    for f in ("densityScale", "invMaxMagnitude", "gradientFactor"):
+        assert getattr(r.volume, f) == getattr(stored, f), f
+    assert r.volume.bbox.vmin.tuple() == stored.bbox.vmin.tuple() and r.volume.bbox.invSize.tuple() == stored.bbox.invSize.tuple()
+    r.set_transfer_function(g[f"{name}_tf"])
+    r.set_camera(L.Camera.from_buffer_copy(bytes(g[f"{name}_camera"])))
+    lb = bytes(g[f"{name}_lights"])
+    r.set_area_lights([L.AreaLight.from_buffer_copy(lb[i * 44:(i + 1) * 44]) for i in range(nl)])
+    r.set_env_light(S.constant_env_light(), enabled=False)
+    return float(g[f"{name}_step"]), depth, frames
+
+
 REFSCENE_LIB = os.path.join(REF_DIR, "libsvr_refscene.so")
 
 

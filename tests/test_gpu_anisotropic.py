@@ -2,7 +2,8 @@
 macrocell edge (70 x 52 x 37 voxels) and anisotropic spacing (0.7, 1.0, 1.9) -- what VolumeReader hands over
 for a MetaImage file (core/VolumeReader.cpp:174-201: bbox = +-dim*spacing/2, step size from the spacing).
 Ray caster against the reference's float twin (1e-4), path tracer against the reference path for path (twin
-mode) and statistically (product mode), acceleration toggles bit-exact."""
+mode) -- against the CPU oracle where the reference's kernels are not built -- and statistically (product mode, see
+_statistical_parity for its reference arm), acceleration toggles bit-exact."""
 import numpy as np
 import pytest
 import torch
@@ -10,7 +11,7 @@ import torch
 from sunvolumerender_b200 import _lib as L
 from sunvolumerender_b200 import scene as S
 
-from _gpu_common import raycast_f32, reference
+from _gpu_common import check_paths, check_rgba, check_u8, oracle_reference, raycast_f32
 from test_gpu_pathtrace import _frames, _statistical_parity
 
 pytestmark = pytest.mark.gpu
@@ -21,7 +22,7 @@ W, H = 128, 128   # a canvas size the reference is compiled for (WIDTH/HEIGHT ar
 
 
 class _Cfg:  # what reference() and the helpers read from a Config
-    width, height, name = W, H, "aniso"
+    width, height, name, fmt, dims = W, H, "aniso", L.VOXEL_U16, DIMS
 
 
 def _voxels():
@@ -86,13 +87,12 @@ def test_raycaster_matches_reference(renderer, tf):
         assert torch.equal(im, imgs[0])  # skipping removes zero contributions only
     mine = imgs[0].cpu().numpy()
     assert mine[..., 3].max() > 0.5
-    twin = reference(renderer, _Cfg, f32=True)
+    twin = oracle_reference(renderer, _Cfg, f32=True)
     twin.render_raycasting(step)
-    ref_f = twin.ldr_image().cpu().numpy() / 255.0
-    assert np.abs(mine - ref_f).max() <= 1e-4
-    ref = reference(renderer, _Cfg)
+    check_rgba(mine, twin)
+    ref = oracle_reference(renderer, _Cfg)
     ref.render_raycasting(step)
-    assert np.abs(renderer.ldr_image().cpu().numpy().astype(int) - ref.ldr_image().cpu().numpy().astype(int)).max() <= 1
+    check_u8(renderer.ldr_image().cpu().numpy(), ref)
 
 
 def test_path_tracer_twin_mode_matches_reference(renderer):
@@ -100,15 +100,13 @@ def test_path_tracer_twin_mode_matches_reference(renderer):
     _setup(renderer, depth)
     renderer.set_option(L.OPT_PT_MODE, 0)
     renderer.set_option(L.OPT_PT_KERNEL, 1)
-    ref = reference(renderer, _Cfg)
+    ref = oracle_reference(renderer, _Cfg)
     mine = _frames(renderer, 4, depth)
     ref.frame_no = 0
     ref.render_pathtracer(4, depth)
     theirs = ref.hdr_image().cpu().numpy()
     assert theirs.max() > 0
-    d = np.abs(mine - theirs).max(axis=2)
-    assert (d <= 1e-4).mean() >= 0.999, (d.max(), (d <= 1e-4).mean())
-    assert abs(mine.mean() - theirs.mean()) <= 1e-3 * theirs.mean()
+    check_paths(mine, theirs, ref, frac=0.999, mean_rel=1e-3)
 
 
 def test_path_tracer_product_mode_is_statistically_the_reference(renderer):

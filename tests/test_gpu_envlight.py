@@ -2,16 +2,18 @@
 the C ABI.  The reference left its only call site commented out (pathtracer.cu:233); the checker is the
 environment-light twin of the reference -- the same sources with that one line re-enabled at build time
 (oracle/Makefile) -- so constant skies and HDR maps are compared path for path in the twin mode and
-statistically in the product mode."""
+statistically in the product mode.  Where the twin is not built, constant skies are compared path for path with the CPU
+oracle, and the statistical comparisons take the product's twin mode as their reference arm (see _statistical_parity)."""
 import numpy as np
 import pytest
 import torch
 
+from oracle import binding as B
 from oracle import hdr_oracle as H
 from sunvolumerender_b200 import _lib as L
 from sunvolumerender_b200 import scene as S
 
-from _gpu_common import reference, setup, small_config
+from _gpu_common import OracleRef, check_paths, oracle_reference, reference, setup, small_config
 from test_gpu_pathtrace import _frames, _statistical_parity
 
 pytestmark = pytest.mark.gpu
@@ -25,15 +27,22 @@ def _sky_file(tmp_path, w=128, h=64):
 
 
 def _twin_check(renderer, cfg, depth, frames=3):
+    """Path for path against the environment-light twin of the reference; where it is not built, against the CPU oracle,
+    whose environment light is the constant sky: an HDR map is then compared only statistically (_statistical_parity)."""
     renderer.set_option(L.OPT_PT_MODE, 0)
-    ref = reference(renderer, cfg, env=True)
     mine = _frames(renderer, frames, depth)
+    if B.ref(cfg.width, cfg.height, env=True) is None and renderer.env.tex:
+        return mine
+    ref = oracle_reference(renderer, cfg, env=True)
     ref.render_pathtracer(frames, depth)
     theirs = ref.hdr_image().cpu().numpy()
-    d = np.abs(mine - theirs).max(axis=2)
-    tol = 1e-4 * np.maximum(1.0, theirs.max(axis=2))
-    assert (d <= tol).mean() >= 0.998, (d.max(), (d <= tol).mean())
-    assert abs(mine.mean() - theirs.mean()) <= 2e-3 * theirs.mean()
+    if isinstance(ref, OracleRef):
+        check_paths(mine, theirs, ref, scaled=True)
+    else:
+        d = np.abs(mine - theirs).max(axis=2)
+        tol = 1e-4 * np.maximum(1.0, theirs.max(axis=2))
+        assert (d <= tol).mean() >= 0.998, (d.max(), (d <= tol).mean())
+        assert abs(mine.mean() - theirs.mean()) <= 2e-3 * theirs.mean()
     return mine
 
 

@@ -5,7 +5,9 @@ Same estimator as the reference's kernel_pathtracer; the shadow ray draws from a
 random walks than in shapes 1-3: parity with the reference (oracle/_ref) is statistical (tests/test_gpu_pathtrace.py::
 _statistical_parity).  Exact properties: every path is counted once; radiance is summed per pixel in fixed point, so the
 image does not depend on how lanes were scheduled -- bit-identical across re-fill thresholds, run lengths and block sizes.
-"""
+
+Where oracle/_ref is not built, the reference arm of the statistical comparisons is the product's reference-twin
+mode (tests/test_gpu_pathtrace.py::_statistical_parity)."""
 import numpy as np
 import pytest
 import torch

@@ -7,7 +7,9 @@ shapes 1-3: parity with the reference's kernel_pathtracer (oracle/_ref) is stati
 Welch statistic per 16x16 tile <= 4.5 for >= 99.5 % of the tiles, image means within 1-3 %).  What stays exact: the image
 is a deterministic function of (seed, scene, sample range); launch geometry and the refill threshold only change the
 order of float additions; counted paths are exact; the profile is conservative (checked against brute-force fetches).
-"""
+
+Where oracle/_ref is not built, the reference arm of the statistical comparisons is the product's reference-twin
+mode (tests/test_gpu_pathtrace.py::_statistical_parity)."""
 import numpy as np
 import pytest
 import torch

@@ -15,7 +15,7 @@ import torch
 from sunvolumerender_b200 import _lib as L
 from sunvolumerender_b200 import scene as S
 
-from _gpu_common import cpu_oracle, raycast_f32, reference, setup, small_config
+from _gpu_common import check_rgba, check_u8, cpu_oracle, oracle_reference, raycast_f32, setup, small_config
 
 pytestmark = pytest.mark.gpu
 STEP = S.raycast_step_size()
@@ -24,16 +24,13 @@ STEP = S.raycast_step_size()
 def _check_vs_reference(r, cfg):
     setup(r, cfg)
     mine = raycast_f32(r)
-    mine_u8 = r.ldr_image().cpu().numpy().astype(int)
-    ref = reference(r, cfg)
+    mine_u8 = r.ldr_image().cpu().numpy()
+    ref = oracle_reference(r, cfg)
     ref.render_raycasting(STEP)
-    ref_u8 = ref.ldr_image().cpu().numpy().astype(int)
-    assert np.abs(mine_u8 - ref_u8).max() <= 1
-    twin = reference(r, cfg, f32=True)
+    check_u8(mine_u8, ref)
+    twin = oracle_reference(r, cfg, f32=True)
     twin.render_raycasting(STEP)
-    ref_f = twin.ldr_image().cpu().numpy() / 255.0
-    diff = np.abs(mine.cpu().numpy() - ref_f)
-    assert diff.max() <= 1e-4, diff.max()
+    check_rgba(mine.cpu().numpy(), twin)
     assert mine.cpu().numpy()[..., 3].max() > 0.5  # the volume is actually visible
     return mine
 
@@ -131,9 +128,9 @@ def test_clip_planes_and_density_scale(renderer):
     setup(renderer, cfg)
     renderer.set_volume_params(density_scale=0.6, x_clip=(-0.5, 0.9), z_clip=(-1.0, 0.2))
     mine = raycast_f32(renderer).cpu().numpy()
-    twin = reference(renderer, cfg, f32=True)
+    twin = oracle_reference(renderer, cfg, f32=True)
     twin.render_raycasting(STEP)
-    assert np.abs(mine - twin.ldr_image().cpu().numpy() / 255.0).max() <= 1e-4
+    check_rgba(mine, twin)
     renderer.set_option(L.OPT_RC_SKIP, 0)
     assert np.array_equal(raycast_f32(renderer).cpu().numpy(), mine)
 
@@ -144,9 +141,9 @@ def test_camera_inside_the_volume(renderer):
     setup(renderer, cfg)
     renderer.set_camera(S.make_camera((3.0, -2.0, 10.0), (1, 0, 0), (0, 1, 0), (0, 0, 1), 60.0, 0.0, 1.0, 1.0, cfg.width, cfg.height))
     mine = raycast_f32(renderer).cpu().numpy()
-    twin = reference(renderer, cfg, f32=True)
+    twin = oracle_reference(renderer, cfg, f32=True)
     twin.render_raycasting(STEP)
-    assert np.abs(mine - twin.ldr_image().cpu().numpy() / 255.0).max() <= 1e-4
+    check_rgba(mine, twin)
 
 
 def test_empty_volume_and_ragged_image_size(renderer):
