@@ -195,6 +195,31 @@ int svr_pathtracer_accumulate(svr_vec4* sum, uint32_t traceDepth, uint32_t first
 int svr_pathtracer_accumulate_bands(svr_vec4* sum, uint32_t traceDepth, uint32_t firstSample, uint32_t nSamples, int clear,
                                     uint32_t phase, uint32_t stride, uint32_t* bandRows);
 int svr_pathtracer_resolve(svr_u8vec4* img, svr_vec3* hdrOut, const svr_vec4* sum);
+/* Adaptive sampling.  Clears sum and halfSum, then renders samples [firstSample, firstSample + n_p) of every pixel p into
+ * them, n_p in {minSamples, minSamples + batch, ..., maxSamples}: sum as svr_pathtracer_accumulate (rgb += samples, w += count),
+ * halfSum the samples whose offset from firstSample is odd (rgb, w = n_p / 2).  Resolve sum with svr_pathtracer_resolve.
+ * The loop: every pixel takes minSamples; then, after each round, a pass over the image computes per pixel
+ *     d_p   = max over r, g, b of |tone_map(even mean) - tone_map(odd mean)| / 2, with exposure cam.exposure,
+ *             even mean = (sum - halfSum) / (w - halfSum.w), odd mean = halfSum / halfSum.w
+ *             (the two halves differ by twice the standard error of the full mean: d_p estimates the displayed value's),
+ *     err_p = RMS of d over the 3 x 3 window around p, coordinates clamped to the image,
+ * and a pixel keeps sampling iff it took the last round, err_p >= threshold and w_p < maxSamples; those pixels take
+ * min(batch, maxSamples - w) more samples.  A pixel that has stopped never restarts, so every round renders one sample range.
+ * The loop ends when no pixel is left; reading each pass's counts costs one stream synchronisation per round.
+ * threshold = 0 stops no pixel before maxSamples (err >= 0 always).  A pixel's samples are a function of (seed, pixel, sample),
+ * and each pixel is summed by one warp in a fixed order: sum equals, bit for bit, the uniform svr_pathtracer_accumulate
+ * sequence (firstSample, minSamples, clear) + (firstSample + minSamples + k batch, batch, no clear) truncated where the
+ * pixel's w stops.
+ * Kernel: the sample-parallel shape over a list of pixels, for every traceDepth (deep paths pay that shape's cost: the
+ * scatter queue's per-lane order does not split samples by parity); SVR_OPT_PT_KERNEL, _PROFILE, _BLOCK_SPLIT and
+ * _WARP_PIXELS do not apply.  Estimator modes 0-2 and SVR_OPT_ENV_NEE as elsewhere.  hdr buffers are not touched.
+ * errOrNull: err_p of the final pass (imageW*imageH floats).  *roundsOut = render launches, *samplesOut = sum of w,
+ * *unconvergedOut = pixels with err_p >= threshold in the final pass (any may be NULL).
+ * Errors: null sum / halfSum; minSamples, maxSamples or batch not a positive multiple of 32; maxSamples < minSamples or
+ * above 2^24; threshold < 0 or NaN; SVR_OPT_COUNTERS = 1; the scene checks of the other render calls. */
+int svr_pathtracer_accumulate_adaptive(svr_vec4* sum, svr_vec4* halfSum, float* errOrNull, uint32_t traceDepth,
+                                       uint32_t firstSample, uint32_t minSamples, uint32_t maxSamples, uint32_t batch,
+                                       float threshold, uint32_t* roundsOut, uint64_t* samplesOut, uint32_t* unconvergedOut);
 
 /* Staging buffers for streaming volumes to replicated scenes (SURVEY.md section 8e: the volume is replicated
  * per GPU; the reference is single-device, main.cpp:7-33, and has no counterpart).  One process per GPU:

@@ -132,6 +132,8 @@ SIGNATURES = [
     ("svr_pathtracer_accumulate", C.c_int, [_P, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int]),
     ("svr_pathtracer_accumulate_bands", C.c_int, [_P, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32)]),
     ("svr_pathtracer_resolve", C.c_int, [_P, _P, _P]),
+    ("svr_pathtracer_accumulate_adaptive", C.c_int, [_P, _P, _P, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float,
+                                                     C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
     ("svr_render_raycasting_f32", C.c_int, [_P, C.POINTER(Volume), C.POINTER(TransferFunction), C.POINTER(Camera), C.c_float]),
     ("svr_render_raycasting_rows", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(TransferFunction), C.POINTER(Camera), C.c_float, C.c_uint32, C.c_uint32]),
     ("svr_volume_create", C.c_int, [C.POINTER(Volume), _P, C.c_int, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float, C.c_float, C.c_float, C.c_float]),

@@ -177,6 +177,10 @@ extern "C" int svr_set_device(int device)
     cudaFree(st.dPixelCache);
     st.dPixelCache = nullptr;
     st.pixelCacheCap = 0;
+    cudaFree(st.dAdaptiveList);
+    cudaFree(st.dAdaptiveCounts);
+    st.dAdaptiveList = st.dAdaptiveCounts = nullptr;
+    st.adaptiveListCap = 0;
     cudaFree(st.dAhead);
     st.dAhead = nullptr;
     st.aheadCapFloats = 0;

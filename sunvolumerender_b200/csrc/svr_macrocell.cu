@@ -533,28 +533,6 @@ __global__ void mailbox_kernel(const unsigned int* src, unsigned int* mailbox, i
     __threadfence_system();
 }
 
-int ensure_mailbox(HostState& st)
-{
-    if (!st.hMailbox) {
-        SVR_TRY(cudaHostAlloc(&st.hMailbox, 64, cudaHostAllocMapped | cudaHostAllocPortable));
-        SVR_TRY(cudaHostGetDevicePointer(&st.dMailbox, st.hMailbox, 0));
-    }
-    return 0;
-}
-
-// host <- device, at most 32 bytes, synchronous with respect to the library's stream
-int read_small(HostState& st, void* host, const void* dev, size_t bytes)
-{
-    if (bytes > 32 || (bytes & 3)) return fail_msg("read_small: at most 32 bytes, a multiple of 4");  // bytes 32..63 of the mailbox: tf_check_launch
-    if (int rc = ensure_mailbox(st)) return rc;
-    mailbox_kernel<<<1, 32, 0, st.stream>>>((const unsigned int*)dev, (unsigned int*)st.dMailbox, (int)(bytes / 4));
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    SVR_TRY(cudaStreamSynchronize(st.stream));
-    memcpy(host, st.hMailbox, bytes);
-    return 0;
-}
-
 int launch_fingerprint(HostState& st, int slot)
 {
     if (!st.dFingerprint) SVR_TRY(cudaMalloc(&st.dFingerprint, 2 * sizeof(unsigned long long)));
@@ -614,6 +592,28 @@ int create_point_view(HostState& st, const cudaResourceDesc& vrd, const cudaChan
 }
 
 }  // namespace
+
+int ensure_mailbox(HostState& st)
+{
+    if (!st.hMailbox) {
+        SVR_TRY(cudaHostAlloc(&st.hMailbox, 64, cudaHostAllocMapped | cudaHostAllocPortable));
+        SVR_TRY(cudaHostGetDevicePointer(&st.dMailbox, st.hMailbox, 0));
+    }
+    return 0;
+}
+
+// host <- device, at most 32 bytes, synchronous with respect to the library's stream
+int read_small(HostState& st, void* host, const void* dev, size_t bytes)
+{
+    if (bytes > 32 || (bytes & 3)) return fail_msg("read_small: at most 32 bytes, a multiple of 4");  // bytes 32..63 of the mailbox: tf_check_launch
+    if (int rc = ensure_mailbox(st)) return rc;
+    mailbox_kernel<<<1, 32, 0, st.stream>>>((const unsigned int*)dev, (unsigned int*)st.dMailbox, (int)(bytes / 4));
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+    SVR_TRY(cudaStreamSynchronize(st.stream));
+    memcpy(host, st.hMailbox, bytes);
+    return 0;
+}
 
 void release_grid(HostState& st)
 {

@@ -896,6 +896,55 @@ __global__ void __launch_bounds__(SVR_PT_MAX_THREADS, SVR_PT_MIN_BLOCKS) pathtra
     lc.flush(cnt);
 }
 
+// Adaptive sampling (svr_pathtracer_accumulate_adaptive): shape 2 over a list of pixels.  Warp w of the grid renders the pixel
+// list[w] exactly as pathtrace_warp_kernel does -- same samples per lane, same butterfly, so `sum` receives the same bits -- and
+// also adds the sum of the samples with an odd offset from firstSample to `half` (rgb, w = nSamples / 2).  Lane j traces the
+// offsets j, j + 32, ...: odd lanes hold odd offsets, and before the butterfly's last step (xor 1) every even lane holds the
+// even lanes' sum and receives the odd lanes' sum from its neighbour.  nSamples is a multiple of 32; no counters.
+template <int MODE>
+__global__ void __launch_bounds__(SVR_PT_MAX_THREADS, SVR_PT_MIN_BLOCKS) pathtrace_list_kernel(const __grid_constant__ DevScene s, const PtLaunch a,
+                                                                                           const uint32_t* __restrict__ list, uint32_t count, float4* half)
+{
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t item = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (item >= count) return;  // whole warps
+    const uint32_t offset = list[item];
+    const uint32_t idy = offset / s.cam.imageW, idx = offset - idy * s.cam.imageW;
+    const PixelInfo pi = load_pixel_info(a.pixelInfo, offset);
+    LocalCounters<false> lc;
+    if (pi.empty && !pi.lights && (!s.envEnabled || s.env.tex == 0)) {
+        // the constant sky, as pathtrace_warp_kernel writes it; half of it is the odd samples' share (exactly half the sum)
+        if (lane == 0) {
+            const float3 sky = (a.traceDepth != 0 && s.envEnabled) ? f3(s.env.defaultRadiance) * s.env.intensity : f3(0.f);
+            write_pixel(s, a, offset, sky * (float)a.nSamples);
+            const float3 o = sky * (float)(a.nSamples / 2u);
+            const float4 prev = half[offset];
+            half[offset] = make_float4(prev.x + o.x, prev.y + o.y, prev.z + o.z, prev.w + (float)(a.nSamples / 2u));
+        }
+        return;
+    }
+    PathState<MODE> ps;
+    pixel_begin<MODE>(ps);
+    for (uint32_t n = lane; n < a.nSamples; n += 32u) trace_sample<MODE, false>(s, a, ps, idx, idy, offset, a.firstSample + n, pi, lc);
+    float3 sum = pixel_sum<MODE>(ps);
+    __syncwarp();
+#pragma unroll
+    for (int o = 16; o > 1; o >>= 1) {
+        sum.x += __shfl_xor_sync(0xffffffffu, sum.x, o);
+        sum.y += __shfl_xor_sync(0xffffffffu, sum.y, o);
+        sum.z += __shfl_xor_sync(0xffffffffu, sum.z, o);
+    }
+    const float3 other = f3(__shfl_xor_sync(0xffffffffu, sum.x, 1), __shfl_xor_sync(0xffffffffu, sum.y, 1), __shfl_xor_sync(0xffffffffu, sum.z, 1));
+    sum.x += other.x;
+    sum.y += other.y;
+    sum.z += other.z;
+    write_pixel_warp(s, a, offset, sum, lane);
+    if (lane == 0) {  // an even lane: `other` is the odd lanes' sum
+        const float4 prev = half[offset];
+        half[offset] = make_float4(prev.x + other.x, prev.y + other.y, prev.z + other.z, prev.w + (float)(a.nSamples / 2u));
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // kernel shape 3: sample-parallel warp with a scatter queue (deep paths).  In a high-albedo medium most
 // samples of a pixel leave after no or one scatter event and a few bounce traceDepth times; with the loop
@@ -2046,6 +2095,79 @@ __global__ void resolve_kernel(const float4* __restrict__ sum, float* __restrict
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// adaptive sampling: the start of a render and the convergence pass between its rounds
+// ---------------------------------------------------------------------------------------------
+// clears the two accumulators, lists every pixel, clears both count slots
+__global__ void adaptive_start_kernel(float4* __restrict__ sum, float4* __restrict__ half, uint32_t* __restrict__ list, uint32_t* __restrict__ counts,
+                                      uint32_t npix)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < 4u) counts[i] = 0u;
+    if (i >= npix) return;
+    sum[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    half[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    list[i] = i;
+}
+
+// d = max over channels of |tone_map(even half's mean) - tone_map(odd half's mean)| / 2: the standard error of the displayed
+// value, estimated from the two halves (they differ by twice the standard error of the full mean)
+SVR_DEV float half_difference(const float4* __restrict__ sum, const float4* __restrict__ half, uint32_t i, float exposure)
+{
+    const float4 s = sum[i], h = half[i];
+    const float we = s.w - h.w;
+    if (!(h.w > 0.f) || !(we > 0.f)) return 0.f;
+    const float3 even = tone_map(f3((s.x - h.x) / we, (s.y - h.y) / we, (s.z - h.z) / we), exposure);
+    const float3 odd = tone_map(f3(h.x / h.w, h.y / h.w, h.z / h.w), exposure);
+    return 0.5f * fmaxf(fmaxf(fabsf(even.x - odd.x), fabsf(even.y - odd.y)), fabsf(even.z - odd.z));
+}
+
+// One pass over the image after a round: err = RMS of d over the 3 x 3 window (coordinates clamped to the image), optionally
+// stored; a pixel stays listed iff it took the last round (w == wActive), err >= threshold and w < maxSamples.  Blocks of
+// 32 x 8 pixels: d of the block and its one-pixel rim goes through shared memory, and each warp (one row of 32 pixels) appends
+// its active pixels to the list with one atomicAdd.  counts[slot] = {active, err >= threshold}; the other slot is cleared for
+// the next pass (the previous pass's counts have been read by then).
+__global__ void __launch_bounds__(256) adaptive_converge_kernel(const float4* __restrict__ sum, const float4* __restrict__ half, float* __restrict__ err,
+                                                                uint32_t* __restrict__ list, uint32_t* __restrict__ counts, uint32_t slot, uint32_t W,
+                                                                uint32_t H, float wActive, float maxSamples, float threshold, float exposure)
+{
+    __shared__ float d[10][34];
+    const int x0 = (int)(blockIdx.x * 32u) - 1, y0 = (int)(blockIdx.y * 8u) - 1;
+    for (uint32_t t = threadIdx.y * 32u + threadIdx.x; t < 10u * 34u; t += 256u) {
+        const int ty = (int)(t / 34u), tx = (int)(t % 34u);
+        const uint32_t x = (uint32_t)min(max(x0 + tx, 0), (int)W - 1), y = (uint32_t)min(max(y0 + ty, 0), (int)H - 1);
+        d[ty][tx] = half_difference(sum, half, y * W + x, exposure);
+    }
+    if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.y == 0 && threadIdx.x < 2u) counts[2u * (slot ^ 1u) + threadIdx.x] = 0u;
+    __syncthreads();
+    const uint32_t x = blockIdx.x * 32u + threadIdx.x, y = blockIdx.y * 8u + threadIdx.y;
+    bool active = false, unconverged = false;
+    if (x < W && y < H) {
+        float e2 = 0.f;
+#pragma unroll
+        for (int j = 0; j < 3; ++j)
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+                const float v = d[threadIdx.y + j][threadIdx.x + i];
+                e2 += v * v;
+            }
+        const float e = sqrtf(e2 * (1.f / 9.f));
+        const uint32_t offset = y * W + x;
+        if (err) err[offset] = e;
+        const float w = sum[offset].w;
+        unconverged = e >= threshold;
+        active = unconverged && w == wActive && w < maxSamples;
+    }
+    const uint32_t ballot = __ballot_sync(0xffffffffu, active), late = __ballot_sync(0xffffffffu, unconverged);
+    uint32_t base = 0u;
+    if (threadIdx.x == 0) {
+        if (ballot) base = atomicAdd(counts + 2u * slot, (uint32_t)__popc(ballot));
+        if (late) atomicAdd(counts + 2u * slot + 1u, (uint32_t)__popc(late));
+    }
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (active) list[base + (uint32_t)__popc(ballot & ((1u << threadIdx.x) - 1u))] = y * W + x;
+}
+
 template <int MODE>
 void launch_mode(int shape, dim3 grid, int block, cudaStream_t stream, const DevScene& sc, const PtLaunch& a, Counters* cnt)
 {
@@ -2082,7 +2204,15 @@ void launch_mode(int shape, dim3 grid, int block, cudaStream_t stream, const Dev
     }
 }
 
-int launch_pathtrace(PtLaunch& a)
+// The pixels an adaptive render still samples (svr_pathtracer_accumulate_adaptive): offsets list[0 .. count), odd samples' sums into half
+struct PixelList {
+    const uint32_t* list;
+    uint32_t count;
+    float4* half;
+};
+
+// pl != null: the sample-parallel shape over the listed pixels (pathtrace_list_kernel), whatever the options would pick
+int launch_pathtrace(PtLaunch& a, const PixelList* pl = nullptr)
 {
     HostState& st = state();
     DevScene sc = st.scene;
@@ -2132,6 +2262,7 @@ int launch_pathtrace(PtLaunch& a)
     if (shape == 5 && mode != 2) shape = 2;
     if (sc.envNee && shape >= 3) shape = 2;  // environment next-event estimation lives in the shared event code of shapes 0-2
     if (shape >= 2 && a.nSamples < (uint32_t)st.options[SVR_OPT_PT_WARP_MIN_SPP] && !a.perSample) shape = 1;
+    if (pl) shape = 2;  // (the adaptive entry point has ruled out counters)
     if (a.perSample && (shape != 2 || cnt || a.nSamples > 32u)) {
         a.perSample = nullptr;  // look-ahead is for the plain sample-parallel shape: the caller renders this frame the ordinary way
         return 0;
@@ -2182,6 +2313,19 @@ int launch_pathtrace(PtLaunch& a)
         }
         a.pixelCache = 2;
         a.pixelInfo = st.dPixelCache;
+    }
+    if (pl) {
+        if (pl->count == 0) return 0;
+        const dim3 lg((pl->count + (uint32_t)block / 32u - 1u) / ((uint32_t)block / 32u));
+        switch (sc.envNee ? 3 : mode) {
+            case 0: pathtrace_list_kernel<0><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
+            case 1: pathtrace_list_kernel<1><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
+            case 2: pathtrace_list_kernel<2><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
+            default: pathtrace_list_kernel<3><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
+        }
+        count_launch();
+        SVR_TRY(cudaGetLastError());
+        return 0;
     }
     a.blockSplit = shape == 2 && st.options[SVR_OPT_PT_BLOCK_SPLIT] != 0 && a.nSamples >= 32u * ((uint32_t)block / 32u);
     if (a.blockSplit) tileH = 1u;
@@ -2416,6 +2560,73 @@ extern "C" int svr_pathtracer_accumulate_bands(svr_vec4* sum, uint32_t traceDept
     int rc = launch_pathtrace(a);
     if (bandRows) *bandRows = a.bandRows;
     return rc;
+}
+
+// Adaptive sampling (include/svr_render.h).  Every round renders one sample range for all listed pixels -- a pixel that has
+// stopped never restarts, so the listed pixels share one sample count -- and reads the pass's two counts through the mailbox:
+// one stream synchronisation per round.
+extern "C" int svr_pathtracer_accumulate_adaptive(svr_vec4* sum, svr_vec4* halfSum, float* errOrNull, uint32_t traceDepth, uint32_t firstSample,
+                                                  uint32_t minSamples, uint32_t maxSamples, uint32_t batch, float threshold, uint32_t* roundsOut,
+                                                  uint64_t* samplesOut, uint32_t* unconvergedOut)
+{
+    HostState& st = state();
+    if (!sum || !halfSum) return fail_msg("svr_pathtracer_accumulate_adaptive: sum and halfSum must not be null");
+    if (minSamples == 0 || maxSamples == 0 || batch == 0 || (minSamples | maxSamples | batch) % 32u != 0u)
+        return fail_msg("svr_pathtracer_accumulate_adaptive: minSamples, maxSamples and batch must be positive multiples of 32");
+    if (maxSamples < minSamples) return fail_msg("svr_pathtracer_accumulate_adaptive: maxSamples is below minSamples");
+    if (maxSamples > (1u << 24)) return fail_msg("svr_pathtracer_accumulate_adaptive: maxSamples above 2^24 (sample counts are floats)");
+    if (!(threshold >= 0.f)) return fail_msg("svr_pathtracer_accumulate_adaptive: threshold must be >= 0");
+    if (st.options[SVR_OPT_COUNTERS]) return fail_msg("svr_pathtracer_accumulate_adaptive: SVR_OPT_COUNTERS must be 0");
+    if (!st.scene.vol.tex || !st.scene.tf.tex) return fail_msg("render_pathtracer: setup_volume / setup_transferfunction not called");
+    const uint32_t W = st.scene.cam.imageW, H = st.scene.cam.imageH, npix = W * H;
+    if (!npix) return fail_msg("render_pathtracer: setup_camera not called");
+    if (st.adaptiveListCap < npix) {
+        cudaFree(st.dAdaptiveList);
+        st.dAdaptiveList = nullptr;
+        st.adaptiveListCap = 0;
+        SVR_TRY(cudaMalloc(&st.dAdaptiveList, (size_t)npix * sizeof(uint32_t)));
+        st.adaptiveListCap = npix;
+    }
+    if (!st.dAdaptiveCounts) SVR_TRY(cudaMalloc(&st.dAdaptiveCounts, 4 * sizeof(uint32_t)));
+    float4* s4 = (float4*)sum;
+    float4* h4 = (float4*)halfSum;
+    adaptive_start_kernel<<<(npix + 255u) / 256u, 256, 0, st.stream>>>(s4, h4, st.dAdaptiveList, st.dAdaptiveCounts, npix);
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+
+    PtLaunch a;
+    memset(&a, 0, sizeof(a));
+    a.traceDepth = traceDepth;
+    a.y0 = 0;
+    a.y1 = 0xffffffffu;
+    a.sum = s4;
+    PixelList pl = {st.dAdaptiveList, npix, h4};
+    uint32_t w = 0, n = minSamples, rounds = 0, unconverged = 0;
+    uint64_t samples = 0;
+    for (uint32_t pass = 0;; ++pass) {
+        a.firstSample = firstSample + w;
+        a.nSamples = n;
+        if (int rc = launch_pathtrace(a, &pl)) return rc;
+        rounds++;
+        samples += (uint64_t)pl.count * n;
+        w += n;
+        const dim3 cb((W + 31u) / 32u, (H + 7u) / 8u);
+        const uint32_t slot = pass & 1u;
+        adaptive_converge_kernel<<<cb, dim3(32, 8), 0, st.stream>>>(s4, h4, errOrNull, st.dAdaptiveList, st.dAdaptiveCounts, slot, W, H, (float)w,
+                                                                   (float)maxSamples, threshold, st.scene.cam.exposure);
+        count_launch();
+        SVR_TRY(cudaGetLastError());
+        uint32_t c[2];
+        if (int rc = read_small(st, c, st.dAdaptiveCounts + 2u * slot, sizeof(c))) return rc;
+        pl.count = c[0];
+        unconverged = c[1];
+        if (pl.count == 0) break;
+        n = std::min(batch, maxSamples - w);
+    }
+    if (roundsOut) *roundsOut = rounds;
+    if (samplesOut) *samplesOut = samples;
+    if (unconvergedOut) *unconvergedOut = unconverged;
+    return 0;
 }
 
 extern "C" int svr_pathtracer_resolve(svr_u8vec4* img, svr_vec3* hdrOut, const svr_vec4* sum)

@@ -85,6 +85,12 @@ struct HostState {
     unsigned long long aheadSingleEpoch = 0, aheadTimedEpoch = 0, aheadOffEpoch = 0;
     uint32_t aheadTimedBatch = 0;
 
+    // Adaptive sampling (svr_pathtracer_accumulate_adaptive): the offsets of the pixels still taking samples, and the counts
+    // of the convergence pass (two slots of {active, unconverged}: a pass fills one and clears the other)
+    uint32_t* dAdaptiveList = nullptr;
+    size_t adaptiveListCap = 0;
+    uint32_t* dAdaptiveCounts = nullptr;
+
     Counters* dCounters = nullptr;
     unsigned long long launches = 0;
     std::string lastError;
@@ -134,6 +140,11 @@ int upload_with_ranges(cudaArray_t arr, const cudaChannelFormatDesc& ch, const c
 
 // Builds / refreshes the environment light's importance sampler for scene->env and fills scene->envS.
 int ensure_env_sampler(DevScene* scene);
+
+// Small results for the host through the mapped mailbox (svr_macrocell.cu): at most 32 bytes, synchronous with respect to
+// the library's stream
+int ensure_mailbox(HostState& st);
+int read_small(HostState& st, void* host, const void* dev, size_t bytes);
 
 inline void count_launch(int n = 1) { state().launches += (unsigned long long)n; }
 

@@ -237,6 +237,17 @@ class Renderer:
                 "svr_pathtracer_accumulate_bands")
         return int(rows.value)
 
+    def accumulate_adaptive(self, sum_buf, half_buf, trace_depth, first_sample, min_samples, max_samples, batch, threshold, err=None):
+        """Adaptive sampling (svr_pathtracer_accumulate_adaptive): every pixel takes min_samples, then batches of `batch` until its
+        display-space error estimate falls below `threshold` or it has max_samples.  sum_buf / half_buf: float4 per pixel (all
+        samples / the odd ones); err: optional float per pixel, the final error estimate.  Returns {"rounds", "samples",
+        "unconverged"}."""
+        rounds, samples, unconverged = C.c_uint32(0), C.c_uint64(0), C.c_uint32(0)
+        L.check(self.lib.svr_pathtracer_accumulate_adaptive(_ptr(sum_buf), _ptr(half_buf), _ptr(err), trace_depth, first_sample, min_samples, max_samples,
+                                                            batch, threshold, C.byref(rounds), C.byref(samples), C.byref(unconverged)),
+                "svr_pathtracer_accumulate_adaptive")
+        return {"rounds": int(rounds.value), "samples": int(samples.value), "unconverged": int(unconverged.value)}
+
     def resolve(self, sum_buf, want_hdr=True):
         ptr = sum_buf if isinstance(sum_buf, C.c_void_p) else _ptr(sum_buf)
         L.check(self.lib.svr_pathtracer_resolve(_ptr(self.img), _ptr(self.hdr if want_hdr else None), ptr), "svr_pathtracer_resolve")
