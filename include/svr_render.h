@@ -220,6 +220,50 @@ int svr_pathtracer_resolve(svr_u8vec4* img, svr_vec3* hdrOut, const svr_vec4* su
 int svr_pathtracer_accumulate_adaptive(svr_vec4* sum, svr_vec4* halfSum, float* errOrNull, uint32_t traceDepth,
                                        uint32_t firstSample, uint32_t minSamples, uint32_t maxSamples, uint32_t batch,
                                        float threshold, uint32_t* roundsOut, uint64_t* samplesOut, uint32_t* unconvergedOut);
+/* Denoising: guide images of the bound scene, then an edge-avoiding a-trous filter of an accumulated image (DESIGN.md 7f).
+ * Guides.  Writes albedoCoverage and normalDepth (imageW*imageH float4 each, row-major like sum): the noise-free mean of what
+ * a camera ray's first collision sees.  Delta tracking collides at density T(t) sigma(t), sigma = TF opacity per world unit
+ * (the path tracer's extinction), so each ray marches from the volume's near face (clip planes included) to its far face or
+ * the nearest area-light disk, whichever comes first, with step h = 0.5 min(spacing), samples at t0 + (k + 1/2) h, cells of
+ * majorant <= 0 skipped through the macrocell grid; per sample p = T (1 - exp(-sigma h)), alpha += p, A += p rgb(TF),
+ * Z += p dot(x - cam.pos, -cam.w) (view-space depth), N += p n (n = normalised gradient turned to face the ray's origin;
+ * a zero gradient adds nothing), T *= exp(-sigma h); a ray stops at T < 1e-3.  raysPerPixel (1, 4 or 16) rays on a
+ * sqrt(k) x sqrt(k) grid of sub-pixel positions ((i + 1/2) / sqrt(k), (j + 1/2) / sqrt(k)); with apeture > 0 the same
+ * grid position is mapped to the lens disk (concentric mapping) and the ray passes through the focal plane as in
+ * render_pathtracer.  Summed over the pixel's rays: albedoCoverage = (A / alpha, alpha / k), normalDepth = (normalize(N),
+ * Z / alpha); 0 for all eight where alpha = 0.  Estimator modes and SVR_OPT_COUNTERS do not apply; one launch.
+ * Errors: null outputs; raysPerPixel not 1, 4 or 16; the scene checks of the other render calls. */
+int svr_pathtracer_guides(svr_vec4* albedoCoverage, svr_vec4* normalDepth, uint32_t raysPerPixel);
+/* Filter parameters (svr_denoise_defaults fills the defaults: 5, 4, 128, 1, 0.1). */
+typedef struct svr_denoise_params {
+    uint32_t iterations;   /* a-trous iterations, 0..8 (steps 1, 2, 4, ...) */
+    float sigmaLuminance;  /* luminance stop, in standard deviations of the pixel's estimate */
+    float sigmaNormal;     /* normal stop exponent (0 = off) */
+    float sigmaDepth;      /* depth stop, in pixel footprints per unit step */
+    float sigmaCoverage;   /* coverage stop */
+} svr_denoise_params;
+int svr_denoise_defaults(svr_denoise_params* out);
+/* Filter.  sum / halfSum as svr_pathtracer_accumulate_adaptive leaves them (for a uniform render: that call with
+ * minSamples = maxSamples and threshold 0 -- one round, bit-identical to svr_pathtracer_accumulate -- fills halfSum), the
+ * guides of svr_pathtracer_guides.  Outputs as svr_pathtracer_resolve: packed vec3 HDR and / or the tone-mapped image.
+ *   demodulate: c = sum.rgb / sum.w, m = alpha albedo + (1 - alpha) per channel (at least 1e-3), e = c / m;
+ *   variance:   Var = (l(even / m) - l(odd / m))^2 / 4, l = Rec. 709 luminance, even = (sum - halfSum) / (w - halfSum.w),
+ *               odd = halfSum / halfSum.w; +inf where either half is empty (the luminance stop is then off); then the
+ *               3 x 3 binomial filter, coordinates clamped;
+ *   iteration i < iterations, step s = 2^i: 5 x 5 taps q = p + s (dx, dy), kernel h = [1/16, 1/4, 3/8, 1/4, 1/16] x h,
+ *               taps outside the image dropped, weight w = h w_l w_n w_z w_a with
+ *                 w_l = exp(-|l(e_p) - l(e_q)| / (sigmaLuminance sqrt(Var_p) + 1e-10)),
+ *                 w_n = max(0, n_p . n_q)^sigmaNormal (1 if both normals are 0, 0 if one is; 1 for sigmaNormal = 0),
+ *                 w_z = exp(-|z_p - z_q| / (sigmaDepth s f_p + 1e-10)), f_p = 2 z_p tanFovxOverTwo / (imageH - 1),
+ *                 w_a = exp(-|alpha_p - alpha_q| / sigmaCoverage);
+ *               e' = sum w e_q / sum w, Var' = sum w^2 Var_q / (sum w)^2 (taps of weight 0 add nothing);
+ *   resolve:    hdr = m e, then the tone map and u8 packing of svr_pathtracer_resolve.
+ * iterations = 0 is svr_pathtracer_resolve, bit for bit (that case skips the demodulation: m (c / m) is not c in float).
+ * paramsOrNull = NULL: svr_denoise_defaults.  The filter's buffers are the library's (2 x 16 bytes per pixel, kept).
+ * Errors, all reported before any CUDA call: null sum, halfSum or guide; both outputs null; iterations > 8; sigmaLuminance,
+ * sigmaDepth or sigmaCoverage not positive or not finite; sigmaNormal negative or not finite; setup_camera not called. */
+int svr_pathtracer_denoise(svr_u8vec4* imgOrNull, svr_vec3* hdrOutOrNull, const svr_vec4* sum, const svr_vec4* halfSum,
+                           const svr_vec4* albedoCoverage, const svr_vec4* normalDepth, const svr_denoise_params* paramsOrNull);
 
 /* Staging buffers for streaming volumes to replicated scenes (SURVEY.md section 8e: the volume is replicated
  * per GPU; the reference is single-device, main.cpp:7-33, and has no counterpart).  One process per GPU:

@@ -96,6 +96,14 @@ assert C.sizeof(Disk) == 28 and C.sizeof(AreaLight) == 44
 assert C.sizeof(EnvLight) == 32 and EnvLight.intensity.offset == 20
 assert C.sizeof(RenderParams) == 16 and RenderParams.hdrBuffer.offset == 8
 
+
+class DenoiseParams(C.Structure):  # svr_denoise_params
+    _fields_ = [("iterations", C.c_uint32), ("sigmaLuminance", C.c_float), ("sigmaNormal", C.c_float), ("sigmaDepth", C.c_float),
+                ("sigmaCoverage", C.c_float)]
+
+
+assert C.sizeof(DenoiseParams) == 20
+
 # enum svr_option
 (OPT_PT_MODE, OPT_SHADOW_ESTIMATOR, OPT_ENV_ENABLED, OPT_MACROCELL_SIZE, OPT_RC_SKIP, OPT_SEED, OPT_COUNTERS,
  OPT_PT_BLOCK, OPT_RC_BLOCK, OPT_PT_KERNEL, OPT_PT_ROUNDS, OPT_LEAP, OPT_PT_ENTRY_CACHE, OPT_PT_WARP_PIXELS,
@@ -134,6 +142,9 @@ SIGNATURES = [
     ("svr_pathtracer_resolve", C.c_int, [_P, _P, _P]),
     ("svr_pathtracer_accumulate_adaptive", C.c_int, [_P, _P, _P, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float,
                                                      C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
+    ("svr_pathtracer_guides", C.c_int, [_P, _P, C.c_uint32]),
+    ("svr_denoise_defaults", C.c_int, [C.POINTER(DenoiseParams)]),
+    ("svr_pathtracer_denoise", C.c_int, [_P, _P, _P, _P, _P, _P, C.POINTER(DenoiseParams)]),
     ("svr_render_raycasting_f32", C.c_int, [_P, C.POINTER(Volume), C.POINTER(TransferFunction), C.POINTER(Camera), C.c_float]),
     ("svr_render_raycasting_rows", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(TransferFunction), C.POINTER(Camera), C.c_float, C.c_uint32, C.c_uint32]),
     ("svr_volume_create", C.c_int, [C.POINTER(Volume), _P, C.c_int, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float, C.c_float, C.c_float, C.c_float]),

@@ -181,6 +181,10 @@ extern "C" int svr_set_device(int device)
     cudaFree(st.dAdaptiveCounts);
     st.dAdaptiveList = st.dAdaptiveCounts = nullptr;
     st.adaptiveListCap = 0;
+    cudaFree(st.dDenoise[0]);
+    cudaFree(st.dDenoise[1]);
+    st.dDenoise[0] = st.dDenoise[1] = nullptr;
+    st.denoiseCap = 0;
     cudaFree(st.dAhead);
     st.dAhead = nullptr;
     st.aheadCapFloats = 0;

@@ -91,6 +91,10 @@ struct HostState {
     size_t adaptiveListCap = 0;
     uint32_t* dAdaptiveCounts = nullptr;
 
+    // Denoising (svr_pathtracer_denoise, svr_denoise.cu): the filter's ping-pong buffers, float4 (demodulated rgb, variance) per pixel
+    float4* dDenoise[2] = {nullptr, nullptr};
+    size_t denoiseCap = 0;
+
     Counters* dCounters = nullptr;
     unsigned long long launches = 0;
     std::string lastError;

@@ -248,6 +248,32 @@ class Renderer:
                 "svr_pathtracer_accumulate_adaptive")
         return {"rounds": int(rounds.value), "samples": int(samples.value), "unconverged": int(unconverged.value)}
 
+    def guides(self, albedo_cov=None, normal_depth=None, rays_per_pixel=4):
+        """Guide images of the bound scene for denoise() (svr_pathtracer_guides): float4 (albedo rgb, coverage) and float4
+        (normal xyz, view-space depth) per pixel, allocated here when not given.  Returns (albedo_cov, normal_depth)."""
+        n = self.camera.imageW * self.camera.imageH * 4
+        if albedo_cov is None:
+            albedo_cov = torch.empty(n, dtype=torch.float32, device=self.device)
+        if normal_depth is None:
+            normal_depth = torch.empty(n, dtype=torch.float32, device=self.device)
+        L.check(self.lib.svr_pathtracer_guides(_ptr(albedo_cov), _ptr(normal_depth), rays_per_pixel), "svr_pathtracer_guides")
+        return albedo_cov, normal_depth
+
+    def denoise(self, sum_buf, half_buf, guides, iterations=None, sigma_luminance=None, sigma_normal=None, sigma_depth=None,
+                sigma_coverage=None, want_hdr=True):
+        """Filtered resolve of an adaptive render (svr_pathtracer_denoise) into self.img and, with want_hdr, self.hdr, as
+        resolve() writes them.  sum_buf / half_buf: float4 per pixel as accumulate_adaptive leaves them; guides: the pair
+        guides() returns.  Parameters not given take the library's defaults."""
+        p = L.DenoiseParams()
+        L.check(self.lib.svr_denoise_defaults(C.byref(p)), "svr_denoise_defaults")
+        for field, value in (("iterations", iterations), ("sigmaLuminance", sigma_luminance), ("sigmaNormal", sigma_normal),
+                             ("sigmaDepth", sigma_depth), ("sigmaCoverage", sigma_coverage)):
+            if value is not None:
+                setattr(p, field, value)
+        albedo_cov, normal_depth = guides
+        L.check(self.lib.svr_pathtracer_denoise(_ptr(self.img), _ptr(self.hdr if want_hdr else None), _ptr(sum_buf), _ptr(half_buf),
+                                                _ptr(albedo_cov), _ptr(normal_depth), C.byref(p)), "svr_pathtracer_denoise")
+
     def resolve(self, sum_buf, want_hdr=True):
         ptr = sum_buf if isinstance(sum_buf, C.c_void_p) else _ptr(sum_buf)
         L.check(self.lib.svr_pathtracer_resolve(_ptr(self.img), _ptr(self.hdr if want_hdr else None), ptr), "svr_pathtracer_resolve")
