@@ -166,17 +166,38 @@ enum svr_option {
      * Not used with SVR_OPT_COUNTERS, nor where the scatter-queue kernel would run (traceDepth >= SVR_OPT_PT_QUEUE_MIN_DEPTH).
      * Memory: batch x pixels x 12 bytes (at most 1 GiB; larger canvases get smaller batches). */
     SVR_OPT_PT_LOOKAHEAD = 25,
+    /* Denoised progressive display (DESIGN.md section 7g).  0 (default) = off.  1, 4 or 16 = on, with that many guide rays per
+     * pixel (svr_pathtracer_guides) at the start of a render; other values are rejected.  While on, a render_pathtracer call
+     * produces a DENOISED FRAME when SVR_OPT_COUNTERS is 0 and the call continues the render the library follows: frameNo == 0,
+     * or frameNo is the previous call's plus 1 with the same hdrBuffer, imageW x imageH and traceDepth.  A denoised frame
+     *   - traces one sample as the option-off call does: hdrBuffer is bit-identical to the option-off run;
+     *   - adds the sample to library-owned float4 sums, one for the even frames and one for the odd ones (both cleared at
+     *     frameNo == 0);
+     *   - uses library-owned guide images made by svr_pathtracer_guides with the option's ray count before frame 16 and with
+     *     16 rays from frame 16 on; they are remade when the scene has changed since they were made (any setup_*, upload or
+     *     option) or the frame wants another ray count (so once at the first denoised frame >= 16, one hitch);
+     *   - writes img as svr_pathtracer_denoise(img, NULL, even + odd, odd, guides, params) does, bit for bit, params as set
+     *     by svr_pathtracer_set_denoise_params.  At frame 0 the odd half is empty: the luminance stop is off and the first
+     *     frame after a change is an edge-avoiding blur guided by the guides alone.
+     * Any other call renders as with the option off, and the library follows no render until the next frameNo == 0 (so turning
+     * the option on in the middle of a render takes effect at the next restart).  svr_render_pathtracer_spp also ends it.
+     * If the library cannot allocate its buffers the call renders as with the option off.  Look-ahead (SVR_OPT_PT_LOOKAHEAD)
+     * is not used for denoised frames.  Memory: 4 x 16 bytes per pixel, kept, besides the filter's 2 x 16 bytes. */
+    SVR_OPT_PT_DENOISE = 26,
     SVR_OPT_COUNT_
 };
 /* Defaults can also come from the environment, read once at first use, for hosts that only know the
  * seven reference entry points: SVR_PT_MODE, SVR_SHADOW_ESTIMATOR, SVR_ENV_ENABLED, SVR_RC_SKIP,
- * SVR_SEED, SVR_PT_KERNEL (same values as the options). */
+ * SVR_SEED, SVR_PT_KERNEL, SVR_PT_DENOISE (same values as the options; SVR_PT_DENOISE=4 gives the reference GUI a
+ * denoised progressive display). */
 int svr_set_option(int key, int value);
 int svr_get_option(int key);
 
 /* Equivalent to `spp` consecutive render_pathtracer calls with frameNo, frameNo+1, ... but in one
  * launch: samples accumulate in registers, hdrBuffer is read and written once, the tone map
- * runs once.  frameNo == 0 clears first.  img may be NULL (no tone map). */
+ * runs once.  frameNo == 0 clears first.  img may be NULL (no tone map).  The equivalence holds for
+ * hdrBuffer always and for img while SVR_OPT_PT_DENOISE is 0: this call ignores that option and ends the
+ * render it follows (the next render_pathtracer call renders as with the option off until frameNo == 0). */
 int svr_render_pathtracer_spp(svr_u8vec4* img, const svr_render_params* renderParams, uint32_t spp);
 
 /* Multi-GPU building blocks (SURVEY.md section 8e).  `sum` is imageW*imageH float4: rgb = sum of
@@ -264,6 +285,10 @@ int svr_denoise_defaults(svr_denoise_params* out);
  * sigmaDepth or sigmaCoverage not positive or not finite; sigmaNormal negative or not finite; setup_camera not called. */
 int svr_pathtracer_denoise(svr_u8vec4* imgOrNull, svr_vec3* hdrOutOrNull, const svr_vec4* sum, const svr_vec4* halfSum,
                            const svr_vec4* albedoCoverage, const svr_vec4* normalDepth, const svr_denoise_params* paramsOrNull);
+/* The filter parameters of the denoised progressive display (SVR_OPT_PT_DENOISE); NULL restores svr_denoise_defaults.  Checked
+ * as svr_pathtracer_denoise checks them, before any CUDA call.  Takes effect at the next denoised frame; the guides do not
+ * depend on it, so the render goes on. */
+int svr_pathtracer_set_denoise_params(const svr_denoise_params* paramsOrNull);
 
 /* Staging buffers for streaming volumes to replicated scenes (SURVEY.md section 8e: the volume is replicated
  * per GPU; the reference is single-device, main.cpp:7-33, and has no counterpart).  One process per GPU:

@@ -108,7 +108,7 @@ assert C.sizeof(DenoiseParams) == 20
 (OPT_PT_MODE, OPT_SHADOW_ESTIMATOR, OPT_ENV_ENABLED, OPT_MACROCELL_SIZE, OPT_RC_SKIP, OPT_SEED, OPT_COUNTERS,
  OPT_PT_BLOCK, OPT_RC_BLOCK, OPT_PT_KERNEL, OPT_PT_ROUNDS, OPT_LEAP, OPT_PT_ENTRY_CACHE, OPT_PT_WARP_PIXELS,
  OPT_PT_WARP_MIN_SPP, OPT_PT_QUEUE_MIN_DEPTH, OPT_SETUP_SYNC, OPT_PT_LIGHT_CULL, OPT_PT_PROFILE, OPT_PT_REFILL, OPT_PT_POOL_PIXELS, OPT_ENV_NEE, OPT_PT_BLOCK_SPLIT, OPT_PT_PIXEL_CACHE,
- OPT_FUSED_UPLOAD, OPT_PT_LOOKAHEAD) = range(26)
+ OPT_FUSED_UPLOAD, OPT_PT_LOOKAHEAD, OPT_PT_DENOISE) = range(27)
 # enum svr_voxel_format
 VOXEL_U8, VOXEL_U16, VOXEL_F16, VOXEL_F32 = range(4)
 VOXEL_BYTES = {VOXEL_U8: 1, VOXEL_U16: 2, VOXEL_F16: 2, VOXEL_F32: 4}
@@ -145,6 +145,7 @@ SIGNATURES = [
     ("svr_pathtracer_guides", C.c_int, [_P, _P, C.c_uint32]),
     ("svr_denoise_defaults", C.c_int, [C.POINTER(DenoiseParams)]),
     ("svr_pathtracer_denoise", C.c_int, [_P, _P, _P, _P, _P, _P, C.POINTER(DenoiseParams)]),
+    ("svr_pathtracer_set_denoise_params", C.c_int, [C.POINTER(DenoiseParams)]),
     ("svr_render_raycasting_f32", C.c_int, [_P, C.POINTER(Volume), C.POINTER(TransferFunction), C.POINTER(Camera), C.c_float]),
     ("svr_render_raycasting_rows", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(TransferFunction), C.POINTER(Camera), C.c_float, C.c_uint32, C.c_uint32]),
     ("svr_volume_create", C.c_int, [C.POINTER(Volume), _P, C.c_int, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float, C.c_float, C.c_float, C.c_float]),

@@ -11,6 +11,9 @@
 
 namespace svr {
 
+// SVR_OPT_PT_DENOISE: off, or the guide rays per pixel svr_pathtracer_guides takes
+static bool denoise_value_ok(long v) { return v == 0 || v == 1 || v == 4 || v == 16; }
+
 HostState& state()
 {
     static HostState* s = [] {
@@ -46,18 +49,21 @@ HostState& state()
         p->options[SVR_OPT_PT_PIXEL_CACHE] = 1;
         p->options[SVR_OPT_FUSED_UPLOAD] = 1;
         p->options[SVR_OPT_PT_LOOKAHEAD] = 32;
+        p->options[SVR_OPT_PT_DENOISE] = 0;
+        svr_denoise_defaults(&p->progParams);
         // A host that only knows the reference's seven entry points (gui/canvas.cpp) cannot call
-        // svr_set_option: the same switches are read once from the environment.
-        static const struct { const char* name; int key, lo, hi; } kEnv[] = {
+        // svr_set_option: the same switches are read once from the environment.  `ok`, where given, replaces the range.
+        static const struct { const char* name; int key, lo, hi; bool (*ok)(long); } kEnv[] = {
             {"SVR_PT_MODE", SVR_OPT_PT_MODE, 0, 2},           {"SVR_SHADOW_ESTIMATOR", SVR_OPT_SHADOW_ESTIMATOR, 0, 1},
             {"SVR_ENV_ENABLED", SVR_OPT_ENV_ENABLED, 0, 1},   {"SVR_RC_SKIP", SVR_OPT_RC_SKIP, 0, 1},
             {"SVR_SEED", SVR_OPT_SEED, INT32_MIN, INT32_MAX}, {"SVR_PT_KERNEL", SVR_OPT_PT_KERNEL, 0, 5},
+            {"SVR_PT_DENOISE", SVR_OPT_PT_DENOISE, 0, 16, denoise_value_ok},
         };
         for (const auto& e : kEnv) {
             const char* v = getenv(e.name);
             if (!v || !*v) continue;
             long x = strtol(v, nullptr, 0);
-            if (x >= e.lo && x <= e.hi) p->options[e.key] = (int)x;
+            if (e.ok ? e.ok(x) : (x >= e.lo && x <= e.hi)) p->options[e.key] = (int)x;
             else fprintf(stderr, "libsvr_b200: ignoring %s=%s (out of range)\n", e.name, v);
         }
         return p;
@@ -185,6 +191,7 @@ extern "C" int svr_set_device(int device)
     cudaFree(st.dDenoise[1]);
     st.dDenoise[0] = st.dDenoise[1] = nullptr;
     st.denoiseCap = 0;
+    release_progressive(st);
     cudaFree(st.dAhead);
     st.dAhead = nullptr;
     st.aheadCapFloats = 0;
@@ -262,6 +269,9 @@ extern "C" int svr_set_option(int key, int value)
             break;
         case SVR_OPT_PT_ROUNDS:
             if (value < 0) return fail_msg("SVR_OPT_PT_ROUNDS must be >= 0");
+            break;
+        case SVR_OPT_PT_DENOISE:
+            if (!denoise_value_ok(value)) return fail_msg("SVR_OPT_PT_DENOISE must be 0 (off), 1, 4 or 16");
             break;
         default: break;
     }

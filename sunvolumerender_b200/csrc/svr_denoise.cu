@@ -244,7 +244,138 @@ __global__ void __launch_bounds__(256) denoise_iter_kernel(const float4* __restr
     }
 }
 
+// sum = even + odd, component by component: the full sums of a progressive render whose frames went into two halves by parity
+__global__ void __launch_bounds__(256) sum_halves_kernel(const float4* __restrict__ even, const float4* __restrict__ odd, float4* __restrict__ sum,
+                                                         uint32_t n)
+{
+    const uint32_t i = blockIdx.x * 256u + threadIdx.x;
+    if (i >= n) return;
+    const float4 e = __ldg(even + i), o = __ldg(odd + i);
+    sum[i] = make_float4(e.x + o.x, e.y + o.y, e.z + o.z, e.w + o.w);
+}
+
 }  // namespace
+
+int check_denoise_params(const char* who, const svr_denoise_params* paramsOrNull, svr_denoise_params* out)
+{
+    svr_denoise_params p;
+    if (paramsOrNull) p = *paramsOrNull;
+    else svr_denoise_defaults(&p);
+    const char* err = nullptr;
+    if (p.iterations > 8u) err = "iterations above 8";
+    else if (!(p.sigmaLuminance > 0.f) || !std::isfinite(p.sigmaLuminance) || !(p.sigmaDepth > 0.f) || !std::isfinite(p.sigmaDepth) ||
+             !(p.sigmaCoverage > 0.f) || !std::isfinite(p.sigmaCoverage))
+        err = "sigmaLuminance, sigmaDepth and sigmaCoverage must be positive and finite";
+    else if (!(p.sigmaNormal >= 0.f) || !std::isfinite(p.sigmaNormal)) err = "sigmaNormal must be >= 0 and finite";
+    if (err) {
+        char msg[192];
+        snprintf(msg, sizeof(msg), "%s: %s", who, err);
+        return fail_msg(msg);
+    }
+    *out = p;
+    return 0;
+}
+
+namespace {
+
+// The filter's two ping-pong buffers for npix pixels
+int ensure_filter_buffers(HostState& st, size_t npix)
+{
+    if (st.denoiseCap >= npix) return 0;
+    cudaFree(st.dDenoise[0]);
+    cudaFree(st.dDenoise[1]);
+    st.dDenoise[0] = st.dDenoise[1] = nullptr;
+    st.denoiseCap = 0;
+    SVR_TRY(cudaMalloc(&st.dDenoise[0], npix * sizeof(float4)));
+    SVR_TRY(cudaMalloc(&st.dDenoise[1], npix * sizeof(float4)));
+    st.denoiseCap = npix;
+    return 0;
+}
+
+// The filter for checked parameters and a camera of W x H pixels.  `sum` may be dDenoise[1]: the prep pass reads it before the
+// first iteration writes there.
+int run_filter(uint32_t* img, float* hdr, const float4* sum, const float4* half, const float4* ac, const float4* nd, const svr_denoise_params& p)
+{
+    HostState& st = state();
+    const uint32_t W = st.scene.cam.imageW, H = st.scene.cam.imageH;
+    if (p.iterations == 0u) return svr_pathtracer_resolve((svr_u8vec4*)img, (svr_vec3*)hdr, (const svr_vec4*)sum);  // the identity, bit for bit
+
+    if (hdr && (const void*)hdr == st.aheadHdr) st.aheadCount = 0;  // as svr_pathtracer_resolve
+    if (int rc = ensure_filter_buffers(st, (size_t)W * H)) return rc;
+    const dim3 blocks((W + 31u) / 32u, (H + 7u) / 8u), threads(32, 8);
+    denoise_prep_kernel<<<blocks, threads, 0, st.stream>>>(sum, half, ac, st.dDenoise[0], W, H);
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+    DenoiseStops k;
+    k.sigmaL = p.sigmaLuminance;
+    k.sigmaN = p.sigmaNormal;
+    k.sigmaZ = p.sigmaDepth;
+    k.invSigmaA = 1.f / p.sigmaCoverage;
+    k.pixelAngle = 2.f * st.scene.cam.tanFovxOverTwo / ((float)H - 1.f);
+    for (uint32_t i = 0; i < p.iterations; ++i) {
+        const bool last = i + 1u == p.iterations;
+        denoise_iter_kernel<<<blocks, threads, 0, st.stream>>>(st.dDenoise[i & 1u], st.dDenoise[(i + 1u) & 1u], ac, nd, W, H, 1 << i, k,
+                                                               last ? hdr : nullptr, last ? img : nullptr, st.scene.cam.exposure);
+        count_launch();
+        SVR_TRY(cudaGetLastError());
+    }
+    return 0;
+}
+
+}  // namespace
+
+// dProg[0..3] (even sum, odd sum, albedoCoverage, normalDepth) and the filter's buffers; on failure nothing is kept allocated
+// but what was there before, and the CUDA error is cleared
+bool ensure_progressive_buffers(HostState& st, size_t npix)
+{
+    if (st.progCap < npix) {
+        release_progressive(st);
+        for (int i = 0; i < 4; ++i)
+            if (cudaMalloc(&st.dProg[i], npix * sizeof(float4)) != cudaSuccess) {
+                cudaGetLastError();
+                release_progressive(st);
+                return false;
+            }
+        st.progCap = npix;
+    }
+    if (ensure_filter_buffers(st, npix)) {
+        cudaGetLastError();
+        return false;
+    }
+    return true;
+}
+
+void release_progressive(HostState& st)
+{
+    for (int i = 0; i < 4; ++i) {
+        cudaFree(st.dProg[i]);
+        st.dProg[i] = nullptr;
+    }
+    st.progCap = 0;
+    st.progActive = false;
+    st.progGuideEpoch = 0;
+    st.progGuideRays = 0;
+}
+
+// Guides made with SVR_OPT_PT_DENOISE rays before frame 16 and with 16 from there on, kept while the scene epoch stays where it
+// was after the frame that made them; then the filter of (even + odd, odd).  The caller has traced the frame's sample.
+int progressive_denoise(uint32_t* img, uint32_t frameNo)
+{
+    HostState& st = state();
+    const uint32_t rays = frameNo >= 16u ? 16u : (uint32_t)st.options[SVR_OPT_PT_DENOISE];
+    if (st.progGuideEpoch != st.sceneEpoch || st.progGuideRays != rays) {
+        if (int rc = svr_pathtracer_guides((svr_vec4*)st.dProg[2], (svr_vec4*)st.dProg[3], rays)) return rc;
+        st.progGuideRays = rays;
+    }
+    const uint32_t npix = st.scene.cam.imageW * st.scene.cam.imageH;
+    sum_halves_kernel<<<(npix + 255u) / 256u, 256, 0, st.stream>>>(st.dProg[0], st.dProg[1], st.dDenoise[1], npix);
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+    if (int rc = run_filter(img, nullptr, st.dDenoise[1], st.dProg[1], st.dProg[2], st.dProg[3], st.progParams)) return rc;
+    st.progGuideEpoch = st.sceneEpoch;  // after the frame's launches: refreshing the majorants moves the epoch
+    return 0;
+}
+
 }  // namespace svr
 
 using namespace svr;
@@ -286,47 +417,16 @@ extern "C" int svr_pathtracer_denoise(svr_u8vec4* imgOrNull, svr_vec3* hdrOutOrN
     if (!albedoCoverage || !normalDepth) return fail_msg("svr_pathtracer_denoise: the guides (albedoCoverage, normalDepth) must not be null");
     if (!imgOrNull && !hdrOutOrNull) return fail_msg("svr_pathtracer_denoise: img and hdrOut are both null");
     svr_denoise_params p;
-    if (paramsOrNull) p = *paramsOrNull;
-    else svr_denoise_defaults(&p);
-    if (p.iterations > 8u) return fail_msg("svr_pathtracer_denoise: iterations above 8");
-    if (!(p.sigmaLuminance > 0.f) || !std::isfinite(p.sigmaLuminance) || !(p.sigmaDepth > 0.f) || !std::isfinite(p.sigmaDepth) ||
-        !(p.sigmaCoverage > 0.f) || !std::isfinite(p.sigmaCoverage))
-        return fail_msg("svr_pathtracer_denoise: sigmaLuminance, sigmaDepth and sigmaCoverage must be positive and finite");
-    if (!(p.sigmaNormal >= 0.f) || !std::isfinite(p.sigmaNormal)) return fail_msg("svr_pathtracer_denoise: sigmaNormal must be >= 0 and finite");
-    const uint32_t W = st.scene.cam.imageW, H = st.scene.cam.imageH;
-    const size_t npix = (size_t)W * H;
-    if (!npix) return fail_msg("svr_pathtracer_denoise: setup_camera not called");
-    if (p.iterations == 0u) return svr_pathtracer_resolve(imgOrNull, hdrOutOrNull, sum);  // the identity, bit for bit
+    if (int rc = check_denoise_params("svr_pathtracer_denoise", paramsOrNull, &p)) return rc;
+    if (!st.scene.cam.imageW || !st.scene.cam.imageH) return fail_msg("svr_pathtracer_denoise: setup_camera not called");
+    return run_filter((uint32_t*)imgOrNull, (float*)hdrOutOrNull, (const float4*)sum, (const float4*)halfSum, (const float4*)albedoCoverage,
+                      (const float4*)normalDepth, p);
+}
 
-    if (hdrOutOrNull && (const void*)hdrOutOrNull == st.aheadHdr) st.aheadCount = 0;  // as svr_pathtracer_resolve
-    if (st.denoiseCap < npix) {
-        cudaFree(st.dDenoise[0]);
-        cudaFree(st.dDenoise[1]);
-        st.dDenoise[0] = st.dDenoise[1] = nullptr;
-        st.denoiseCap = 0;
-        SVR_TRY(cudaMalloc(&st.dDenoise[0], npix * sizeof(float4)));
-        SVR_TRY(cudaMalloc(&st.dDenoise[1], npix * sizeof(float4)));
-        st.denoiseCap = npix;
-    }
-    const float4* ac = (const float4*)albedoCoverage;
-    const float4* nd = (const float4*)normalDepth;
-    const dim3 blocks((W + 31u) / 32u, (H + 7u) / 8u), threads(32, 8);
-    denoise_prep_kernel<<<blocks, threads, 0, st.stream>>>((const float4*)sum, (const float4*)halfSum, ac, st.dDenoise[0], W, H);
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    DenoiseStops k;
-    k.sigmaL = p.sigmaLuminance;
-    k.sigmaN = p.sigmaNormal;
-    k.sigmaZ = p.sigmaDepth;
-    k.invSigmaA = 1.f / p.sigmaCoverage;
-    k.pixelAngle = 2.f * st.scene.cam.tanFovxOverTwo / ((float)H - 1.f);
-    for (uint32_t i = 0; i < p.iterations; ++i) {
-        const bool last = i + 1u == p.iterations;
-        denoise_iter_kernel<<<blocks, threads, 0, st.stream>>>(st.dDenoise[i & 1u], st.dDenoise[(i + 1u) & 1u], ac, nd, W, H, 1 << i, k,
-                                                               last ? (float*)hdrOutOrNull : nullptr, last ? (uint32_t*)imgOrNull : nullptr,
-                                                               st.scene.cam.exposure);
-        count_launch();
-        SVR_TRY(cudaGetLastError());
-    }
+extern "C" int svr_pathtracer_set_denoise_params(const svr_denoise_params* paramsOrNull)
+{
+    svr_denoise_params p;
+    if (int rc = check_denoise_params("svr_pathtracer_set_denoise_params", paramsOrNull, &p)) return rc;
+    state().progParams = p;  // the guides do not depend on it: the scene epoch stays
     return 0;
 }

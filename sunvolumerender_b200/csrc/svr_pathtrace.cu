@@ -2480,10 +2480,49 @@ static int lookahead_frame(uint32_t* img, float* hdr, uint32_t traceDepth, uint3
     return 0;
 }
 
+// SVR_OPT_PT_DENOISE (include/svr_render.h).  *done = the call was a denoised frame: one sample traced by the ordinary launch into
+// hdr (bit-identical to the option-off call) and into the even or odd sum by the parity of frameNo, then guides and filter into
+// img (svr_denoise.cu).  A call that does not continue the followed render drops it; so does a failed allocation, and the call
+// then renders as with the option off.
+static int denoised_frame(uint32_t* img, float* hdr, uint32_t traceDepth, uint32_t frameNo, bool* done)
+{
+    HostState& st = state();
+    *done = false;
+    const uint32_t W = st.scene.cam.imageW, H = st.scene.cam.imageH;
+    const bool follows = frameNo == 0u || (st.progActive && frameNo == st.progNext && hdr == st.progHdr && W == st.progW && H == st.progH &&
+                                           traceDepth == st.progDepth);
+    st.progActive = false;
+    if (!st.options[SVR_OPT_PT_DENOISE] || st.options[SVR_OPT_COUNTERS] || !follows || !img || !hdr || !W || !H) return 0;
+    const size_t npix = (size_t)W * H;
+    if (!ensure_progressive_buffers(st, npix)) return 0;
+    if (frameNo == 0u) SVR_TRY(cudaMemsetAsync(st.dProg[1], 0, npix * sizeof(float4), st.stream));
+    PtLaunch a;
+    memset(&a, 0, sizeof(a));
+    a.traceDepth = traceDepth;
+    a.firstSample = frameNo;
+    a.nSamples = 1;
+    a.y0 = 0;
+    a.y1 = 0xffffffffu;
+    a.hdr = hdr;
+    a.sum = st.dProg[frameNo & 1u];
+    a.clearSum = frameNo == 0u;
+    if (int rc = launch_pathtrace(a)) return rc;
+    if (int rc = progressive_denoise(img, frameNo)) return rc;
+    st.progActive = true;
+    st.progNext = frameNo + 1u;
+    st.progW = W;
+    st.progH = H;
+    st.progDepth = traceDepth;
+    st.progHdr = hdr;
+    *done = true;
+    return 0;
+}
+
 extern "C" void render_pathtracer(svr_u8vec4* img, const svr_render_params* renderParams)
 {
     bool done = false;
-    int rc = lookahead_frame((uint32_t*)img, (float*)renderParams->hdrBuffer, renderParams->traceDepth, renderParams->frameNo, &done);
+    int rc = denoised_frame((uint32_t*)img, (float*)renderParams->hdrBuffer, renderParams->traceDepth, renderParams->frameNo, &done);
+    if (!rc && !done) rc = lookahead_frame((uint32_t*)img, (float*)renderParams->hdrBuffer, renderParams->traceDepth, renderParams->frameNo, &done);
     if (!rc && !done) {
         PtLaunch a;
         memset(&a, 0, sizeof(a));
@@ -2515,6 +2554,7 @@ extern "C" void render_pathtracer(svr_u8vec4* img, const svr_render_params* rend
 extern "C" int svr_render_pathtracer_spp(svr_u8vec4* img, const svr_render_params* renderParams, uint32_t spp)
 {
     if (!renderParams || !renderParams->hdrBuffer) return fail_msg("svr_render_pathtracer_spp: hdrBuffer is null");
+    state().progActive = false;  // SVR_OPT_PT_DENOISE does not apply: the render it followed has moved on without its sums
     PtLaunch a;
     memset(&a, 0, sizeof(a));
     a.traceDepth = renderParams->traceDepth;

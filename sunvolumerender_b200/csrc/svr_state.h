@@ -95,6 +95,17 @@ struct HostState {
     float4* dDenoise[2] = {nullptr, nullptr};
     size_t denoiseCap = 0;
 
+    // Denoised progressive display (SVR_OPT_PT_DENOISE, render_pathtracer): the even and odd frames' sample sums and the guides
+    // (albedoCoverage, normalDepth) of the render being followed; progNext is the frame the next call must ask for
+    float4* dProg[4] = {nullptr, nullptr, nullptr, nullptr};
+    size_t progCap = 0;
+    bool progActive = false;
+    uint32_t progNext = 0, progW = 0, progH = 0, progDepth = 0;
+    const void* progHdr = nullptr;
+    unsigned long long progGuideEpoch = 0;  // sceneEpoch after the frame that made the guides; 0 = none
+    uint32_t progGuideRays = 0;
+    svr_denoise_params progParams;          // svr_pathtracer_set_denoise_params (state(): the defaults)
+
     Counters* dCounters = nullptr;
     unsigned long long launches = 0;
     std::string lastError;
@@ -149,6 +160,14 @@ int ensure_env_sampler(DevScene* scene);
 // the library's stream
 int ensure_mailbox(HostState& st);
 int read_small(HostState& st, void* host, const void* dev, size_t bytes);
+
+// Denoising (svr_denoise.cu).  check_denoise_params: 0, or the error of `who` (before any CUDA call).  progressive_denoise: the
+// guides and the filter of one denoised frame of render_pathtracer (SVR_OPT_PT_DENOISE) into img, after its sample has gone
+// into dProg[frameNo & 1]; ensure_progressive_buffers: false when they cannot be allocated.
+int check_denoise_params(const char* who, const svr_denoise_params* paramsOrNull, svr_denoise_params* out);
+bool ensure_progressive_buffers(HostState& st, size_t npix);
+int progressive_denoise(uint32_t* img, uint32_t frameNo);
+void release_progressive(HostState& st);
 
 inline void count_launch(int n = 1) { state().launches += (unsigned long long)n; }
 

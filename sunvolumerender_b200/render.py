@@ -274,6 +274,21 @@ class Renderer:
         L.check(self.lib.svr_pathtracer_denoise(_ptr(self.img), _ptr(self.hdr if want_hdr else None), _ptr(sum_buf), _ptr(half_buf),
                                                 _ptr(albedo_cov), _ptr(normal_depth), C.byref(p)), "svr_pathtracer_denoise")
 
+    def set_denoise_params(self, params=None):
+        """Filter parameters of the denoised progressive display (OPT_PT_DENOISE, svr_pathtracer_set_denoise_params): a dict
+        with any of iterations, sigma_luminance, sigma_normal, sigma_depth, sigma_coverage (the others take the library's
+        defaults), or None for the defaults."""
+        if params is None:
+            L.check(self.lib.svr_pathtracer_set_denoise_params(None), "svr_pathtracer_set_denoise_params")
+            return
+        p = L.DenoiseParams()
+        L.check(self.lib.svr_denoise_defaults(C.byref(p)), "svr_denoise_defaults")
+        names = {"iterations": "iterations", "sigma_luminance": "sigmaLuminance", "sigma_normal": "sigmaNormal", "sigma_depth": "sigmaDepth",
+                 "sigma_coverage": "sigmaCoverage"}
+        for key, value in params.items():
+            setattr(p, names[key], value)
+        L.check(self.lib.svr_pathtracer_set_denoise_params(C.byref(p)), "svr_pathtracer_set_denoise_params")
+
     def resolve(self, sum_buf, want_hdr=True):
         ptr = sum_buf if isinstance(sum_buf, C.c_void_p) else _ptr(sum_buf)
         L.check(self.lib.svr_pathtracer_resolve(_ptr(self.img), _ptr(self.hdr if want_hdr else None), ptr), "svr_pathtracer_resolve")

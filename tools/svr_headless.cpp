@@ -12,6 +12,8 @@
 //   press X Y BUTTONS | move X Y BUTTONS | wheel DELTA | key left|right|down      (BUTTONS: 1 left, 4 middle)
 //   mode pt|rc | depth D | density S | gradient G | fov F | exposure E | apeture A | focal L | clip x|y|z LO HI
 //   envcolor R G B | envintensity I | envmap file.hdr | repaint 0|1 | paint N | save prefix
+//   denoise 0|1|4|16      (SVR_OPT_PT_DENOISE: the denoised progressive display from the next restart of the render on)
+// The whole script is parsed before the device is touched: a malformed line fails with exit code 2.
 //
 // --volume loads a MetaImage file the way Canvas::LoadVolume does (core/VolumeReader.cpp:13-94) instead of
 // generating the configuration's synthetic volume; camera and light are framed on its extent.
@@ -89,6 +91,59 @@ static void tf_table(const std::string& kind, std::vector<float>& t)
     }
 }
 
+// One line of an --interact script.  canvas == nullptr: parse only (non-zero = malformed); otherwise run it (non-zero = a call
+// failed).  Blank lines and lines starting with '#' do nothing.
+static int interact_line(svr_canvas* canvas, const std::string& line, int npix, int W, int H)
+{
+#define RUN(x)                   \
+    do {                         \
+        if (canvas) SVR(x);      \
+    } while (0)
+    std::istringstream ls(line);
+    std::string cmd;
+    if (!(ls >> cmd) || cmd[0] == '#') return 0;
+    float a = 0.f, b = 0.f, c3 = 0.f;
+    int n = 0;
+    std::string word;
+    if (cmd == "press" && ls >> a >> b >> n) RUN(svr_canvas_mouse_press(canvas, a, b, n));
+    else if (cmd == "move" && ls >> a >> b >> n) RUN(svr_canvas_mouse_move(canvas, a, b, n));
+    else if (cmd == "wheel" && ls >> n) RUN(svr_canvas_wheel(canvas, n));
+    else if (cmd == "key" && ls >> word) RUN(svr_canvas_key(canvas, word == "left" ? SVR_KEY_LEFT : word == "right" ? SVR_KEY_RIGHT : SVR_KEY_DOWN));
+    else if (cmd == "mode" && ls >> word) RUN(svr_canvas_set_render_mode(canvas, word == "pt" ? SVR_RENDER_MODE_PATHTRACER : SVR_RENDER_MODE_RAYCASTING));
+    else if (cmd == "depth" && ls >> a) RUN(svr_canvas_set_scatter_times(canvas, a));
+    else if (cmd == "density" && ls >> a) RUN(svr_canvas_set_density_scale(canvas, a));
+    else if (cmd == "gradient" && ls >> a) RUN(svr_canvas_set_gradient_factor(canvas, a));
+    else if (cmd == "fov" && ls >> a) RUN(svr_canvas_set_fov(canvas, a));
+    else if (cmd == "exposure" && ls >> a) RUN(svr_canvas_set_exposure(canvas, a));
+    else if (cmd == "apeture" && ls >> a) RUN(svr_canvas_set_apeture(canvas, a));
+    else if (cmd == "focal" && ls >> a) RUN(svr_canvas_set_focal_length(canvas, a));
+    else if (cmd == "clip" && ls >> word >> a >> b) RUN(svr_canvas_set_clip_plane(canvas, word == "x" ? 0 : word == "y" ? 1 : 2, a, b));
+    else if (cmd == "envcolor" && ls >> a >> b >> c3) RUN(svr_canvas_set_env_background(canvas, a, b, c3));
+    else if (cmd == "envintensity" && ls >> a) RUN(svr_canvas_set_env_intensity(canvas, a));
+    else if (cmd == "envmap" && ls >> word) RUN(svr_canvas_set_env_map(canvas, word.c_str()));
+    else if (cmd == "denoise" && ls >> n && (n == 0 || n == 1 || n == 4 || n == 16)) RUN(svr_set_option(SVR_OPT_PT_DENOISE, n));
+    else if (cmd == "repaint" && ls >> n) {
+        if (canvas) svr_canvas_set_immediate_repaint(canvas, n);
+    } else if (cmd == "paint" && ls >> n) {
+        for (int i = 0; i < n; ++i) RUN(svr_canvas_paint(canvas));
+    } else if (cmd == "save" && ls >> word) {
+        if (!canvas) return 0;
+        std::vector<unsigned char> px((size_t)npix * 4);
+        SVR(svr_canvas_read_image(canvas, px.data()));
+        FILE* f = fopen((word + ".ppm").c_str(), "wb");
+        if (f) {
+            fprintf(f, "P6\n%d %d\n255\n", W, H);
+            for (int y = H - 1; y >= 0; --y)
+                for (int x = 0; x < W; ++x) fwrite(&px[4 * ((size_t)y * W + x)], 1, 3, f);
+            fclose(f);
+        }
+    } else {
+        return 2;
+    }
+    return 0;
+#undef RUN
+}
+
 int main(int argc, char** argv)
 {
     Config cfg = kConfigs[0];
@@ -116,6 +171,22 @@ int main(int argc, char** argv)
         else if (k == "--reps") reps = atoi(v.c_str());
         else if (k == "--interact") interactPath = v;
         else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
+    }
+    std::vector<std::string> script;
+    if (!interactPath.empty()) {
+        std::ifstream in(interactPath);
+        if (!in) {
+            fprintf(stderr, "cannot open %s\n", interactPath.c_str());
+            return 1;
+        }
+        std::string line;
+        for (int lineNo = 1; std::getline(in, line); ++lineNo) {
+            if (interact_line(nullptr, line, 0, 0, 0)) {
+                fprintf(stderr, "%s:%d: cannot parse '%s'\n", interactPath.c_str(), lineNo, line.c_str());
+                return 2;
+            }
+            script.push_back(line);
+        }
     }
     if (sppArg > 0) cfg.spp = sppArg;
     if (depthArg >= 0) cfg.depth = depthArg;
@@ -207,54 +278,9 @@ int main(int argc, char** argv)
         SVR(svr_canvas_set_volume(canvas, &vol, size, radius));
         SVR(svr_canvas_set_transfer_function(canvas, &tf));
         SVR(svr_canvas_set_area_lights(canvas, &light, 1));
-        std::ifstream in(interactPath);
-        if (!in) {
-            fprintf(stderr, "cannot open %s\n", interactPath.c_str());
-            return 1;
-        }
-        std::string line;
-        int lineNo = 0;
-        while (std::getline(in, line)) {
-            ++lineNo;
-            std::istringstream ls(line);
-            std::string cmd;
-            if (!(ls >> cmd) || cmd[0] == '#') continue;
-            float a = 0.f, b = 0.f, c3 = 0.f;
-            int n = 0;
-            std::string word;
-            if (cmd == "press" && ls >> a >> b >> n) SVR(svr_canvas_mouse_press(canvas, a, b, n));
-            else if (cmd == "move" && ls >> a >> b >> n) SVR(svr_canvas_mouse_move(canvas, a, b, n));
-            else if (cmd == "wheel" && ls >> n) SVR(svr_canvas_wheel(canvas, n));
-            else if (cmd == "key" && ls >> word) SVR(svr_canvas_key(canvas, word == "left" ? SVR_KEY_LEFT : word == "right" ? SVR_KEY_RIGHT : SVR_KEY_DOWN));
-            else if (cmd == "mode" && ls >> word) SVR(svr_canvas_set_render_mode(canvas, word == "pt" ? SVR_RENDER_MODE_PATHTRACER : SVR_RENDER_MODE_RAYCASTING));
-            else if (cmd == "depth" && ls >> a) SVR(svr_canvas_set_scatter_times(canvas, a));
-            else if (cmd == "density" && ls >> a) SVR(svr_canvas_set_density_scale(canvas, a));
-            else if (cmd == "gradient" && ls >> a) SVR(svr_canvas_set_gradient_factor(canvas, a));
-            else if (cmd == "fov" && ls >> a) SVR(svr_canvas_set_fov(canvas, a));
-            else if (cmd == "exposure" && ls >> a) SVR(svr_canvas_set_exposure(canvas, a));
-            else if (cmd == "apeture" && ls >> a) SVR(svr_canvas_set_apeture(canvas, a));
-            else if (cmd == "focal" && ls >> a) SVR(svr_canvas_set_focal_length(canvas, a));
-            else if (cmd == "clip" && ls >> word >> a >> b) SVR(svr_canvas_set_clip_plane(canvas, word == "x" ? 0 : word == "y" ? 1 : 2, a, b));
-            else if (cmd == "envcolor" && ls >> a >> b >> c3) SVR(svr_canvas_set_env_background(canvas, a, b, c3));
-            else if (cmd == "envintensity" && ls >> a) SVR(svr_canvas_set_env_intensity(canvas, a));
-            else if (cmd == "envmap" && ls >> word) SVR(svr_canvas_set_env_map(canvas, word.c_str()));
-            else if (cmd == "repaint" && ls >> n) svr_canvas_set_immediate_repaint(canvas, n);
-            else if (cmd == "paint" && ls >> n) {
-                for (int i = 0; i < n; ++i) SVR(svr_canvas_paint(canvas));
-            } else if (cmd == "save" && ls >> word) {
-                std::vector<unsigned char> px(npix * 4);
-                SVR(svr_canvas_read_image(canvas, px.data()));
-                FILE* f = fopen((word + ".ppm").c_str(), "wb");
-                if (f) {
-                    fprintf(f, "P6\n%d %d\n255\n", W, H);
-                    for (int y = H - 1; y >= 0; --y)
-                        for (int x = 0; x < W; ++x) fwrite(&px[4 * ((size_t)y * W + x)], 1, 3, f);
-                    fclose(f);
-                }
-            } else {
-                fprintf(stderr, "%s:%d: cannot parse '%s'\n", interactPath.c_str(), lineNo, line.c_str());
-                return 2;
-            }
+        for (size_t i = 0; i < script.size(); ++i) {
+            const int rc = interact_line(canvas, script[i], (int)npix, W, H);
+            if (rc) return rc;
         }
         svr_camera cc;
         svr_canvas_get_camera(canvas, &cc);
