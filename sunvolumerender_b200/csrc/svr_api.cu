@@ -71,6 +71,17 @@ HostState& state()
     return *s;
 }
 
+void DeviceState::reset()
+{
+    if (volPointTex) cudaDestroyTextureObject(volPointTex);
+    if (uploadSurf) cudaDestroySurfaceObject(uploadSurf);
+    if (aheadEvReady)
+        for (cudaEvent_t e : aheadEv) cudaEventDestroy(e);  // events belong to the device they were created on
+    if (tfCheckEvent) cudaEventDestroy(tfCheckEvent);
+    if (hMailbox) cudaFreeHost(hMailbox);
+    *this = DeviceState();  // the DevBufs swapped out here free themselves
+}
+
 int fail(const char* where, cudaError_t e)
 {
     char buf[512];
@@ -113,11 +124,11 @@ extern "C" void setup_volume(const svr_volume* vol)
     // nothing: any change of texture handle, box, spacing or gradient normalisation drops the cache (ranges,
     // dims and the point-sampled view bound to the old array); and when the struct is unchanged in all of those a
     // sampled fingerprint of the voxels is compared against the one taken when the ranges were built.
-    if (st.gridArray && !same_volume_resource(st.scene.vol, *vol)) release_grid(st);
+    if (st.dev.gridArray && !same_volume_resource(st.scene.vol, *vol)) release_grid(st);
     st.scene.vol = *vol;
     st.sceneEpoch++;
-    st.majorantValid = false;  // densityScale / array may have changed
-    st.fingerprintDue = true;  // checked at the next grid use (needs the stream; setup_* must stay cheap)
+    st.dev.majorantValid = false;  // densityScale / array may have changed
+    st.dev.fingerprintDue = true;  // checked at the next grid use (needs the stream; setup_* must stay cheap)
     if (st.options[SVR_OPT_SETUP_SYNC]) SVR_FATAL(cudaDeviceSynchronize());
 }
 
@@ -126,7 +137,7 @@ extern "C" void setup_transferfunction(const svr_transfer_function* tf)
     HostState& st = state();
     st.scene.tf = *tf;
     st.sceneEpoch++;
-    st.majorantValid = false;  // every TF edit invalidates the local majorants
+    st.dev.majorantValid = false;  // every TF edit invalidates the local majorants
     if (st.options[SVR_OPT_SETUP_SYNC]) SVR_FATAL(cudaDeviceSynchronize());
 }
 
@@ -172,57 +183,9 @@ extern "C" int svr_set_device(int device)
 {
     HostState& st = state();
     SVR_TRY(cudaSetDevice(device));
-    // derived data lives on the previous device: drop it
-    release_grid(st);
-    cudaFree(st.dTfSparse);
-    cudaFree(st.dTfTable);
-    cudaFree(st.dCounters);
-    cudaFree(st.dStats);
-    cudaFree(st.dFingerprint);
-    cudaFree(st.dTfHash);
-    cudaFree(st.dPixelCache);
-    st.dPixelCache = nullptr;
-    st.pixelCacheCap = 0;
-    cudaFree(st.dAdaptiveList);
-    cudaFree(st.dAdaptiveCounts);
-    st.dAdaptiveList = st.dAdaptiveCounts = nullptr;
-    st.adaptiveListCap = 0;
-    cudaFree(st.dDenoise[0]);
-    cudaFree(st.dDenoise[1]);
-    st.dDenoise[0] = st.dDenoise[1] = nullptr;
-    st.denoiseCap = 0;
-    release_progressive(st);
-    cudaFree(st.dAhead);
-    st.dAhead = nullptr;
-    st.aheadCapFloats = 0;
-    st.aheadCount = 0;
-    if (st.aheadEvReady)
-        for (int i = 0; i < 6; ++i) cudaEventDestroy(st.aheadEv[i]);  // events belong to the device they were created on
-    st.aheadEvReady = false;
-    st.aheadSingleEpoch = st.aheadTimedEpoch = st.aheadOffEpoch = 0;
-    if (st.tfCheckEvent) cudaEventDestroy(st.tfCheckEvent);
-    st.tfCheckEvent = nullptr;
-    st.tfCheckPending = false;
-    cudaFreeHost(st.hMailbox);
-    st.hMailbox = st.dMailbox = nullptr;
-    if (st.uploadSurf) cudaDestroySurfaceObject(st.uploadSurf);
-    st.uploadSurf = 0;
-    st.uploadSurfArray = nullptr;
+    st.dev.reset();  // derived data lives on the previous device: drop it
     cudaGetLastError();
     st.sceneEpoch++;
-    cudaFree(st.dEnvMarg);
-    cudaFree(st.dEnvCond);
-    st.dEnvMarg = st.dEnvCond = nullptr;
-    st.envSamplerValid = false;
-    st.dFingerprint = nullptr;
-    st.dTfHash = nullptr;
-    st.dStats = nullptr;
-    st.autoCell = 0;
-    st.dTfSparse = nullptr;
-    st.dTfTable = nullptr;
-    st.tfEntries = 0;
-    st.dCounters = nullptr;
-    cudaGetLastError();
     return 0;
 }
 
@@ -239,7 +202,7 @@ extern "C" int svr_set_option(int key, int value)
                 return fail_msg("SVR_OPT_MACROCELL_SIZE must be 0 (automatic) or a power of two in 2..64");
             if (value != st.options[key]) {
                 release_grid(st);
-                st.autoCell = 0;
+                st.dev.autoCell = 0;
             }
             break;
         case SVR_OPT_PT_BLOCK:
@@ -303,11 +266,11 @@ namespace svr {
 Counters* device_counters()
 {
     HostState& st = state();
-    if (!st.dCounters) {
-        if (cudaMalloc(&st.dCounters, sizeof(Counters)) != cudaSuccess) return nullptr;
-        cudaMemset(st.dCounters, 0, sizeof(Counters));
+    if (!st.dev.counters.p) {
+        if (st.dev.counters.reserve(1) != cudaSuccess) return nullptr;
+        cudaMemset(st.dev.counters.p, 0, sizeof(Counters));
     }
-    return st.dCounters;
+    return st.dev.counters.p;
 }
 }  // namespace svr
 
@@ -470,9 +433,9 @@ extern "C" int svr_volume_upload(const svr_volume* vol, const void* data, int da
         cp.srcPtr = make_cudaPitchedPtr(const_cast<void*>(data), ext.width * bpe, ext.width, ext.height);
         SVR_TRY(cudaMemcpy3DAsync(&cp, st.stream));
         // same dims, new contents: the grid's allocations stay, its range stage reruns at the next render
-        if (rd.res.array.array == st.gridArray) st.rangeValid = false;
+        if (rd.res.array.array == st.dev.gridArray) st.dev.rangeValid = false;
     }
-    st.uploadEpoch++;
+    st.dev.uploadEpoch++;
     st.sceneEpoch++;
     return 0;
 }
@@ -546,8 +509,8 @@ extern "C" int svr_tf_upload(svr_transfer_function* tf, const float* host_rgba, 
     float maxOpacity = 0.f;
     for (uint32_t i = 0; i < n; ++i) maxOpacity = fmaxf(maxOpacity, host_rgba[4 * i + 3]);
     tf->maxOpacity = maxOpacity;
-    st.majorantValid = false;
-    st.uploadEpoch++;
+    st.dev.majorantValid = false;
+    st.dev.uploadEpoch++;
     st.sceneEpoch++;
     return 0;
 }
@@ -559,7 +522,7 @@ extern "C" int svr_volume_destroy(svr_volume* vol)
     cudaResourceDesc rd;
     SVR_TRY(cudaGetTextureObjectResourceDesc(&rd, vol->tex));
     SVR_TRY(cudaDeviceSynchronize());
-    if (rd.resType == cudaResourceTypeArray && rd.res.array.array == st.gridArray) release_grid(st);
+    if (rd.resType == cudaResourceTypeArray && rd.res.array.array == st.dev.gridArray) release_grid(st);
     SVR_TRY(cudaDestroyTextureObject(vol->tex));
     if (rd.resType == cudaResourceTypeArray) SVR_TRY(cudaFreeArray(rd.res.array.array));
     vol->tex = 0;
@@ -611,9 +574,9 @@ extern "C" int svr_tf_destroy(svr_transfer_function* tf)
     cudaResourceDesc rd;
     SVR_TRY(cudaGetTextureObjectResourceDesc(&rd, tf->tex));
     SVR_TRY(cudaDeviceSynchronize());
-    if (rd.resType == cudaResourceTypeArray && rd.res.array.array == state().majorantTfArray) {
-        state().majorantTfArray = nullptr;
-        state().majorantValid = false;
+    if (rd.resType == cudaResourceTypeArray && rd.res.array.array == state().dev.majorantTfArray) {
+        state().dev.majorantTfArray = nullptr;
+        state().dev.majorantValid = false;
     }
     SVR_TRY(cudaDestroyTextureObject(tf->tex));
     if (rd.resType == cudaResourceTypeArray) SVR_TRY(cudaFreeArray(rd.res.array.array));

@@ -278,32 +278,19 @@ int check_denoise_params(const char* who, const svr_denoise_params* paramsOrNull
 
 namespace {
 
-// The filter's two ping-pong buffers for npix pixels
-int ensure_filter_buffers(HostState& st, size_t npix)
-{
-    if (st.denoiseCap >= npix) return 0;
-    cudaFree(st.dDenoise[0]);
-    cudaFree(st.dDenoise[1]);
-    st.dDenoise[0] = st.dDenoise[1] = nullptr;
-    st.denoiseCap = 0;
-    SVR_TRY(cudaMalloc(&st.dDenoise[0], npix * sizeof(float4)));
-    SVR_TRY(cudaMalloc(&st.dDenoise[1], npix * sizeof(float4)));
-    st.denoiseCap = npix;
-    return 0;
-}
-
-// The filter for checked parameters and a camera of W x H pixels.  `sum` may be dDenoise[1]: the prep pass reads it before the
-// first iteration writes there.
+// The filter for checked parameters and a camera of W x H pixels, ping-ponging between the two halves of st.dev.denoise.  `sum`
+// may be the second half: the prep pass reads it before the first iteration writes there.
 int run_filter(uint32_t* img, float* hdr, const float4* sum, const float4* half, const float4* ac, const float4* nd, const svr_denoise_params& p)
 {
     HostState& st = state();
     const uint32_t W = st.scene.cam.imageW, H = st.scene.cam.imageH;
     if (p.iterations == 0u) return svr_pathtracer_resolve((svr_u8vec4*)img, (svr_vec3*)hdr, (const svr_vec4*)sum);  // the identity, bit for bit
 
-    if (hdr && (const void*)hdr == st.aheadHdr) st.aheadCount = 0;  // as svr_pathtracer_resolve
-    if (int rc = ensure_filter_buffers(st, (size_t)W * H)) return rc;
+    hdr_written_outside(st.dev, hdr, false);  // as svr_pathtracer_resolve
+    SVR_TRY(st.dev.denoise.reserve(2 * (size_t)W * H));
+    float4* const buf[2] = {st.dev.denoise.p, st.dev.denoise.p + (size_t)W * H};
     const dim3 blocks((W + 31u) / 32u, (H + 7u) / 8u), threads(32, 8);
-    denoise_prep_kernel<<<blocks, threads, 0, st.stream>>>(sum, half, ac, st.dDenoise[0], W, H);
+    denoise_prep_kernel<<<blocks, threads, 0, st.stream>>>(sum, half, ac, buf[0], W, H);
     count_launch();
     SVR_TRY(cudaGetLastError());
     DenoiseStops k;
@@ -314,7 +301,7 @@ int run_filter(uint32_t* img, float* hdr, const float4* sum, const float4* half,
     k.pixelAngle = 2.f * st.scene.cam.tanFovxOverTwo / ((float)H - 1.f);
     for (uint32_t i = 0; i < p.iterations; ++i) {
         const bool last = i + 1u == p.iterations;
-        denoise_iter_kernel<<<blocks, threads, 0, st.stream>>>(st.dDenoise[i & 1u], st.dDenoise[(i + 1u) & 1u], ac, nd, W, H, 1 << i, k,
+        denoise_iter_kernel<<<blocks, threads, 0, st.stream>>>(buf[i & 1u], buf[(i + 1u) & 1u], ac, nd, W, H, 1 << i, k,
                                                                last ? hdr : nullptr, last ? img : nullptr, st.scene.cam.exposure);
         count_launch();
         SVR_TRY(cudaGetLastError());
@@ -324,37 +311,15 @@ int run_filter(uint32_t* img, float* hdr, const float4* sum, const float4* half,
 
 }  // namespace
 
-// dProg[0..3] (even sum, odd sum, albedoCoverage, normalDepth) and the filter's buffers; on failure nothing is kept allocated
-// but what was there before, and the CUDA error is cleared
+// st.dev.prog (even sum, odd sum, albedoCoverage, normalDepth) and the filter's buffers; on failure the CUDA error is cleared
 bool ensure_progressive_buffers(HostState& st, size_t npix)
 {
-    if (st.progCap < npix) {
-        release_progressive(st);
-        for (int i = 0; i < 4; ++i)
-            if (cudaMalloc(&st.dProg[i], npix * sizeof(float4)) != cudaSuccess) {
-                cudaGetLastError();
-                release_progressive(st);
-                return false;
-            }
-        st.progCap = npix;
-    }
-    if (ensure_filter_buffers(st, npix)) {
+    if (st.dev.prog.cap < 4 * npix) st.dev.progGuideEpoch = 0;  // new memory holds no guides
+    if (st.dev.prog.reserve(4 * npix) != cudaSuccess || st.dev.denoise.reserve(2 * npix) != cudaSuccess) {
         cudaGetLastError();
         return false;
     }
     return true;
-}
-
-void release_progressive(HostState& st)
-{
-    for (int i = 0; i < 4; ++i) {
-        cudaFree(st.dProg[i]);
-        st.dProg[i] = nullptr;
-    }
-    st.progCap = 0;
-    st.progActive = false;
-    st.progGuideEpoch = 0;
-    st.progGuideRays = 0;
 }
 
 // Guides made with SVR_OPT_PT_DENOISE rays before frame 16 and with 16 from there on, kept while the scene epoch stays where it
@@ -363,16 +328,17 @@ int progressive_denoise(uint32_t* img, uint32_t frameNo)
 {
     HostState& st = state();
     const uint32_t rays = frameNo >= 16u ? 16u : (uint32_t)st.options[SVR_OPT_PT_DENOISE];
-    if (st.progGuideEpoch != st.sceneEpoch || st.progGuideRays != rays) {
-        if (int rc = svr_pathtracer_guides((svr_vec4*)st.dProg[2], (svr_vec4*)st.dProg[3], rays)) return rc;
-        st.progGuideRays = rays;
-    }
     const uint32_t npix = st.scene.cam.imageW * st.scene.cam.imageH;
-    sum_halves_kernel<<<(npix + 255u) / 256u, 256, 0, st.stream>>>(st.dProg[0], st.dProg[1], st.dDenoise[1], npix);
+    float4* const prog = st.dev.prog.p;
+    if (st.dev.progGuideEpoch != st.sceneEpoch || st.dev.progGuideRays != rays) {
+        if (int rc = svr_pathtracer_guides((svr_vec4*)(prog + 2 * npix), (svr_vec4*)(prog + 3 * npix), rays)) return rc;
+        st.dev.progGuideRays = rays;
+    }
+    sum_halves_kernel<<<(npix + 255u) / 256u, 256, 0, st.stream>>>(prog, prog + npix, st.dev.denoise.p + npix, npix);
     count_launch();
     SVR_TRY(cudaGetLastError());
-    if (int rc = run_filter(img, nullptr, st.dDenoise[1], st.dProg[1], st.dProg[2], st.dProg[3], st.progParams)) return rc;
-    st.progGuideEpoch = st.sceneEpoch;  // after the frame's launches: refreshing the majorants moves the epoch
+    if (int rc = run_filter(img, nullptr, st.dev.denoise.p + npix, prog + npix, prog + 2 * npix, prog + 3 * npix, st.progParams)) return rc;
+    st.dev.progGuideEpoch = st.sceneEpoch;  // after the frame's launches: refreshing the majorants moves the epoch
     return 0;
 }
 

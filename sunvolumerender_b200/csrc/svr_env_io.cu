@@ -272,23 +272,23 @@ int ensure_env_sampler(DevScene* scene)
 {
     HostState& st = state();
     const svr_env_light& e = scene->env;
-    if (!st.envSamplerValid || memcmp(&st.envSamplerKey, &e, sizeof(e)) != 0) {
-        if (!st.dEnvMarg) SVR_TRY(cudaMalloc(&st.dEnvMarg, (ENV_H + 1) * sizeof(float)));
-        if (!st.dEnvCond) SVR_TRY(cudaMalloc(&st.dEnvCond, (size_t)ENV_H * (ENV_W + 1) * sizeof(float)));
-        if (!st.dStats) SVR_TRY(cudaMalloc(&st.dStats, 16));
-        SVR_TRY(cudaMemsetAsync(st.dStats, 0, 16, st.stream));
+    if (!st.dev.envSamplerValid || memcmp(&st.dev.envSamplerKey, &e, sizeof(e)) != 0) {
+        SVR_TRY(st.dev.envMarg.reserve(ENV_H + 1));
+        SVR_TRY(st.dev.envCond.reserve((size_t)ENV_H * (ENV_W + 1)));
+        SVR_TRY(st.dev.stats.reserve(2));
+        SVR_TRY(cudaMemsetAsync(st.dev.stats.p, 0, 16, st.stream));
         double sinSum = 0.0;
         for (int j = 0; j < ENV_H; ++j) sinSum += (double)sinf(SVR_PI_F * ((float)j + 0.5f) / (float)ENV_H);
-        env_lum_kernel<<<ENV_H, ENV_W, 0, st.stream>>>(e, st.dEnvCond, st.dEnvMarg, (double*)st.dStats);
-        env_cond_kernel<<<ENV_H, ENV_W, 0, st.stream>>>(st.dEnvCond, st.dEnvMarg, (const double*)st.dStats, sinSum);
-        env_marg_kernel<<<1, ENV_H, 0, st.stream>>>(st.dEnvMarg);
+        env_lum_kernel<<<ENV_H, ENV_W, 0, st.stream>>>(e, st.dev.envCond.p, st.dev.envMarg.p, (double*)st.dev.stats.p);
+        env_cond_kernel<<<ENV_H, ENV_W, 0, st.stream>>>(st.dev.envCond.p, st.dev.envMarg.p, (const double*)st.dev.stats.p, sinSum);
+        env_marg_kernel<<<1, ENV_H, 0, st.stream>>>(st.dev.envMarg.p);
         count_launch(3);
         SVR_TRY(cudaGetLastError());
-        st.envSamplerKey = e;
-        st.envSamplerValid = true;
+        st.dev.envSamplerKey = e;
+        st.dev.envSamplerValid = true;
     }
-    scene->envS.marg = st.dEnvMarg;
-    scene->envS.cond = st.dEnvCond;
+    scene->envS.marg = st.dev.envMarg.p;
+    scene->envS.cond = st.dev.envCond.p;
     scene->envS.w = ENV_W;
     scene->envS.h = ENV_H;
     return 0;
@@ -305,7 +305,7 @@ extern "C" int svr_env_sampler_copy(float* host_marg, float* host_cond, uint32_t
     SVR_TRY(cudaStreamSynchronize(st.stream));
     if (w) *w = ENV_W;
     if (h) *h = ENV_H;
-    if (host_marg) SVR_TRY(cudaMemcpy(host_marg, st.dEnvMarg, (ENV_H + 1) * sizeof(float), cudaMemcpyDeviceToHost));
-    if (host_cond) SVR_TRY(cudaMemcpy(host_cond, st.dEnvCond, (size_t)ENV_H * (ENV_W + 1) * sizeof(float), cudaMemcpyDeviceToHost));
+    if (host_marg) SVR_TRY(cudaMemcpy(host_marg, st.dev.envMarg.p, (ENV_H + 1) * sizeof(float), cudaMemcpyDeviceToHost));
+    if (host_cond) SVR_TRY(cudaMemcpy(host_cond, st.dev.envCond.p, (size_t)ENV_H * (ENV_W + 1) * sizeof(float), cudaMemcpyDeviceToHost));
     return 0;
 }

@@ -179,10 +179,10 @@ int launch_range_brick_cell(HostState& st, Fetch fetch)
     constexpr int BX = 32 / CELL, BY = CELL <= 8 ? 8 / CELL : 1, BZ = BY;
     constexpr int TX = BX * CELL + 2, TY = BY * CELL + 2, TZ = BZ * CELL + 2;
     constexpr size_t shm = sizeof(float) * ((size_t)TX * TY * TZ + 2 * (size_t)BX * TY * TZ + 2 * (size_t)BX * BY * TZ);
-    dim3 g((st.gridDims.x + BX - 1) / BX, (st.gridDims.y + BY - 1) / BY, (st.gridDims.z + BZ - 1) / BZ);
+    dim3 g((st.dev.gridDims.x + BX - 1) / BX, (st.dev.gridDims.y + BY - 1) / BY, (st.dev.gridDims.z + BZ - 1) / BZ);
     if (shm > 48 * 1024)
         SVR_TRY(cudaFuncSetAttribute(range_brick_kernel<Fetch, CELL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm));
-    range_brick_kernel<Fetch, CELL><<<g, 256, shm, st.stream>>>(fetch, st.gridDims, st.dRange);
+    range_brick_kernel<Fetch, CELL><<<g, 256, shm, st.stream>>>(fetch, st.dev.gridDims, st.dev.range.p);
     count_launch();
     SVR_TRY(cudaGetLastError());
     return 0;
@@ -191,7 +191,7 @@ int launch_range_brick_cell(HostState& st, Fetch fetch)
 template <class Fetch>
 int launch_range_brick(HostState& st, Fetch fetch)
 {
-    switch (st.gridCell) {
+    switch (st.dev.gridCell) {
         case 2: return launch_range_brick_cell<Fetch, 2>(st, fetch);
         case 4: return launch_range_brick_cell<Fetch, 4>(st, fetch);
         case 8: return launch_range_brick_cell<Fetch, 8>(st, fetch);
@@ -355,15 +355,15 @@ int launch_upload_range_cell(HostState& st, const void* src, cudaSurfaceObject_t
     constexpr int BX = 32 / CELL, BY = CELL <= 8 ? 8 / CELL : 1, BZ = BY;
     constexpr int TX = BX * CELL + 2, TY = BY * CELL + 2, TZ = BZ * CELL + 2;
     constexpr size_t shm = sizeof(float) * ((size_t)TX * TY * TZ + 2 * (size_t)BX * TY * TZ + 2 * (size_t)BX * BY * TZ);
-    dim3 g((st.gridDims.x + BX - 1) / BX, (st.gridDims.y + BY - 1) / BY, (st.gridDims.z + BZ - 1) / BZ);
-    if (st.volDims.x % 32 == 0 && ((uintptr_t)src & 15u) == 0) {
+    dim3 g((st.dev.gridDims.x + BX - 1) / BX, (st.dev.gridDims.y + BY - 1) / BY, (st.dev.gridDims.z + BZ - 1) / BZ);
+    if (st.dev.volDims.x % 32 == 0 && ((uintptr_t)src & 15u) == 0) {
         if (shm > 48 * 1024)
             SVR_TRY(cudaFuncSetAttribute(upload_range_vec_kernel<V, CELL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm));
-        upload_range_vec_kernel<V, CELL><<<g, 256, shm, st.stream>>>((const typename V::raw*)src, surf, st.volDims, st.gridDims, st.dRange);
+        upload_range_vec_kernel<V, CELL><<<g, 256, shm, st.stream>>>((const typename V::raw*)src, surf, st.dev.volDims, st.dev.gridDims, st.dev.range.p);
     } else {
         if (shm > 48 * 1024)
             SVR_TRY(cudaFuncSetAttribute(upload_range_kernel<V, CELL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm));
-        upload_range_kernel<V, CELL><<<g, 256, shm, st.stream>>>((const typename V::raw*)src, surf, st.volDims, st.gridDims, st.dRange);
+        upload_range_kernel<V, CELL><<<g, 256, shm, st.stream>>>((const typename V::raw*)src, surf, st.dev.volDims, st.dev.gridDims, st.dev.range.p);
     }
     count_launch();
     SVR_TRY(cudaGetLastError());
@@ -373,7 +373,7 @@ int launch_upload_range_cell(HostState& st, const void* src, cudaSurfaceObject_t
 template <class V>
 int launch_upload_range(HostState& st, const void* src, cudaSurfaceObject_t surf)
 {
-    switch (st.gridCell) {
+    switch (st.dev.gridCell) {
         case 2: return launch_upload_range_cell<V, 2>(st, src, surf);
         case 4: return launch_upload_range_cell<V, 4>(st, src, surf);
         case 8: return launch_upload_range_cell<V, 8>(st, src, surf);
@@ -535,9 +535,9 @@ __global__ void mailbox_kernel(const unsigned int* src, unsigned int* mailbox, i
 
 int launch_fingerprint(HostState& st, int slot)
 {
-    if (!st.dFingerprint) SVR_TRY(cudaMalloc(&st.dFingerprint, 2 * sizeof(unsigned long long)));
-    if (int rc = zero_words(st, st.dFingerprint + slot, sizeof(unsigned long long))) return rc;
-    fingerprint_kernel<<<64, 128, 0, st.stream>>>(st.volPointTex, st.volDims, st.dFingerprint + slot);
+    SVR_TRY(st.dev.fingerprint.reserve(2));
+    if (int rc = zero_words(st, st.dev.fingerprint.p + slot, sizeof(unsigned long long))) return rc;
+    fingerprint_kernel<<<64, 128, 0, st.stream>>>(st.dev.volPointTex, st.dev.volDims, st.dev.fingerprint.p + slot);
     count_launch();
     SVR_TRY(cudaGetLastError());
     return 0;
@@ -578,8 +578,8 @@ __global__ void tf_hash_kernel(const float4* table, cudaTextureObject_t tex, int
 
 int create_point_view(HostState& st, const cudaResourceDesc& vrd, const cudaChannelFormatDesc& ch)
 {
-    if (st.volPointTex) cudaDestroyTextureObject(st.volPointTex);
-    st.volPointTex = 0;
+    if (st.dev.volPointTex) cudaDestroyTextureObject(st.dev.volPointTex);
+    st.dev.volPointTex = 0;
     cudaGetLastError();  // destroying a view whose array the host has freed may report an error: the view is gone either way
     cudaTextureDesc td;
     memset(&td, 0, sizeof(td));
@@ -587,7 +587,7 @@ int create_point_view(HostState& st, const cudaResourceDesc& vrd, const cudaChan
     td.filterMode = cudaFilterModePoint;
     td.readMode = (ch.f == cudaChannelFormatKindFloat) ? cudaReadModeElementType : cudaReadModeNormalizedFloat;
     td.normalizedCoords = 0;
-    SVR_TRY(cudaCreateTextureObject(&st.volPointTex, &vrd, &td, nullptr));
+    SVR_TRY(cudaCreateTextureObject(&st.dev.volPointTex, &vrd, &td, nullptr));
     return 0;
 }
 
@@ -595,9 +595,9 @@ int create_point_view(HostState& st, const cudaResourceDesc& vrd, const cudaChan
 
 int ensure_mailbox(HostState& st)
 {
-    if (!st.hMailbox) {
-        SVR_TRY(cudaHostAlloc(&st.hMailbox, 64, cudaHostAllocMapped | cudaHostAllocPortable));
-        SVR_TRY(cudaHostGetDevicePointer(&st.dMailbox, st.hMailbox, 0));
+    if (!st.dev.hMailbox) {
+        SVR_TRY(cudaHostAlloc(&st.dev.hMailbox, 64, cudaHostAllocMapped | cudaHostAllocPortable));
+        SVR_TRY(cudaHostGetDevicePointer(&st.dev.dMailbox, st.dev.hMailbox, 0));
     }
     return 0;
 }
@@ -607,36 +607,33 @@ int read_small(HostState& st, void* host, const void* dev, size_t bytes)
 {
     if (bytes > 32 || (bytes & 3)) return fail_msg("read_small: at most 32 bytes, a multiple of 4");  // bytes 32..63 of the mailbox: tf_check_launch
     if (int rc = ensure_mailbox(st)) return rc;
-    mailbox_kernel<<<1, 32, 0, st.stream>>>((const unsigned int*)dev, (unsigned int*)st.dMailbox, (int)(bytes / 4));
+    mailbox_kernel<<<1, 32, 0, st.stream>>>((const unsigned int*)dev, (unsigned int*)st.dev.dMailbox, (int)(bytes / 4));
     count_launch();
     SVR_TRY(cudaGetLastError());
     SVR_TRY(cudaStreamSynchronize(st.stream));
-    memcpy(host, st.hMailbox, bytes);
+    memcpy(host, st.dev.hMailbox, bytes);
     return 0;
 }
 
 void release_grid(HostState& st)
 {
-    if (st.volPointTex) cudaDestroyTextureObject(st.volPointTex);
-    st.volPointTex = 0;
-    if (st.uploadSurf) cudaDestroySurfaceObject(st.uploadSurf);
-    st.uploadSurf = 0;
-    st.uploadSurfArray = nullptr;
+    DeviceState& d = st.dev;
+    if (d.volPointTex) cudaDestroyTextureObject(d.volPointTex);
+    d.volPointTex = 0;
+    if (d.uploadSurf) cudaDestroySurfaceObject(d.uploadSurf);
+    d.uploadSurf = 0;
+    d.uploadSurfArray = nullptr;
     cudaGetLastError();  // as for the view: the array behind it may be gone already
-    cudaFree(st.dRange);
-    cudaFree(st.dMajorant);
-    cudaFree(st.dDist[0]);
-    cudaFree(st.dDist[1]);
-    cudaFree(st.dOcc);
-    st.dRange = nullptr;
-    st.dMajorant = nullptr;
-    st.dDist[0] = st.dDist[1] = nullptr;
-    st.dOcc = nullptr;
+    d.range.release();
+    d.majorant.release();
+    d.dist[0].release();
+    d.dist[1].release();
+    d.occ.release();
     st.sceneEpoch++;
-    st.gridArray = nullptr;
-    st.autoArray = nullptr;  // the automatic cell size is re-derived for whatever volume comes next
-    st.rangeValid = false;
-    st.majorantValid = false;
+    d.gridArray = nullptr;
+    d.autoArray = nullptr;  // the automatic cell size is re-derived for whatever volume comes next
+    d.rangeValid = false;
+    d.majorantValid = false;
 }
 
 // svr_volume_upload's fast path (see upload_range_kernel).  *done stays false when the array, the grid or the options do
@@ -646,33 +643,33 @@ int upload_with_ranges(cudaArray_t arr, const cudaChannelFormatDesc& ch, const c
     HostState& st = state();
     *done = false;
     if (!st.options[SVR_OPT_FUSED_UPLOAD] || !(flags & cudaArraySurfaceLoadStore)) return 0;
-    if (arr != st.gridArray || !st.dRange || !st.volPointTex || st.gridCell > 16) return 0;
+    if (arr != st.dev.gridArray || !st.dev.range.p || !st.dev.volPointTex || st.dev.gridCell > 16) return 0;
     // setup_volume since the last render: the array behind the handle may be a new one (build_grid looks first)
-    if (st.fingerprintDue) return 0;
-    if ((int)ext.width != st.volDims.x || (int)ext.height != st.volDims.y || (int)ext.depth != st.volDims.z) return 0;
+    if (st.dev.fingerprintDue) return 0;
+    if ((int)ext.width != st.dev.volDims.x || (int)ext.height != st.dev.volDims.y || (int)ext.depth != st.dev.volDims.z) return 0;
     if (ch.y || ch.z || ch.w) return 0;
     const bool isFloat = ch.f == cudaChannelFormatKindFloat, isUint = ch.f == cudaChannelFormatKindUnsigned;
     if (!((isUint && (ch.x == 8 || ch.x == 16)) || (isFloat && (ch.x == 16 || ch.x == 32)))) return 0;
-    if (st.uploadSurfArray != arr) {
-        if (st.uploadSurf) cudaDestroySurfaceObject(st.uploadSurf);
-        st.uploadSurf = 0;
-        st.uploadSurfArray = nullptr;
+    if (st.dev.uploadSurfArray != arr) {
+        if (st.dev.uploadSurf) cudaDestroySurfaceObject(st.dev.uploadSurf);
+        st.dev.uploadSurf = 0;
+        st.dev.uploadSurfArray = nullptr;
         cudaGetLastError();
         cudaResourceDesc rd;
         memset(&rd, 0, sizeof(rd));
         rd.resType = cudaResourceTypeArray;
         rd.res.array.array = arr;
-        SVR_TRY(cudaCreateSurfaceObject(&st.uploadSurf, &rd));
-        st.uploadSurfArray = arr;
+        SVR_TRY(cudaCreateSurfaceObject(&st.dev.uploadSurf, &rd));
+        st.dev.uploadSurfArray = arr;
     }
     int rc;
-    if (isUint && ch.x == 8) rc = launch_upload_range<VoxU8>(st, devData, st.uploadSurf);
-    else if (isUint) rc = launch_upload_range<VoxU16>(st, devData, st.uploadSurf);
-    else if (ch.x == 16) rc = launch_upload_range<VoxF16>(st, devData, st.uploadSurf);
-    else rc = launch_upload_range<VoxF32>(st, devData, st.uploadSurf);
+    if (isUint && ch.x == 8) rc = launch_upload_range<VoxU8>(st, devData, st.dev.uploadSurf);
+    else if (isUint) rc = launch_upload_range<VoxU16>(st, devData, st.dev.uploadSurf);
+    else if (ch.x == 16) rc = launch_upload_range<VoxF16>(st, devData, st.dev.uploadSurf);
+    else rc = launch_upload_range<VoxF32>(st, devData, st.dev.uploadSurf);
     if (rc) return rc;
-    st.rangeValid = true;
-    st.majorantValid = false;
+    st.dev.rangeValid = true;
+    st.dev.majorantValid = false;
     rc = launch_fingerprint(st, 0);  // of the voxels these ranges describe
     if (rc) return rc;
     st.fusedUploads++;
@@ -723,67 +720,67 @@ static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebu
     unsigned int flags = 0;
     SVR_TRY(cudaArrayGetInfo(&ch, &ext, &flags, varr));
     if (ext.depth == 0) return fail_msg("ensure_grid: volume array is not 3-D");
-    if (varr == st.gridArray && st.dRange && st.fingerprintDue) {
+    if (varr == st.dev.gridArray && st.dev.range.p && st.dev.fingerprintDue) {
         // setup_volume was called since the voxels were last looked at, with a struct that names the same resources
         // (svr_api.cu: setup_volume).  The array behind the handle may still be another one (freed and reallocated by
         // the host): compare its dims, take a fresh point-sampled view of it, and compare a sampled hash of its voxels
         // with the one taken when the ranges were built.
-        if ((int)ext.width != st.volDims.x || (int)ext.height != st.volDims.y || (int)ext.depth != st.volDims.z) {
+        if ((int)ext.width != st.dev.volDims.x || (int)ext.height != st.dev.volDims.y || (int)ext.depth != st.dev.volDims.z) {
             release_grid(st);
         } else {
             int rc = create_point_view(st, vrd, ch);
             if (rc) return rc;
-            if (st.rangeValid) {
+            if (st.dev.rangeValid) {
                 rc = launch_fingerprint(st, 1);
                 if (rc) return rc;
                 unsigned long long h[2] = {0, 1};
-                rc = read_small(st, h, st.dFingerprint, sizeof(h));
+                rc = read_small(st, h, st.dev.fingerprint.p, sizeof(h));
                 if (rc) return rc;
-                if (h[0] != h[1]) st.rangeValid = false;
+                if (h[0] != h[1]) st.dev.rangeValid = false;
             }
         }
     }
-    st.fingerprintDue = false;
-    if (varr != st.gridArray || cell != st.gridCell || !st.dRange) {
+    st.dev.fingerprintDue = false;
+    if (varr != st.dev.gridArray || cell != st.dev.gridCell || !st.dev.range.p) {
         // ---- allocate for this (array, cell size)
         release_grid(st);
         int rcv = create_point_view(st, vrd, ch);
         if (rcv) return rcv;
 
-        st.volDims = make_int3((int)ext.width, (int)ext.height, (int)ext.depth);
-        st.gridDims = make_int3((st.volDims.x + cell - 1) / cell, (st.volDims.y + cell - 1) / cell,
-                                (st.volDims.z + cell - 1) / cell);
-        size_t cells = (size_t)st.gridDims.x * st.gridDims.y * st.gridDims.z;
-        size_t padded = (size_t)(st.gridDims.x + 2) * (st.gridDims.y + 2) * (st.gridDims.z + 2);
-        SVR_TRY(cudaMalloc(&st.dRange, cells * sizeof(float2)));
-        SVR_TRY(cudaMalloc(&st.dMajorant, padded * sizeof(float)));
-        SVR_TRY(cudaMalloc(&st.dDist[0], padded));
-        SVR_TRY(cudaMalloc(&st.dDist[1], padded));
-        SVR_TRY(cudaMalloc(&st.dOcc, 6 * sizeof(int)));
-        st.gridArray = varr;
-        st.gridCell = cell;
-        st.rangeValid = false;
+        st.dev.volDims = make_int3((int)ext.width, (int)ext.height, (int)ext.depth);
+        st.dev.gridDims = make_int3((st.dev.volDims.x + cell - 1) / cell, (st.dev.volDims.y + cell - 1) / cell,
+                                (st.dev.volDims.z + cell - 1) / cell);
+        size_t cells = (size_t)st.dev.gridDims.x * st.dev.gridDims.y * st.dev.gridDims.z;
+        size_t padded = (size_t)(st.dev.gridDims.x + 2) * (st.dev.gridDims.y + 2) * (st.dev.gridDims.z + 2);
+        SVR_TRY(st.dev.range.reserve(cells));
+        SVR_TRY(st.dev.majorant.reserve(padded));
+        SVR_TRY(st.dev.dist[0].reserve(padded));
+        SVR_TRY(st.dev.dist[1].reserve(padded));
+        SVR_TRY(st.dev.occ.reserve(6));
+        st.dev.gridArray = varr;
+        st.dev.gridCell = cell;
+        st.dev.rangeValid = false;
     }
-    if (!st.rangeValid) {
+    if (!st.dev.rangeValid) {
         // ---- stage 1: range grid (again after svr_volume_upload: same allocations, new voxels)
         if (cell <= 16) {
-            int rc = launch_range_brick(st, TexFetch{st.volPointTex});
+            int rc = launch_range_brick(st, TexFetch{st.dev.volPointTex});
             if (rc) return rc;
         } else {
-            dim3 g(st.gridDims.x, st.gridDims.y, st.gridDims.z);
-            range_kernel<<<g, 128, 0, st.stream>>>(st.volPointTex, st.volDims, st.gridDims, cell, st.dRange);
+            dim3 g(st.dev.gridDims.x, st.dev.gridDims.y, st.dev.gridDims.z);
+            range_kernel<<<g, 128, 0, st.stream>>>(st.dev.volPointTex, st.dev.volDims, st.dev.gridDims, cell, st.dev.range.p);
             count_launch();
             SVR_TRY(cudaGetLastError());
         }
-        st.rangeValid = true;
-        st.majorantValid = false;
+        st.dev.rangeValid = true;
+        st.dev.majorantValid = false;
         int rc = launch_fingerprint(st, 0);  // of the voxels these ranges describe (stays on the device until it is needed)
         if (rc) return rc;
     }
 
     const int leap = st.options[SVR_OPT_LEAP] != 0;
-    if (force || !st.majorantValid || st.majorantDensityScale != vol.densityScale || st.majorantTfArray != tarr ||
-        st.majorantLeap != leap) {
+    if (force || !st.dev.majorantValid || st.dev.majorantDensityScale != vol.densityScale || st.dev.majorantTfArray != tarr ||
+        st.dev.majorantLeap != leap) {
         // ---- stage 2: majorants from (range, TF, densityScale), into the padded grid
         cudaChannelFormatDesc ch;
         cudaExtent ext;
@@ -792,57 +789,51 @@ static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebu
         int n = (int)ext.width;
         if (n < 2 || ch.x != 32 || ch.w != 32) return fail_msg("ensure_grid: transfer function must be a 1-D float4 array");
         int levels = 32 - __builtin_clz((unsigned)n);
-        if (n != st.tfEntries) {
-            cudaFree(st.dTfSparse);
-            cudaFree(st.dTfTable);
-            st.dTfSparse = nullptr;
-            st.dTfTable = nullptr;
-            SVR_TRY(cudaMalloc(&st.dTfTable, (size_t)n * sizeof(float4)));
-            SVR_TRY(cudaMalloc(&st.dTfSparse, (size_t)levels * n * sizeof(float)));
-            st.tfEntries = n;
-        }
-        SVR_TRY(cudaMemcpy2DFromArrayAsync(st.dTfTable, (size_t)n * sizeof(float4), tarr, 0, 0, (size_t)n * sizeof(float4), 1,
+        SVR_TRY(st.dev.tfTable.reserve((size_t)n));
+        SVR_TRY(st.dev.tfSparse.reserve((size_t)levels * n));
+        st.dev.tfEntries = n;
+        SVR_TRY(cudaMemcpy2DFromArrayAsync(st.dev.tfTable.p, (size_t)n * sizeof(float4), tarr, 0, 0, (size_t)n * sizeof(float4), 1,
                                            cudaMemcpyDeviceToDevice, st.stream));
-        tf_sparse_kernel<<<1, 1024, 0, st.stream>>>(st.dTfTable, n, levels, st.dTfSparse);
-        if (!st.dTfHash) SVR_TRY(cudaMalloc(&st.dTfHash, 4 * sizeof(unsigned long long)));  // [0] built-from, [1] live, [2] stale flag (32 bit)
-        tf_hash_kernel<<<1, 256, 0, st.stream>>>(st.dTfTable, 0, n, st.dTfHash, nullptr, nullptr, nullptr);  // of the table these majorants come from
-        const int px = st.gridDims.x + 2, py = st.gridDims.y + 2, pz = st.gridDims.z + 2;
+        tf_sparse_kernel<<<1, 1024, 0, st.stream>>>(st.dev.tfTable.p, n, levels, st.dev.tfSparse.p);
+        SVR_TRY(st.dev.tfHash.reserve(4));  // [0] built-from, [1] live, [2] stale flag (32 bit)
+        tf_hash_kernel<<<1, 256, 0, st.stream>>>(st.dev.tfTable.p, 0, n, st.dev.tfHash.p, nullptr, nullptr, nullptr);  // of the table these majorants come from
+        const int px = st.dev.gridDims.x + 2, py = st.dev.gridDims.y + 2, pz = st.dev.gridDims.z + 2;
         const size_t padded = (size_t)px * py * pz;
-        if (int rc = zero_words(st, st.dMajorant, padded * sizeof(float))) return rc;
-        occ_init_kernel<<<1, 32, 0, st.stream>>>(st.dOcc);
-        dim3 mb(32, 4, 1), mg((st.gridDims.x + 31) / 32, (st.gridDims.y + 3) / 4, st.gridDims.z);
-        majorant_kernel<<<mg, mb, 0, st.stream>>>(st.dRange, st.gridDims, st.dTfSparse, n, vol.densityScale, st.dMajorant, st.dOcc);
+        if (int rc = zero_words(st, st.dev.majorant.p, padded * sizeof(float))) return rc;
+        occ_init_kernel<<<1, 32, 0, st.stream>>>(st.dev.occ.p);
+        dim3 mb(32, 4, 1), mg((st.dev.gridDims.x + 31) / 32, (st.dev.gridDims.y + 3) / 4, st.dev.gridDims.z);
+        majorant_kernel<<<mg, mb, 0, st.stream>>>(st.dev.range.p, st.dev.gridDims, st.dev.tfSparse.p, n, vol.densityScale, st.dev.majorant.p, st.dev.occ.p);
         // ---- stage 3: leap distances for empty cells (border cells included)
         dim3 pg((px + 31) / 32, (py + 3) / 4, pz);
         const int cap = leap ? SVR_LEAP_CAP : 0;
-        dist_axis_kernel<true, false><<<pg, mb, 0, st.stream>>>(nullptr, st.dDist[0], st.dMajorant, px, py, pz, 0, cap);
-        dist_axis_kernel<false, false><<<pg, mb, 0, st.stream>>>(st.dDist[0], st.dDist[1], nullptr, px, py, pz, 1, cap);
-        dist_axis_kernel<false, true><<<pg, mb, 0, st.stream>>>(st.dDist[1], nullptr, st.dMajorant, px, py, pz, 2, cap);
+        dist_axis_kernel<true, false><<<pg, mb, 0, st.stream>>>(nullptr, st.dev.dist[0].p, st.dev.majorant.p, px, py, pz, 0, cap);
+        dist_axis_kernel<false, false><<<pg, mb, 0, st.stream>>>(st.dev.dist[0].p, st.dev.dist[1].p, nullptr, px, py, pz, 1, cap);
+        dist_axis_kernel<false, true><<<pg, mb, 0, st.stream>>>(st.dev.dist[1].p, nullptr, st.dev.majorant.p, px, py, pz, 2, cap);
         count_launch(7);
         SVR_TRY(cudaGetLastError());
         if (majorantsRebuilt) *majorantsRebuilt = true;
         st.sceneEpoch++;
-        st.majorantValid = true;
-        st.majorantDensityScale = vol.densityScale;
-        st.majorantTfArray = tarr;
-        st.majorantLeap = leap;
+        st.dev.majorantValid = true;
+        st.dev.majorantDensityScale = vol.densityScale;
+        st.dev.majorantTfArray = tarr;
+        st.dev.majorantLeap = leap;
     }
 
-    scene->volDim = st.volDims;
+    scene->volDim = st.dev.volDims;
     DevGrid& g = scene->grid;
-    g.px = st.gridDims.x + 2;
-    g.pxy = g.px * (st.gridDims.y + 2);
-    g.pyF = (float)(st.gridDims.y + 2);
-    g.cells = st.dMajorant + g.pxy + g.px + 1;  // interior cell (0,0,0)
-    g.range = st.dRange;
-    g.occ = st.dOcc;
-    g.gx = st.gridDims.x;
-    g.gy = st.gridDims.y;
-    g.gz = st.gridDims.z;
-    g.cell = st.gridCell;
-    g.scale = f3((float)st.volDims.x / (float)st.gridCell, (float)st.volDims.y / (float)st.gridCell,
-                 (float)st.volDims.z / (float)st.gridCell);
-    g.invScale = f3((float)st.gridCell / (float)st.volDims.x, (float)st.gridCell / (float)st.volDims.y, (float)st.gridCell / (float)st.volDims.z);
+    g.px = st.dev.gridDims.x + 2;
+    g.pxy = g.px * (st.dev.gridDims.y + 2);
+    g.pyF = (float)(st.dev.gridDims.y + 2);
+    g.cells = st.dev.majorant.p + g.pxy + g.px + 1;  // interior cell (0,0,0)
+    g.range = st.dev.range.p;
+    g.occ = st.dev.occ.p;
+    g.gx = st.dev.gridDims.x;
+    g.gy = st.dev.gridDims.y;
+    g.gz = st.dev.gridDims.z;
+    g.cell = st.dev.gridCell;
+    g.scale = f3((float)st.dev.volDims.x / (float)st.dev.gridCell, (float)st.dev.volDims.y / (float)st.dev.gridCell,
+                 (float)st.dev.volDims.z / (float)st.dev.gridCell);
+    g.invScale = f3((float)st.dev.gridCell / (float)st.dev.volDims.x, (float)st.dev.gridCell / (float)st.dev.volDims.y, (float)st.dev.gridCell / (float)st.dev.volDims.z);
     g.toCell = f3(vol.bbox.invSize) * g.scale;
     g.cellOff = f3(vol.bbox.vmin) * g.toCell;
     return 0;
@@ -855,16 +846,16 @@ static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebu
 // thin transfer function, 0.009 -> 32).  The statistic is the mean non-zero majorant of the current grid.
 static int auto_cell(HostState& st, int current, int* want)
 {
-    const size_t padded = (size_t)(st.gridDims.x + 2) * (st.gridDims.y + 2) * (st.gridDims.z + 2);
-    if (!st.dStats) SVR_TRY(cudaMalloc(&st.dStats, 16));
-    if (int rc = zero_words(st, st.dStats, 16)) return rc;
-    majorant_stats_kernel<<<148 * 4, 256, 0, st.stream>>>(st.dMajorant, padded, (double*)st.dStats, (unsigned long long*)((char*)st.dStats + 8));
+    const size_t padded = (size_t)(st.dev.gridDims.x + 2) * (st.dev.gridDims.y + 2) * (st.dev.gridDims.z + 2);
+    SVR_TRY(st.dev.stats.reserve(2));
+    if (int rc = zero_words(st, st.dev.stats.p, 16)) return rc;
+    majorant_stats_kernel<<<148 * 4, 256, 0, st.stream>>>(st.dev.majorant.p, padded, (double*)st.dev.stats.p, (unsigned long long*)((char*)st.dev.stats.p + 8));
     count_launch();
     struct {
         double sum;
         unsigned long long count;
     } h;
-    if (int rc = read_small(st, &h, st.dStats, 16)) return rc;
+    if (int rc = read_small(st, &h, st.dev.stats.p, 16)) return rc;
     *want = current;
     if (h.count == 0 || !(h.sum > 0.0)) return 0;  // nothing to track through: any size will do
     const double ideal = log2(2.0 / (h.sum / (double)h.count));  // log2 of twice the mean free path, in voxels
@@ -886,11 +877,11 @@ int tf_check_collect(bool* changed)
 {
     HostState& st = state();
     *changed = false;
-    if (!st.tfCheckPending) return 0;
-    st.tfCheckPending = false;
-    SVR_TRY(cudaEventSynchronize(st.tfCheckEvent));
+    if (!st.dev.tfCheckPending) return 0;
+    st.dev.tfCheckPending = false;
+    SVR_TRY(cudaEventSynchronize(st.dev.tfCheckEvent));
     unsigned long long h[2];
-    memcpy(h, (const char*)st.hMailbox + 32, sizeof(h));
+    memcpy(h, (const char*)st.dev.hMailbox + 32, sizeof(h));
     *changed = h[0] != h[1];
     return 0;
 }
@@ -900,18 +891,18 @@ int tf_check_launch(const svr_transfer_function& tf, const unsigned int** staleF
 {
     HostState& st = state();
     *staleFlag = nullptr;
-    if (!tf.tex || !st.majorantValid || !st.dTfHash || !st.tfEntries) return 0;
+    if (!tf.tex || !st.dev.majorantValid || !st.dev.tfHash.p || !st.dev.tfEntries) return 0;
     cudaResourceDesc trd;
     SVR_TRY(cudaGetTextureObjectResourceDesc(&trd, tf.tex));
-    if (trd.resType != cudaResourceTypeArray || trd.res.array.array != st.majorantTfArray) return 0;
+    if (trd.resType != cudaResourceTypeArray || trd.res.array.array != st.dev.majorantTfArray) return 0;
     if (int rc = ensure_mailbox(st)) return rc;
-    if (!st.tfCheckEvent) SVR_TRY(cudaEventCreateWithFlags(&st.tfCheckEvent, cudaEventDisableTiming));
-    unsigned int* flag = (unsigned int*)(st.dTfHash + 2);
-    tf_hash_kernel<<<1, 256, 0, st.stream>>>(nullptr, tf.tex, st.tfEntries, st.dTfHash + 1, st.dTfHash, (unsigned long long*)((char*)st.dMailbox + 32), flag);
+    if (!st.dev.tfCheckEvent) SVR_TRY(cudaEventCreateWithFlags(&st.dev.tfCheckEvent, cudaEventDisableTiming));
+    unsigned int* flag = (unsigned int*)(st.dev.tfHash.p + 2);
+    tf_hash_kernel<<<1, 256, 0, st.stream>>>(nullptr, tf.tex, st.dev.tfEntries, st.dev.tfHash.p + 1, st.dev.tfHash.p, (unsigned long long*)((char*)st.dev.dMailbox + 32), flag);
     count_launch();
     SVR_TRY(cudaGetLastError());
-    SVR_TRY(cudaEventRecord(st.tfCheckEvent, st.stream));
-    st.tfCheckPending = true;
+    SVR_TRY(cudaEventRecord(st.dev.tfCheckEvent, st.stream));
+    st.dev.tfCheckPending = true;
     *staleFlag = flag;
     return 0;
 }
@@ -921,14 +912,14 @@ int ensure_grid(DevScene* scene, bool force, int maxAutoCell)
     HostState& st = state();
     const int opt = st.options[SVR_OPT_MACROCELL_SIZE];
     if (opt != 0) return build_grid(scene, force, opt, nullptr);
-    int cell = st.autoCell ? st.autoCell : 8;
+    int cell = st.dev.autoCell ? st.dev.autoCell : 8;
     if (cell > maxAutoCell) cell = maxAutoCell;
     int rc = build_grid(scene, force, cell, nullptr);
     if (rc) return rc;
     // re-evaluate when the scene behind the grid changed, not on every forced refresh (ray caster)
-    const bool sceneChanged = st.autoArray != st.gridArray || st.autoTfArray != st.majorantTfArray ||
-                              st.autoDensityScale != scene->vol.densityScale || st.autoEpoch != st.uploadEpoch;
-    if (st.autoCell && !sceneChanged) return 0;
+    const bool sceneChanged = st.dev.autoArray != st.dev.gridArray || st.dev.autoTfArray != st.dev.majorantTfArray ||
+                              st.dev.autoDensityScale != scene->vol.densityScale || st.dev.autoEpoch != st.dev.uploadEpoch;
+    if (st.dev.autoCell && !sceneChanged) return 0;
     // majorants grow with the cell they are taken over, so the statistic is looked at again on the grid of
     // the size it suggested (at most twice; the 0.75-octave hysteresis in auto_cell settles it)
     for (int round = 0; round < 3; ++round) {
@@ -941,11 +932,11 @@ int ensure_grid(DevScene* scene, bool force, int maxAutoCell)
         rc = build_grid(scene, force, cell, nullptr);
         if (rc) return rc;
     }
-    st.autoCell = cell;
-    st.autoArray = st.gridArray;
-    st.autoTfArray = st.majorantTfArray;
-    st.autoDensityScale = scene->vol.densityScale;
-    st.autoEpoch = st.uploadEpoch;
+    st.dev.autoCell = cell;
+    st.dev.autoArray = st.dev.gridArray;
+    st.dev.autoTfArray = st.dev.majorantTfArray;
+    st.dev.autoDensityScale = scene->vol.densityScale;
+    st.dev.autoEpoch = st.dev.uploadEpoch;
     return 0;
 }
 
@@ -990,31 +981,31 @@ extern "C" int svr_debug_sample_tf(const svr_transfer_function* tf, const float*
 extern "C" int svr_grid_info(int32_t* dims, int32_t* cell)
 {
     svr::HostState& st = svr::state();
-    if (!st.dRange) return svr::fail_msg("svr_grid_info: no grid has been built yet");
+    if (!st.dev.range.p) return svr::fail_msg("svr_grid_info: no grid has been built yet");
     if (dims) {
-        dims[0] = st.gridDims.x;
-        dims[1] = st.gridDims.y;
-        dims[2] = st.gridDims.z;
+        dims[0] = st.dev.gridDims.x;
+        dims[1] = st.dev.gridDims.y;
+        dims[2] = st.dev.gridDims.z;
     }
-    if (cell) *cell = st.gridCell;
+    if (cell) *cell = st.dev.gridCell;
     return 0;
 }
 
 extern "C" int svr_grid_copy(float* host_majorant, float* host_range)
 {
     svr::HostState& st = svr::state();
-    if (!st.dRange || !st.dMajorant) return svr::fail_msg("svr_grid_copy: no grid has been built yet");
-    const int gx = st.gridDims.x, gy = st.gridDims.y, gz = st.gridDims.z;
+    if (!st.dev.range.p || !st.dev.majorant.p) return svr::fail_msg("svr_grid_copy: no grid has been built yet");
+    const int gx = st.dev.gridDims.x, gy = st.dev.gridDims.y, gz = st.dev.gridDims.z;
     size_t cells = (size_t)gx * gy * gz;
     SVR_TRY(cudaStreamSynchronize(st.stream));
     if (host_majorant) {
         const int px = gx + 2, py = gy + 2, pz = gz + 2;
         std::vector<float> padded((size_t)px * py * pz);
-        SVR_TRY(cudaMemcpy(padded.data(), st.dMajorant, padded.size() * sizeof(float), cudaMemcpyDeviceToHost));
+        SVR_TRY(cudaMemcpy(padded.data(), st.dev.majorant.p, padded.size() * sizeof(float), cudaMemcpyDeviceToHost));
         for (int z = 0; z < gz; ++z)
             for (int y = 0; y < gy; ++y)
                 memcpy(host_majorant + ((size_t)z * gy + y) * gx, &padded[((size_t)(z + 1) * py + (y + 1)) * px + 1], gx * sizeof(float));
     }
-    if (host_range) SVR_TRY(cudaMemcpy(host_range, st.dRange, cells * sizeof(float2), cudaMemcpyDeviceToHost));
+    if (host_range) SVR_TRY(cudaMemcpy(host_range, st.dev.range.p, cells * sizeof(float2), cudaMemcpyDeviceToHost));
     return 0;
 }

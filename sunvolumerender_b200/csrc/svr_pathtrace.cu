@@ -31,6 +31,8 @@
 #include "svr_rng.cuh"
 #include "svr_state.h"
 
+#include <type_traits>
+
 // Launch bounds of the path-tracing kernels: at most SVR_PT_MAX_THREADS threads per block and at least
 // SVR_PT_MIN_BLOCKS resident blocks per SM, i.e. a register budget of 65536 / (128 * 9) = 56 per thread
 // (36 warps per SM).  Chosen by measurement (DESIGN.md section 3.1, round 2, C3 per 256-spp launch): 6 blocks (80
@@ -2168,39 +2170,55 @@ __global__ void __launch_bounds__(256) adaptive_converge_kernel(const float4* __
     if (active) list[base + (uint32_t)__popc(ballot & ((1u << threadIdx.x) - 1u))] = y * W + x;
 }
 
+// dynamic shared memory of pathtrace_pool_kernel for blocks of `threads`
+constexpr size_t pool_shared_bytes(int threads) { return sizeof(float) * SVR_ITEM_WORDS * (SVR_POOL_CAP + SVR_EVQ_CAP) * (size_t)(threads / 32); }
+
+typedef void (*PtKernel)(const DevScene, const PtLaunch, Counters*);
+
+// the kernel's COUNT = true instance with counters, its COUNT = false instance without
+void launch_counted(PtKernel counted, PtKernel plain, dim3 grid, int block, size_t shm, cudaStream_t stream, const DevScene& sc, const PtLaunch& a,
+                    Counters* cnt)
+{
+    (cnt ? counted : plain)<<<grid, block, shm, stream>>>(sc, a, cnt);
+}
+
 template <int MODE>
 void launch_mode(int shape, dim3 grid, int block, cudaStream_t stream, const DevScene& sc, const PtLaunch& a, Counters* cnt)
 {
-    if (shape == 5) {  // launch_pathtrace() only picks it for MODE 2
-        const size_t shm = sizeof(float) * SVR_ITEM_WORDS * (SVR_POOL_CAP + SVR_EVQ_CAP) * (size_t)(block / 32);
+    if (shape == 5) {  // choose_shape() only picks it for MODE 2
         static bool attr = false;
         if (!attr) {
-            cudaFuncSetAttribute(pathtrace_pool_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(float) * SVR_ITEM_WORDS * (SVR_POOL_CAP + SVR_EVQ_CAP) * (SVR_PT_MAX_THREADS / 32)));
-            cudaFuncSetAttribute(pathtrace_pool_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(float) * SVR_ITEM_WORDS * (SVR_POOL_CAP + SVR_EVQ_CAP) * (SVR_PT_MAX_THREADS / 32)));
+            for (PtKernel k : {pathtrace_pool_kernel<true>, pathtrace_pool_kernel<false>})
+                cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pool_shared_bytes(SVR_PT_MAX_THREADS));
             attr = true;
         }
-        if (cnt) pathtrace_pool_kernel<true><<<grid, block, shm, stream>>>(sc, a, cnt);
-        else pathtrace_pool_kernel<false><<<grid, block, shm, stream>>>(sc, a, cnt);
-    } else if (shape == 4) {  // launch_pathtrace() only picks it for MODE 2 with a pinhole camera
-        if (cnt) pathtrace_profile_kernel<true><<<grid, block, 0, stream>>>(sc, a, cnt);
-        else pathtrace_profile_kernel<false><<<grid, block, 0, stream>>>(sc, a, cnt);
-    } else if (shape == 3) {  // launch_pathtrace() only picks it for MODE 2
-        if (cnt) pathtrace_queue_kernel<true><<<grid, block, 0, stream>>>(sc, a, cnt);
-        else pathtrace_queue_kernel<false><<<grid, block, 0, stream>>>(sc, a, cnt);
+        launch_counted(pathtrace_pool_kernel<true>, pathtrace_pool_kernel<false>, grid, block, pool_shared_bytes(block), stream, sc, a, cnt);
+    } else if (shape == 4) {  // choose_shape() only picks it for MODE 2 with a pinhole camera
+        launch_counted(pathtrace_profile_kernel<true>, pathtrace_profile_kernel<false>, grid, block, 0, stream, sc, a, cnt);
+    } else if (shape == 3) {  // choose_shape() only picks it for MODE 2
+        launch_counted(pathtrace_queue_kernel<true>, pathtrace_queue_kernel<false>, grid, block, 0, stream, sc, a, cnt);
     } else if (shape == 2 && a.perSample) {  // launch_pathtrace() only sets it without counters and without the block split
         pathtrace_warp_kernel<MODE, false, false, true><<<grid, block, 0, stream>>>(sc, a, cnt);
     } else if (shape == 2 && a.blockSplit) {
-        if (cnt) pathtrace_warp_kernel<MODE, true, true><<<grid, block, 0, stream>>>(sc, a, cnt);
-        else pathtrace_warp_kernel<MODE, false, true><<<grid, block, 0, stream>>>(sc, a, cnt);
+        launch_counted(pathtrace_warp_kernel<MODE, true, true>, pathtrace_warp_kernel<MODE, false, true>, grid, block, 0, stream, sc, a, cnt);
     } else if (shape == 2) {
-        if (cnt) pathtrace_warp_kernel<MODE, true, false><<<grid, block, 0, stream>>>(sc, a, cnt);
-        else pathtrace_warp_kernel<MODE, false, false><<<grid, block, 0, stream>>>(sc, a, cnt);
+        launch_counted(pathtrace_warp_kernel<MODE, true, false>, pathtrace_warp_kernel<MODE, false, false>, grid, block, 0, stream, sc, a, cnt);
     } else if (shape == 1) {
-        if (cnt) pathtrace_mega_kernel<MODE, true><<<grid, block, 0, stream>>>(sc, a, cnt);
-        else pathtrace_mega_kernel<MODE, false><<<grid, block, 0, stream>>>(sc, a, cnt);
+        launch_counted(pathtrace_mega_kernel<MODE, true>, pathtrace_mega_kernel<MODE, false>, grid, block, 0, stream, sc, a, cnt);
     } else {
-        if (cnt) pathtrace_sched_kernel<MODE, true><<<grid, block, 0, stream>>>(sc, a, cnt);
-        else pathtrace_sched_kernel<MODE, false><<<grid, block, 0, stream>>>(sc, a, cnt);
+        launch_counted(pathtrace_sched_kernel<MODE, true>, pathtrace_sched_kernel<MODE, false>, grid, block, 0, stream, sc, a, cnt);
+    }
+}
+
+// f(std::integral_constant<int, MODE>()) for the kernels' MODE: SVR_OPT_PT_MODE, or 3 for local majorants with environment NEE
+template <class F>
+void with_mode(int mode, F&& f)
+{
+    switch (mode) {
+        case 0: f(std::integral_constant<int, 0>()); break;
+        case 1: f(std::integral_constant<int, 1>()); break;
+        case 2: f(std::integral_constant<int, 2>()); break;
+        default: f(std::integral_constant<int, 3>()); break;
     }
 }
 
@@ -2210,6 +2228,73 @@ struct PixelList {
     uint32_t count;
     float4* half;
 };
+
+// The kernel shape a launch runs: SVR_OPT_PT_KERNEL (`requested`) where the estimator, the camera and the launch allow it.
+int choose_shape(int requested, int mode, uint32_t traceDepth, int queueMinDepth, bool profile, bool pinhole, bool envNee, uint32_t nSamples,
+                 uint32_t warpMinSpp, bool perSample, bool list)
+{
+    if (list) return 2;  // the adaptive entry point's list kernel is a sample-parallel sibling (it has ruled out counters)
+    int shape = requested;
+    if (mode != 2 || envNee) {
+        // shapes 3-5 serve local-majorant Philox paths, and environment next-event estimation lives in the shared event code
+        // of shapes 0-2: the plain sample-parallel shape stands in for them
+        shape = std::min(shape, 2);
+    } else if (shape == 2 || shape == 3) {
+        // camera rays against the pixel's majorant profile (shape 4) when the camera is a pinhole (one origin per pixel); it has
+        // shape 3's scatter queue built in.  Otherwise deep paths get the scatter queue (DESIGN.md section 3.1)
+        const bool deep = shape == 3 || (queueMinDepth > 0 && traceDepth >= (uint32_t)queueMinDepth);
+        shape = profile && pinhole ? 4 : (deep ? 3 : 2);
+    } else if (shape == 4 && !pinhole) {
+        shape = 2;
+    }
+    // the sample-parallel shapes need a warp's worth of samples per pixel; below that one lane per pixel
+    if (shape >= 2 && nSamples < warpMinSpp && !perSample) shape = 1;
+    return shape;
+}
+
+// Per-pixel classification for shapes 1-3: made for the whole image by a kernel of its own and, with SVR_OPT_PT_PIXEL_CACHE,
+// kept until something a pixel can see changes (sceneEpoch); without it, made again for every launch.  The render kernels only
+// read it.  A kept classification includes the entry walk whenever the option allows one: its cost is paid once, so it also
+// serves single-sample launches, for which a walk per launch does not pay (images are bit-identical either way: only empty
+// space is skipped).
+int ensure_pixel_classification(HostState& st, const DevScene& sc, int mode, PtLaunch& a)
+{
+    DeviceState& d = st.dev;
+    const bool keep = st.options[SVR_OPT_PT_PIXEL_CACHE] != 0;
+    const int walk = keep ? (st.options[SVR_OPT_PT_ENTRY_CACHE] != 0) : a.entryCache;
+    const size_t npix = (size_t)sc.cam.imageW * sc.cam.imageH;
+    if (d.pixelCache.cap < npix) d.pixelCacheEpoch = 0;  // new memory holds no classification
+    SVR_TRY(d.pixelCache.reserve(npix));
+    const int key = (sc.envNee ? 3 : mode) * 2 + walk;
+    const bool valid = keep && d.pixelCacheEpoch == st.sceneEpoch && d.pixelCacheW == sc.cam.imageW && d.pixelCacheH == sc.cam.imageH &&
+                       d.pixelCacheMode == key;
+    if (!valid) {
+        dim3 cg((sc.cam.imageW + 15u) / 16u, (sc.cam.imageH + 7u) / 8u);
+        classify_pixels_kernel<<<cg, 128, 0, st.stream>>>(sc, d.pixelCache.p, mode >= 2 ? 1 : 0, walk, a.lightCull);
+        count_launch();
+        SVR_TRY(cudaGetLastError());
+        d.pixelCacheEpoch = keep ? st.sceneEpoch : 0;
+        d.pixelCacheW = sc.cam.imageW;
+        d.pixelCacheH = sc.cam.imageH;
+        d.pixelCacheMode = key;
+    }
+    a.pixelCache = 2;
+    a.pixelInfo = d.pixelCache.p;
+    return 0;
+}
+
+// A launch over every row of the image, everything else zero
+PtLaunch full_frame(uint32_t traceDepth, uint32_t firstSample, uint32_t nSamples)
+{
+    PtLaunch a;
+    memset(&a, 0, sizeof(a));
+    a.traceDepth = traceDepth;
+    a.firstSample = firstSample;
+    a.nSamples = nSamples;
+    a.y0 = 0;
+    a.y1 = 0xffffffffu;
+    return a;
+}
 
 // pl != null: the sample-parallel shape over the listed pixels (pathtrace_list_kernel), whatever the options would pick
 int launch_pathtrace(PtLaunch& a, const PixelList* pl = nullptr)
@@ -2248,29 +2333,16 @@ int launch_pathtrace(PtLaunch& a, const PixelList* pl = nullptr)
         if (!cnt) return fail_msg("render_pathtracer: counter allocation failed");
     }
     const int block = st.options[SVR_OPT_PT_BLOCK];
-    int shape = st.options[SVR_OPT_PT_KERNEL];
-    // the sample-parallel shape needs a warp's worth of samples per pixel; below that one lane per pixel
-    // deep paths: the sample-parallel shape gets its scatter queue (DESIGN.md section 3.1)
-    const int queueDepth = st.options[SVR_OPT_PT_QUEUE_MIN_DEPTH];
-    if (shape == 2 && queueDepth > 0 && a.traceDepth >= (uint32_t)queueDepth) shape = 3;
-    // the scatter queue serves local-majorant Philox paths; the other estimators run the plain sample-parallel shape
-    if (shape == 3 && mode != 2) shape = 2;
-    // camera rays against the pixel's majorant profile (shape 4) whenever the sample-parallel shape would run with
-    // local majorants and the camera is a pinhole (one origin per pixel); it has shape 3's scatter queue built in
-    if ((shape == 2 || shape == 3) && mode == 2 && st.options[SVR_OPT_PT_PROFILE] && sc.cam.apeture == 0.f) shape = 4;
-    if (shape == 4 && (mode != 2 || sc.cam.apeture != 0.f)) shape = 2;
-    if (shape == 5 && mode != 2) shape = 2;
-    if (sc.envNee && shape >= 3) shape = 2;  // environment next-event estimation lives in the shared event code of shapes 0-2
-    if (shape >= 2 && a.nSamples < (uint32_t)st.options[SVR_OPT_PT_WARP_MIN_SPP] && !a.perSample) shape = 1;
-    if (pl) shape = 2;  // (the adaptive entry point has ruled out counters)
+    const int shape = choose_shape(st.options[SVR_OPT_PT_KERNEL], mode, a.traceDepth, st.options[SVR_OPT_PT_QUEUE_MIN_DEPTH], st.options[SVR_OPT_PT_PROFILE] != 0,
+                                   sc.cam.apeture == 0.f, sc.envNee != 0, a.nSamples, (uint32_t)st.options[SVR_OPT_PT_WARP_MIN_SPP], a.perSample != nullptr,
+                                   pl != nullptr);
     if (a.perSample && (shape != 2 || cnt || a.nSamples > 32u)) {
         a.perSample = nullptr;  // look-ahead is for the plain sample-parallel shape: the caller renders this frame the ordinary way
         return 0;
     }
-    if (a.hdr) st.aheadCount = 0;  // an ordinary launch moves the running mean on: samples kept for later frames no longer follow it
-    // shape 4: idle lanes take new camera samples together, once this many wait (SVR_OPT_PT_REFILL)
-    if (shape == 4) a.marchBurst = st.options[SVR_OPT_PT_REFILL] > 0 ? st.options[SVR_OPT_PT_REFILL] : 8;
-    if (shape == 5) a.marchBurst = st.options[SVR_OPT_PT_REFILL] > 0 ? st.options[SVR_OPT_PT_REFILL] : 8;
+    hdr_written_outside(st.dev, a.hdr, true);
+    // shapes 4 and 5: idle lanes take new camera samples together, once this many wait (SVR_OPT_PT_REFILL)
+    if (shape >= 4) a.marchBurst = st.options[SVR_OPT_PT_REFILL] > 0 ? st.options[SVR_OPT_PT_REFILL] : 8;
     a.warpPixels = st.options[SVR_OPT_PT_WARP_PIXELS];
     if (a.warpPixels <= 0) a.warpPixels = a.nSamples >= 128u ? 1 : 2;  // automatic: see the option's default (svr_api.cu)
     if (shape == 5) a.warpPixels = st.options[SVR_OPT_PT_POOL_PIXELS] > 0 ? st.options[SVR_OPT_PT_POOL_PIXELS] : 16;
@@ -2279,50 +2351,16 @@ int launch_pathtrace(PtLaunch& a, const PixelList* pl = nullptr)
         tileW = (uint32_t)a.warpPixels;
         tileH = (uint32_t)block / 32u;
     }
-    // Per-pixel classification (shapes 1-3): made for the whole image by a kernel of its own and, with SVR_OPT_PT_PIXEL_CACHE, kept
-    // until something a pixel can see changes (sceneEpoch); without it, made again for every launch.  The render kernels only
-    // read it.  A kept classification includes the entry walk whenever the option allows one: its cost is paid once, so it also
-    // serves single-sample launches, for which a walk per launch does not pay (images are bit-identical either way: only empty
-    // space is skipped).
     a.pixelCache = 0;
     a.pixelInfo = nullptr;
     if (shape >= 1 && shape <= 3) {
-        const bool keep = st.options[SVR_OPT_PT_PIXEL_CACHE] != 0;
-        const int walk = keep ? (st.options[SVR_OPT_PT_ENTRY_CACHE] != 0) : a.entryCache;
-        const size_t npix = (size_t)sc.cam.imageW * sc.cam.imageH;
-        if (st.pixelCacheCap < npix) {
-            cudaFree(st.dPixelCache);
-            st.dPixelCache = nullptr;
-            st.pixelCacheCap = 0;
-            SVR_TRY(cudaMalloc(&st.dPixelCache, npix * sizeof(float2)));
-            st.pixelCacheCap = npix;
-            st.pixelCacheEpoch = 0;
-        }
-        const int key = (sc.envNee ? 3 : mode) * 2 + walk;
-        const bool valid = keep && st.pixelCacheEpoch == st.sceneEpoch && st.pixelCacheW == sc.cam.imageW && st.pixelCacheH == sc.cam.imageH &&
-                           st.pixelCacheMode == key;
-        if (!valid) {
-            dim3 cg((sc.cam.imageW + 15u) / 16u, (sc.cam.imageH + 7u) / 8u);
-            classify_pixels_kernel<<<cg, 128, 0, st.stream>>>(sc, st.dPixelCache, mode >= 2 ? 1 : 0, walk, a.lightCull);
-            count_launch();
-            SVR_TRY(cudaGetLastError());
-            st.pixelCacheEpoch = keep ? st.sceneEpoch : 0;
-            st.pixelCacheW = sc.cam.imageW;
-            st.pixelCacheH = sc.cam.imageH;
-            st.pixelCacheMode = key;
-        }
-        a.pixelCache = 2;
-        a.pixelInfo = st.dPixelCache;
+        if (int rc = ensure_pixel_classification(st, sc, mode, a)) return rc;
     }
+    const int kernelMode = sc.envNee ? 3 : mode;
     if (pl) {
         if (pl->count == 0) return 0;
         const dim3 lg((pl->count + (uint32_t)block / 32u - 1u) / ((uint32_t)block / 32u));
-        switch (sc.envNee ? 3 : mode) {
-            case 0: pathtrace_list_kernel<0><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
-            case 1: pathtrace_list_kernel<1><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
-            case 2: pathtrace_list_kernel<2><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
-            default: pathtrace_list_kernel<3><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); break;
-        }
+        with_mode(kernelMode, [&](auto m) { pathtrace_list_kernel<decltype(m)::value><<<lg, block, 0, st.stream>>>(sc, a, pl->list, pl->count, pl->half); });
         count_launch();
         SVR_TRY(cudaGetLastError());
         return 0;
@@ -2335,12 +2373,7 @@ int launch_pathtrace(PtLaunch& a, const PixelList* pl = nullptr)
     if (a.bandPhase >= bands) return 0;
     a.bandRows = tileH;
     dim3 grid((sc.cam.imageW + tileW - 1u) / tileW, (bands - a.bandPhase + a.bandStride - 1u) / a.bandStride);
-    switch (sc.envNee ? 3 : mode) {
-        case 0: launch_mode<0>(shape, grid, block, st.stream, sc, a, cnt); break;
-        case 1: launch_mode<1>(shape, grid, block, st.stream, sc, a, cnt); break;
-        case 2: launch_mode<2>(shape, grid, block, st.stream, sc, a, cnt); break;
-        default: launch_mode<3>(shape, grid, block, st.stream, sc, a, cnt); break;
-    }
+    with_mode(kernelMode, [&](auto m) { launch_mode<decltype(m)::value>(shape, grid, block, st.stream, sc, a, cnt); });
     count_launch();
     SVR_TRY(cudaGetLastError());
     return 0;
@@ -2359,13 +2392,13 @@ using namespace svr;
 // look-ahead switches itself off until the scene changes.  Images do not depend on the decision (the two paths are bit-equal).
 static bool lookahead_events(HostState& st)
 {
-    if (!st.aheadEvReady) {
+    if (!st.dev.aheadEvReady) {
         for (int i = 0; i < 6; ++i)
-            if (cudaEventCreate(&st.aheadEv[i]) != cudaSuccess) {
+            if (cudaEventCreate(&st.dev.aheadEv[i]) != cudaSuccess) {
                 cudaGetLastError();
                 return false;
             }
-        st.aheadEvReady = true;
+        st.dev.aheadEvReady = true;
     }
     return true;
 }
@@ -2373,19 +2406,19 @@ static bool lookahead_events(HostState& st)
 // true = measured, and batches do not pay for the current scene
 static bool lookahead_does_not_pay(HostState& st)
 {
-    if (st.aheadTimedEpoch != st.sceneEpoch || st.aheadSingleEpoch != st.sceneEpoch || st.aheadTimeFold || !st.aheadTimedBatch) return false;
+    if (st.dev.aheadTimedEpoch != st.sceneEpoch || st.dev.aheadSingleEpoch != st.sceneEpoch || st.dev.aheadTimeFold || !st.dev.aheadTimedBatch) return false;
     for (int i = 1; i < 6; i += 2)
-        if (cudaEventQuery(st.aheadEv[i]) != cudaSuccess) {
+        if (cudaEventQuery(st.dev.aheadEv[i]) != cudaSuccess) {
             cudaGetLastError();
             return false;  // not there yet: ask again at the next batch
         }
     float single = 0.f, batch = 0.f, fold = 0.f;
-    if (cudaEventElapsedTime(&single, st.aheadEv[0], st.aheadEv[1]) != cudaSuccess || cudaEventElapsedTime(&batch, st.aheadEv[2], st.aheadEv[3]) != cudaSuccess ||
-        cudaEventElapsedTime(&fold, st.aheadEv[4], st.aheadEv[5]) != cudaSuccess) {
+    if (cudaEventElapsedTime(&single, st.dev.aheadEv[0], st.dev.aheadEv[1]) != cudaSuccess || cudaEventElapsedTime(&batch, st.dev.aheadEv[2], st.dev.aheadEv[3]) != cudaSuccess ||
+        cudaEventElapsedTime(&fold, st.dev.aheadEv[4], st.dev.aheadEv[5]) != cudaSuccess) {
         cudaGetLastError();
         return false;
     }
-    return batch / (float)st.aheadTimedBatch + fold > 0.97f * single;
+    return batch / (float)st.dev.aheadTimedBatch + fold > 0.97f * single;
 }
 
 // *done = the frame has been produced (from samples kept by an earlier call, or by a batch launched now).
@@ -2397,63 +2430,47 @@ static int lookahead_frame(uint32_t* img, float* hdr, uint32_t traceDepth, uint3
     const int opt = st.options[SVR_OPT_PT_LOOKAHEAD];
     const bool adaptive = opt > 0;
     const uint32_t maxBatch = (uint32_t)std::min(opt < 0 ? -opt : opt, 32);
-    if (maxBatch < 2u || !hdr || !W || !H || st.options[SVR_OPT_COUNTERS] || (adaptive && st.aheadOffEpoch == st.sceneEpoch)) {
-        st.aheadCount = 0;
+    if (maxBatch < 2u || !hdr || !W || !H || st.options[SVR_OPT_COUNTERS] || (adaptive && st.dev.aheadOffEpoch == st.sceneEpoch)) {
+        st.dev.aheadCount = 0;
         return 0;
     }
     const size_t npix = (size_t)W * H;
-    const bool kept = st.aheadCount != 0 && st.aheadEpoch == st.sceneEpoch && st.aheadW == W && st.aheadH == H && st.aheadDepth == traceDepth &&
-                      st.aheadHdr == hdr && frameNo == st.aheadNext && frameNo < st.aheadFirst + st.aheadCount;
+    const bool kept = st.dev.aheadCount != 0 && st.dev.aheadEpoch == st.sceneEpoch && st.dev.aheadRender.continues(frameNo, hdr, W, H, traceDepth) &&
+                      frameNo < st.dev.aheadFirst + st.dev.aheadCount;
     if (!kept) {
-        st.aheadCount = 0;
+        st.dev.aheadCount = 0;
         // a render that has come this far without a change is likely to go on (whoever moves the camera every few frames never
         // gets here and pays nothing)
         if (frameNo < 16u) return 0;
         if (adaptive && lookahead_does_not_pay(st)) {
-            st.aheadOffEpoch = st.sceneEpoch;
+            st.dev.aheadOffEpoch = st.sceneEpoch;
             return 0;
         }
         uint32_t batch = maxBatch;
         while (batch >= 2u && (size_t)batch * npix * 3 * sizeof(float) > ((size_t)1 << 30)) batch >>= 1;
         if (batch < 2u) return 0;
         const size_t need = (size_t)batch * npix * 3 + (npix + 3) / 4;  // records, then one flag byte per pixel
-        if (st.aheadCapFloats < need) {
-            cudaFree(st.dAhead);
-            st.dAhead = nullptr;
-            st.aheadCapFloats = 0;
-            if (cudaMalloc(&st.dAhead, need * sizeof(float)) != cudaSuccess) {
-                cudaGetLastError();
-                return 0;  // no memory for it: one sample per call as before
-            }
-            st.aheadCapFloats = need;
+        if (st.dev.ahead.reserve(need) != cudaSuccess) {
+            cudaGetLastError();
+            return 0;  // no memory for it: one sample per call as before
         }
-        PtLaunch a;
-        memset(&a, 0, sizeof(a));
-        a.traceDepth = traceDepth;
-        a.firstSample = frameNo;
-        a.nSamples = batch;
-        a.y0 = 0;
-        a.y1 = 0xffffffffu;
-        a.perSample = st.dAhead;
-        a.constantPixel = (uint8_t*)(st.dAhead + (size_t)batch * npix * 3);
-        const bool timeIt = adaptive && st.aheadTimedEpoch != st.sceneEpoch && lookahead_events(st);
-        if (timeIt) SVR_TRY(cudaEventRecord(st.aheadEv[2], st.stream));
+        PtLaunch a = full_frame(traceDepth, frameNo, batch);
+        a.perSample = st.dev.ahead.p;
+        a.constantPixel = (uint8_t*)(st.dev.ahead.p + (size_t)batch * npix * 3);
+        const bool timeIt = adaptive && st.dev.aheadTimedEpoch != st.sceneEpoch && lookahead_events(st);
+        if (timeIt) SVR_TRY(cudaEventRecord(st.dev.aheadEv[2], st.stream));
         int rc = launch_pathtrace(a);
         if (rc) return rc;
         if (!a.perSample) return 0;  // another kernel shape serves this scene
         if (timeIt) {
-            SVR_TRY(cudaEventRecord(st.aheadEv[3], st.stream));
-            st.aheadTimedEpoch = st.sceneEpoch;
-            st.aheadTimedBatch = batch;
-            st.aheadTimeFold = true;
+            SVR_TRY(cudaEventRecord(st.dev.aheadEv[3], st.stream));
+            st.dev.aheadTimedEpoch = st.sceneEpoch;
+            st.dev.aheadTimedBatch = batch;
+            st.dev.aheadTimeFold = true;
         }
-        st.aheadFirst = st.aheadNext = frameNo;
-        st.aheadCount = batch;
-        st.aheadEpoch = st.sceneEpoch;  // after the launch: refreshing the majorants moves the epoch
-        st.aheadW = W;
-        st.aheadH = H;
-        st.aheadDepth = traceDepth;
-        st.aheadHdr = hdr;
+        st.dev.aheadFirst = frameNo;
+        st.dev.aheadCount = batch;
+        st.dev.aheadEpoch = st.sceneEpoch;  // after the launch: refreshing the majorants moves the epoch
         st.aheadBatches++;
     }
     PtLaunch c;
@@ -2465,17 +2482,17 @@ static int lookahead_frame(uint32_t* img, float* hdr, uint32_t traceDepth, uint3
     c.img = img;
     DevScene sc = st.scene;
     sc.envEnabled = st.options[SVR_OPT_ENV_ENABLED];  // as launch_pathtrace sets it
-    const bool timeFold = st.aheadTimeFold && st.aheadTimedEpoch == st.sceneEpoch;
-    if (timeFold) SVR_TRY(cudaEventRecord(st.aheadEv[4], st.stream));
-    lookahead_consume_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st.stream>>>(sc, c, st.dAhead, (const uint8_t*)(st.dAhead + (size_t)st.aheadCount * npix * 3),
-                                                                                   st.aheadCount, frameNo - st.aheadFirst);
+    const bool timeFold = st.dev.aheadTimeFold && st.dev.aheadTimedEpoch == st.sceneEpoch;
+    if (timeFold) SVR_TRY(cudaEventRecord(st.dev.aheadEv[4], st.stream));
+    lookahead_consume_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st.stream>>>(sc, c, st.dev.ahead.p, (const uint8_t*)(st.dev.ahead.p + (size_t)st.dev.aheadCount * npix * 3),
+                                                                                   st.dev.aheadCount, frameNo - st.dev.aheadFirst);
     count_launch();
     SVR_TRY(cudaGetLastError());
     if (timeFold) {
-        SVR_TRY(cudaEventRecord(st.aheadEv[5], st.stream));
-        st.aheadTimeFold = false;
+        SVR_TRY(cudaEventRecord(st.dev.aheadEv[5], st.stream));
+        st.dev.aheadTimeFold = false;
     }
-    st.aheadNext = frameNo + 1u;
+    st.dev.aheadRender.follow(frameNo, hdr, W, H, traceDepth);
     *done = true;
     return 0;
 }
@@ -2489,31 +2506,20 @@ static int denoised_frame(uint32_t* img, float* hdr, uint32_t traceDepth, uint32
     HostState& st = state();
     *done = false;
     const uint32_t W = st.scene.cam.imageW, H = st.scene.cam.imageH;
-    const bool follows = frameNo == 0u || (st.progActive && frameNo == st.progNext && hdr == st.progHdr && W == st.progW && H == st.progH &&
-                                           traceDepth == st.progDepth);
-    st.progActive = false;
+    const bool follows = frameNo == 0u || st.dev.progRender.continues(frameNo, hdr, W, H, traceDepth);
+    st.dev.progRender = FollowedRender();
     if (!st.options[SVR_OPT_PT_DENOISE] || st.options[SVR_OPT_COUNTERS] || !follows || !img || !hdr || !W || !H) return 0;
     const size_t npix = (size_t)W * H;
     if (!ensure_progressive_buffers(st, npix)) return 0;
-    if (frameNo == 0u) SVR_TRY(cudaMemsetAsync(st.dProg[1], 0, npix * sizeof(float4), st.stream));
-    PtLaunch a;
-    memset(&a, 0, sizeof(a));
-    a.traceDepth = traceDepth;
-    a.firstSample = frameNo;
-    a.nSamples = 1;
-    a.y0 = 0;
-    a.y1 = 0xffffffffu;
+    float4* const sums = st.dev.prog.p;  // even, odd
+    if (frameNo == 0u) SVR_TRY(cudaMemsetAsync(sums + npix, 0, npix * sizeof(float4), st.stream));
+    PtLaunch a = full_frame(traceDepth, frameNo, 1);
     a.hdr = hdr;
-    a.sum = st.dProg[frameNo & 1u];
+    a.sum = sums + (frameNo & 1u) * npix;
     a.clearSum = frameNo == 0u;
     if (int rc = launch_pathtrace(a)) return rc;
     if (int rc = progressive_denoise(img, frameNo)) return rc;
-    st.progActive = true;
-    st.progNext = frameNo + 1u;
-    st.progW = W;
-    st.progH = H;
-    st.progDepth = traceDepth;
-    st.progHdr = hdr;
+    st.dev.progRender.follow(frameNo, hdr, W, H, traceDepth);
     *done = true;
     return 0;
 }
@@ -2524,24 +2530,18 @@ extern "C" void render_pathtracer(svr_u8vec4* img, const svr_render_params* rend
     int rc = denoised_frame((uint32_t*)img, (float*)renderParams->hdrBuffer, renderParams->traceDepth, renderParams->frameNo, &done);
     if (!rc && !done) rc = lookahead_frame((uint32_t*)img, (float*)renderParams->hdrBuffer, renderParams->traceDepth, renderParams->frameNo, &done);
     if (!rc && !done) {
-        PtLaunch a;
-        memset(&a, 0, sizeof(a));
-        a.traceDepth = renderParams->traceDepth;
-        a.firstSample = renderParams->frameNo;
-        a.nSamples = 1;
-        a.y0 = 0;
-        a.y1 = 0xffffffffu;
+        PtLaunch a = full_frame(renderParams->traceDepth, renderParams->frameNo, 1);
         a.hdr = (float*)renderParams->hdrBuffer;
         a.img = (uint32_t*)img;
         // look-ahead's yardstick: one steady-state single-sample launch per scene (classification cached, nothing to refresh)
         HostState& st = state();
-        const bool timeIt = st.options[SVR_OPT_PT_LOOKAHEAD] > 1 && a.firstSample >= 8u && a.firstSample < 16u && st.aheadSingleEpoch != st.sceneEpoch &&
-                            st.pixelCacheEpoch == st.sceneEpoch && lookahead_events(st);
-        if (timeIt) cudaEventRecord(st.aheadEv[0], st.stream);
+        const bool timeIt = st.options[SVR_OPT_PT_LOOKAHEAD] > 1 && a.firstSample >= 8u && a.firstSample < 16u && st.dev.aheadSingleEpoch != st.sceneEpoch &&
+                            st.dev.pixelCacheEpoch == st.sceneEpoch && lookahead_events(st);
+        if (timeIt) cudaEventRecord(st.dev.aheadEv[0], st.stream);
         rc = launch_pathtrace(a);
         if (timeIt && !rc) {
-            cudaEventRecord(st.aheadEv[1], st.stream);
-            st.aheadSingleEpoch = st.sceneEpoch;
+            cudaEventRecord(st.dev.aheadEv[1], st.stream);
+            st.dev.aheadSingleEpoch = st.sceneEpoch;
         }
     }
     if (rc) {
@@ -2554,14 +2554,8 @@ extern "C" void render_pathtracer(svr_u8vec4* img, const svr_render_params* rend
 extern "C" int svr_render_pathtracer_spp(svr_u8vec4* img, const svr_render_params* renderParams, uint32_t spp)
 {
     if (!renderParams || !renderParams->hdrBuffer) return fail_msg("svr_render_pathtracer_spp: hdrBuffer is null");
-    state().progActive = false;  // SVR_OPT_PT_DENOISE does not apply: the render it followed has moved on without its sums
-    PtLaunch a;
-    memset(&a, 0, sizeof(a));
-    a.traceDepth = renderParams->traceDepth;
-    a.firstSample = renderParams->frameNo;
-    a.nSamples = spp;
-    a.y0 = 0;
-    a.y1 = 0xffffffffu;
+    state().dev.progRender = FollowedRender();  // SVR_OPT_PT_DENOISE does not apply: the render it followed has moved on without its sums
+    PtLaunch a = full_frame(renderParams->traceDepth, renderParams->frameNo, spp);
     a.hdr = (float*)renderParams->hdrBuffer;
     a.img = (uint32_t*)img;
     return launch_pathtrace(a);
@@ -2570,13 +2564,7 @@ extern "C" int svr_render_pathtracer_spp(svr_u8vec4* img, const svr_render_param
 extern "C" int svr_pathtracer_accumulate(svr_vec4* sum, uint32_t traceDepth, uint32_t firstSample, uint32_t nSamples, int clear)
 {
     if (!sum) return fail_msg("svr_pathtracer_accumulate: sum is null");
-    PtLaunch a;
-    memset(&a, 0, sizeof(a));
-    a.traceDepth = traceDepth;
-    a.firstSample = firstSample;
-    a.nSamples = nSamples;
-    a.y0 = 0;
-    a.y1 = 0xffffffffu;
+    PtLaunch a = full_frame(traceDepth, firstSample, nSamples);
     a.sum = (float4*)sum;
     a.clearSum = clear;
     return launch_pathtrace(a);
@@ -2586,13 +2574,7 @@ extern "C" int svr_pathtracer_accumulate_bands(svr_vec4* sum, uint32_t traceDept
                                                uint32_t phase, uint32_t stride, uint32_t* bandRows)
 {
     if (!sum) return fail_msg("svr_pathtracer_accumulate_bands: sum is null");
-    PtLaunch a;
-    memset(&a, 0, sizeof(a));
-    a.traceDepth = traceDepth;
-    a.firstSample = firstSample;
-    a.nSamples = nSamples;
-    a.y0 = 0;
-    a.y1 = 0xffffffffu;
+    PtLaunch a = full_frame(traceDepth, firstSample, nSamples);
     a.sum = (float4*)sum;
     a.clearSum = clear;
     a.bandPhase = phase;
@@ -2620,27 +2602,17 @@ extern "C" int svr_pathtracer_accumulate_adaptive(svr_vec4* sum, svr_vec4* halfS
     if (!st.scene.vol.tex || !st.scene.tf.tex) return fail_msg("render_pathtracer: setup_volume / setup_transferfunction not called");
     const uint32_t W = st.scene.cam.imageW, H = st.scene.cam.imageH, npix = W * H;
     if (!npix) return fail_msg("render_pathtracer: setup_camera not called");
-    if (st.adaptiveListCap < npix) {
-        cudaFree(st.dAdaptiveList);
-        st.dAdaptiveList = nullptr;
-        st.adaptiveListCap = 0;
-        SVR_TRY(cudaMalloc(&st.dAdaptiveList, (size_t)npix * sizeof(uint32_t)));
-        st.adaptiveListCap = npix;
-    }
-    if (!st.dAdaptiveCounts) SVR_TRY(cudaMalloc(&st.dAdaptiveCounts, 4 * sizeof(uint32_t)));
+    SVR_TRY(st.dev.adaptiveList.reserve(npix));
+    SVR_TRY(st.dev.adaptiveCounts.reserve(4));
     float4* s4 = (float4*)sum;
     float4* h4 = (float4*)halfSum;
-    adaptive_start_kernel<<<(npix + 255u) / 256u, 256, 0, st.stream>>>(s4, h4, st.dAdaptiveList, st.dAdaptiveCounts, npix);
+    adaptive_start_kernel<<<(npix + 255u) / 256u, 256, 0, st.stream>>>(s4, h4, st.dev.adaptiveList.p, st.dev.adaptiveCounts.p, npix);
     count_launch();
     SVR_TRY(cudaGetLastError());
 
-    PtLaunch a;
-    memset(&a, 0, sizeof(a));
-    a.traceDepth = traceDepth;
-    a.y0 = 0;
-    a.y1 = 0xffffffffu;
+    PtLaunch a = full_frame(traceDepth, 0, 0);
     a.sum = s4;
-    PixelList pl = {st.dAdaptiveList, npix, h4};
+    PixelList pl = {st.dev.adaptiveList.p, npix, h4};
     uint32_t w = 0, n = minSamples, rounds = 0, unconverged = 0;
     uint64_t samples = 0;
     for (uint32_t pass = 0;; ++pass) {
@@ -2652,12 +2624,12 @@ extern "C" int svr_pathtracer_accumulate_adaptive(svr_vec4* sum, svr_vec4* halfS
         w += n;
         const dim3 cb((W + 31u) / 32u, (H + 7u) / 8u);
         const uint32_t slot = pass & 1u;
-        adaptive_converge_kernel<<<cb, dim3(32, 8), 0, st.stream>>>(s4, h4, errOrNull, st.dAdaptiveList, st.dAdaptiveCounts, slot, W, H, (float)w,
+        adaptive_converge_kernel<<<cb, dim3(32, 8), 0, st.stream>>>(s4, h4, errOrNull, st.dev.adaptiveList.p, st.dev.adaptiveCounts.p, slot, W, H, (float)w,
                                                                    (float)maxSamples, threshold, st.scene.cam.exposure);
         count_launch();
         SVR_TRY(cudaGetLastError());
         uint32_t c[2];
-        if (int rc = read_small(st, c, st.dAdaptiveCounts + 2u * slot, sizeof(c))) return rc;
+        if (int rc = read_small(st, c, st.dev.adaptiveCounts.p + 2u * slot, sizeof(c))) return rc;
         pl.count = c[0];
         unconverged = c[1];
         if (pl.count == 0) break;
@@ -2675,7 +2647,7 @@ extern "C" int svr_pathtracer_resolve(svr_u8vec4* img, svr_vec3* hdrOut, const s
     if (!sum) return fail_msg("svr_pathtracer_resolve: sum is null");
     uint32_t npix = st.scene.cam.imageW * st.scene.cam.imageH;
     if (!npix) return fail_msg("svr_pathtracer_resolve: setup_camera not called");
-    if (hdrOut && (const void*)hdrOut == st.aheadHdr) st.aheadCount = 0;  // the running mean render_pathtracer's kept samples follow is overwritten
+    hdr_written_outside(st.dev, hdrOut, false);
     resolve_kernel<<<(npix + 255u) / 256u, 256, 0, st.stream>>>((const float4*)sum, (float*)hdrOut, (uint32_t*)img, npix,
                                                                st.scene.cam.exposure);
     count_launch();

@@ -10,44 +10,97 @@
 #include <cstdio>
 #include <cstdlib>
 #include <string>
+#include <utility>
 
 #include "../../include/svr_render.h"
 #include "svr_scene.cuh"
 
 namespace svr {
 
-struct HostState {
-    cudaStream_t stream = nullptr;
-    DevScene scene;  // what setup_* stored (zero-initialised in state())
-    int options[SVR_OPT_COUNT_];
+// A device allocation that only grows.  reserve(n) keeps the buffer when it holds n elements already, and otherwise replaces
+// it; a failed allocation leaves {nullptr, 0} and returns the error.  A DevBuf of function scope frees its buffer on return.
+template <class T>
+struct DevBuf {
+    T* p = nullptr;
+    size_t cap = 0;  // elements
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf& operator=(DevBuf&& o) noexcept
+    {
+        std::swap(p, o.p);
+        std::swap(cap, o.cap);
+        return *this;
+    }
+    ~DevBuf() { release(); }
+    cudaError_t reserve(size_t n)
+    {
+        if (cap >= n) return cudaSuccess;
+        release();
+        const cudaError_t e = cudaMalloc(&p, n * sizeof(T));
+        if (e != cudaSuccess) {
+            p = nullptr;
+            return e;
+        }
+        cap = n;
+        return cudaSuccess;
+    }
+    void release()
+    {
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+};
 
+// The render a sequence of render_pathtracer calls builds in one running mean: the next frame, the hdrBuffer, the image size
+// and traceDepth.  A default record follows nothing.
+struct FollowedRender {
+    uint32_t next = 0, W = 0, H = 0, depth = 0;
+    const void* hdr = nullptr;
+    bool continues(uint32_t frameNo, const void* hdr_, uint32_t W_, uint32_t H_, uint32_t depth_) const
+    {
+        return hdr && frameNo == next && hdr_ == hdr && W_ == W && H_ == H && depth_ == depth;
+    }
+    void follow(uint32_t frameNo, const void* hdr_, uint32_t W_, uint32_t H_, uint32_t depth_)
+    {
+        next = frameNo + 1u;
+        hdr = hdr_;
+        W = W_;
+        H = H_;
+        depth = depth_;
+    }
+};
+
+// Everything bound to the current device: its allocations, events and views, and the keys and flags that say what they hold
+// (svr_set_device resets it)
+struct DeviceState {
     // macrocell cache -- callee-owned derived data, keyed on the caller's cudaArray handle
     cudaArray_t gridArray = nullptr;      // volume array the range grid was built from
     int gridCell = 0;
     int3 gridDims = {0, 0, 0};
     int3 volDims = {0, 0, 0};
-    float2* dRange = nullptr;
-    float* dMajorant = nullptr;              // padded: (gx+2)(gy+2)(gz+2), one empty cell around the grid
-    uint8_t* dDist[2] = {nullptr, nullptr};  // ping-pong Chebyshev distance to the nearest non-empty cell
-    int* dOcc = nullptr;                     // bounding box of the non-empty cells: lo xyz, hi xyz
+    DevBuf<float2> range;
+    DevBuf<float> majorant;                // padded: (gx+2)(gy+2)(gz+2), one empty cell around the grid
+    DevBuf<uint8_t> dist[2];               // ping-pong Chebyshev distance to the nearest non-empty cell
+    DevBuf<int> occ;                       // bounding box of the non-empty cells: lo xyz, hi xyz
     int majorantLeap = -1;
-    float* dTfSparse = nullptr;           // range-max sparse table over the TF opacity
-    float4* dTfTable = nullptr;           // linear copy of the TF array
+    DevBuf<float> tfSparse;               // range-max sparse table over the TF opacity
+    DevBuf<float4> tfTable;               // linear copy of the TF array
     int tfEntries = 0;
     cudaTextureObject_t volPointTex = 0;  // point-sampled view of gridArray
     cudaSurfaceObject_t uploadSurf = 0;   // store view of uploadSurfArray (svr_volume_upload from a device buffer, svr_macrocell.cu)
     cudaArray_t uploadSurfArray = nullptr;
-    unsigned long long fusedUploads = 0;
     void* hMailbox = nullptr;             // 64 bytes of mapped pinned memory: small results reach the host without a copy engine
     void* dMailbox = nullptr;
     bool rangeValid = false;              // false until the range grid reflects the array's current voxels
     bool fingerprintDue = false;          // setup_volume was called since the voxels were last looked at
-    unsigned long long* dFingerprint = nullptr;  // [0] sampled hash of the voxels the ranges were built from, [1] scratch
+    DevBuf<unsigned long long> fingerprint;  // [0] sampled hash of the voxels the ranges were built from, [1] scratch
     bool majorantValid = false;           // false after setup_volume/setup_transferfunction
     float majorantDensityScale = 0.f;
     cudaArray_t majorantTfArray = nullptr;
-    unsigned long long* dTfHash = nullptr;  // [0] hash of the TF table the majorants were built from, [1] of the live table, [2] stale flag
-    cudaEvent_t tfCheckEvent = nullptr;     // behind the ray caster's per-call hash of the live table (svr_macrocell.cu: tf_check_*)
+    DevBuf<unsigned long long> tfHash;    // [0] hash of the TF table the majorants were built from, [1] of the live table, [2] stale flag
+    cudaEvent_t tfCheckEvent = nullptr;   // behind the ray caster's per-call hash of the live table (svr_macrocell.cu: tf_check_*)
     bool tfCheckPending = false;
 
     // automatic macrocell size (SVR_OPT_MACROCELL_SIZE = 0): the choice and the scene it was made for
@@ -55,30 +108,27 @@ struct HostState {
     cudaArray_t autoArray = nullptr, autoTfArray = nullptr;
     float autoDensityScale = 0.f;
     unsigned autoEpoch = 0, uploadEpoch = 0;  // uploadEpoch counts svr_volume_upload / svr_tf_upload calls
-    void* dStats = nullptr;
+    DevBuf<unsigned long long> stats;
 
     // importance sampler of the environment light (svr_env_io.cu), keyed on what it was built from
-    float* dEnvMarg = nullptr;
-    float* dEnvCond = nullptr;
+    DevBuf<float> envMarg;
+    DevBuf<float> envCond;
     svr_env_light envSamplerKey = {};
     bool envSamplerValid = false;
 
     // Per-pixel classification (classify_pixel: entry skip, light cull, all-sky flag) kept across the 1-sample-per-call frames
     // of a progressive render: valid while sceneEpoch has not moved since it was stored
-    float2* dPixelCache = nullptr;
-    size_t pixelCacheCap = 0;
-    unsigned long long sceneEpoch = 1, pixelCacheEpoch = 0;  // sceneEpoch: bumped by everything that can change what a pixel sees
+    DevBuf<float2> pixelCache;
+    unsigned long long pixelCacheEpoch = 0;
     uint32_t pixelCacheW = 0, pixelCacheH = 0;
     int pixelCacheMode = -1;
 
     // Sample look-ahead of the 1-sample-per-call protocol (SVR_OPT_PT_LOOKAHEAD, svr_pathtrace.cu): the radiance of the samples
-    // [aheadFirst, aheadFirst + aheadCount) of every pixel, computed in one sample-parallel launch; aheadNext is the frame the
-    // next call must ask for
-    float* dAhead = nullptr;
-    size_t aheadCapFloats = 0;
-    uint32_t aheadFirst = 0, aheadCount = 0, aheadNext = 0, aheadW = 0, aheadH = 0, aheadDepth = 0;
-    unsigned long long aheadEpoch = 0, aheadBatches = 0;
-    const void* aheadHdr = nullptr;
+    // [aheadFirst, aheadFirst + aheadCount) of every pixel of aheadRender, computed in one sample-parallel launch
+    DevBuf<float> ahead;
+    FollowedRender aheadRender;
+    uint32_t aheadFirst = 0, aheadCount = 0;
+    unsigned long long aheadEpoch = 0;
     // does it pay for this scene?  timed once per scene epoch: a single-sample launch [0,1], the first batch [2,3], one fold [4,5]
     cudaEvent_t aheadEv[6] = {};
     bool aheadEvReady = false, aheadTimeFold = false;
@@ -87,27 +137,41 @@ struct HostState {
 
     // Adaptive sampling (svr_pathtracer_accumulate_adaptive): the offsets of the pixels still taking samples, and the counts
     // of the convergence pass (two slots of {active, unconverged}: a pass fills one and clears the other)
-    uint32_t* dAdaptiveList = nullptr;
-    size_t adaptiveListCap = 0;
-    uint32_t* dAdaptiveCounts = nullptr;
+    DevBuf<uint32_t> adaptiveList;
+    DevBuf<uint32_t> adaptiveCounts;
 
-    // Denoising (svr_pathtracer_denoise, svr_denoise.cu): the filter's ping-pong buffers, float4 (demodulated rgb, variance) per pixel
-    float4* dDenoise[2] = {nullptr, nullptr};
-    size_t denoiseCap = 0;
+    // Denoising (svr_pathtracer_denoise, svr_denoise.cu): the filter's two ping-pong buffers of npix float4 (demodulated rgb,
+    // variance), one after the other
+    DevBuf<float4> denoise;
 
     // Denoised progressive display (SVR_OPT_PT_DENOISE, render_pathtracer): the even and odd frames' sample sums and the guides
-    // (albedoCoverage, normalDepth) of the render being followed; progNext is the frame the next call must ask for
-    float4* dProg[4] = {nullptr, nullptr, nullptr, nullptr};
-    size_t progCap = 0;
-    bool progActive = false;
-    uint32_t progNext = 0, progW = 0, progH = 0, progDepth = 0;
-    const void* progHdr = nullptr;
+    // (albedoCoverage, normalDepth) of progRender, four blocks of npix float4
+    DevBuf<float4> prog;
+    FollowedRender progRender;
     unsigned long long progGuideEpoch = 0;  // sceneEpoch after the frame that made the guides; 0 = none
     uint32_t progGuideRays = 0;
-    svr_denoise_params progParams;          // svr_pathtracer_set_denoise_params (state(): the defaults)
 
-    Counters* dCounters = nullptr;
-    unsigned long long launches = 0;
+    DevBuf<Counters> counters;
+
+    // Frees every allocation, event, view and the mailbox, and returns every key and flag to its default (svr_api.cu)
+    void reset();
+};
+
+// The running mean `hdr` (null: none) was written outside the render look-ahead follows: the samples kept for that render no
+// longer follow it.  anyHdr: whichever running mean it was (an ordinary path-tracing launch moves the one it writes on).
+inline void hdr_written_outside(DeviceState& d, const void* hdr, bool anyHdr)
+{
+    if (hdr && (anyHdr || hdr == d.aheadRender.hdr)) d.aheadCount = 0;
+}
+
+struct HostState {
+    cudaStream_t stream = nullptr;
+    DevScene scene;  // what setup_* stored (zero-initialised in state())
+    int options[SVR_OPT_COUNT_];
+    DeviceState dev;
+    unsigned long long sceneEpoch = 1;  // bumped by everything that can change what a pixel sees
+    svr_denoise_params progParams;      // svr_pathtracer_set_denoise_params (state(): the defaults)
+    unsigned long long launches = 0, fusedUploads = 0, aheadBatches = 0;
     std::string lastError;
 };
 
@@ -163,11 +227,10 @@ int read_small(HostState& st, void* host, const void* dev, size_t bytes);
 
 // Denoising (svr_denoise.cu).  check_denoise_params: 0, or the error of `who` (before any CUDA call).  progressive_denoise: the
 // guides and the filter of one denoised frame of render_pathtracer (SVR_OPT_PT_DENOISE) into img, after its sample has gone
-// into dProg[frameNo & 1]; ensure_progressive_buffers: false when they cannot be allocated.
+// into the even or odd sum of dev.prog (frameNo & 1); ensure_progressive_buffers: false when they cannot be allocated.
 int check_denoise_params(const char* who, const svr_denoise_params* paramsOrNull, svr_denoise_params* out);
 bool ensure_progressive_buffers(HostState& st, size_t npix);
 int progressive_denoise(uint32_t* img, uint32_t frameNo);
-void release_progressive(HostState& st);
 
 inline void count_launch(int n = 1) { state().launches += (unsigned long long)n; }
 

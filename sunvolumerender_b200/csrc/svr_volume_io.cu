@@ -175,11 +175,6 @@ __global__ void rescale_kernel(short* __restrict__ data, size_t n, float dataMin
     }
 }
 
-struct DevBuf {
-    void* p = nullptr;
-    ~DevBuf() { cudaFree(p); }
-};
-
 }  // namespace
 }  // namespace svr
 
@@ -289,17 +284,19 @@ extern "C" int svr_volume_from_raw(const void* host_data, int met_type, int msb,
         return fail_msg("svr_volume_from_raw: dimension exceeds the 3-D texture limit (16384 per axis)");
     HostState& st = state();
     const size_t n = (size_t)nx * ny * nz;
-    DevBuf raw, data, aux, hist;
-    SVR_TRY(cudaMalloc(&raw.p, n * es));
-    SVR_TRY(cudaMalloc(&data.p, n * sizeof(short)));
-    SVR_TRY(cudaMalloc(&aux.p, 32));
+    DevBuf<uint8_t> raw, aux;
+    DevBuf<short> data;
+    DevBuf<unsigned int> hist;
+    SVR_TRY(raw.reserve(n * es));
+    SVR_TRY(data.reserve(n));
+    SVR_TRY(aux.reserve(32));
     SVR_TRY(cudaMemcpyAsync(raw.p, host_data, n * es, cudaMemcpyHostToDevice, st.stream));
     int* dMinMax = (int*)aux.p;        // [0] min, [1] max, [2] max gradient magnitude
     unsigned long long* dTotal = (unsigned long long*)((char*)aux.p + 16);
     const int init[8] = {INT_MAX, INT_MIN, INT_MIN, 0, 0, 0, 0, 0};
     SVR_TRY(cudaMemcpyAsync(aux.p, init, sizeof(init), cudaMemcpyHostToDevice, st.stream));
     const int blocks = 148 * 8, threads = 256;
-    short* d = (short*)data.p;
+    short* d = data.p;
     const int swap = msb && es > 1;
     switch (met_type) {
         case SVR_MET_UCHAR: cast_minmax_kernel<unsigned char><<<blocks, threads, 0, st.stream>>>((const unsigned char*)raw.p, swap, n, d, dMinMax); break;
@@ -316,15 +313,14 @@ extern "C" int svr_volume_from_raw(const void* host_data, int met_type, int msb,
     int h[3];
     SVR_TRY(cudaMemcpyAsync(h, aux.p, sizeof(h), cudaMemcpyDeviceToHost, st.stream));
     SVR_TRY(cudaStreamSynchronize(st.stream));
-    cudaFree(raw.p);
-    raw.p = nullptr;
+    raw.release();
     const int dataMin = h[0], dataMax = h[1];
     const int bins = dataMax - dataMin;  // SetComponentExtent(0, max - min - 1, ...)
     unsigned long long total = 0;
     if (bins > 0) {
-        SVR_TRY(cudaMalloc(&hist.p, (size_t)bins * sizeof(unsigned int)));
+        SVR_TRY(hist.reserve((size_t)bins));
         SVR_TRY(cudaMemsetAsync(hist.p, 0, (size_t)bins * sizeof(unsigned int), st.stream));
-        histogram_kernel<<<blocks, threads, 0, st.stream>>>(d, n, dataMin, bins, (unsigned int*)hist.p, dTotal);
+        histogram_kernel<<<blocks, threads, 0, st.stream>>>(d, n, dataMin, bins, hist.p, dTotal);
         count_launch();
         if (histogram && histogram_capacity)
             SVR_TRY(cudaMemcpyAsync(histogram, hist.p, sizeof(unsigned int) * std::min<size_t>((size_t)bins, histogram_capacity),
