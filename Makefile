@@ -14,7 +14,7 @@ ARCH     := -gencode arch=compute_100a,code=sm_100a
 NVFLAGS  := -std=c++17 -O3 -use_fast_math -lineinfo $(ARCH) -Xcompiler -fPIC -Xptxas -v -cudart shared
 CSRC     := sunvolumerender_b200/csrc
 OBJDIR   := build/obj
-SRCS     := $(CSRC)/svr_api.cu $(CSRC)/svr_macrocell.cu $(CSRC)/svr_raycast.cu $(CSRC)/svr_pathtrace.cu $(CSRC)/svr_volume_io.cu $(CSRC)/svr_tf_io.cu $(CSRC)/svr_env_io.cu $(CSRC)/svr_canvas.cu $(CSRC)/svr_denoise.cu
+SRCS     := $(CSRC)/svr_api.cu $(CSRC)/svr_macrocell.cu $(CSRC)/svr_raycast.cu $(CSRC)/svr_pathtrace.cu $(CSRC)/svr_volume_io.cu $(CSRC)/svr_tf_io.cu $(CSRC)/svr_env_io.cu $(CSRC)/svr_canvas.cu $(CSRC)/svr_denoise.cu $(CSRC)/svr_project.cu
 OBJS     := $(patsubst $(CSRC)/%.cu,$(OBJDIR)/%.o,$(SRCS))
 HDRS     := $(wildcard $(CSRC)/*.cuh $(CSRC)/*.h include/*.h)
 LIB      := sunvolumerender_b200/libsvr_b200.so

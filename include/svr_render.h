@@ -77,7 +77,8 @@ enum svr_option {
     /* macrocell edge in voxels: 0 (default) = chosen from the scene, about twice the mean free path inside
      * the medium, re-evaluated when volume, transfer function or density scale change; or a power of two in 2..64 */
     SVR_OPT_MACROCELL_SIZE = 3,
-    /* ray caster empty-space skipping through the macrocell grid: 0 off, 1 on (default) */
+    /* skipping in the two ray-marching kernels: the ray caster's empty-space skipping through the macrocell grid, and the
+     * projection's skipping of cells that cannot change the projected value (svr_render_projection): 0 off, 1 on (default) */
     SVR_OPT_RC_SKIP = 4,
     /* Philox key */
     SVR_OPT_SEED = 5,
@@ -335,6 +336,32 @@ int svr_render_raycasting_rows(svr_u8vec4* img, svr_vec4* outOrNull, const svr_v
 int svr_render_raycasting_bands(svr_u8vec4* img, svr_vec4* outOrNull, const svr_volume* volume,
                                 const svr_transfer_function* tf, const svr_camera* camera, float stepSize,
                                 uint32_t phase, uint32_t stride, uint32_t* bandRows);
+
+/* Intensity projections (DESIGN.md section 7h): maximum (MIP), minimum (MinIP) and average (AIP) of the volume along each
+ * pixel-centre ray, no transfer function and no setup_* needed.  The ray is camera_ray_center's (pinhole, as
+ * render_raycasting), clipped to the volume box and its clip planes (the axis-aligned slab) and to t >= 0: with
+ * t0 = max(tNear, 0), h = 0.5 * stepSize and K = floor((tFar - t0) / h + 0.5), sample k (0 <= k < K) lies at
+ * t0 + (k + 0.5) h and has the value v_k = tex3D(volume, p) * densityScale (the hardware trilinear fetch).  The projected value
+ *   MAX:  P = max_k v_k        MIN:  P = min_k v_k        MEAN:  P = (v_0 + v_1 + ... + v_{K-1}) / K (fp32 sum in k order)
+ * and P = 0 when K = 0 (a ray that misses the box, or a box behind the camera).  The divisions in K and g are fp32 with
+ * fast-math rounding (within 2 ulp).  valueOrNull receives P (imageW*imageH floats);
+ * imgOrNull the grey image g = clamp((P - (windowCenter - windowWidth / 2)) / windowWidth, 0, 1), packed as trunc(255 g) in
+ * r, g and b with alpha 255.  Both are full-frame buffers; phase 0, stride 1 renders the frame, other values the bands of
+ * svr_render_raycasting_bands (*bandRows = the band height; pixels outside the call's bands are not touched).
+ * SVR_OPT_RC_SKIP = 1 (default) skips the samples of macrocells that cannot change P (MAX: cell maximum at or below the running
+ * maximum; MIN: cell minimum at or above the running minimum; MEAN: a cell of zero voxels), from a range grid kept per volume
+ * array (SVR_OPT_MACROCELL_SIZE, else the edge already built for that array, else 8); P is bit-identical either way.
+ * Errors, all reported before any CUDA call: a null volume, camera or params; both outputs null; a mode out of range;
+ * stepSize or windowWidth not positive or not finite; windowCenter not finite; phase >= stride. */
+enum svr_projection_mode { SVR_PROJECT_MAX = 0, SVR_PROJECT_MIN = 1, SVR_PROJECT_MEAN = 2 };
+typedef struct svr_projection_params {
+    int32_t mode;        /* svr_projection_mode */
+    float stepSize;      /* as render_raycasting: samples 0.5 * stepSize apart */
+    float windowCenter;  /* display window on the projected value */
+    float windowWidth;
+} svr_projection_params;
+int svr_render_projection(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_camera* camera,
+                          const svr_projection_params* params, uint32_t phase, uint32_t stride, uint32_t* bandRows);
 
 /* ---- resource builders (the input contract of the path) ---- */
 enum svr_voxel_format { SVR_VOXEL_U8 = 0, SVR_VOXEL_U16 = 1, SVR_VOXEL_F16 = 2, SVR_VOXEL_F32 = 3 };

@@ -104,6 +104,16 @@ class DenoiseParams(C.Structure):  # svr_denoise_params
 
 assert C.sizeof(DenoiseParams) == 20
 
+
+class ProjectionParams(C.Structure):  # svr_projection_params
+    _fields_ = [("mode", C.c_int32), ("stepSize", C.c_float), ("windowCenter", C.c_float), ("windowWidth", C.c_float)]
+
+
+assert C.sizeof(ProjectionParams) == 16
+# enum svr_projection_mode
+PROJECT_MAX, PROJECT_MIN, PROJECT_MEAN = range(3)
+PROJECT_MODES = {"max": PROJECT_MAX, "min": PROJECT_MIN, "mean": PROJECT_MEAN}
+
 # enum svr_option
 (OPT_PT_MODE, OPT_SHADOW_ESTIMATOR, OPT_ENV_ENABLED, OPT_MACROCELL_SIZE, OPT_RC_SKIP, OPT_SEED, OPT_COUNTERS,
  OPT_PT_BLOCK, OPT_RC_BLOCK, OPT_PT_KERNEL, OPT_PT_ROUNDS, OPT_LEAP, OPT_PT_ENTRY_CACHE, OPT_PT_WARP_PIXELS,
@@ -181,6 +191,8 @@ SIGNATURES = [
     ("svr_debug_sample_tf", C.c_int, [C.POINTER(TransferFunction), _P, C.c_uint32, _P]),
     ("svr_grid_info", C.c_int, [C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     ("svr_grid_copy", C.c_int, [_P, _P]),
+    ("svr_render_projection", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(Camera), C.POINTER(ProjectionParams), C.c_uint32, C.c_uint32,
+                                        C.POINTER(C.c_uint32)]),
 ]
 
 
@@ -258,7 +270,7 @@ class View(C.Structure):  # svr_view: the camera-related members of Canvas (gui/
 
 BUTTON_LEFT, BUTTON_MID = 1, 4
 KEY_LEFT, KEY_RIGHT, KEY_DOWN = 0, 1, 2
-RENDER_MODE_PATHTRACER, RENDER_MODE_RAYCASTING = 0, 1
+RENDER_MODE_PATHTRACER, RENDER_MODE_RAYCASTING, RENDER_MODE_PROJECTION = 0, 1, 2
 _F3 = C.POINTER(C.c_float * 3)
 _V = C.POINTER(View)
 
@@ -292,6 +304,7 @@ SIGNATURES_CANVAS = [
     ("svr_canvas_set_focal_length", C.c_int, [_P, C.c_float]),
     ("svr_canvas_set_exposure", C.c_int, [_P, C.c_float]),
     ("svr_canvas_set_clip_plane", C.c_int, [_P, C.c_int, C.c_double, C.c_double]),
+    ("svr_canvas_set_projection", C.c_int, [_P, C.c_int, C.c_float, C.c_float]),
     ("svr_canvas_mouse_press", C.c_int, [_P, C.c_float, C.c_float, C.c_int]),
     ("svr_canvas_mouse_move", C.c_int, [_P, C.c_float, C.c_float, C.c_int]),
     ("svr_canvas_wheel", C.c_int, [_P, C.c_int]),

@@ -99,6 +99,11 @@ class Canvas:
                 rc = getattr(lib, "svr_canvas_set_" + k)(c, v)
             self._ck(rc, "svr_canvas_set_" + k)
 
+    def set_projection(self, mode="max", window=(0.5, 1.0)):
+        """Projection mode's settings (svr_canvas_set_projection): mode "max", "min" or "mean", window (center, width);
+        select the mode with set(render_mode=L.RENDER_MODE_PROJECTION)."""
+        self._ck(self.lib.svr_canvas_set_projection(self.c, L.PROJECT_MODES[mode], float(window[0]), float(window[1])), "svr_canvas_set_projection")
+
     def set_immediate_repaint(self, on):
         self.lib.svr_canvas_set_immediate_repaint(self.c, 1 if on else 0)
 

@@ -208,6 +208,7 @@ struct svr_canvas {
     svr_render_params renderParams;
     svr_u8vec4* img = nullptr;
     int renderMode = SVR_RENDER_MODE_RAYCASTING;  // canvas.h:226
+    svr_projection_params projection = {SVR_PROJECT_MAX, 0.f, 0.5f, 1.f};  // stepSize: elementRadius at paint time
     bool ready = false;
     bool immediate = true;
     uint64_t paints = 0;
@@ -218,8 +219,13 @@ namespace {
 int paint_into(svr_canvas* c, svr_u8vec4* img)
 {
     if (!c->ready) return 0;  // canvas.cpp:67
-    if (!c->tf.tex) return fail_msg("svr_canvas_paint: no transfer function set");
-    if (c->renderMode == SVR_RENDER_MODE_RAYCASTING)
+    if (c->renderMode == SVR_RENDER_MODE_PROJECTION) {
+        svr_projection_params p = c->projection;
+        p.stepSize = c->elementRadius;
+        if (int rc = svr_render_projection(img, nullptr, &c->volume, &c->camera, &p, 0, 1, nullptr)) return rc;
+    } else if (!c->tf.tex) {
+        return fail_msg("svr_canvas_paint: no transfer function set");
+    } else if (c->renderMode == SVR_RENDER_MODE_RAYCASTING)
         render_raycasting(img, &c->volume, &c->tf, &c->camera, c->elementRadius);  // canvas.cpp:92
     else
         render_pathtracer(img, &c->renderParams);                                 // canvas.cpp:96
@@ -386,8 +392,21 @@ extern "C" int svr_canvas_set_scatter_times(svr_canvas* c, double depth)
 extern "C" int svr_canvas_set_render_mode(svr_canvas* c, int mode)
 {
     if (!c) return fail_msg("svr_canvas_set_render_mode: null canvas");
-    if (mode != SVR_RENDER_MODE_PATHTRACER && mode != SVR_RENDER_MODE_RAYCASTING) return fail_msg("svr_canvas_set_render_mode: bad mode");
+    if (mode != SVR_RENDER_MODE_PATHTRACER && mode != SVR_RENDER_MODE_RAYCASTING && mode != SVR_RENDER_MODE_PROJECTION)
+        return fail_msg("svr_canvas_set_render_mode: bad mode");
     c->renderMode = mode;  // the timer that repaints in path-tracer mode (canvas.h:80-93) is the host's paint loop
+    return restart(c);
+}
+
+extern "C" int svr_canvas_set_projection(svr_canvas* c, int mode, float windowCenter, float windowWidth)
+{
+    if (!c) return fail_msg("svr_canvas_set_projection: null canvas");
+    if (mode < SVR_PROJECT_MAX || mode > SVR_PROJECT_MEAN) return fail_msg("svr_canvas_set_projection: mode must be 0 (max), 1 (min) or 2 (mean)");
+    if (!(windowWidth > 0.f) || !std::isfinite(windowWidth) || !std::isfinite(windowCenter))
+        return fail_msg("svr_canvas_set_projection: windowWidth must be positive and finite, windowCenter finite");
+    c->projection.mode = mode;
+    c->projection.windowCenter = windowCenter;
+    c->projection.windowWidth = windowWidth;
     return restart(c);
 }
 

@@ -700,21 +700,15 @@ __global__ void majorant_stats_kernel(const float* __restrict__ majorant, size_t
     }
 }
 
-static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebuilt)
+int ensure_ranges(const svr_volume& vol, int cell)
 {
     HostState& st = state();
-    const svr_volume& vol = scene->vol;
-    const svr_transfer_function& tf = scene->tf;
-    if (!vol.tex || !tf.tex) return fail_msg("ensure_grid: volume or transfer function texture is not set");
-
-    cudaResourceDesc vrd, trd;
+    if (!vol.tex) return fail_msg("ensure_ranges: volume texture is not set");
+    cudaResourceDesc vrd;
     SVR_TRY(cudaGetTextureObjectResourceDesc(&vrd, vol.tex));
-    SVR_TRY(cudaGetTextureObjectResourceDesc(&trd, tf.tex));
-    if (vrd.resType != cudaResourceTypeArray || trd.resType != cudaResourceTypeArray)
-        return fail_msg("ensure_grid: textures must be bound to cudaArrays");
-    cudaArray_t varr = vrd.res.array.array, tarr = trd.res.array.array;
+    if (vrd.resType != cudaResourceTypeArray) return fail_msg("ensure_grid: textures must be bound to cudaArrays");
+    cudaArray_t varr = vrd.res.array.array;
 
-    if (majorantsRebuilt) *majorantsRebuilt = false;
     cudaChannelFormatDesc ch;
     cudaExtent ext;
     unsigned int flags = 0;
@@ -741,6 +735,7 @@ static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebu
         }
     }
     st.dev.fingerprintDue = false;
+    if (cell == 0) cell = varr == st.dev.gridArray && st.dev.range.p ? st.dev.gridCell : 8;
     if (varr != st.dev.gridArray || cell != st.dev.gridCell || !st.dev.range.p) {
         // ---- allocate for this (array, cell size)
         release_grid(st);
@@ -751,12 +746,7 @@ static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebu
         st.dev.gridDims = make_int3((st.dev.volDims.x + cell - 1) / cell, (st.dev.volDims.y + cell - 1) / cell,
                                 (st.dev.volDims.z + cell - 1) / cell);
         size_t cells = (size_t)st.dev.gridDims.x * st.dev.gridDims.y * st.dev.gridDims.z;
-        size_t padded = (size_t)(st.dev.gridDims.x + 2) * (st.dev.gridDims.y + 2) * (st.dev.gridDims.z + 2);
         SVR_TRY(st.dev.range.reserve(cells));
-        SVR_TRY(st.dev.majorant.reserve(padded));
-        SVR_TRY(st.dev.dist[0].reserve(padded));
-        SVR_TRY(st.dev.dist[1].reserve(padded));
-        SVR_TRY(st.dev.occ.reserve(6));
         st.dev.gridArray = varr;
         st.dev.gridCell = cell;
         st.dev.rangeValid = false;
@@ -777,6 +767,29 @@ static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebu
         int rc = launch_fingerprint(st, 0);  // of the voxels these ranges describe (stays on the device until it is needed)
         if (rc) return rc;
     }
+    return 0;
+}
+
+static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebuilt)
+{
+    HostState& st = state();
+    const svr_volume& vol = scene->vol;
+    const svr_transfer_function& tf = scene->tf;
+    if (!vol.tex || !tf.tex) return fail_msg("ensure_grid: volume or transfer function texture is not set");
+
+    cudaResourceDesc trd;
+    SVR_TRY(cudaGetTextureObjectResourceDesc(&trd, tf.tex));
+    if (trd.resType != cudaResourceTypeArray) return fail_msg("ensure_grid: textures must be bound to cudaArrays");
+    cudaArray_t tarr = trd.res.array.array;
+
+    if (majorantsRebuilt) *majorantsRebuilt = false;
+    if (int rc = ensure_ranges(vol, cell)) return rc;
+    // the majorant grid and its helpers, for the grid ensure_ranges settled on (release_grid frees them with the ranges)
+    const size_t padded = (size_t)(st.dev.gridDims.x + 2) * (st.dev.gridDims.y + 2) * (st.dev.gridDims.z + 2);
+    SVR_TRY(st.dev.majorant.reserve(padded));
+    SVR_TRY(st.dev.dist[0].reserve(padded));
+    SVR_TRY(st.dev.dist[1].reserve(padded));
+    SVR_TRY(st.dev.occ.reserve(6));
 
     const int leap = st.options[SVR_OPT_LEAP] != 0;
     if (force || !st.dev.majorantValid || st.dev.majorantDensityScale != vol.densityScale || st.dev.majorantTfArray != tarr ||

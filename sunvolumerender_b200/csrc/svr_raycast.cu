@@ -23,17 +23,8 @@ __global__ void __launch_bounds__(256) raycast_kernel(const __grid_constant__ De
                                                       float4* __restrict__ outf, uint32_t y0, uint32_t y1, uint32_t bandPhase,
                                                       uint32_t bandStride, Counters* cnt, const unsigned int* __restrict__ staleGrid)
 {
-    // warp = 8x4 pixel tile; block = 16 pixels wide, 2 warps across.  Row bands of the block's height are dealt out
-    // round robin: this launch renders bands bandPhase, bandPhase + bandStride, ... (1 GPU: phase 0, stride 1)
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t idx = blockIdx.x * 16u + (warp & 1u) * 8u + (lane & 7u);
-    // Bands are issued from the middle of the image outwards: blocks launch in blockIdx order, the camera looks at
-    // the volume's centre (Canvas::ZoomToExtent), so the long rays start first and the short ones fill the tail.
-    const uint32_t nBands = ((y1 - y0) + (blockDim.x >> 4) - 1u) / (blockDim.x >> 4);
-    const uint32_t k = blockIdx.y * bandStride + bandPhase;  // k-th band counted from the middle
-    const uint32_t mid = nBands >> 1;
-    const uint32_t band = (k & 1u) ? mid - ((k + 1u) >> 1) : mid + (k >> 1);
-    const uint32_t idy = y0 + band * (blockDim.x >> 4) + (warp >> 1) * 4u + (lane >> 3);
+    const uint2 pix = band_pixel(y0, y1, bandPhase, bandStride);
+    const uint32_t idx = pix.x, idy = pix.y;
     const bool inside = idx < s.cam.imageW && idy < y1;
     LocalCounters<COUNT> lc;
 

@@ -140,6 +140,23 @@ SVR_DEV Ray camera_ray_center(const svr_camera& c, uint32_t x, uint32_t y)
     return r;
 }
 
+// Pixel of this thread in the image layout of the ray-marching kernels (ray caster, projection): a warp is an 8x4 pixel
+// tile, a block 16 pixels wide (2 warps across) and blockDim/16 rows high.  Row bands of the block's height are dealt out
+// round robin from the middle of the image outwards: this launch renders bands bandPhase, bandPhase + bandStride, ...
+// (1 GPU: phase 0, stride 1).  Blocks launch in blockIdx order and the camera looks at the volume's centre
+// (Canvas::ZoomToExtent), so the long rays start first and the short ones fill the tail.
+SVR_DEV uint2 band_pixel(uint32_t y0, uint32_t y1, uint32_t bandPhase, uint32_t bandStride)
+{
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t idx = blockIdx.x * 16u + (warp & 1u) * 8u + (lane & 7u);
+    const uint32_t nBands = ((y1 - y0) + (blockDim.x >> 4) - 1u) / (blockDim.x >> 4);
+    const uint32_t k = blockIdx.y * bandStride + bandPhase;  // k-th band counted from the middle
+    const uint32_t mid = nBands >> 1;
+    const uint32_t band = (k & 1u) ? mid - ((k + 1u) >> 1) : mid + (k >> 1);
+    const uint32_t idy = y0 + band * (blockDim.x >> 4) + (warp >> 1) * 4u + (lane >> 3);
+    return make_uint2(idx, idy);
+}
+
 // sampling.h:26-32.  EXACT_PI: the reference evaluates 2.f * M_PI * u in double.
 template <bool EXACT_PI>
 SVR_DEV float two_pi_times(float u)

@@ -210,6 +210,11 @@ int fail_msg(const char* msg);
 // ray caster (which only skips empty space with the grid) never gains from cells above 8 voxels.
 int ensure_grid(DevScene* scene, bool force, int maxAutoCell = 32);
 
+// Stage 1 of the macrocell grid alone: the range grid of `vol`'s voxels (dev.range, dev.gridDims, dev.gridCell), which needs
+// no transfer function.  cell = 0: the edge the cache holds for this array, else 8.  A new array or edge releases the whole
+// grid; new voxels (svr_volume_upload, a setup_volume whose array holds other voxels) rebuild the ranges.
+int ensure_ranges(const svr_volume& vol, int cell);
+
 // true when the transfer-function table behind `tf` differs from the one the majorants were built from (one small
 // launch + an 16-byte read-back; the ray caster's drop-in entry point, whose host may edit the table behind an unchanged
 // handle, gui/transferfunction.cpp:128-151).  Also true when no majorants exist yet.

@@ -317,6 +317,19 @@ class Renderer:
                                                      phase, stride, C.byref(rows)), "svr_render_raycasting_bands")
         return int(rows.value)
 
+    def render_projection(self, mode="max", window=(0.5, 1.0), step_size=None, out=None, img_ptr=None, phase=0, stride=1):
+        """Maximum, minimum or average intensity projection (svr_render_projection) of the bound volume from the bound camera:
+        mode "max", "min" or "mean"; window (center, width) maps the projected value to the grey u8 image; out: optional
+        float tensor, one value per pixel.  The u8 image goes to self.img, or to img_ptr, a raw device pointer (e.g.
+        distributed.PeerFrame.img_ptr).  phase / stride: the row bands of render_raycasting_bands.  Returns the band height."""
+        if step_size is None:
+            step_size = S.raycast_step_size(self.volume.spacing.tuple())
+        p = L.ProjectionParams(L.PROJECT_MODES[mode], step_size, window[0], window[1])
+        rows = C.c_uint32(0)
+        L.check(self.lib.svr_render_projection(img_ptr if img_ptr is not None else _ptr(self.img), _ptr(out), C.byref(self.volume), C.byref(self.camera),
+                                               C.byref(p), phase, stride, C.byref(rows)), "svr_render_projection")
+        return int(rows.value)
+
     # ---- results
     def hdr_image(self):
         return self.hdr.view(self.camera.imageH, self.camera.imageW, 3)

@@ -4,7 +4,7 @@
 // render_raycasting -- on the synthetic configurations of SURVEY.md section 8d, times the loop with
 // CUDA events and writes the image as PPM (tone-mapped u8) and PFM (float accumulator).
 //
-//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc] [--spp N] [--depth D] [--batched 0|1]
+//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip] [--window C,W] [--spp N] [--depth D] [--batched 0|1]
 //                [--pt-mode 0|1|2] [--n N --w W --h H] [--out prefix] [--reps R] [--volume file.mhd|.mha] [--tf file.tf|app]
 //                [--interact script.txt]
 // --interact replays an interaction script through the windowless Canvas (include/svr_canvas.h: gui/canvas.cpp's
@@ -15,6 +15,8 @@
 //   denoise 0|1|4|16      (SVR_OPT_PT_DENOISE: the denoised progressive display from the next restart of the render on)
 // The whole script is parsed before the device is touched: a malformed line fails with exit code 2.
 //
+// --mode mip|minip|aip renders the maximum / minimum / average intensity projection (svr_render_projection) with the ray
+// caster's step size, grey through the display window --window C,W (default 0.5,1); the .pfm then holds the projected values.
 // --volume loads a MetaImage file the way Canvas::LoadVolume does (core/VolumeReader.cpp:13-94) instead of
 // generating the configuration's synthetic volume; camera and light are framed on its extent.
 // --tf loads a transfer function saved by the application (gui/transferfunction.cpp:55-88); `app` is the
@@ -150,6 +152,7 @@ int main(int argc, char** argv)
     std::string mode = "pt", out = "svr_out", volumePath, tfPath;
     std::string interactPath;
     int batched = 1, ptMode = 2, reps = 3, sppArg = -1, depthArg = -1;
+    float windowC = 0.5f, windowW = 1.f;
     for (int i = 1; i + 1 < argc; i += 2) {
         std::string k = argv[i], v = argv[i + 1];
         if (k == "--config") {
@@ -170,7 +173,9 @@ int main(int argc, char** argv)
         else if (k == "--tf") tfPath = v;
         else if (k == "--reps") reps = atoi(v.c_str());
         else if (k == "--interact") interactPath = v;
-        else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
+        else if (k == "--window") {
+            if (sscanf(v.c_str(), "%f,%f", &windowC, &windowW) != 2) { fprintf(stderr, "--window wants C,W\n"); return 2; }
+        } else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
     }
     std::vector<std::string> script;
     if (!interactPath.empty()) {
@@ -188,6 +193,7 @@ int main(int argc, char** argv)
             script.push_back(line);
         }
     }
+    const int projMode = mode == "mip" ? SVR_PROJECT_MAX : mode == "minip" ? SVR_PROJECT_MIN : mode == "aip" ? SVR_PROJECT_MEAN : -1;
     if (sppArg > 0) cfg.spp = sppArg;
     if (depthArg >= 0) cfg.depth = depthArg;
     const int W = cfg.w, H = cfg.h;
@@ -301,17 +307,22 @@ int main(int argc, char** argv)
     CK(cudaMemset(rp.hdrBuffer, 0, npix * sizeof(svr_vec3)));
     svr_u8vec4* dImg = nullptr;
     CK(cudaMalloc((void**)&dImg, npix * 4));
+    float* dValue = nullptr;
+    if (projMode >= 0) CK(cudaMalloc((void**)&dValue, npix * sizeof(float)));
 
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
     CK(cudaEventCreate(&e1));
     // VolumeReader::GetElementBoundingSphereRadius (core/VolumeReader.cpp:198-201): half the voxel diagonal
     const float stepSize = 0.5f * sqrtf(vol.spacing.x * vol.spacing.x + vol.spacing.y * vol.spacing.y + vol.spacing.z * vol.spacing.z);
+    const svr_projection_params proj = {projMode, stepSize, windowC, windowW};
     float best = 1e30f;
     for (int rep = 0; rep < reps + 1; ++rep) {  // first pass warms up (and builds the macrocell grid)
         CK(cudaEventRecord(e0, 0));
         if (mode == "rc") {
             render_raycasting(dImg, &vol, &tf, &cam, stepSize);
+        } else if (projMode >= 0) {
+            SVR(svr_render_projection(dImg, dValue, &vol, &cam, &proj, 0, 1, nullptr));
         } else if (batched) {
             rp.frameNo = 0;
             SVR(svr_render_pathtracer_spp(dImg, &rp, (uint32_t)cfg.spp));
@@ -327,9 +338,9 @@ int main(int argc, char** argv)
         CK(cudaEventElapsedTime(&ms, e0, e1));
         if (rep > 0 && ms < best) best = ms;
     }
-    if (mode == "rc")
-        printf("{\"config\": \"%s\", \"mode\": \"rc\", \"ms\": %.4f, \"mrays_per_s\": %.2f, \"launches\": %llu}\n", cfg.name, best,
-               npix / (best * 1e-3) / 1e6, (unsigned long long)svr_launch_count());
+    if (mode == "rc" || projMode >= 0)
+        printf("{\"config\": \"%s\", \"mode\": \"%s\", \"ms\": %.4f, \"mrays_per_s\": %.2f, \"launches\": %llu}\n", cfg.name, mode.c_str(),
+               best, npix / (best * 1e-3) / 1e6, (unsigned long long)svr_launch_count());
     else
         printf("{\"config\": \"%s\", \"mode\": \"pt\", \"pt_mode\": %d, \"batched\": %d, \"spp\": %d, \"depth\": %d, \"ms\": %.4f, "
                "\"msamples_per_s\": %.2f, \"launches\": %llu}\n",
@@ -348,7 +359,16 @@ int main(int argc, char** argv)
             fclose(f);
         }
     }
-    if (mode != "rc") {
+    if (projMode >= 0) {
+        std::vector<float> value(npix);
+        CK(cudaMemcpy(value.data(), dValue, npix * sizeof(float), cudaMemcpyDeviceToHost));
+        FILE* f = fopen((out + ".pfm").c_str(), "wb");
+        if (f) {
+            fprintf(f, "Pf\n%d %d\n-1.0\n", W, H);
+            fwrite(value.data(), sizeof(float), value.size(), f);
+            fclose(f);
+        }
+    } else if (mode != "rc") {
         std::vector<float> hdr(npix * 3);
         CK(cudaMemcpy(hdr.data(), rp.hdrBuffer, npix * 12, cudaMemcpyDeviceToHost));
         FILE* f = fopen((out + ".pfm").c_str(), "wb");
@@ -362,5 +382,6 @@ int main(int argc, char** argv)
     svr_tf_destroy(&tf);
     cudaFree(rp.hdrBuffer);
     cudaFree(dImg);
+    cudaFree(dValue);
     return 0;
 }
