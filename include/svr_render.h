@@ -77,8 +77,9 @@ enum svr_option {
     /* macrocell edge in voxels: 0 (default) = chosen from the scene, about twice the mean free path inside
      * the medium, re-evaluated when volume, transfer function or density scale change; or a power of two in 2..64 */
     SVR_OPT_MACROCELL_SIZE = 3,
-    /* skipping in the two ray-marching kernels: the ray caster's empty-space skipping through the macrocell grid, and the
-     * projection's skipping of cells that cannot change the projected value (svr_render_projection): 0 off, 1 on (default) */
+    /* skipping in the ray-marching kernels: the ray caster's empty-space skipping through the macrocell grid, the
+     * projection's skipping of cells that cannot change the projected value (svr_render_projection) and the isosurface's
+     * skipping of cells below the threshold (svr_render_isosurface): 0 off, 1 on (default) */
     SVR_OPT_RC_SKIP = 4,
     /* Philox key */
     SVR_OPT_SEED = 5,
@@ -362,6 +363,39 @@ typedef struct svr_projection_params {
 } svr_projection_params;
 int svr_render_projection(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_camera* camera,
                           const svr_projection_params* params, uint32_t phase, uint32_t stride, uint32_t* bandRows);
+
+/* Isosurface (DESIGN.md section 7i): the first place along each pixel-centre ray where the volume reaches isoValue, shaded as a
+ * surface with the ray caster's headlight; no transfer function and no setup_* needed.  Rays and samples are
+ * svr_render_projection's: t0 = max(tNear, 0), h = 0.5 * stepSize, K = floor((tFar - t0) / h + 0.5), sample k (0 <= k < K) at
+ * t_k = t0 + (k + 0.5) h with the value v(t_k), v(t) = tex3D(volume, orig + t dir) * densityScale.
+ *   hit:        k* = the smallest k with v_k >= isoValue; none: the ray misses.
+ *   refinement: k* = 0: t_hit = t_0 (half a step past the entry: the cap where a clip plane or the camera cuts the solid).
+ *               k* > 0: lo = t_{k*-1}, hi = t_{k*} (v_lo < isoValue <= v_hi), then 4 bisection steps m = (lo + hi) / 2,
+ *               hi = m if v(m) >= isoValue, else lo = m (v_lo, v_hi follow), then
+ *               t_hit = lo + (hi - lo) (isoValue - v_lo) / (v_hi - v_lo).  x_hit = orig + t_hit dir.
+ *   normal:     g = the ray caster's 6-tap central-difference gradient at x_hit; n = normalize(g) turned to face the ray's
+ *               origin if |g| > 1e-3, else n = 0.
+ *   shading:    l = normalize(cam.pos - x_hit); n != 0: c = |n . l|, s = c^30; n = 0: c = 1, s = 0;
+ *               rgb = min(color c 0.8 + s 0.2, 1).
+ * imgOrNull receives (trunc(255 rgb), 255) for a hit and (0, 0, 0, 0) for a miss; surfaceOrNull (imageW*imageH float4)
+ * receives (n, z) with z = dot(x_hit - cam.pos, -cam.w), the view-space depth of svr_pathtracer_guides, and (0, 0, 0, +inf)
+ * for a miss.  Both are full-frame buffers; phase 0, stride 1 renders the frame, other values the bands of
+ * svr_render_raycasting_bands (*bandRows = the band height; pixels outside the call's bands are not touched).  The divisions
+ * in K and t_hit are fp32 with fast-math rounding (within 2 ulp).
+ * SVR_OPT_RC_SKIP = 1 (default) skips the samples of macrocells whose maximum is below isoValue, from the range grid of
+ * svr_render_projection (SVR_OPT_MACROCELL_SIZE, else the edge already built for that array, else 8); img and surface are
+ * bit-identical either way.  With SVR_OPT_COUNTERS: paths = rays, steps = samples enumerated up to and including k* (K on a
+ * miss), skipped = those of them dropped, shade_taps = those taken (steps = shade_taps + skipped), cells = cell visits; the
+ * 4 refinement and 6 gradient taps of each hit are not counted.
+ * Errors, all reported before any CUDA call: a null volume, camera or params; both outputs null; stepSize not positive or
+ * not finite; isoValue not finite; a colour component not finite or outside [0, 1]; phase >= stride. */
+typedef struct svr_isosurface_params {
+    float isoValue;   /* threshold on tex3D * densityScale */
+    float stepSize;   /* as render_raycasting / svr_render_projection: samples 0.5 * stepSize apart */
+    float color[3];   /* surface colour, each in [0, 1] */
+} svr_isosurface_params;
+int svr_render_isosurface(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrNull, const svr_volume* volume, const svr_camera* camera,
+                          const svr_isosurface_params* params, uint32_t phase, uint32_t stride, uint32_t* bandRows);
 
 /* ---- resource builders (the input contract of the path) ---- */
 enum svr_voxel_format { SVR_VOXEL_U8 = 0, SVR_VOXEL_U16 = 1, SVR_VOXEL_F16 = 2, SVR_VOXEL_F32 = 3 };

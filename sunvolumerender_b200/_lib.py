@@ -114,6 +114,13 @@ assert C.sizeof(ProjectionParams) == 16
 PROJECT_MAX, PROJECT_MIN, PROJECT_MEAN = range(3)
 PROJECT_MODES = {"max": PROJECT_MAX, "min": PROJECT_MIN, "mean": PROJECT_MEAN}
 
+
+class IsosurfaceParams(C.Structure):  # svr_isosurface_params
+    _fields_ = [("isoValue", C.c_float), ("stepSize", C.c_float), ("color", C.c_float * 3)]
+
+
+assert C.sizeof(IsosurfaceParams) == 20
+
 # enum svr_option
 (OPT_PT_MODE, OPT_SHADOW_ESTIMATOR, OPT_ENV_ENABLED, OPT_MACROCELL_SIZE, OPT_RC_SKIP, OPT_SEED, OPT_COUNTERS,
  OPT_PT_BLOCK, OPT_RC_BLOCK, OPT_PT_KERNEL, OPT_PT_ROUNDS, OPT_LEAP, OPT_PT_ENTRY_CACHE, OPT_PT_WARP_PIXELS,
@@ -192,6 +199,8 @@ SIGNATURES = [
     ("svr_grid_info", C.c_int, [C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     ("svr_grid_copy", C.c_int, [_P, _P]),
     ("svr_render_projection", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(Camera), C.POINTER(ProjectionParams), C.c_uint32, C.c_uint32,
+                                        C.POINTER(C.c_uint32)]),
+    ("svr_render_isosurface", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(Camera), C.POINTER(IsosurfaceParams), C.c_uint32, C.c_uint32,
                                         C.POINTER(C.c_uint32)]),
 ]
 

@@ -330,6 +330,20 @@ class Renderer:
                                                C.byref(p), phase, stride, C.byref(rows)), "svr_render_projection")
         return int(rows.value)
 
+    def render_isosurface(self, iso, step_size=None, color=(1.0, 1.0, 1.0), surface=None, img_ptr=None, phase=0, stride=1):
+        """Isosurface (svr_render_isosurface) of the bound volume from the bound camera: the first point along each pixel-centre
+        ray where tex3D * densityScale reaches iso, shaded in color with the ray caster's headlight.  surface: optional float
+        tensor, four values per pixel (normal facing the camera, view-space depth; (0, 0, 0, +inf) where the ray misses).  The
+        u8 image goes to self.img, or to img_ptr, a raw device pointer.  phase / stride: the row bands of
+        render_raycasting_bands.  Returns the band height."""
+        if step_size is None:
+            step_size = S.raycast_step_size(self.volume.spacing.tuple())
+        p = L.IsosurfaceParams(iso, step_size, (C.c_float * 3)(*color))
+        rows = C.c_uint32(0)
+        L.check(self.lib.svr_render_isosurface(img_ptr if img_ptr is not None else _ptr(self.img), _ptr(surface), C.byref(self.volume),
+                                               C.byref(self.camera), C.byref(p), phase, stride, C.byref(rows)), "svr_render_isosurface")
+        return int(rows.value)
+
     # ---- results
     def hdr_image(self):
         return self.hdr.view(self.camera.imageH, self.camera.imageW, 3)

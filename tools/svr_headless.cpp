@@ -4,7 +4,7 @@
 // render_raycasting -- on the synthetic configurations of SURVEY.md section 8d, times the loop with
 // CUDA events and writes the image as PPM (tone-mapped u8) and PFM (float accumulator).
 //
-//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip] [--window C,W] [--spp N] [--depth D] [--batched 0|1]
+//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip|iso] [--window C,W] [--iso V] [--spp N] [--depth D] [--batched 0|1]
 //                [--pt-mode 0|1|2] [--n N --w W --h H] [--out prefix] [--reps R] [--volume file.mhd|.mha] [--tf file.tf|app]
 //                [--interact script.txt]
 // --interact replays an interaction script through the windowless Canvas (include/svr_canvas.h: gui/canvas.cpp's
@@ -17,6 +17,7 @@
 //
 // --mode mip|minip|aip renders the maximum / minimum / average intensity projection (svr_render_projection) with the ray
 // caster's step size, grey through the display window --window C,W (default 0.5,1); the .pfm then holds the projected values.
+// --mode iso renders the white isosurface at --iso V (default 0.5; svr_render_isosurface) with the ray caster's step size.
 // --volume loads a MetaImage file the way Canvas::LoadVolume does (core/VolumeReader.cpp:13-94) instead of
 // generating the configuration's synthetic volume; camera and light are framed on its extent.
 // --tf loads a transfer function saved by the application (gui/transferfunction.cpp:55-88); `app` is the
@@ -152,7 +153,7 @@ int main(int argc, char** argv)
     std::string mode = "pt", out = "svr_out", volumePath, tfPath;
     std::string interactPath;
     int batched = 1, ptMode = 2, reps = 3, sppArg = -1, depthArg = -1;
-    float windowC = 0.5f, windowW = 1.f;
+    float windowC = 0.5f, windowW = 1.f, isoValue = 0.5f;
     for (int i = 1; i + 1 < argc; i += 2) {
         std::string k = argv[i], v = argv[i + 1];
         if (k == "--config") {
@@ -175,6 +176,8 @@ int main(int argc, char** argv)
         else if (k == "--interact") interactPath = v;
         else if (k == "--window") {
             if (sscanf(v.c_str(), "%f,%f", &windowC, &windowW) != 2) { fprintf(stderr, "--window wants C,W\n"); return 2; }
+        } else if (k == "--iso") {
+            if (sscanf(v.c_str(), "%f", &isoValue) != 1) { fprintf(stderr, "--iso wants a value\n"); return 2; }
         } else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
     }
     std::vector<std::string> script;
@@ -316,6 +319,7 @@ int main(int argc, char** argv)
     // VolumeReader::GetElementBoundingSphereRadius (core/VolumeReader.cpp:198-201): half the voxel diagonal
     const float stepSize = 0.5f * sqrtf(vol.spacing.x * vol.spacing.x + vol.spacing.y * vol.spacing.y + vol.spacing.z * vol.spacing.z);
     const svr_projection_params proj = {projMode, stepSize, windowC, windowW};
+    const svr_isosurface_params iso = {isoValue, stepSize, {1.f, 1.f, 1.f}};
     float best = 1e30f;
     for (int rep = 0; rep < reps + 1; ++rep) {  // first pass warms up (and builds the macrocell grid)
         CK(cudaEventRecord(e0, 0));
@@ -323,6 +327,8 @@ int main(int argc, char** argv)
             render_raycasting(dImg, &vol, &tf, &cam, stepSize);
         } else if (projMode >= 0) {
             SVR(svr_render_projection(dImg, dValue, &vol, &cam, &proj, 0, 1, nullptr));
+        } else if (mode == "iso") {
+            SVR(svr_render_isosurface(dImg, nullptr, &vol, &cam, &iso, 0, 1, nullptr));
         } else if (batched) {
             rp.frameNo = 0;
             SVR(svr_render_pathtracer_spp(dImg, &rp, (uint32_t)cfg.spp));
@@ -338,7 +344,7 @@ int main(int argc, char** argv)
         CK(cudaEventElapsedTime(&ms, e0, e1));
         if (rep > 0 && ms < best) best = ms;
     }
-    if (mode == "rc" || projMode >= 0)
+    if (mode == "rc" || mode == "iso" || projMode >= 0)
         printf("{\"config\": \"%s\", \"mode\": \"%s\", \"ms\": %.4f, \"mrays_per_s\": %.2f, \"launches\": %llu}\n", cfg.name, mode.c_str(),
                best, npix / (best * 1e-3) / 1e6, (unsigned long long)svr_launch_count());
     else
@@ -368,7 +374,7 @@ int main(int argc, char** argv)
             fwrite(value.data(), sizeof(float), value.size(), f);
             fclose(f);
         }
-    } else if (mode != "rc") {
+    } else if (mode != "rc" && mode != "iso") {
         std::vector<float> hdr(npix * 3);
         CK(cudaMemcpy(hdr.data(), rp.hdrBuffer, npix * 12, cudaMemcpyDeviceToHost));
         FILE* f = fopen((out + ".pfm").c_str(), "wb");
