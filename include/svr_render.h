@@ -79,7 +79,8 @@ enum svr_option {
     SVR_OPT_MACROCELL_SIZE = 3,
     /* skipping in the ray-marching kernels: the ray caster's empty-space skipping through the macrocell grid, the
      * projection's skipping of cells that cannot change the projected value (svr_render_projection) and the isosurface's
-     * skipping of cells below the threshold (svr_render_isosurface): 0 off, 1 on (default) */
+     * skipping of cells below the threshold (svr_render_isosurface), and the same projection skipping across a thick slab
+     * (svr_render_slices): 0 off, 1 on (default) */
     SVR_OPT_RC_SKIP = 4,
     /* Philox key */
     SVR_OPT_SEED = 5,
@@ -396,6 +397,42 @@ typedef struct svr_isosurface_params {
 } svr_isosurface_params;
 int svr_render_isosurface(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrNull, const svr_volume* volume, const svr_camera* camera,
                           const svr_isosurface_params* params, uint32_t phase, uint32_t stride, uint32_t* bandRows);
+
+/* Slices (DESIGN.md section 7j): a stack of `count` planar images of the volume, imageW x imageH each, in parallel projection:
+ * thin slices (multi-planar reformatting: axial, coronal, sagittal or oblique) or thick slabs projected along the plane's
+ * normal with svr_projection_mode; no transfer function, no camera and no setup_* needed.  In fp32:
+ *   pixel centre: c = center + (x + 1/2 - W/2) axisU + (y + 1/2 - H/2) axisV + j axisW   (slice j, pixel (x, y))
+ *   slab:         n = normalize(cross(axisU, axisV)); h = sampleSpacing; K = thickness > 0 ? max(1, floor(thickness / h + 1/2)) : 1;
+ *                 t0 = -K h / 2; sample k (0 <= k < K) at x_k = c + s_k n, s_k = t0 + (k + 1/2) h (from k, as the projection
+ *                 computes its samples).  A thin slice (thickness 0) is K = 1 with s_0 = 0: x_0 = c.
+ *   value:        v_k = tex3D(volume, x_k) * densityScale (the hardware trilinear fetch).
+ *   inclusion:    sample k is included iff cmin <= x_k <= cmax componentwise, cmin = vmin * (-x_clip.x, -y_clip.x, -z_clip.x),
+ *                 cmax = vmax * (x_clip.y, y_clip.y, z_clip.y) (the clipped box of the projection).  Each component of x_k is
+ *                 monotone in k, so the included samples are one index range [kLo, kHi), found by binary search.
+ *   P:            MAX: max v_k; MIN: min v_k; MEAN: (fp32 sum in k order) / (kHi - kLo), over the included samples; 0 if none.
+ * valueOrNull receives P at [(j * imageH + y) * imageW + x] (count * imageH * imageW floats); imgOrNull the grey image of
+ * svr_render_projection (trunc(255 g) in r, g, b, alpha 255), and (0, 0, 0, 0) for a pixel with no included sample, so
+ * "outside the volume" differs from "below the window".  The divisions in MEAN and g are svr_render_projection's.
+ * SVR_OPT_RC_SKIP = 1 (default) walks slabs with K > 1 through svr_render_projection's range grid and drops samples by its
+ * per-mode rules; P is bit-identical either way.  A thin slice takes its one fetch and never walks.  With SVR_OPT_COUNTERS:
+ * paths = pixels * slices, steps = included samples, skipped = those dropped, shade_taps = those fetched
+ * (steps = shade_taps + skipped), cells = cell visits.  SVR_OPT_RC_BLOCK sets the threads per block.
+ * Errors, all reported before any CUDA call: a null volume or params; both outputs null; axisU or axisV not finite, or
+ * cross(axisU, axisV) zero or not finite; axisW not finite when count > 1; imageW or imageH 0 or above 16384; count 0 or above
+ * 65535; a mode out of range; thickness negative or not finite; sampleSpacing not positive or not finite while thickness > 0;
+ * thickness / sampleSpacing above 65536; windowWidth not positive or not finite; windowCenter not finite. */
+typedef struct svr_slice_params {
+    float center[3];        /* world position of the centre of slice 0 */
+    float axisU[3];         /* world step from a pixel to the next one in its row (x + 1) */
+    float axisV[3];         /* world step from a row to the next (y + 1) */
+    float axisW[3];         /* world step from a slice to the next (j + 1); ignored when count == 1 */
+    uint32_t imageW, imageH, count;
+    int32_t mode;           /* svr_projection_mode across the slab */
+    float thickness;        /* slab thickness along n = normalize(cross(axisU, axisV)), world units; 0 = a thin slice */
+    float sampleSpacing;    /* world distance between slab samples; used when thickness > 0 */
+    float windowCenter, windowWidth;
+} svr_slice_params;
+int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_slice_params* params);
 
 /* ---- resource builders (the input contract of the path) ---- */
 enum svr_voxel_format { SVR_VOXEL_U8 = 0, SVR_VOXEL_U16 = 1, SVR_VOXEL_F16 = 2, SVR_VOXEL_F32 = 3 };

@@ -121,6 +121,15 @@ class IsosurfaceParams(C.Structure):  # svr_isosurface_params
 
 assert C.sizeof(IsosurfaceParams) == 20
 
+
+class SliceParams(C.Structure):  # svr_slice_params
+    _fields_ = [("center", C.c_float * 3), ("axisU", C.c_float * 3), ("axisV", C.c_float * 3), ("axisW", C.c_float * 3),
+                ("imageW", C.c_uint32), ("imageH", C.c_uint32), ("count", C.c_uint32), ("mode", C.c_int32), ("thickness", C.c_float),
+                ("sampleSpacing", C.c_float), ("windowCenter", C.c_float), ("windowWidth", C.c_float)]
+
+
+assert C.sizeof(SliceParams) == 80
+
 # enum svr_option
 (OPT_PT_MODE, OPT_SHADOW_ESTIMATOR, OPT_ENV_ENABLED, OPT_MACROCELL_SIZE, OPT_RC_SKIP, OPT_SEED, OPT_COUNTERS,
  OPT_PT_BLOCK, OPT_RC_BLOCK, OPT_PT_KERNEL, OPT_PT_ROUNDS, OPT_LEAP, OPT_PT_ENTRY_CACHE, OPT_PT_WARP_PIXELS,
@@ -202,6 +211,7 @@ SIGNATURES = [
                                         C.POINTER(C.c_uint32)]),
     ("svr_render_isosurface", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(Camera), C.POINTER(IsosurfaceParams), C.c_uint32, C.c_uint32,
                                         C.POINTER(C.c_uint32)]),
+    ("svr_render_slices", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(SliceParams)]),
 ]
 
 

@@ -344,6 +344,18 @@ class Renderer:
                                                C.byref(self.camera), C.byref(p), phase, stride, C.byref(rows)), "svr_render_isosurface")
         return int(rows.value)
 
+    def render_slices(self, params, value=None, img=None):
+        """Slices or slabs (svr_render_slices) of the bound volume; params: an L.SliceParams (scene.axis_slice,
+        scene.oblique_slice).  value: float32 (count, H, W) and img: uint8 (count, H, W, 4) device tensors, allocated when not
+        given.  Returns (value, img)."""
+        shape = (params.count, params.imageH, params.imageW)
+        if value is None:
+            value = torch.empty(shape, dtype=torch.float32, device=self.device)
+        if img is None:
+            img = torch.empty(shape + (4,), dtype=torch.uint8, device=self.device)
+        L.check(self.lib.svr_render_slices(_ptr(img), _ptr(value), C.byref(self.volume), C.byref(params)), "svr_render_slices")
+        return value, img
+
     # ---- results
     def hdr_image(self):
         return self.hdr.view(self.camera.imageH, self.camera.imageW, 3)

@@ -195,6 +195,57 @@ def host_volume_struct(n_xyz, spacing=(1.0, 1.0, 1.0), max_grad_mag=1.0):
     return v
 
 
+# slice orientations (svr_render_slices): the world axes of a pixel row (U) and of a row step (V) per slice normal axis
+_SLICE_AXES = {"z": (0, 1), "y": (0, 2), "x": (1, 2)}  # axial, coronal, sagittal
+
+
+def axis_slice(dims, spacing, axis, index, thickness_voxels=0, count=1, mode="max", window=(0.5, 1.0)):
+    """svr_slice_params of an axial (axis "z": U = +x, V = +y), coronal ("y": U = +x, V = +z) or sagittal ("x": U = +y,
+    V = +z) slice through voxel `index` of a dims (x, y, z) volume with the given spacing (the box of host_volume_struct,
+    centred on the origin).  Pixel centres lie on voxel centres; a stack of `count` slices advances one voxel per slice.  A
+    slab of thickness_voxels > 0 voxels is projected with `mode` and a sample spacing of one voxel, centred on the slice."""
+    a = "xyz".index(axis)
+    iu, iv = _SLICE_AXES[axis]
+    sp = [np.float32(x) for x in spacing]
+    p = L.SliceParams()
+    center = [0.0, 0.0, 0.0]
+    center[a] = float((np.float32(index) + np.float32(0.5) - np.float32(0.5) * np.float32(dims[a])) * sp[a])
+    p.center[:] = center
+    p.axisU[:] = [float(sp[iu]) if i == iu else 0.0 for i in range(3)]
+    p.axisV[:] = [float(sp[iv]) if i == iv else 0.0 for i in range(3)]
+    p.axisW[:] = [float(sp[a]) if i == a else 0.0 for i in range(3)]
+    p.imageW, p.imageH, p.count = int(dims[iu]), int(dims[iv]), int(count)
+    p.mode = L.PROJECT_MODES[mode]
+    p.thickness = float(np.float32(thickness_voxels) * sp[a])
+    p.sampleSpacing = float(sp[a])
+    p.windowCenter, p.windowWidth = window
+    return p
+
+
+def oblique_slice(center, normal, up, pixel_size, image_w, image_h, count=1, slice_step=None, thickness=0.0, sample_spacing=None,
+                  mode="max", window=(0.5, 1.0)):
+    """svr_slice_params of a slice centred on `center` with the given normal: U = pixel_size * normalize(cross(up, normal)),
+    V = pixel_size * cross(normalize(normal), normalize(U)), so cross(U, V) points along the normal and V along the part of
+    `up` across it.  A stack steps slice_step (default pixel_size) along the normal; a slab of `thickness` world units is
+    sampled every sample_spacing (default pixel_size)."""
+    n = np.asarray(normal, np.float64)
+    n = n / np.linalg.norm(n)
+    u = np.cross(np.asarray(up, np.float64), n)
+    u = u / np.linalg.norm(u)
+    v = np.cross(n, u)
+    p = L.SliceParams()
+    p.center[:] = [float(x) for x in center]
+    p.axisU[:] = [float(x) for x in pixel_size * u]
+    p.axisV[:] = [float(x) for x in pixel_size * v]
+    p.axisW[:] = [float(x) for x in (pixel_size if slice_step is None else slice_step) * n]
+    p.imageW, p.imageH, p.count = int(image_w), int(image_h), int(count)
+    p.mode = L.PROJECT_MODES[mode]
+    p.thickness = float(thickness)
+    p.sampleSpacing = float(pixel_size if sample_spacing is None else sample_spacing)
+    p.windowCenter, p.windowWidth = window
+    return p
+
+
 @dataclass
 class Config:
     """One BASELINE.json configuration."""

@@ -1,0 +1,41 @@
+"""TEST INFRASTRUCTURE -- the CPU restatement of svr_render_slices (tests/slice_oracle.cpp, on the CPU oracle's texture
+filter), compiled on first use into a temporary directory."""
+import ctypes as C
+import os
+import subprocess
+import tempfile
+
+import numpy as np
+
+from oracle import binding as B
+from sunvolumerender_b200 import _lib as L
+from sunvolumerender_b200 import scene as S
+
+SRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "slice_oracle.cpp")
+_lib = None
+
+
+def lib():
+    global _lib
+    if _lib is None:
+        out = os.path.join(tempfile.mkdtemp(prefix="svr_slice_oracle_"), "libsvr_slice_oracle.so")
+        # the flags of oracle/Makefile's cpu target (the distro compiler: it has libgomp)
+        subprocess.check_call(["/usr/bin/g++", "-O3", "-fopenmp", "-fno-fast-math", "-shared", "-fPIC", "-o", out, SRC])
+        lib_ = C.CDLL(out)
+        lib_.svr_oracle_slices.argtypes = [C.POINTER(B.OracleScene), C.POINTER(L.SliceParams), C.c_void_p, C.c_void_p]
+        _lib = lib_
+    return _lib
+
+
+def oracle(voxels, fmt, dims, volume):
+    """A CpuOracle scene for slices (no transfer function or camera is used: a zero table and a default camera stand in)."""
+    return B.CpuOracle(voxels, fmt, dims, volume, np.zeros((2, 4), np.float32), S.default_camera(dims, 8, 8))
+
+
+def slices(orc, params):
+    """(value (count, H, W) float32, u8 (count, H, W, 4))."""
+    shape = (params.count, params.imageH, params.imageW)
+    value = np.zeros(shape, np.float32)
+    u8 = np.zeros(shape + (4,), np.uint8)
+    lib().svr_oracle_slices(C.byref(orc.scene), C.byref(params), value.ctypes.data, u8.ctypes.data)
+    return value, u8

@@ -4,7 +4,8 @@
 // render_raycasting -- on the synthetic configurations of SURVEY.md section 8d, times the loop with
 // CUDA events and writes the image as PPM (tone-mapped u8) and PFM (float accumulator).
 //
-//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip|iso] [--window C,W] [--iso V] [--spp N] [--depth D] [--batched 0|1]
+//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip|iso|slice] [--window C,W] [--iso V] [--axis x|y|z --index I --slab N]
+//                [--spp N] [--depth D] [--batched 0|1]
 //                [--pt-mode 0|1|2] [--n N --w W --h H] [--out prefix] [--reps R] [--volume file.mhd|.mha] [--tf file.tf|app]
 //                [--interact script.txt]
 // --interact replays an interaction script through the windowless Canvas (include/svr_canvas.h: gui/canvas.cpp's
@@ -18,6 +19,9 @@
 // --mode mip|minip|aip renders the maximum / minimum / average intensity projection (svr_render_projection) with the ray
 // caster's step size, grey through the display window --window C,W (default 0.5,1); the .pfm then holds the projected values.
 // --mode iso renders the white isosurface at --iso V (default 0.5; svr_render_isosurface) with the ray caster's step size.
+// --mode slice renders the --w x --h slice (svr_render_slices) normal to --axis (default z: axial; y coronal, x sagittal) through
+// voxel --index (default the middle one), one voxel per pixel, centred on the volume in the plane and oriented as
+// scene.axis_slice; --slab N makes it the MIP of a slab of N voxels (one sample per voxel), grey through --window.
 // --volume loads a MetaImage file the way Canvas::LoadVolume does (core/VolumeReader.cpp:13-94) instead of
 // generating the configuration's synthetic volume; camera and light are framed on its extent.
 // --tf loads a transfer function saved by the application (gui/transferfunction.cpp:55-88); `app` is the
@@ -154,6 +158,7 @@ int main(int argc, char** argv)
     std::string interactPath;
     int batched = 1, ptMode = 2, reps = 3, sppArg = -1, depthArg = -1;
     float windowC = 0.5f, windowW = 1.f, isoValue = 0.5f;
+    int sliceAxis = 2, sliceIndex = -1, slab = 0;
     for (int i = 1; i + 1 < argc; i += 2) {
         std::string k = argv[i], v = argv[i + 1];
         if (k == "--config") {
@@ -178,7 +183,12 @@ int main(int argc, char** argv)
             if (sscanf(v.c_str(), "%f,%f", &windowC, &windowW) != 2) { fprintf(stderr, "--window wants C,W\n"); return 2; }
         } else if (k == "--iso") {
             if (sscanf(v.c_str(), "%f", &isoValue) != 1) { fprintf(stderr, "--iso wants a value\n"); return 2; }
-        } else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
+        } else if (k == "--axis") {
+            if (v != "x" && v != "y" && v != "z") { fprintf(stderr, "--axis wants x, y or z\n"); return 2; }
+            sliceAxis = v[0] - 'x';
+        } else if (k == "--index") sliceIndex = atoi(v.c_str());
+        else if (k == "--slab") slab = atoi(v.c_str());
+        else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
     }
     std::vector<std::string> script;
     if (!interactPath.empty()) {
@@ -209,11 +219,13 @@ int main(int argc, char** argv)
 
     // ---- Canvas::LoadVolume (gui/canvas.cpp:27-41) with a synthetic volume instead of a MetaImage file
     svr_volume vol;
+    uint32_t dims[3] = {(uint32_t)N, (uint32_t)N, (uint32_t)N};
     if (!volumePath.empty()) {
         svr_volume_stats vs;
         SVR(svr_volume_load_metaimage(volumePath.c_str(), &vol, &vs, nullptr, 0));
         const float ex = vs.dim[0] * vs.spacing[0], ey = vs.dim[1] * vs.spacing[1], ez = vs.dim[2] * vs.spacing[2];
         N = (int)fmaxf(ex, fmaxf(ey, ez));  // the extent the camera and the light are framed on (gui/canvas.cpp:191-197)
+        for (int a = 0; a < 3; ++a) dims[a] = vs.dim[a];
         fprintf(stderr, "loaded %s: %u x %u x %u, spacing %g %g %g, range [%g, %g], max |grad| %g, %u histogram bins\n", volumePath.c_str(),
                 vs.dim[0], vs.dim[1], vs.dim[2], vs.spacing[0], vs.spacing[1], vs.spacing[2], vs.data_min, vs.data_max,
                 vs.max_gradient_magnitude, vs.histogram_bins);
@@ -311,7 +323,7 @@ int main(int argc, char** argv)
     svr_u8vec4* dImg = nullptr;
     CK(cudaMalloc((void**)&dImg, npix * 4));
     float* dValue = nullptr;
-    if (projMode >= 0) CK(cudaMalloc((void**)&dValue, npix * sizeof(float)));
+    if (projMode >= 0 || mode == "slice") CK(cudaMalloc((void**)&dValue, npix * sizeof(float)));
 
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
@@ -320,6 +332,26 @@ int main(int argc, char** argv)
     const float stepSize = 0.5f * sqrtf(vol.spacing.x * vol.spacing.x + vol.spacing.y * vol.spacing.y + vol.spacing.z * vol.spacing.z);
     const svr_projection_params proj = {projMode, stepSize, windowC, windowW};
     const svr_isosurface_params iso = {isoValue, stepSize, {1.f, 1.f, 1.f}};
+    svr_slice_params slice;
+    memset(&slice, 0, sizeof(slice));
+    {
+        static const int kU[3] = {1, 0, 0}, kV[3] = {2, 2, 1};  // sagittal U = +y, V = +z; coronal U = +x, V = +z; axial U = +x, V = +y
+        const float sp[3] = {vol.spacing.x, vol.spacing.y, vol.spacing.z};
+        const int a = sliceAxis;
+        const int index = sliceIndex >= 0 ? sliceIndex : (int)dims[a] / 2;
+        slice.center[a] = ((float)index + 0.5f - 0.5f * (float)dims[a]) * sp[a];
+        slice.axisU[kU[a]] = sp[kU[a]];
+        slice.axisV[kV[a]] = sp[kV[a]];
+        slice.axisW[a] = sp[a];
+        slice.imageW = (uint32_t)W;
+        slice.imageH = (uint32_t)H;
+        slice.count = 1;
+        slice.mode = SVR_PROJECT_MAX;
+        slice.thickness = (float)slab * sp[a];
+        slice.sampleSpacing = sp[a];
+        slice.windowCenter = windowC;
+        slice.windowWidth = windowW;
+    }
     float best = 1e30f;
     for (int rep = 0; rep < reps + 1; ++rep) {  // first pass warms up (and builds the macrocell grid)
         CK(cudaEventRecord(e0, 0));
@@ -329,6 +361,8 @@ int main(int argc, char** argv)
             SVR(svr_render_projection(dImg, dValue, &vol, &cam, &proj, 0, 1, nullptr));
         } else if (mode == "iso") {
             SVR(svr_render_isosurface(dImg, nullptr, &vol, &cam, &iso, 0, 1, nullptr));
+        } else if (mode == "slice") {
+            SVR(svr_render_slices(dImg, dValue, &vol, &slice));
         } else if (batched) {
             rp.frameNo = 0;
             SVR(svr_render_pathtracer_spp(dImg, &rp, (uint32_t)cfg.spp));
@@ -344,7 +378,7 @@ int main(int argc, char** argv)
         CK(cudaEventElapsedTime(&ms, e0, e1));
         if (rep > 0 && ms < best) best = ms;
     }
-    if (mode == "rc" || mode == "iso" || projMode >= 0)
+    if (mode == "rc" || mode == "iso" || mode == "slice" || projMode >= 0)
         printf("{\"config\": \"%s\", \"mode\": \"%s\", \"ms\": %.4f, \"mrays_per_s\": %.2f, \"launches\": %llu}\n", cfg.name, mode.c_str(),
                best, npix / (best * 1e-3) / 1e6, (unsigned long long)svr_launch_count());
     else
@@ -365,7 +399,7 @@ int main(int argc, char** argv)
             fclose(f);
         }
     }
-    if (projMode >= 0) {
+    if (projMode >= 0 || mode == "slice") {
         std::vector<float> value(npix);
         CK(cudaMemcpy(value.data(), dValue, npix * sizeof(float), cudaMemcpyDeviceToHost));
         FILE* f = fopen((out + ".pfm").c_str(), "wb");
@@ -374,7 +408,7 @@ int main(int argc, char** argv)
             fwrite(value.data(), sizeof(float), value.size(), f);
             fclose(f);
         }
-    } else if (mode != "rc" && mode != "iso") {
+    } else if (mode != "rc" && mode != "iso" && mode != "slice") {
         std::vector<float> hdr(npix * 3);
         CK(cudaMemcpy(hdr.data(), rp.hdrBuffer, npix * 12, cudaMemcpyDeviceToHost));
         FILE* f = fopen((out + ".pfm").c_str(), "wb");
