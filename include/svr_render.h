@@ -80,7 +80,7 @@ enum svr_option {
     /* skipping in the ray-marching kernels: the ray caster's empty-space skipping through the macrocell grid, the
      * projection's skipping of cells that cannot change the projected value (svr_render_projection) and the isosurface's
      * skipping of cells below the threshold (svr_render_isosurface), and the same projection skipping across a thick slab
-     * (svr_render_slices): 0 off, 1 on (default) */
+     * (svr_render_slices; svr_render_curved for slabs of 32 samples or more): 0 off, 1 on (default) */
     SVR_OPT_RC_SKIP = 4,
     /* Philox key */
     SVR_OPT_SEED = 5,
@@ -433,6 +433,63 @@ typedef struct svr_slice_params {
     float windowCenter, windowWidth;
 } svr_slice_params;
 int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_slice_params* params);
+
+/* Curved planar reformation (DESIGN.md section 7k): images of the volume along a centerline, for tubular structures (vessels,
+ * airways, colon, spinal canal, dental arch).  `points` is a host array of nPoints xyz triples in world coordinates, a
+ * polyline (callers pass a dense one: no spline is fitted).
+ * Frame rule, on the host in double precision, the results rounded to float:
+ *   1. every point equal to its predecessor is dropped; at least 2 points must remain, P_0 .. P_{M-1}.  S_0 = 0,
+ *      S_{m+1} = S_m + |P_{m+1} - P_m|, L = S_{M-1}.
+ *   2. c(s), s in [0, L], is linear on segment m, the last m <= M - 2 with S_m <= s: P_m + ((s - S_m) / (S_{m+1} - S_m)) (P_{m+1} - P_m).
+ *   3. station i lies at s_i = (i + 1/2) stationSpacing, c_i = c(s_i); it is valid iff s_i <= L.  The valid stations are a prefix.
+ *   4. t_i = normalize(c(min(s_i + D, L)) - c(max(s_i - D, 0))), D = stationSpacing; where that difference is zero (a curve
+ *      that doubles back), the direction of the segment of s_i (rule 2).
+ *   5. the rotation-minimising frame by double reflection (Wang, Juttler, Zheng and Liu 2008): r_0 = normalize(up - (up.t_0) t_0);
+ *      r_{i+1} from r_i: v1 = c_{i+1} - c_i, r^L = r_i - (2 / v1.v1)(v1.r_i) v1, t^L = t_i - (2 / v1.v1)(v1.t_i) v1;
+ *      v2 = t_{i+1} - t^L, r' = r^L - (2 / v2.v2)(v2.r^L) v2 (a zero v1 or v2 skips its reflection); r_{i+1} =
+ *      normalize(r' - (r'.t_{i+1}) t_{i+1}).  b_i = t_i x r_i.
+ *   6. an invalid station has zero vectors and valid = 0.
+ * svr_curve_frames writes, per station, 4 svr_vec4: (c, valid), (t, 0), (r, 0), (b, 0).  It makes no CUDA call: a viewer maps
+ * a CPR pixel back to a world position with it.
+ * Pixel rule, fp32 on the device (fx = (x + 1/2) - W/2, fy = (y + 1/2) - H/2, ps = pixelSpacing):
+ *   straightened (SVR_CURVED_STRAIGHTENED): N = imageH stations, row y is station y; image j (0 <= j < count) has
+ *     theta_j = angle0 + j angleStep, (cos theta_j, sin theta_j) computed in double on the host and rounded to float.
+ *     a = cos r + sin b, n = cos b - sin r (= t x a); pixel (x, y) of image j is at p = c_y + (fx ps) a; the slab runs along n.
+ *     count > 1 is the rotational CPR stack.
+ *   cross-sections (SVR_CURVED_CROSS): N = count stations, image j is station j, theta = angle0 (angleStep is ignored);
+ *     a = cos r + sin b, e = cos b - sin r (= t x a); p = c_j + (fx ps) a + (fy ps) e; the slab runs along t (= a x e).
+ *   slab, inclusion, fold and outputs: those of svr_render_slices on the ray (p, n) or (p, t): K, t0, s_k from k, the clipped
+ *     box, the one index range [kLo, kHi), MAX / MIN / MEAN, the window, value[(j * imageH + y) * imageW + x], and alpha 0 for
+ *     a pixel with no included sample.  A pixel of an invalid station gets P = 0 and alpha 0.
+ * Counters as for svr_render_slices.  SVR_OPT_RC_SKIP = 1 (default) walks slabs with K >= 32 through the range grid with
+ * svr_render_slices' rules (shorter slabs are faster without the walk, DESIGN.md section 7k); thin images and shorter slabs
+ * never walk.  P is bit-identical with skipping on and off.  The frames and the (cos, sin) table go to the device through a library-owned
+ * pinned staging buffer; a call waits on the host only for the copy that last read that buffer.
+ * Errors, all reported before any CUDA call: a null volume, params or points; both outputs null; nPoints below 2 or above
+ * 2^20; a point not finite; fewer than 2 distinct points; up not finite, zero, or parallel to t_0
+ * (|up - (up.t_0) t_0| <= 1e-6 |up|); no valid station (the curve is shorter than half a station); layout out of range;
+ * imageW or imageH 0 or above 16384; count 0 or above 65535; mode out of range; pixelSpacing or stationSpacing not positive or
+ * not finite; angle0 or angleStep not finite; and the thickness, sampleSpacing and window errors of svr_render_slices.
+ * svr_curve_frames makes the same checks on its arguments (a null up or hostFrames, or nStations 0, is an error). */
+enum svr_curved_layout { SVR_CURVED_STRAIGHTENED = 0, SVR_CURVED_CROSS = 1 };
+typedef struct svr_curved_params {
+    float up[3];             /* fixes the roll of the frame at station 0 */
+    int32_t layout;          /* svr_curved_layout */
+    uint32_t imageW, imageH, count;
+    int32_t mode;            /* svr_projection_mode across the slab */
+    float pixelSpacing;      /* world distance between neighbouring pixels across the curve */
+    float stationSpacing;    /* arc length between stations */
+    float angle0, angleStep; /* radians, about the tangent */
+    float thickness;         /* slab thickness, world units; 0 = thin */
+    float sampleSpacing;     /* used when thickness > 0 */
+    float windowCenter, windowWidth;
+} svr_curved_params;
+
+/* host only, no CUDA call: the frames of nStations stations, 4 svr_vec4 each: (c, valid), (t, 0), (r, 0), (b, 0) */
+int svr_curve_frames(const float* points, uint32_t nPoints, const float up[3], float stationSpacing, uint32_t nStations,
+                     svr_vec4* hostFrames);
+int svr_render_curved(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_curved_params* params,
+                      const float* points, uint32_t nPoints);
 
 /* ---- resource builders (the input contract of the path) ---- */
 enum svr_voxel_format { SVR_VOXEL_U8 = 0, SVR_VOXEL_U16 = 1, SVR_VOXEL_F16 = 2, SVR_VOXEL_F32 = 3 };

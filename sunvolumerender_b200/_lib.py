@@ -130,6 +130,20 @@ class SliceParams(C.Structure):  # svr_slice_params
 
 assert C.sizeof(SliceParams) == 80
 
+
+class CurvedParams(C.Structure):  # svr_curved_params
+    _fields_ = [("up", C.c_float * 3), ("layout", C.c_int32), ("imageW", C.c_uint32), ("imageH", C.c_uint32), ("count", C.c_uint32),
+                ("mode", C.c_int32), ("pixelSpacing", C.c_float), ("stationSpacing", C.c_float), ("angle0", C.c_float),
+                ("angleStep", C.c_float), ("thickness", C.c_float), ("sampleSpacing", C.c_float), ("windowCenter", C.c_float),
+                ("windowWidth", C.c_float)]
+
+
+assert C.sizeof(CurvedParams) == 64
+
+# enum svr_curved_layout
+CURVED_STRAIGHTENED, CURVED_CROSS = 0, 1
+CURVED_LAYOUTS = {"straightened": CURVED_STRAIGHTENED, "cross": CURVED_CROSS}
+
 # enum svr_option
 (OPT_PT_MODE, OPT_SHADOW_ESTIMATOR, OPT_ENV_ENABLED, OPT_MACROCELL_SIZE, OPT_RC_SKIP, OPT_SEED, OPT_COUNTERS,
  OPT_PT_BLOCK, OPT_RC_BLOCK, OPT_PT_KERNEL, OPT_PT_ROUNDS, OPT_LEAP, OPT_PT_ENTRY_CACHE, OPT_PT_WARP_PIXELS,
@@ -212,6 +226,8 @@ SIGNATURES = [
     ("svr_render_isosurface", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(Camera), C.POINTER(IsosurfaceParams), C.c_uint32, C.c_uint32,
                                         C.POINTER(C.c_uint32)]),
     ("svr_render_slices", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(SliceParams)]),
+    ("svr_curve_frames", C.c_int, [_P, C.c_uint32, _P, C.c_float, C.c_uint32, _P]),
+    ("svr_render_curved", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(CurvedParams), _P, C.c_uint32]),
 ]
 
 

@@ -79,6 +79,11 @@ void DeviceState::reset()
         for (cudaEvent_t e : aheadEv) cudaEventDestroy(e);  // events belong to the device they were created on
     if (tfCheckEvent) cudaEventDestroy(tfCheckEvent);
     if (hMailbox) cudaFreeHost(hMailbox);
+    if (curveStageEvent) {
+        cudaEventSynchronize(curveStageEvent);  // the copy that last read the staging buffer may still be in flight
+        cudaEventDestroy(curveStageEvent);
+    }
+    if (curveStage) cudaFreeHost(curveStage);
     *this = DeviceState();  // the DevBufs swapped out here free themselves
 }
 

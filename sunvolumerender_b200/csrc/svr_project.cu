@@ -1,6 +1,7 @@
 // svr_project.cu -- maximum, minimum and average intensity projection (svr_render_projection), the isosurface
-// (svr_render_isosurface), which samples the volume the same way (iso_kernel), and slices and slabs (svr_render_slices), which
-// fold samples along a plane's normal as the projection folds them along a camera ray (slice_kernel).
+// (svr_render_isosurface), which samples the volume the same way (iso_kernel), slices and slabs (svr_render_slices), which
+// fold samples along a plane's normal as the projection folds them along a camera ray (slice_kernel), and the curved planar
+// reformation (svr_render_curved), which folds them along rays set by a frame per station of a centerline (curved_kernel).
 //
 // The reference has no projection mode; the sampling rule is this library's own (include/svr_render.h).  Per pixel-centre
 // ray, clipped to the volume box and its clip planes and to t >= 0: K = floor((tFar - t0) / h + 1/2) samples at
@@ -21,6 +22,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <vector>
 
 #include "svr_state.h"
 
@@ -309,9 +311,58 @@ __global__ void __launch_bounds__(256) iso_kernel(const __grid_constant__ ProjSc
     if (surface) surface[offset] = surf;
 }
 
+// The clipped box [cmin, cmax] turned so that the samples of a ray along dir move up it: per component sg = -1 where
+// dir < 0, else +1, and sg x in [lo, hi] (lo = sg cmin, hi = sg cmax, swapped where sg = -1) iff x in [cmin, cmax].
+struct TurnedBox {
+    float3 sg, lo, hi;
+};
+
+SVR_HD float turned_sign(float d) { return d < 0.f ? -1.f : 1.f; }
+
+SVR_HD TurnedBox turn_box(float3 dir, float3 cmin, float3 cmax)
+{
+    TurnedBox b;
+    b.sg = f3(turned_sign(dir.x), turned_sign(dir.y), turned_sign(dir.z));
+    b.lo = f3(dir.x < 0.f ? -cmax.x : cmin.x, dir.y < 0.f ? -cmax.y : cmin.y, dir.z < 0.f ? -cmax.z : cmin.z);
+    b.hi = f3(dir.x < 0.f ? -cmin.x : cmax.x, dir.y < 0.f ? -cmin.y : cmax.y, dir.z < 0.f ? -cmin.z : cmax.z);
+    return b;
+}
+
+// The included samples [kLo, kHi) of the slab rule (include/svr_render.h, svr_render_slices) on the ray (orig, dir), sample k
+// at orig + (t0 + (k + 1/2) h) dir, against the box turned for dir.  Each component of x_k is monotone in k (s_k and the
+// rounded products and sums are), so the lower bounds of the turned box hold from kLo on and its upper bounds below kHi; two
+// binary searches find both.  A component with dir = 0 is constant: its two conditions hold for every k or for none.
+SVR_DEV uint2 included_range(const Ray& ray, float t0, float h, uint32_t K, const float3& sg, const float3& bLo, const float3& bHi)
+{
+    // sg * x_k is non-decreasing in k on every component: "sg x_k >= lo" holds from some k on, "sg x_k <= hi" up to some k
+    auto at = [&](uint32_t k) { return sg * (ray.orig + __fadd_rn(t0, __fmul_rn((float)k + 0.5f, h)) * ray.dir); };
+    auto rises = [&](uint32_t k) {
+        const float3 x = at(k);
+        return x.x >= bLo.x && x.y >= bLo.y && x.z >= bLo.z;
+    };
+    auto falls = [&](uint32_t k) {
+        const float3 x = at(k);
+        return x.x <= bHi.x && x.y <= bHi.y && x.z <= bHi.z;
+    };
+    // kLo = the first k in [0, K] with rises(k) (K: none), kHi = the first k in [0, K] without falls(k)
+    uint32_t lo = 0u, hi = K;
+    while (lo < hi) {
+        const uint32_t m = (lo + hi) >> 1;
+        if (rises(m)) hi = m;
+        else lo = m + 1u;
+    }
+    const uint32_t kLo = lo;
+    hi = K;
+    while (lo < hi) {
+        const uint32_t m = (lo + hi) >> 1;
+        if (falls(m)) lo = m + 1u;
+        else hi = m;
+    }
+    return make_uint2(kLo, lo);
+}
+
 // The plane geometry of svr_render_slices (include/svr_render.h), from the host: n, K, t0 and h of the slab rule, and the
-// clipped box [cmin, cmax] turned so that the samples move up it: per component sg = -1 where n < 0, else +1, and
-// sg x in [lo, hi] (lo = sg cmin, hi = sg cmax, swapped where sg = -1) iff x in [cmin, cmax].
+// clipped box turned for n (TurnedBox).
 struct SliceGeom {
     float3 center, u, v, w, n;
     float3 sg, lo, hi;
@@ -320,9 +371,7 @@ struct SliceGeom {
 };
 
 // Slices and slabs (include/svr_render.h): pixel (x, y) of slice blockIdx.z folds the included samples [kLo, kHi) of the ray
-// (c, n) with fold_samples.  Each component of x_k = c + s_k n is monotone in k (s_k and the rounded products and sums are), so
-// the lower bounds of the turned box hold from kLo on and its upper bounds below kHi; two binary searches find both.  A
-// component with n = 0 is constant: its two conditions hold for every k or for none.
+// (c, n) with fold_samples.
 template <int OP, bool SKIP, bool COUNT>
 __global__ void __launch_bounds__(256) slice_kernel(const __grid_constant__ ProjScene s, const __grid_constant__ SliceGeom g, float windowCenter,
                                                     float windowWidth, uint32_t* __restrict__ img, float* __restrict__ value, Counters* cnt)
@@ -336,31 +385,8 @@ __global__ void __launch_bounds__(256) slice_kernel(const __grid_constant__ Proj
         Ray ray;
         ray.orig = g.center + fx * g.u + fy * g.v + (float)j * g.w;
         ray.dir = g.n;
-        // sg * x_k is non-decreasing in k on every component: "sg x_k >= lo" holds from some k on, "sg x_k <= hi" up to some k
-        auto at = [&](uint32_t k) { return g.sg * (ray.orig + __fadd_rn(g.t0, __fmul_rn((float)k + 0.5f, g.h)) * ray.dir); };
-        auto rises = [&](uint32_t k) {
-            const float3 x = at(k);
-            return x.x >= g.lo.x && x.y >= g.lo.y && x.z >= g.lo.z;
-        };
-        auto falls = [&](uint32_t k) {
-            const float3 x = at(k);
-            return x.x <= g.hi.x && x.y <= g.hi.y && x.z <= g.hi.z;
-        };
-        // kLo = the first k in [0, K] with rises(k) (K: none), kHi = the first k in [0, K] without falls(k)
-        uint32_t lo = 0u, hi = g.K;
-        while (lo < hi) {
-            const uint32_t m = (lo + hi) >> 1;
-            if (rises(m)) hi = m;
-            else lo = m + 1u;
-        }
-        const uint32_t kLo = lo;
-        hi = g.K;
-        while (lo < hi) {
-            const uint32_t m = (lo + hi) >> 1;
-            if (falls(m)) lo = m + 1u;
-            else hi = m;
-        }
-        const uint32_t kHi = lo;
+        const uint2 kr = included_range(ray, g.t0, g.h, g.K, g.sg, g.lo, g.hi);
+        const uint32_t kLo = kr.x, kHi = kr.y;
         const uint32_t taken = kHi > kLo ? kHi - kLo : 0u;
         float P = 0.f;
         if (taken > 0u) {
@@ -370,6 +396,75 @@ __global__ void __launch_bounds__(256) slice_kernel(const __grid_constant__ Proj
         }
         // the pixel's place from the launch geometry again: nothing but P and the count stays live across the division, which
         // is a subroutine call (else the MEAN variant spills the pixel around it)
+        const uint2 q = band_pixel(0u, g.H, 0u, 1u);
+        const size_t offset = ((size_t)blockIdx.z * g.H + q.y) * g.W + q.x;
+        if (value) value[offset] = P;
+        if (img) {
+            uint32_t rgba = 0u;
+            if (taken > 0u) {
+                const float gr = fminf(fmaxf((P - (windowCenter - 0.5f * windowWidth)) / windowWidth, 0.f), 1.f);
+                const float grey = 255.f * gr;
+                rgba = pack_u8x4(grey, grey, grey, 255.f);
+            }
+            img[offset] = rgba;
+        }
+    }
+    lc.flush(cnt);
+}
+
+// The geometry of svr_render_curved (include/svr_render.h) that all pixels share, from the host: the slab rule's K, t0 and h,
+// the clipped box, and where the per-image (cos, sin) table starts in the frame table (after the 4 float4 of every station).
+// the fewest slab samples for which svr_render_curved walks the range grid (SVR_OPT_RC_SKIP)
+constexpr uint32_t CURVED_WALK_MIN_K = 32u;
+
+struct CurveGeom {
+    float3 cmin, cmax;
+    uint32_t W, H, K, trig;
+    float t0, h, ps;
+    int cross;  // SVR_CURVED_CROSS: image j is station j; else row y is station y and image j the angle j
+};
+
+// Curved planar reformation (include/svr_render.h): pixel (x, y) of image blockIdx.z reads its station's frame (c, t, r, b),
+// forms its ray (p, n) or (p, t), turns the clipped box for that direction and folds the included samples with fold_samples.
+template <int OP, bool SKIP, bool COUNT>
+__global__ void __launch_bounds__(256) curved_kernel(const __grid_constant__ ProjScene s, const __grid_constant__ CurveGeom g,
+                                                     const float4* __restrict__ frames, float windowCenter, float windowWidth,
+                                                     uint32_t* __restrict__ img, float* __restrict__ value, Counters* cnt)
+{
+    const uint2 pix = band_pixel(0u, g.H, 0u, 1u);
+    const uint32_t idx = pix.x, idy = pix.y, j = blockIdx.z;
+    LocalCounters<COUNT> lc;
+    if (idx < g.W && idy < g.H) {
+        lc.add(SVR_CNT_PATHS, 1);
+        const float4* f = frames + 4u * (g.cross ? j : idy);
+        const float4 c = __ldg(f);
+        uint32_t taken = 0u;
+        float P = 0.f;
+        if (c.w != 0.f) {  // a valid station
+            const float4 t = __ldg(f + 1), r = __ldg(f + 2), b = __ldg(f + 3);
+            const float4 cs = __ldg(frames + g.trig + (g.cross ? 0u : j));
+            const float3 a = cs.x * f3(r.x, r.y, r.z) + cs.y * f3(b.x, b.y, b.z);
+            const float3 e = cs.x * f3(b.x, b.y, b.z) - cs.y * f3(r.x, r.y, r.z);  // t x a
+            const float fx = __fsub_rn((float)idx + 0.5f, 0.5f * (float)g.W);
+            Ray ray;
+            if (g.cross) {
+                const float fy = __fsub_rn((float)idy + 0.5f, 0.5f * (float)g.H);
+                ray.orig = f3(c.x, c.y, c.z) + (fx * g.ps) * a + (fy * g.ps) * e;
+                ray.dir = f3(t.x, t.y, t.z);
+            } else {
+                ray.orig = f3(c.x, c.y, c.z) + (fx * g.ps) * a;
+                ray.dir = e;
+            }
+            const TurnedBox box = turn_box(ray.dir, g.cmin, g.cmax);
+            const uint2 kr = included_range(ray, g.t0, g.h, g.K, box.sg, box.lo, box.hi);
+            taken = kr.y > kr.x ? kr.y - kr.x : 0u;
+            if (taken > 0u) {
+                lc.add(SVR_CNT_STEPS, taken);
+                const float acc = fold_samples<OP, SKIP>(s, ray, g.t0, g.h, kr.x, kr.y, lc);
+                P = OP == SVR_PROJECT_MEAN ? __fdiv_rn(acc, (float)taken) : acc;
+            }
+        }
+        // as slice_kernel: the pixel's place from the launch geometry again, after the division
         const uint2 q = band_pixel(0u, g.H, 0u, 1u);
         const size_t offset = ((size_t)blockIdx.z * g.H + q.y) * g.W + q.x;
         if (value) value[offset] = P;
@@ -577,16 +672,10 @@ extern "C" int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, cons
     const svr_volume& vo = *volume;
     const float cmin[3] = {vo.bbox.vmin.x * -vo.x_clip.x, vo.bbox.vmin.y * -vo.y_clip.x, vo.bbox.vmin.z * -vo.z_clip.x};
     const float cmax[3] = {vo.bbox.vmax.x * vo.x_clip.y, vo.bbox.vmax.y * vo.y_clip.y, vo.bbox.vmax.z * vo.z_clip.y};
-    const float n3[3] = {g.n.x, g.n.y, g.n.z};
-    float sg[3], lo[3], hi[3];
-    for (int c = 0; c < 3; ++c) {
-        sg[c] = n3[c] < 0.f ? -1.f : 1.f;
-        lo[c] = n3[c] < 0.f ? -cmax[c] : cmin[c];
-        hi[c] = n3[c] < 0.f ? -cmin[c] : cmax[c];
-    }
-    g.sg = f3(sg[0], sg[1], sg[2]);
-    g.lo = f3(lo[0], lo[1], lo[2]);
-    g.hi = f3(hi[0], hi[1], hi[2]);
+    const TurnedBox box = turn_box(g.n, f3(cmin[0], cmin[1], cmin[2]), f3(cmax[0], cmax[1], cmax[2]));
+    g.sg = box.sg;
+    g.lo = box.lo;
+    g.hi = box.hi;
 
     const int block = st.options[SVR_OPT_RC_BLOCK];
     const uint32_t tileH = (uint32_t)block / 16u;
@@ -601,6 +690,221 @@ extern "C" int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, cons
     if (p.mode == SVR_PROJECT_MAX) launch_slice_mode<SVR_PROJECT_MAX>(skip, count, grid, block, st.stream, sc, g, p, img, valueOrNull, cnt);
     else if (p.mode == SVR_PROJECT_MIN) launch_slice_mode<SVR_PROJECT_MIN>(skip, count, grid, block, st.stream, sc, g, p, img, valueOrNull, cnt);
     else launch_slice_mode<SVR_PROJECT_MEAN>(skip, count, grid, block, st.stream, sc, g, p, img, valueOrNull, cnt);
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+    return 0;
+}
+
+namespace {
+
+struct D3 {
+    double x, y, z;
+};
+D3 operator+(D3 a, D3 b) { return {a.x + b.x, a.y + b.y, a.z + b.z}; }
+D3 operator-(D3 a, D3 b) { return {a.x - b.x, a.y - b.y, a.z - b.z}; }
+D3 operator*(double s, D3 a) { return {s * a.x, s * a.y, s * a.z}; }
+double dot(D3 a, D3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
+D3 cross(D3 a, D3 b) { return {a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x}; }
+D3 normalize(D3 a) { return (1.0 / std::sqrt(dot(a, a))) * a; }
+bool is_zero(D3 a) { return a.x == 0.0 && a.y == 0.0 && a.z == 0.0; }
+svr_vec4 v4(D3 a, float w) { return {(float)a.x, (float)a.y, (float)a.z, w}; }
+
+// The frame rule of include/svr_render.h: nStations frames, 4 svr_vec4 each, into out; `who` names the entry point in an error.
+// No CUDA call.
+int curve_frames(const char* who, const float* points, uint32_t nPoints, const float* up, float stationSpacing, uint32_t nStations,
+                 svr_vec4* out)
+{
+    auto err = [&](const char* what) { return fail_msg((std::string(who) + ": " + what).c_str()); };
+    if (!points || !up) return err("null points or up");
+    if (nPoints < 2u || nPoints > (1u << 20)) return err("nPoints must be in 2..2^20");
+    if (!(stationSpacing > 0.f) || !std::isfinite(stationSpacing)) return err("stationSpacing must be positive and finite");
+    if (nStations == 0u) return err("nStations must be at least 1");
+    for (size_t i = 0; i < 3 * (size_t)nPoints; ++i)
+        if (!std::isfinite(points[i])) return err("every point must be finite");
+    // 1. drop repeats; cumulative arc length
+    std::vector<D3> P;
+    std::vector<double> S;
+    P.reserve(nPoints);
+    S.reserve(nPoints);
+    for (uint32_t i = 0; i < nPoints; ++i) {
+        const D3 q = {points[3 * i], points[3 * i + 1], points[3 * i + 2]};
+        if (!P.empty() && q.x == P.back().x && q.y == P.back().y && q.z == P.back().z) continue;
+        S.push_back(P.empty() ? 0.0 : S.back() + std::sqrt(dot(q - P.back(), q - P.back())));
+        P.push_back(q);
+    }
+    if (P.size() < 2) return err("the curve needs at least 2 distinct points");
+    if (!std::isfinite(up[0]) || !std::isfinite(up[1]) || !std::isfinite(up[2])) return err("up must be finite");
+    const D3 upv = {up[0], up[1], up[2]};
+    if (is_zero(upv)) return err("up must not be zero");
+    const double L = S.back(), D = stationSpacing;
+    if (0.5 * D > L) return err("no valid station: the curve is shorter than half a station");
+    // 2. c(s) on segment m, the last m <= M - 2 with S_m <= s
+    const size_t M = P.size();
+    auto seg = [&](double s) {
+        const size_t m = (size_t)(std::upper_bound(S.begin(), S.end(), s) - S.begin());
+        return std::min(m == 0 ? 0 : m - 1, M - 2);
+    };
+    auto at = [&](double s) {
+        const size_t m = seg(s);
+        return P[m] + ((s - S[m]) / (S[m + 1] - S[m])) * (P[m + 1] - P[m]);
+    };
+    // 3., 4. station position and tangent
+    auto station = [&](uint32_t i, D3* c, D3* t) {
+        const double s = ((double)i + 0.5) * D;
+        *c = at(s);
+        D3 d = at(std::min(s + D, L)) - at(std::max(s - D, 0.0));
+        if (is_zero(d)) {
+            const size_t m = seg(s);
+            d = P[m + 1] - P[m];
+        }
+        *t = normalize(d);
+    };
+    D3 c, t;
+    station(0, &c, &t);
+    const D3 r0 = upv - dot(upv, t) * t;
+    if (std::sqrt(dot(r0, r0)) <= 1e-6 * std::sqrt(dot(upv, upv))) return err("up must not be parallel to the tangent at station 0");
+    // 5. double reflection from station to station
+    D3 r = normalize(r0);
+    for (uint32_t i = 0; i < nStations; ++i) {
+        svr_vec4* o = out + 4 * (size_t)i;
+        if (((double)i + 0.5) * D > L) {  // 6.
+            o[0] = o[1] = o[2] = o[3] = svr_vec4{0.f, 0.f, 0.f, 0.f};
+            continue;
+        }
+        if (i > 0) {
+            D3 cn, tn;
+            station(i, &cn, &tn);
+            const D3 v1 = cn - c;
+            const double c1 = dot(v1, v1);
+            D3 rL = r, tL = t;
+            if (c1 != 0.0) {
+                rL = r - (2.0 / c1 * dot(v1, r)) * v1;
+                tL = t - (2.0 / c1 * dot(v1, t)) * v1;
+            }
+            const D3 v2 = tn - tL;
+            const double c2 = dot(v2, v2);
+            if (c2 != 0.0) rL = rL - (2.0 / c2 * dot(v2, rL)) * v2;
+            r = normalize(rL - dot(rL, tn) * tn);
+            c = cn;
+            t = tn;
+        }
+        o[0] = v4(c, 1.f);
+        o[1] = v4(t, 0.f);
+        o[2] = v4(r, 0.f);
+        o[3] = v4(cross(t, r), 0.f);
+    }
+    return 0;
+}
+
+// The frame table into curveFrames through the pinned staging buffer, on the library stream.  The host waits only for the
+// copy that last read the staging buffer; that copy is stream-ordered after the earlier renders.
+int stage_curve_table(HostState& st, const std::vector<svr_vec4>& table)
+{
+    DeviceState& d = st.dev;
+    const size_t n = table.size();
+    if (!d.curveStageEvent) SVR_TRY(cudaEventCreateWithFlags(&d.curveStageEvent, cudaEventDisableTiming));
+    SVR_TRY(cudaEventSynchronize(d.curveStageEvent));
+    if (d.curveStageCap < n) {
+        if (d.curveStage) cudaFreeHost(d.curveStage);
+        d.curveStage = nullptr;
+        d.curveStageCap = 0;
+        SVR_TRY(cudaHostAlloc((void**)&d.curveStage, n * sizeof(float4), cudaHostAllocPortable));
+        d.curveStageCap = n;
+    }
+    SVR_TRY(d.curveFrames.reserve(n));
+    memcpy(d.curveStage, table.data(), n * sizeof(float4));
+    SVR_TRY(cudaMemcpyAsync(d.curveFrames.p, d.curveStage, n * sizeof(float4), cudaMemcpyHostToDevice, st.stream));
+    SVR_TRY(cudaEventRecord(d.curveStageEvent, st.stream));
+    return 0;
+}
+
+template <int OP, bool SKIP>
+void launch_curved(bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const CurveGeom& g, const float4* frames,
+                   const svr_curved_params& p, uint32_t* img, float* value, Counters* cnt)
+{
+    if (count) curved_kernel<OP, SKIP, true><<<grid, block, 0, stream>>>(sc, g, frames, p.windowCenter, p.windowWidth, img, value, cnt);
+    else curved_kernel<OP, SKIP, false><<<grid, block, 0, stream>>>(sc, g, frames, p.windowCenter, p.windowWidth, img, value, cnt);
+}
+
+template <int OP>
+void launch_curved_mode(bool skip, bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const CurveGeom& g,
+                        const float4* frames, const svr_curved_params& p, uint32_t* img, float* value, Counters* cnt)
+{
+    if (skip) launch_curved<OP, true>(count, grid, block, stream, sc, g, frames, p, img, value, cnt);
+    else launch_curved<OP, false>(count, grid, block, stream, sc, g, frames, p, img, value, cnt);
+}
+
+}  // namespace
+
+extern "C" int svr_curve_frames(const float* points, uint32_t nPoints, const float up[3], float stationSpacing, uint32_t nStations,
+                                svr_vec4* hostFrames)
+{
+    if (!hostFrames) return fail_msg("svr_curve_frames: null hostFrames");
+    return curve_frames("svr_curve_frames", points, nPoints, up, stationSpacing, nStations, hostFrames);
+}
+
+extern "C" int svr_render_curved(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_curved_params* params,
+                                 const float* points, uint32_t nPoints)
+{
+    HostState& st = state();
+    if (!volume || !params || !points) return fail_msg("svr_render_curved: null volume, params or points");
+    if (!imgOrNull && !valueOrNull) return fail_msg("svr_render_curved: both outputs are null");
+    const svr_curved_params p = *params;
+    if (p.layout != SVR_CURVED_STRAIGHTENED && p.layout != SVR_CURVED_CROSS)
+        return fail_msg("svr_render_curved: layout must be 0 (straightened) or 1 (cross-sections)");
+    if (p.imageW == 0u || p.imageW > 16384u || p.imageH == 0u || p.imageH > 16384u)
+        return fail_msg("svr_render_curved: imageW and imageH must be in 1..16384");
+    if (p.count == 0u || p.count > 65535u) return fail_msg("svr_render_curved: count must be in 1..65535");
+    if (p.mode < SVR_PROJECT_MAX || p.mode > SVR_PROJECT_MEAN) return fail_msg("svr_render_curved: mode must be 0 (max), 1 (min) or 2 (mean)");
+    if (!(p.pixelSpacing > 0.f) || !std::isfinite(p.pixelSpacing)) return fail_msg("svr_render_curved: pixelSpacing must be positive and finite");
+    if (!std::isfinite(p.angle0) || !std::isfinite(p.angleStep)) return fail_msg("svr_render_curved: angle0 and angleStep must be finite");
+    if (!(p.thickness >= 0.f) || !std::isfinite(p.thickness)) return fail_msg("svr_render_curved: thickness must be finite and not negative");
+    if (p.thickness > 0.f) {
+        if (!(p.sampleSpacing > 0.f) || !std::isfinite(p.sampleSpacing))
+            return fail_msg("svr_render_curved: sampleSpacing must be positive and finite for a slab");
+        if (!(p.thickness / p.sampleSpacing <= 65536.f)) return fail_msg("svr_render_curved: thickness / sampleSpacing must be at most 65536");
+    }
+    if (!(p.windowWidth > 0.f) || !std::isfinite(p.windowWidth) || !std::isfinite(p.windowCenter))
+        return fail_msg("svr_render_curved: windowWidth must be positive and finite, windowCenter finite");
+    const bool cross = p.layout == SVR_CURVED_CROSS;
+    const uint32_t nStations = cross ? p.count : p.imageH, nTrig = cross ? 1u : p.count;
+    std::vector<svr_vec4> table(4 * (size_t)nStations + nTrig);
+    if (int rc = curve_frames("svr_render_curved", points, nPoints, p.up, p.stationSpacing, nStations, table.data())) return rc;
+    for (uint32_t j = 0; j < nTrig; ++j) {
+        const double theta = (double)p.angle0 + (double)j * (double)p.angleStep;
+        table[4 * (size_t)nStations + j] = svr_vec4{(float)std::cos(theta), (float)std::sin(theta), 0.f, 0.f};
+    }
+
+    CurveGeom g;
+    const svr_volume& vo = *volume;
+    g.cmin = f3(vo.bbox.vmin.x * -vo.x_clip.x, vo.bbox.vmin.y * -vo.y_clip.x, vo.bbox.vmin.z * -vo.z_clip.x);
+    g.cmax = f3(vo.bbox.vmax.x * vo.x_clip.y, vo.bbox.vmax.y * vo.y_clip.y, vo.bbox.vmax.z * vo.z_clip.y);
+    g.W = p.imageW;
+    g.H = p.imageH;
+    g.h = p.thickness > 0.f ? p.sampleSpacing : 0.f;
+    g.K = p.thickness > 0.f ? (uint32_t)std::max(1.f, std::floor(p.thickness / g.h + 0.5f)) : 1u;
+    g.t0 = -((float)g.K * g.h) * 0.5f;
+    g.ps = p.pixelSpacing;
+    g.trig = 4u * nStations;
+    g.cross = cross ? 1 : 0;
+
+    const int block = st.options[SVR_OPT_RC_BLOCK];
+    const uint32_t tileH = (uint32_t)block / 16u;
+    ProjScene sc;
+    // slabs of fewer than CURVED_WALK_MIN_K samples, and thin images, do not walk: 16-sample slabs measured slower with the walk,
+    // 64-sample ones faster (DESIGN.md section 7k)
+    const bool skip = st.options[SVR_OPT_RC_SKIP] != 0 && g.K >= CURVED_WALK_MIN_K;
+    const bool count = st.options[SVR_OPT_COUNTERS] != 0;
+    if (int rc = make_scene(&sc, *volume, nullptr, skip)) return rc;
+    Counters* cnt = count ? device_counters() : nullptr;
+    if (count && !cnt) return fail_msg("svr_render_curved: counter allocation failed");
+    if (int rc = stage_curve_table(st, table)) return rc;
+    const float4* frames = st.dev.curveFrames.p;
+    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + tileH - 1u) / tileH, p.count);
+    uint32_t* img = (uint32_t*)imgOrNull;
+    if (p.mode == SVR_PROJECT_MAX) launch_curved_mode<SVR_PROJECT_MAX>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
+    else if (p.mode == SVR_PROJECT_MIN) launch_curved_mode<SVR_PROJECT_MIN>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
+    else launch_curved_mode<SVR_PROJECT_MEAN>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
     count_launch();
     SVR_TRY(cudaGetLastError());
     return 0;

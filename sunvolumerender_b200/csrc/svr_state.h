@@ -151,6 +151,14 @@ struct DeviceState {
     unsigned long long progGuideEpoch = 0;  // sceneEpoch after the frame that made the guides; 0 = none
     uint32_t progGuideRays = 0;
 
+    // Curved planar reformation (svr_render_curved, svr_project.cu): the stations' frames and the per-image (cos, sin) table,
+    // copied from curveStage (pinned, curveStageCap float4) on the library stream; curveStageEvent follows the copy that last
+    // read curveStage, and is all a call waits on before refilling it
+    DevBuf<float4> curveFrames;
+    float4* curveStage = nullptr;
+    size_t curveStageCap = 0;
+    cudaEvent_t curveStageEvent = nullptr;
+
     DevBuf<Counters> counters;
 
     // Frees every allocation, event, view and the mailbox, and returns every key and flag to its default (svr_api.cu)

@@ -356,6 +356,20 @@ class Renderer:
         L.check(self.lib.svr_render_slices(_ptr(img), _ptr(value), C.byref(self.volume), C.byref(params)), "svr_render_slices")
         return value, img
 
+    def render_curved(self, points, params, value=None, img=None):
+        """Curved planar reformation (svr_render_curved) of the bound volume along the polyline `points` ((n, 3) world xyz on
+        the host); params: an L.CurvedParams (scene.straightened_curve, scene.curve_cross_sections).  value: float32
+        (count, H, W) and img: uint8 (count, H, W, 4) device tensors, allocated when not given.  Returns (value, img)."""
+        pts = np.ascontiguousarray(np.asarray(points, np.float32).reshape(-1, 3))
+        shape = (params.count, params.imageH, params.imageW)
+        if value is None:
+            value = torch.empty(shape, dtype=torch.float32, device=self.device)
+        if img is None:
+            img = torch.empty(shape + (4,), dtype=torch.uint8, device=self.device)
+        L.check(self.lib.svr_render_curved(_ptr(img), _ptr(value), C.byref(self.volume), C.byref(params), pts.ctypes.data, len(pts)),
+                "svr_render_curved")
+        return value, img
+
     # ---- results
     def hdr_image(self):
         return self.hdr.view(self.camera.imageH, self.camera.imageW, 3)

@@ -246,6 +246,61 @@ def oblique_slice(center, normal, up, pixel_size, image_w, image_h, count=1, sli
     return p
 
 
+def _curved(layout, image_w, image_h, count, pixel_spacing, station_spacing, up, angle0, angle_step, thickness, sample_spacing, mode,
+            window):
+    p = L.CurvedParams()
+    p.up[:] = [float(x) for x in up]
+    p.layout = L.CURVED_LAYOUTS[layout]
+    p.imageW, p.imageH, p.count = int(image_w), int(image_h), int(count)
+    p.mode = L.PROJECT_MODES[mode]
+    p.pixelSpacing, p.stationSpacing = float(pixel_spacing), float(station_spacing)
+    p.angle0, p.angleStep = float(angle0), float(angle_step)
+    p.thickness = float(thickness)
+    p.sampleSpacing = float(pixel_spacing if sample_spacing is None else sample_spacing)
+    p.windowCenter, p.windowWidth = window
+    return p
+
+
+def straightened_curve(image_w, n_stations, pixel_spacing, station_spacing=None, up=(0.0, 0.0, 1.0), count=1, angle0=0.0,
+                       angle_step=None, thickness=0.0, sample_spacing=None, mode="max", window=(0.5, 1.0)):
+    """svr_curved_params of a straightened CPR (svr_render_curved): one row per station (n_stations rows, station_spacing apart
+    along the curve, default pixel_spacing), image_w columns pixel_spacing apart across it.  count > 1 is the rotational stack,
+    image j at angle0 + j angle_step about the tangent (default a full turn over the count).  A slab of `thickness` world units
+    across the image plane is sampled every sample_spacing (default pixel_spacing)."""
+    step = 2.0 * math.pi / count if angle_step is None else angle_step
+    return _curved("straightened", image_w, n_stations, count, pixel_spacing, pixel_spacing if station_spacing is None else station_spacing,
+                   up, angle0, step, thickness, sample_spacing, mode, window)
+
+
+def curve_cross_sections(image_w, image_h, count, pixel_spacing, station_spacing, up=(0.0, 0.0, 1.0), angle=0.0, thickness=0.0,
+                         sample_spacing=None, mode="max", window=(0.5, 1.0)):
+    """svr_curved_params of `count` cross-sections (svr_render_curved): image j is the image_w x image_h plane perpendicular to
+    the curve at station j (station_spacing apart), pixel_spacing between pixels, its columns along the frame's
+    cos(angle) r + sin(angle) b.  A slab of `thickness` world units along the tangent is sampled every sample_spacing."""
+    return _curved("cross", image_w, image_h, count, pixel_spacing, station_spacing, up, angle, 0.0, thickness, sample_spacing, mode, window)
+
+
+def polyline_length(points):
+    """Arc length of the polyline `points` ((n, 3)), in float64."""
+    p = np.asarray(points, np.float64).reshape(-1, 3)
+    return float(np.linalg.norm(np.diff(p, axis=0), axis=1).sum())
+
+
+def curve_frames(points, up, station_spacing, n):
+    """The library's frames of n stations of the polyline `points` (svr_curve_frames; no GPU): (n, 4, 4) float32, rows
+    (c, valid), (t, 0), (r, 0), (b, 0).  The world position of CPR pixel column x of a straightened row y at angle theta is
+    c_y + (x + 1/2 - W/2) pixelSpacing (cos(theta) r_y + sin(theta) b_y)."""
+    import ctypes as C
+
+    pts = np.ascontiguousarray(np.asarray(points, np.float32).reshape(-1, 3))
+    upv = np.ascontiguousarray(np.asarray(up, np.float32).reshape(3))
+    out = np.zeros((int(n), 4, 4), np.float32)
+    lib = L.load()
+    L.check(lib.svr_curve_frames(pts.ctypes.data, len(pts), upv.ctypes.data, C.c_float(station_spacing), int(n), out.ctypes.data),
+            "svr_curve_frames")
+    return out
+
+
 @dataclass
 class Config:
     """One BASELINE.json configuration."""

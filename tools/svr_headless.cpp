@@ -4,7 +4,8 @@
 // render_raycasting -- on the synthetic configurations of SURVEY.md section 8d, times the loop with
 // CUDA events and writes the image as PPM (tone-mapped u8) and PFM (float accumulator).
 //
-//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip|iso|slice] [--window C,W] [--iso V] [--axis x|y|z --index I --slab N]
+//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip|iso|slice|cpr] [--window C,W] [--iso V] [--axis x|y|z --index I --slab N]
+//                [--curve FILE] [--up x,y,z]
 //                [--spp N] [--depth D] [--batched 0|1]
 //                [--pt-mode 0|1|2] [--n N --w W --h H] [--out prefix] [--reps R] [--volume file.mhd|.mha] [--tf file.tf|app]
 //                [--interact script.txt]
@@ -22,6 +23,9 @@
 // --mode slice renders the --w x --h slice (svr_render_slices) normal to --axis (default z: axial; y coronal, x sagittal) through
 // voxel --index (default the middle one), one voxel per pixel, centred on the volume in the plane and oriented as
 // scene.axis_slice; --slab N makes it the MIP of a slab of N voxels (one sample per voxel), grey through --window.
+// --mode cpr renders the --w x --h straightened curved planar reformation (svr_render_curved) along the polyline of --curve FILE
+// (whitespace-separated world xyz triples), the frame's roll fixed by --up (default 0,0,1), pixel and station spacing the
+// smallest voxel spacing; --slab N and --window as for slices.
 // --volume loads a MetaImage file the way Canvas::LoadVolume does (core/VolumeReader.cpp:13-94) instead of
 // generating the configuration's synthetic volume; camera and light are framed on its extent.
 // --tf loads a transfer function saved by the application (gui/transferfunction.cpp:55-88); `app` is the
@@ -159,6 +163,8 @@ int main(int argc, char** argv)
     int batched = 1, ptMode = 2, reps = 3, sppArg = -1, depthArg = -1;
     float windowC = 0.5f, windowW = 1.f, isoValue = 0.5f;
     int sliceAxis = 2, sliceIndex = -1, slab = 0;
+    std::string curvePath;
+    float up[3] = {0.f, 0.f, 1.f};
     for (int i = 1; i + 1 < argc; i += 2) {
         std::string k = argv[i], v = argv[i + 1];
         if (k == "--config") {
@@ -188,6 +194,10 @@ int main(int argc, char** argv)
             sliceAxis = v[0] - 'x';
         } else if (k == "--index") sliceIndex = atoi(v.c_str());
         else if (k == "--slab") slab = atoi(v.c_str());
+        else if (k == "--curve") curvePath = v;
+        else if (k == "--up") {
+            if (sscanf(v.c_str(), "%f,%f,%f", &up[0], &up[1], &up[2]) != 3) { fprintf(stderr, "--up wants x,y,z\n"); return 2; }
+        }
         else { fprintf(stderr, "unknown option %s\n", k.c_str()); return 2; }
     }
     std::vector<std::string> script;
@@ -323,7 +333,7 @@ int main(int argc, char** argv)
     svr_u8vec4* dImg = nullptr;
     CK(cudaMalloc((void**)&dImg, npix * 4));
     float* dValue = nullptr;
-    if (projMode >= 0 || mode == "slice") CK(cudaMalloc((void**)&dValue, npix * sizeof(float)));
+    if (projMode >= 0 || mode == "slice" || mode == "cpr") CK(cudaMalloc((void**)&dValue, npix * sizeof(float)));
 
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
@@ -352,6 +362,28 @@ int main(int argc, char** argv)
         slice.windowCenter = windowC;
         slice.windowWidth = windowW;
     }
+    std::vector<float> curve;
+    svr_curved_params cpr;
+    memset(&cpr, 0, sizeof(cpr));
+    if (mode == "cpr") {
+        std::ifstream cf(curvePath);
+        if (curvePath.empty() || !cf) { fprintf(stderr, "--mode cpr wants --curve FILE (whitespace-separated xyz triples)\n"); return 2; }
+        for (float x; cf >> x;) curve.push_back(x);
+        if (curve.size() % 3 != 0) { fprintf(stderr, "%s: the number of values is not a multiple of 3\n", curvePath.c_str()); return 2; }
+        const float sp = fminf(vol.spacing.x, fminf(vol.spacing.y, vol.spacing.z));
+        memcpy(cpr.up, up, sizeof(up));
+        cpr.layout = SVR_CURVED_STRAIGHTENED;
+        cpr.imageW = (uint32_t)W;
+        cpr.imageH = (uint32_t)H;
+        cpr.count = 1;
+        cpr.mode = SVR_PROJECT_MAX;
+        cpr.pixelSpacing = sp;
+        cpr.stationSpacing = sp;
+        cpr.thickness = (float)slab * sp;
+        cpr.sampleSpacing = sp;
+        cpr.windowCenter = windowC;
+        cpr.windowWidth = windowW;
+    }
     float best = 1e30f;
     for (int rep = 0; rep < reps + 1; ++rep) {  // first pass warms up (and builds the macrocell grid)
         CK(cudaEventRecord(e0, 0));
@@ -363,6 +395,8 @@ int main(int argc, char** argv)
             SVR(svr_render_isosurface(dImg, nullptr, &vol, &cam, &iso, 0, 1, nullptr));
         } else if (mode == "slice") {
             SVR(svr_render_slices(dImg, dValue, &vol, &slice));
+        } else if (mode == "cpr") {
+            SVR(svr_render_curved(dImg, dValue, &vol, &cpr, curve.data(), (uint32_t)(curve.size() / 3)));
         } else if (batched) {
             rp.frameNo = 0;
             SVR(svr_render_pathtracer_spp(dImg, &rp, (uint32_t)cfg.spp));
@@ -378,7 +412,7 @@ int main(int argc, char** argv)
         CK(cudaEventElapsedTime(&ms, e0, e1));
         if (rep > 0 && ms < best) best = ms;
     }
-    if (mode == "rc" || mode == "iso" || mode == "slice" || projMode >= 0)
+    if (mode == "rc" || mode == "iso" || mode == "slice" || mode == "cpr" || projMode >= 0)
         printf("{\"config\": \"%s\", \"mode\": \"%s\", \"ms\": %.4f, \"mrays_per_s\": %.2f, \"launches\": %llu}\n", cfg.name, mode.c_str(),
                best, npix / (best * 1e-3) / 1e6, (unsigned long long)svr_launch_count());
     else
@@ -399,7 +433,7 @@ int main(int argc, char** argv)
             fclose(f);
         }
     }
-    if (projMode >= 0 || mode == "slice") {
+    if (projMode >= 0 || mode == "slice" || mode == "cpr") {
         std::vector<float> value(npix);
         CK(cudaMemcpy(value.data(), dValue, npix * sizeof(float), cudaMemcpyDeviceToHost));
         FILE* f = fopen((out + ".pfm").c_str(), "wb");
@@ -408,7 +442,7 @@ int main(int argc, char** argv)
             fwrite(value.data(), sizeof(float), value.size(), f);
             fclose(f);
         }
-    } else if (mode != "rc" && mode != "iso" && mode != "slice") {
+    } else if (mode != "rc" && mode != "iso" && mode != "slice" && mode != "cpr") {
         std::vector<float> hdr(npix * 3);
         CK(cudaMemcpy(hdr.data(), rp.hdrBuffer, npix * 12, cudaMemcpyDeviceToHost));
         FILE* f = fopen((out + ".pfm").c_str(), "wb");
