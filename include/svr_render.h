@@ -80,7 +80,8 @@ enum svr_option {
     /* skipping in the ray-marching kernels: the ray caster's empty-space skipping through the macrocell grid, the
      * projection's skipping of cells that cannot change the projected value (svr_render_projection) and the isosurface's
      * skipping of cells below the threshold (svr_render_isosurface), and the same projection skipping across a thick slab
-     * (svr_render_slices; svr_render_curved for slabs of 32 samples or more): 0 off, 1 on (default) */
+     * (svr_render_slices; svr_render_curved for slabs of 32 samples or more), and the label surfaces' skipping of cells
+     * that hold no visible label (svr_render_labels, through a label presence grid of its own): 0 off, 1 on (default) */
     SVR_OPT_RC_SKIP = 4,
     /* Philox key */
     SVR_OPT_SEED = 5,
@@ -491,6 +492,67 @@ int svr_curve_frames(const float* points, uint32_t nPoints, const float up[3], f
 int svr_render_curved(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_curved_params* params,
                       const float* points, uint32_t nPoints);
 
+/* Label maps (DESIGN.md section 7l): a segmentation, one u8 label id per voxel (0 = background), made by svr_labels_create or
+ * svr_labels_load_metaimage on the grid of its image, drawn as shaded 3D surfaces (svr_render_labels) or as coloured overlays
+ * on slices (svr_render_label_slices).  Only these two entry points read a label volume: the grey renderers do not check for
+ * one and read its texture as if it were an image.  Both reject a volume whose texture is not a point-filtered, unnormalised,
+ * element-type 8-bit unsigned array.
+ * The table: label l is visible iff l != 0 and color[l][3] > 0; label 0 is never drawn.  Every entry, label 0's included, must
+ * be finite and in [0, 1].  The table and its 256-bit visibility mask reach the kernels as a launch parameter: a change of
+ * colours or visibility costs no copy and rebuilds nothing. */
+typedef struct svr_label_params {
+    float color[256][4];  /* per label id: r, g, b in [0, 1]; a in [0, 1], a = 0 hides the label */
+} svr_label_params;
+
+/* 3D label surfaces: the first place along each pixel-centre ray where the visible labels' indicator reaches 1/2, shaded with
+ * the isosurface's headlight in the colour of the label found there.  Rays and samples are svr_render_projection's on the label
+ * volume's box and clip planes: t0 = max(tNear, 0), h = 0.5 * stepSize, K = floor((tFar - t0) / h + 0.5), sample k at
+ * t_k = t0 + (k + 0.5) h.  In fp32:
+ *   indicator:  u = tex_coord(x) * (nx, ny, nz) - 1/2, i = floor(u), f = u - i per axis; vis(i, j, k) = 1 if voxel (i, j, k)
+ *               lies inside the volume and holds a visible label, else 0; m(x) = the trilinear interpolation of vis over the 8
+ *               corners i .. i + 1, lerp(a, b, f) = (1 - f) a + f b along x, then y, then z (8 point fetches; the hardware
+ *               filter's 8-bit weights are not used).
+ *   hit:        k* = the smallest k with m(t_k) >= 1/2; none: the ray misses.
+ *   refinement: svr_render_isosurface's with v = m and isoValue = 1/2: k* = 0: t_hit = t_0; k* > 0: 4 bisection steps between
+ *               t_{k*-1} and t_{k*}, then the linear interpolation.  t_hi = the final bisection upper bound (t_0 when k* = 0).
+ *   label:      the visible label with the largest summed corner weight w = wx wy wz (wx = 1 - f.x or f.x, ...; summed in corner
+ *               order, x fastest) at t_hi, ties to the smaller id.
+ *   normal:     g = the analytic gradient of m at x_hit (the derivative of the trilinear weights) times
+ *               (nx invSize.x, ny invSize.y, nz invSize.z), in world units; n = normalize(g) turned to face the ray's origin if
+ *               |g|^2 > 0, else n = 0.
+ *   shading:    svr_render_isosurface's headlight with color = color[label].rgb.
+ * imgOrNull receives (trunc(255 rgb), 255) for a hit and (0, 0, 0, 0) for a miss; surfaceOrNull (n, view-space depth) as
+ * svr_render_isosurface writes it, (0, 0, 0, +inf) for a miss; labelOrNull (imageW*imageH bytes) the label, 0 for a miss (for
+ * picking).  phase, stride and *bandRows as for svr_render_isosurface.
+ * SVR_OPT_RC_SKIP = 1 (default) drops the samples of macrocells whose label presence mask (the labels of the cell's voxels and
+ * a one-voxel apron, every corner a sample of the cell can read) holds no visible label: m = 0 on all of them.  img, surface
+ * and label are bit-identical either way.  The presence grid is kept per label array and cell edge (SVR_OPT_MACROCELL_SIZE,
+ * else 8), apart from the grey volumes' range grid; svr_volume_upload into the array rebuilds it at the next call,
+ * svr_volume_destroy releases it, and a new table never rebuilds it.  Counters as for svr_render_isosurface (shade_taps counts
+ * indicator evaluations; the refinement, label and gradient work is not counted).
+ * Errors, all reported before any launch or allocation: a null labels volume, camera or table; all three outputs null;
+ * stepSize not positive or not finite; a table entry not finite or outside [0, 1]; phase >= stride; a volume that is not a
+ * label volume (the only check that makes CUDA calls). */
+int svr_render_labels(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrNull, uint8_t* labelOrNull, const svr_volume* labels,
+                      const svr_camera* camera, const svr_label_params* table, float stepSize, uint32_t phase, uint32_t stride,
+                      uint32_t* bandRows);
+
+/* Label overlays on slices: the labels of the pixels of svr_render_slices with the same params, so that the overlay lands on
+ * the grey slice's pixels.  In fp32:
+ *   pixel centre: c = svr_render_slices' (the slab's centre plane).
+ *   label:        L = the label of voxel floor(tex_coord(c) * (nx, ny, nz)) (0 outside the volume), and L = 0 when c lies
+ *                 outside the label volume's clipped box (svr_render_slices' inclusion rule applied to c alone).
+ *   outline:      with outline = 1, a pixel with a visible L is an outline pixel when one of its 4 neighbours in the same image
+ *                 has a different label; neighbours outside the image do not count.
+ * labelOrNull receives L for every pixel at [(j * imageH + y) * imageW + x].  imgOrNull (the grey image of svr_render_slices,
+ * count * imageH * imageW rgba) is composited in place: where L is visible, with a = color[L][3] (1 on an outline pixel), each
+ * colour channel becomes trunc((1 - a) in + a (255 color) + 1/2) in correctly rounded fp32 operations and alpha 255; every other
+ * pixel is left as it was.  No skipping: one fetch per pixel, and four more with outline.
+ * Errors, all reported before any launch: a null labels volume, params or table; both outputs null; every parameter error of
+ * svr_render_slices; a table entry not finite or outside [0, 1]; outline not 0 or 1; a volume that is not a label volume. */
+int svr_render_label_slices(svr_u8vec4* imgOrNull, uint8_t* labelOrNull, const svr_volume* labels, const svr_slice_params* params,
+                            const svr_label_params* table, int outline);
+
 /* ---- resource builders (the input contract of the path) ---- */
 enum svr_voxel_format { SVR_VOXEL_U8 = 0, SVR_VOXEL_U16 = 1, SVR_VOXEL_F16 = 2, SVR_VOXEL_F32 = 3 };
 
@@ -503,6 +565,14 @@ enum svr_voxel_format { SVR_VOXEL_U8 = 0, SVR_VOXEL_U16 = 1, SVR_VOXEL_F16 = 2, 
 int svr_volume_create(svr_volume* out, const void* data, int data_on_device, int format,
                       uint32_t nx, uint32_t ny, uint32_t nz, float sx, float sy, float sz, float maxGradMag);
 int svr_volume_destroy(svr_volume* vol);
+/* A label volume (svr_render_labels, svr_render_label_slices): nx*ny*nz u8 label ids, x fastest, into a 3-D u8 cudaArray
+ * (surface load/store allowed, as svr_volume_create makes it) behind a texture with point filtering, element-type reads,
+ * unnormalised coordinates and border addressing (a voxel outside the volume reads 0, the background).  bbox, spacing,
+ * invSpacing and the clip planes are svr_volume_create's (a centred box), so a segmentation with the dims and spacing of its
+ * image lines up with it; densityScale and gradientFactor are unused.  svr_volume_destroy, svr_volume_upload and
+ * svr_volume_download take it as they take any volume. */
+int svr_labels_create(svr_volume* out, const void* data, int data_on_device, uint32_t nx, uint32_t ny, uint32_t nz, float sx,
+                      float sy, float sz);
 /* Re-uploads voxels (same dims and format, x-fastest) into the array behind vol->tex -- the second
  * half of VolumeReader::CreateTextures (core/VolumeReader.cpp:146-161) for a volume that is already
  * bound -- and drops the macrocell cache built from the old contents.  Asynchronous on the library

@@ -72,6 +72,12 @@ int svr_volume_from_raw(const void* host_data, int met_type, int msb, uint32_t n
 int svr_volume_load_metaimage(const char* path, svr_volume* out, svr_volume_stats* stats,
                               uint32_t* histogram, uint32_t histogram_capacity);
 
+/* A label map from a MetaImage file (the files svr_volume_load_metaimage reads): any integer ElementType whose values all lie
+ * in 0..255, converted to u8 on the host without rescaling, into a label volume as svr_labels_create makes it.  A float or
+ * double ElementType, a value outside 0..255 (the error names it) and more than one channel are errors, all reported before
+ * any CUDA call.  maxLabelOrNull receives the largest label id. */
+int svr_labels_load_metaimage(const char* path, svr_volume* out, uint32_t* maxLabelOrNull);
+
 /* Copies the voxels behind vol->tex back to host memory (x fastest, the array's own element type);
  * `bytes` must be the exact size.  Used by tests and tools. */
 int svr_volume_download(const svr_volume* vol, void* host_out, uint64_t bytes);

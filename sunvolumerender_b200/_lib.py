@@ -140,6 +140,12 @@ class CurvedParams(C.Structure):  # svr_curved_params
 
 assert C.sizeof(CurvedParams) == 64
 
+class LabelParams(C.Structure):  # svr_label_params
+    _fields_ = [("color", (C.c_float * 4) * 256)]
+
+
+assert C.sizeof(LabelParams) == 4096
+
 # enum svr_curved_layout
 CURVED_STRAIGHTENED, CURVED_CROSS = 0, 1
 CURVED_LAYOUTS = {"straightened": CURVED_STRAIGHTENED, "cross": CURVED_CROSS}
@@ -228,6 +234,10 @@ SIGNATURES = [
     ("svr_render_slices", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(SliceParams)]),
     ("svr_curve_frames", C.c_int, [_P, C.c_uint32, _P, C.c_float, C.c_uint32, _P]),
     ("svr_render_curved", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(CurvedParams), _P, C.c_uint32]),
+    ("svr_render_labels", C.c_int, [_P, _P, _P, C.POINTER(Volume), C.POINTER(Camera), C.POINTER(LabelParams), C.c_float, C.c_uint32, C.c_uint32,
+                                    C.POINTER(C.c_uint32)]),
+    ("svr_render_label_slices", C.c_int, [_P, _P, C.POINTER(Volume), C.POINTER(SliceParams), C.POINTER(LabelParams), C.c_int]),
+    ("svr_labels_create", C.c_int, [C.POINTER(Volume), _P, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float, C.c_float, C.c_float]),
 ]
 
 
@@ -268,6 +278,7 @@ SIGNATURES_IO = [
     ("svr_volume_from_raw", C.c_int, [_P, C.c_int, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_float, C.c_float, C.c_float,
                                       C.POINTER(Volume), C.POINTER(VolumeStats), _P, C.c_uint32]),
     ("svr_volume_load_metaimage", C.c_int, [C.c_char_p, C.POINTER(Volume), C.POINTER(VolumeStats), _P, C.c_uint32]),
+    ("svr_labels_load_metaimage", C.c_int, [C.c_char_p, C.POINTER(Volume), C.POINTER(C.c_uint32)]),
     ("svr_volume_download", C.c_int, [C.POINTER(Volume), _P, C.c_uint64]),
 ]
 

@@ -3,6 +3,7 @@
 // generators (SURVEY.md section 8d), gradient-magnitude reduction, counters, tap microbenchmarks.
 #include <cuda_fp16.h>
 
+#include <cmath>
 #include <cstring>
 #include <vector>
 
@@ -261,6 +262,7 @@ extern "C" uint64_t svr_lookahead_batch_count(void) { return state().aheadBatche
 extern "C" int svr_volume_invalidate_cache(void)
 {
     release_grid(state());
+    release_label_grid(state());
     return 0;
 }
 
@@ -324,6 +326,22 @@ static cudaChannelFormatDesc voxel_channel(int format)
 
 extern "C" int svr_max_gradient_magnitude(const void* dev_data, int format, uint32_t nx, uint32_t ny, uint32_t nz,
                                           float sx, float sy, float sz, float* host_out);
+
+// Everything of a new volume but its texture and gradient normalisation: the centred box, the spacing, the clip planes
+static void volume_geometry(svr_volume* out, uint32_t nx, uint32_t ny, uint32_t nz, float sx, float sy, float sz)
+{
+    memset(out, 0, sizeof(*out));
+    float3 size = f3(nx * sx, ny * sy, nz * sz);
+    float3 vmax = size - size * 0.5f;  // VolumeReader.cpp:178-180
+    out->bbox.vmin = {-vmax.x, -vmax.y, -vmax.z};
+    out->bbox.vmax = {vmax.x, vmax.y, vmax.z};
+    out->bbox.invSize = {1.f / (vmax.x + vmax.x), 1.f / (vmax.y + vmax.y), 1.f / (vmax.z + vmax.z)};
+    out->densityScale = 1.f;          // gui/canvas.cpp:32
+    out->gradientFactor = 0.5f;       // gui/canvas.cpp:19
+    out->spacing = {sx, sy, sz};
+    out->invSpacing = {1.f / sx, 1.f / sy, 1.f / sz};
+    out->x_clip = out->y_clip = out->z_clip = {-1.f, 1.f};  // gui/canvas.cpp:31
+}
 
 // core/VolumeReader.cpp:138-185
 extern "C" int svr_volume_create(svr_volume* out, const void* data, int data_on_device, int format, uint32_t nx,
@@ -395,19 +413,61 @@ extern "C" int svr_volume_create(svr_volume* out, const void* data, int data_on_
     e = cudaStreamSynchronize(st.stream);
     if (e != cudaSuccess) return drop(fail("cudaStreamSynchronize(svr_volume_create)", e));
 
-    memset(out, 0, sizeof(*out));
-    float3 size = f3(nx * sx, ny * sy, nz * sz);
-    float3 vmax = size - size * 0.5f;  // VolumeReader.cpp:178-180
-    out->bbox.vmin = {-vmax.x, -vmax.y, -vmax.z};
-    out->bbox.vmax = {vmax.x, vmax.y, vmax.z};
-    out->bbox.invSize = {1.f / (vmax.x + vmax.x), 1.f / (vmax.y + vmax.y), 1.f / (vmax.z + vmax.z)};
+    volume_geometry(out, nx, ny, nz, sx, sy, sz);
     out->tex = tex;
-    out->densityScale = 1.f;          // gui/canvas.cpp:32
     out->invMaxMagnitude = 1.f / maxGradMag;
-    out->gradientFactor = 0.5f;       // gui/canvas.cpp:19
-    out->spacing = {sx, sy, sz};
-    out->invSpacing = {1.f / sx, 1.f / sy, 1.f / sz};
-    out->x_clip = out->y_clip = out->z_clip = {-1.f, 1.f};  // gui/canvas.cpp:31
+    return 0;
+}
+
+extern "C" int svr_labels_create(svr_volume* out, const void* data, int data_on_device, uint32_t nx, uint32_t ny, uint32_t nz, float sx,
+                                 float sy, float sz)
+{
+    if (!out || !data || !nx || !ny || !nz) return fail_msg("svr_labels_create: bad argument");
+    if (nx > 16384u || ny > 16384u || nz > 16384u) return fail_msg("svr_labels_create: dimension exceeds the 3-D texture limit (16384 per axis)");
+    if (!(sx > 0.f) || !(sy > 0.f) || !(sz > 0.f) || !std::isfinite(sx) || !std::isfinite(sy) || !std::isfinite(sz))
+        return fail_msg("svr_labels_create: spacing must be positive and finite");
+    HostState& st = state();
+    const cudaChannelFormatDesc ch = voxel_channel(SVR_VOXEL_U8);
+    const cudaExtent extent = make_cudaExtent(nx, ny, nz);
+    cudaArray_t arr = nullptr;
+    SVR_TRY(cudaMalloc3DArray(&arr, &ch, extent, cudaArraySurfaceLoadStore));
+    cudaMemcpy3DParms cp;
+    memset(&cp, 0, sizeof(cp));
+    cp.dstArray = arr;
+    cp.extent = extent;
+    cp.kind = data_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    cp.srcPtr = make_cudaPitchedPtr(const_cast<void*>(data), nx, nx, ny);
+    cudaError_t e = cudaMemcpy3DAsync(&cp, st.stream);
+    if (e != cudaSuccess) {
+        cudaFreeArray(arr);
+        return fail("cudaMemcpy3DAsync(labels)", e);
+    }
+    cudaResourceDesc rd;
+    memset(&rd, 0, sizeof(rd));
+    rd.resType = cudaResourceTypeArray;
+    rd.res.array.array = arr;
+    cudaTextureDesc td;
+    memset(&td, 0, sizeof(td));
+    // label ids are not blended: point filtering, the stored byte, voxel-index coordinates; outside the volume reads 0
+    td.addressMode[0] = td.addressMode[1] = td.addressMode[2] = cudaAddressModeBorder;
+    td.filterMode = cudaFilterModePoint;
+    td.readMode = cudaReadModeElementType;
+    td.normalizedCoords = 0;
+    cudaTextureObject_t tex = 0;
+    e = cudaCreateTextureObject(&tex, &rd, &td, nullptr);
+    if (e != cudaSuccess) {
+        cudaFreeArray(arr);
+        return fail("cudaCreateTextureObject(labels)", e);
+    }
+    e = cudaStreamSynchronize(st.stream);
+    if (e != cudaSuccess) {
+        cudaDestroyTextureObject(tex);
+        cudaFreeArray(arr);
+        return fail("cudaStreamSynchronize(svr_labels_create)", e);
+    }
+    volume_geometry(out, nx, ny, nz, sx, sy, sz);
+    out->tex = tex;
+    out->invMaxMagnitude = 1.f;
     return 0;
 }
 
@@ -440,6 +500,7 @@ extern "C" int svr_volume_upload(const svr_volume* vol, const void* data, int da
         // same dims, new contents: the grid's allocations stay, its range stage reruns at the next render
         if (rd.res.array.array == st.dev.gridArray) st.dev.rangeValid = false;
     }
+    if (rd.res.array.array == st.dev.labelArray) st.dev.labelValid = false;  // the label presence masks, likewise
     st.dev.uploadEpoch++;
     st.sceneEpoch++;
     return 0;
@@ -528,6 +589,7 @@ extern "C" int svr_volume_destroy(svr_volume* vol)
     SVR_TRY(cudaGetTextureObjectResourceDesc(&rd, vol->tex));
     SVR_TRY(cudaDeviceSynchronize());
     if (rd.resType == cudaResourceTypeArray && rd.res.array.array == st.dev.gridArray) release_grid(st);
+    if (rd.resType == cudaResourceTypeArray && rd.res.array.array == st.dev.labelArray) release_label_grid(st);
     SVR_TRY(cudaDestroyTextureObject(vol->tex));
     if (rd.resType == cudaResourceTypeArray) SVR_TRY(cudaFreeArray(rd.res.array.array));
     vol->tex = 0;

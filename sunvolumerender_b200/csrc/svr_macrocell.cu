@@ -770,6 +770,67 @@ int ensure_ranges(const svr_volume& vol, int cell)
     return 0;
 }
 
+// Label presence grid (svr_render_labels): one block per cell ORs the label bits of the cell's voxels and a one-voxel apron,
+// [cC - 1, (c+1)C], in shared memory and writes the cell's 8 words once.  The apron holds every corner the indicator of a
+// sample inside the cell reads (u = x - 1/2 lies in [cC - 1/2, (c+1)C - 1/2): corners floor(u) .. floor(u) + 1).  The label
+// texture is point-filtered with unnormalised coordinates: a fetch at the voxel centre is the voxel, outside the border's 0.
+// Label 0 is never visible and is not recorded.  A warp sets each distinct label's bit once (__match_any_sync).
+__global__ void __launch_bounds__(128) label_presence_kernel(cudaTextureObject_t labelTex, int3 grid, int cell, uint32_t* __restrict__ out)
+{
+    __shared__ uint32_t mask[8];
+    if (threadIdx.x < 8) mask[threadIdx.x] = 0u;
+    __syncthreads();
+    const int cx = blockIdx.x, cy = blockIdx.y, cz = blockIdx.z;
+    const int R = cell + 2;
+    const int x0 = cx * cell - 1, y0 = cy * cell - 1, z0 = cz * cell - 1;
+    const int total = R * R * R;
+    for (int base = 0; base < total; base += blockDim.x) {  // the same trip count for every lane: the match is warp-wide
+        const int i = base + (int)threadIdx.x;
+        uint32_t l = 0u;
+        if (i < total) {
+            const int x = i % R, y = (i / R) % R, z = i / (R * R);
+            l = tex3D<unsigned char>(labelTex, (float)(x0 + x) + 0.5f, (float)(y0 + y) + 0.5f, (float)(z0 + z) + 0.5f);
+        }
+        const uint32_t peers = __match_any_sync(0xffffffffu, l);
+        if (l != 0u && (threadIdx.x & 31) == (uint32_t)(__ffs(peers) - 1)) atomicOr(&mask[l >> 5], 1u << (l & 31u));
+    }
+    __syncthreads();
+    if (threadIdx.x < 8) out[(((size_t)cz * grid.y + cy) * grid.x + cx) * 8 + threadIdx.x] = mask[threadIdx.x];
+}
+
+int ensure_label_grid(cudaArray_t arr, cudaTextureObject_t tex, int3 dims, int cell)
+{
+    HostState& st = state();
+    DeviceState& d = st.dev;
+    if (cell == 0) cell = 8;
+    if (arr != d.labelArray || cell != d.labelCell || !d.labelPresence.p) {
+        release_label_grid(st);
+        const int3 g = make_int3((dims.x + cell - 1) / cell, (dims.y + cell - 1) / cell, (dims.z + cell - 1) / cell);
+        SVR_TRY(d.labelPresence.reserve((size_t)g.x * g.y * g.z * 8));
+        d.labelArray = arr;
+        d.labelCell = cell;
+        d.labelGridDims = g;
+    }
+    if (!d.labelValid) {
+        const dim3 g(d.labelGridDims.x, d.labelGridDims.y, d.labelGridDims.z);
+        label_presence_kernel<<<g, 128, 0, st.stream>>>(tex, d.labelGridDims, cell, d.labelPresence.p);
+        count_launch();
+        SVR_TRY(cudaGetLastError());
+        d.labelValid = true;
+    }
+    return 0;
+}
+
+void release_label_grid(HostState& st)
+{
+    DeviceState& d = st.dev;
+    d.labelPresence.release();
+    d.labelArray = nullptr;
+    d.labelCell = 0;
+    d.labelGridDims = make_int3(0, 0, 0);
+    d.labelValid = false;
+}
+
 static int build_grid(DevScene* scene, bool force, int cell, bool* majorantsRebuilt)
 {
     HostState& st = state();

@@ -1,7 +1,8 @@
 // svr_project.cu -- maximum, minimum and average intensity projection (svr_render_projection), the isosurface
 // (svr_render_isosurface), which samples the volume the same way (iso_kernel), slices and slabs (svr_render_slices), which
-// fold samples along a plane's normal as the projection folds them along a camera ray (slice_kernel), and the curved planar
-// reformation (svr_render_curved), which folds them along rays set by a frame per station of a centerline (curved_kernel).
+// fold samples along a plane's normal as the projection folds them along a camera ray (slice_kernel), the curved planar
+// reformation (svr_render_curved), which folds them along rays set by a frame per station of a centerline (curved_kernel),
+// and label maps: 3D label surfaces found like the isosurface (label_kernel) and label overlays on slices (label_slice_kernel).
 //
 // The reference has no projection mode; the sampling rule is this library's own (include/svr_render.h).  Per pixel-centre
 // ray, clipped to the volume box and its clip planes and to t >= 0: K = floor((tFar - t0) / h + 1/2) samples at
@@ -42,24 +43,27 @@ struct ProjScene {
     float3 scale;         // normalised texture coordinate -> cell coordinate
 };
 
-// The walk over the range grid shared by project_kernel, slice_kernel and iso_kernel.  visit(k) is the cell of sample k and
-// kEnd, the first index whose sample lies at or beyond the ray's exit from that cell (at least k + 1, at most K); the caller
-// drops or takes samples [k, kEnd) and continues at kEnd.
+// The walk over a macrocell grid shared by project_kernel, slice_kernel, curved_kernel, iso_kernel (the range grid) and
+// label_kernel (the label presence grid).  visit(k) is the cell of sample k (its index, x fastest) and kEnd, the first index
+// whose sample lies at or beyond the ray's exit from that cell (at least k + 1, at most K); the caller loads what its grid holds
+// for the cell, drops or takes samples [k, kEnd) and continues at kEnd.  S: a scene with vol, scale and gx, gy, gz.
 struct CellVisit {
-    float2 range;   // the cell's (min, max) before densityScale
+    size_t cell;
     uint32_t kEnd;
 };
 
 struct CellWalk {
     float3 dg, invDg;  // the ray in cell coordinates: g(t) = g(t_k) + (t - t_k) dg
 
-    SVR_DEV CellWalk(const ProjScene& s, const Ray& ray)
+    template <class S>
+    SVR_DEV CellWalk(const S& s, const Ray& ray)
     {
         dg = ray.dir * (f3(s.vol.bbox.invSize) * s.scale);
         invDg = 1.f / dg;
     }
 
-    SVR_DEV CellVisit visit(const ProjScene& s, const Ray& ray, float t0, float h, uint32_t k, uint32_t K) const
+    template <class S>
+    SVR_DEV CellVisit visit(const S& s, const Ray& ray, float t0, float h, uint32_t k, uint32_t K) const
     {
         const float t = __fadd_rn(t0, __fmul_rn((float)k + 0.5f, h));
         const float3 g = tex_coord(s.vol, ray.orig + t * ray.dir) * s.scale;
@@ -74,7 +78,7 @@ struct CellWalk {
         const float kf = ceilf((tExit - t0) / h - 0.5f);
         CellVisit c;
         c.kEnd = kf > (float)k ? (kf < (float)K ? (uint32_t)kf : K) : k + 1u;
-        c.range = __ldg(s.range + (((size_t)cz * s.gy + cy) * s.gx + cx));
+        c.cell = ((size_t)cz * s.gy + cy) * s.gx + cx;
         return c;
     }
 };
@@ -120,7 +124,7 @@ SVR_DEV float fold_samples(const ProjScene& s, const Ray& ray, float t0, float h
         while (k < kEnd) {
             const CellVisit c = walk.visit(s, ray, t0, h, k, kEnd);
             const uint32_t kNext = c.kEnd;
-            const float2 r = c.range;
+            const float2 r = __ldg(s.range + c.cell);
             lc.add(SVR_CNT_CELLS, 1);
             bool skip;
             if (OP == SVR_PROJECT_MEAN) {
@@ -181,6 +185,26 @@ __global__ void __launch_bounds__(256) project_kernel(const __grid_constant__ Pr
         }
     }
     lc.flush(cnt);
+}
+
+// The refinement of a first hit (include/svr_render.h, svr_render_isosurface) between lo and hi, value(lo) = vLo < iso <= vHi =
+// value(hi): 4 bisection steps, then the linear interpolation.  Returns (t_hit, the final bisection upper bound).
+template <class V>
+SVR_DEV float2 refine_crossing(const V& value, float iso, float lo, float hi, float vLo, float vHi)
+{
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const float m = (lo + hi) * 0.5f;
+        const float vm = value(m);
+        if (vm >= iso) {
+            hi = m;
+            vHi = vm;
+        } else {
+            lo = m;
+            vLo = vm;
+        }
+    }
+    return make_float2(lo + (hi - lo) * (iso - vLo) / (vHi - vLo), hi);
 }
 
 // Isosurface (include/svr_render.h): the first sample at or above iso along the projection's samples, refined by 4 bisection
@@ -244,7 +268,8 @@ __global__ void __launch_bounds__(256) iso_kernel(const __grid_constant__ ProjSc
                 for (uint32_t k = 0; k < K;) {
                     const CellVisit c = walk.visit(s, ray, t0, h, k, K);
                     lc.add(SVR_CNT_CELLS, 1);
-                    const float top = fmaxf(c.range.x * ds, c.range.y * ds);
+                    const float2 range = __ldg(s.range + c.cell);
+                    const float top = fmaxf(range.x * ds, range.y * ds);
                     if (top + fabsf(top) * RANGE_MARGIN < iso) {
                         lc.add(SVR_CNT_SKIPPED, c.kEnd - k);
                     } else {
@@ -263,20 +288,8 @@ __global__ void __launch_bounds__(256) iso_kernel(const __grid_constant__ ProjSc
                 found = true;
                 tHit = t_of(hit);
                 if (hit > 0u) {
-                    float lo = t_of(hit - 1u), hi = tHit, vLo = value(lo), vHi = vHit;
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const float m = (lo + hi) * 0.5f;
-                        const float vm = value(m);
-                        if (vm >= iso) {
-                            hi = m;
-                            vHi = vm;
-                        } else {
-                            lo = m;
-                            vLo = vm;
-                        }
-                    }
-                    tHit = lo + (hi - lo) * (iso - vLo) / (vHi - vLo);
+                    const float lo = t_of(hit - 1u);
+                    tHit = refine_crossing(value, iso, lo, tHit, value(lo), vHit).x;
                 }
             }
         }
@@ -631,6 +644,30 @@ void launch_slice_mode(bool skip, bool count, dim3 grid, int block, cudaStream_t
 
 bool finite3(const float* a) { return std::isfinite(a[0]) && std::isfinite(a[1]) && std::isfinite(a[2]); }
 
+// svr_render_slices' parameter errors (include/svr_render.h), reported as those of `who`; no CUDA call
+int check_slice_params(const char* who, const svr_slice_params& p)
+{
+    auto err = [&](const char* what) { return fail_msg((std::string(who) + ": " + what).c_str()); };
+    if (!finite3(p.axisU) || !finite3(p.axisV)) return err("axisU and axisV must be finite");
+    const float3 nc = cross(f3(p.axisU[0], p.axisU[1], p.axisU[2]), f3(p.axisV[0], p.axisV[1], p.axisV[2]));
+    const float nn = dot(nc, nc);
+    if (!(nn > 0.f) || !std::isfinite(nn)) return err("cross(axisU, axisV) must be nonzero and finite");
+    if (p.count > 1u && !finite3(p.axisW)) return err("axisW must be finite when count > 1");
+    if (p.imageW == 0u || p.imageW > 16384u || p.imageH == 0u || p.imageH > 16384u)
+        return err("imageW and imageH must be in 1..16384");
+    if (p.count == 0u || p.count > 65535u) return err("count must be in 1..65535");
+    if (p.mode < SVR_PROJECT_MAX || p.mode > SVR_PROJECT_MEAN) return err("mode must be 0 (max), 1 (min) or 2 (mean)");
+    if (!(p.thickness >= 0.f) || !std::isfinite(p.thickness)) return err("thickness must be finite and not negative");
+    if (p.thickness > 0.f) {
+        if (!(p.sampleSpacing > 0.f) || !std::isfinite(p.sampleSpacing))
+            return err("sampleSpacing must be positive and finite for a slab");
+        if (!(p.thickness / p.sampleSpacing <= 65536.f)) return err("thickness / sampleSpacing must be at most 65536");
+    }
+    if (!(p.windowWidth > 0.f) || !std::isfinite(p.windowWidth) || !std::isfinite(p.windowCenter))
+        return err("windowWidth must be positive and finite, windowCenter finite");
+    return 0;
+}
+
 }  // namespace
 
 extern "C" int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_slice_params* params)
@@ -639,24 +676,10 @@ extern "C" int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, cons
     if (!volume || !params) return fail_msg("svr_render_slices: null volume or params");
     if (!imgOrNull && !valueOrNull) return fail_msg("svr_render_slices: both outputs are null");
     const svr_slice_params p = *params;
-    if (!finite3(p.axisU) || !finite3(p.axisV)) return fail_msg("svr_render_slices: axisU and axisV must be finite");
+    if (int rc = check_slice_params("svr_render_slices", p)) return rc;
     const float3 u = f3(p.axisU[0], p.axisU[1], p.axisU[2]), v = f3(p.axisV[0], p.axisV[1], p.axisV[2]);
     const float3 nc = cross(u, v);
     const float nn = dot(nc, nc);
-    if (!(nn > 0.f) || !std::isfinite(nn)) return fail_msg("svr_render_slices: cross(axisU, axisV) must be nonzero and finite");
-    if (p.count > 1u && !finite3(p.axisW)) return fail_msg("svr_render_slices: axisW must be finite when count > 1");
-    if (p.imageW == 0u || p.imageW > 16384u || p.imageH == 0u || p.imageH > 16384u)
-        return fail_msg("svr_render_slices: imageW and imageH must be in 1..16384");
-    if (p.count == 0u || p.count > 65535u) return fail_msg("svr_render_slices: count must be in 1..65535");
-    if (p.mode < SVR_PROJECT_MAX || p.mode > SVR_PROJECT_MEAN) return fail_msg("svr_render_slices: mode must be 0 (max), 1 (min) or 2 (mean)");
-    if (!(p.thickness >= 0.f) || !std::isfinite(p.thickness)) return fail_msg("svr_render_slices: thickness must be finite and not negative");
-    if (p.thickness > 0.f) {
-        if (!(p.sampleSpacing > 0.f) || !std::isfinite(p.sampleSpacing))
-            return fail_msg("svr_render_slices: sampleSpacing must be positive and finite for a slab");
-        if (!(p.thickness / p.sampleSpacing <= 65536.f)) return fail_msg("svr_render_slices: thickness / sampleSpacing must be at most 65536");
-    }
-    if (!(p.windowWidth > 0.f) || !std::isfinite(p.windowWidth) || !std::isfinite(p.windowCenter))
-        return fail_msg("svr_render_slices: windowWidth must be positive and finite, windowCenter finite");
 
     SliceGeom g;
     g.center = f3(p.center[0], p.center[1], p.center[2]);
@@ -905,6 +928,391 @@ extern "C" int svr_render_curved(svr_u8vec4* imgOrNull, float* valueOrNull, cons
     if (p.mode == SVR_PROJECT_MAX) launch_curved_mode<SVR_PROJECT_MAX>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
     else if (p.mode == SVR_PROJECT_MIN) launch_curved_mode<SVR_PROJECT_MIN>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
     else launch_curved_mode<SVR_PROJECT_MEAN>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+    return 0;
+}
+
+namespace svr {
+namespace {
+
+// ---- label maps (include/svr_render.h: svr_render_labels, svr_render_label_slices) ----------------------------------------
+
+// The label table as the kernels read it, a launch parameter (4128 bytes): colours and the 256-bit visibility mask
+struct LabelTable {
+    float4 color[256];
+    uint32_t vis[8];  // bit l: label l is visible (l != 0 and color[l].w > 0)
+};
+
+struct LabelScene {
+    svr_volume vol;          // a label volume: point-filtered u8, unnormalised coordinates, border 0
+    svr_camera cam;
+    float3 dims;             // (nx, ny, nz)
+    const uint4* presence;   // with skipping: per cell 8 words (2 uint4), the labels of the cell and its one-voxel apron
+    int gx, gy, gz;
+    float3 scale;            // normalised texture coordinate -> cell coordinate (CellWalk)
+};
+
+SVR_DEV uint32_t label_at(const svr_volume& v, int i, int j, int k)
+{
+    return tex3D<unsigned char>(v.tex, (float)i + 0.5f, (float)j + 0.5f, (float)k + 0.5f);
+}
+
+SVR_DEV bool label_visible(const LabelTable& t, uint32_t l) { return (t.vis[l >> 5] >> (l & 31u)) & 1u; }
+
+SVR_DEV float lerp_rn(float a, float b, float f) { return __fadd_rn(__fmul_rn(__fsub_rn(1.f, f), a), __fmul_rn(f, b)); }
+
+// The 8 corners around x: u = tex_coord(x) dims - 1/2, i = floor(u), f = u - i; v[c] = vis of corner c (x fastest), lab[c] its label
+struct LabelCorners {
+    float3 f;
+    float v[8];
+    uint32_t lab[8];
+};
+
+SVR_DEV LabelCorners label_corners(const LabelScene& s, const LabelTable& t, float3 x)
+{
+    const float3 tc = tex_coord(s.vol, x);
+    const float ux = __fsub_rn(__fmul_rn(tc.x, s.dims.x), 0.5f), uy = __fsub_rn(__fmul_rn(tc.y, s.dims.y), 0.5f),
+                uz = __fsub_rn(__fmul_rn(tc.z, s.dims.z), 0.5f);
+    const float ix = floorf(ux), iy = floorf(uy), iz = floorf(uz);
+    LabelCorners c;
+    c.f = f3(__fsub_rn(ux, ix), __fsub_rn(uy, iy), __fsub_rn(uz, iz));
+#pragma unroll
+    for (int n = 0; n < 8; ++n) {
+        c.lab[n] = label_at(s.vol, (int)ix + (n & 1), (int)iy + ((n >> 1) & 1), (int)iz + (n >> 2));
+        c.v[n] = label_visible(t, c.lab[n]) ? 1.f : 0.f;
+    }
+    return c;
+}
+
+// m(x): the trilinear interpolation of the visible labels' indicator
+SVR_DEV float label_indicator(const LabelScene& s, const LabelTable& t, float3 x)
+{
+    const LabelCorners c = label_corners(s, t, x);
+    const float y0 = lerp_rn(lerp_rn(c.v[0], c.v[1], c.f.x), lerp_rn(c.v[2], c.v[3], c.f.x), c.f.y);
+    const float y1 = lerp_rn(lerp_rn(c.v[4], c.v[5], c.f.x), lerp_rn(c.v[6], c.v[7], c.f.x), c.f.y);
+    return lerp_rn(y0, y1, c.f.z);
+}
+
+// The visible label with the largest summed corner weight at x, ties to the smaller id (0 if no corner is visible)
+SVR_DEV uint32_t label_pick(const LabelScene& s, const LabelTable& t, float3 x)
+{
+    const LabelCorners c = label_corners(s, t, x);
+    float w[8];
+#pragma unroll
+    for (int n = 0; n < 8; ++n) {
+        const float wx = n & 1 ? c.f.x : __fsub_rn(1.f, c.f.x), wy = (n >> 1) & 1 ? c.f.y : __fsub_rn(1.f, c.f.y),
+                    wz = n >> 2 ? c.f.z : __fsub_rn(1.f, c.f.z);
+        w[n] = c.v[n] != 0.f ? __fmul_rn(__fmul_rn(wx, wy), wz) : 0.f;
+    }
+    uint32_t best = 0u;
+    float bestW = -1.f;
+#pragma unroll
+    for (int a = 0; a < 8; ++a) {
+        if (c.v[a] == 0.f) continue;
+        float sum = 0.f;
+#pragma unroll
+        for (int b = 0; b < 8; ++b)
+            if (c.lab[b] == c.lab[a]) sum = __fadd_rn(sum, w[b]);
+        if (sum > bestW || (sum == bestW && c.lab[a] < best)) {
+            best = c.lab[a];
+            bestW = sum;
+        }
+    }
+    return best;
+}
+
+// The analytic gradient of m at x in world units: the derivative of the trilinear weights times dims * invSize
+SVR_DEV float3 label_gradient(const LabelScene& s, const LabelTable& t, float3 x)
+{
+    const LabelCorners c = label_corners(s, t, x);
+    const float* v = c.v;
+    const float3 f = c.f;
+    const float dx = lerp_rn(lerp_rn(v[1] - v[0], v[3] - v[2], f.y), lerp_rn(v[5] - v[4], v[7] - v[6], f.y), f.z);
+    const float dy = lerp_rn(lerp_rn(v[2] - v[0], v[3] - v[1], f.x), lerp_rn(v[6] - v[4], v[7] - v[5], f.x), f.z);
+    const float dz = lerp_rn(lerp_rn(v[4] - v[0], v[5] - v[1], f.x), lerp_rn(v[6] - v[2], v[7] - v[3], f.x), f.y);
+    return f3(__fmul_rn(dx, __fmul_rn(s.dims.x, s.vol.bbox.invSize.x)), __fmul_rn(dy, __fmul_rn(s.dims.y, s.vol.bbox.invSize.y)),
+              __fmul_rn(dz, __fmul_rn(s.dims.z, s.vol.bbox.invSize.z)));
+}
+
+// 3D label surfaces (include/svr_render.h): iso_kernel's rays, samples, hit search and refinement on m with iso = 1/2.  Skipping
+// drops the samples of cells whose presence mask holds no visible label (m = 0 < 1/2 on all of them); the refinement recomputes
+// the sample before the hit from its index.
+template <bool SKIP, bool COUNT>
+__global__ void __launch_bounds__(256) label_kernel(const __grid_constant__ LabelScene s, const __grid_constant__ LabelTable t, float stepSize,
+                                                    uint32_t* __restrict__ img, float4* __restrict__ surface, uint8_t* __restrict__ label,
+                                                    uint32_t y1, uint32_t bandPhase, uint32_t bandStride, Counters* cnt)
+{
+    const uint2 pix = band_pixel(0u, y1, bandPhase, bandStride);
+    const uint32_t idx = pix.x, idy = pix.y;
+    const bool inside = idx < s.cam.imageW && idy < y1;
+    LocalCounters<COUNT> lc;
+    Ray ray;
+    bool found = false;
+    float tHit = 0.f, tHi = 0.f;
+    if (inside) {
+        ray = camera_ray_center(s.cam, idx, idy);
+        lc.add(SVR_CNT_PATHS, 1);
+        float tNear, tFar;
+        if (intersect_volume(s.vol, ray, &tNear, &tFar)) {
+            const float h = stepSize * 0.5f;
+            const float t0 = fmaxf(tNear, 0.f);
+            const float span = tFar > t0 ? floorf(__fadd_rn(__fsub_rn(tFar, t0) / h, 0.5f)) : 0.f;
+            const uint32_t K = (uint32_t)span;
+            auto t_of = [&](uint32_t k) { return __fadd_rn(t0, __fmul_rn((float)k + 0.5f, h)); };
+            auto value = [&](float tt) { return label_indicator(s, t, ray.orig + tt * ray.dir); };
+            float vHit = 0.f;
+            auto find = [&](uint32_t k, uint32_t kEnd) {
+                for (; k < kEnd; ++k) {
+                    const float v = value(t_of(k));
+                    if (v >= 0.5f) {
+                        vHit = v;
+                        return k;
+                    }
+                }
+                return kEnd;
+            };
+            uint32_t hit = K;
+            if constexpr (!SKIP) {
+                hit = find(0u, K);
+                lc.add(SVR_CNT_SHADE_TAPS, hit < K ? hit + 1u : K);
+            } else {
+                const CellWalk walk(s, ray);
+                for (uint32_t k = 0; k < K;) {
+                    const CellVisit c = walk.visit(s, ray, t0, h, k, K);
+                    lc.add(SVR_CNT_CELLS, 1);
+                    const uint4 p0 = __ldg(s.presence + 2 * c.cell), p1 = __ldg(s.presence + 2 * c.cell + 1);
+                    const uint32_t any = (p0.x & t.vis[0]) | (p0.y & t.vis[1]) | (p0.z & t.vis[2]) | (p0.w & t.vis[3]) | (p1.x & t.vis[4]) |
+                                         (p1.y & t.vis[5]) | (p1.z & t.vis[6]) | (p1.w & t.vis[7]);
+                    if (any == 0u) {
+                        lc.add(SVR_CNT_SKIPPED, c.kEnd - k);
+                    } else {
+                        const uint32_t f = find(k, c.kEnd);
+                        lc.add(SVR_CNT_SHADE_TAPS, (f < c.kEnd ? f + 1u : c.kEnd) - k);
+                        if (f < c.kEnd) {
+                            hit = f;
+                            break;
+                        }
+                    }
+                    k = c.kEnd;
+                }
+            }
+            lc.add(SVR_CNT_STEPS, hit < K ? hit + 1u : K);
+            if (hit < K) {
+                found = true;
+                tHit = tHi = t_of(hit);
+                if (hit > 0u) {
+                    const float lo = t_of(hit - 1u);
+                    const float2 r = refine_crossing(value, 0.5f, lo, tHit, value(lo), vHit);
+                    tHit = r.x;
+                    tHi = r.y;
+                }
+            }
+        }
+    }
+    // as iso_kernel: the counts are complete, flushed before the shading
+    lc.flush(cnt);
+    if (!inside) return;
+    uint32_t rgba = 0u, lab = 0u;
+    float4 surf = make_float4(0.f, 0.f, 0.f, INFINITY);
+    if (found) {
+        lab = label_pick(s, t, ray.orig + tHi * ray.dir);
+        const float3 x = ray.orig + tHit * ray.dir;
+        const float3 camPos = f3(s.cam.pos);
+        const float3 g = label_gradient(s, t, x);
+        float3 n = f3(0.f);
+        float cosTerm = 1.f, specularTerm = 0.f;
+        if (dot(g, g) > 0.f) {
+            n = normalize(g);
+            if (dot(n, ray.dir) > 0.f) n = -n;
+            cosTerm = fabsf(dot(n, normalize(camPos - x)));
+            specularTerm = powf(cosTerm, 30.f);
+        }
+        const float4 color = t.color[lab];
+        const float r = fminf(color.x * cosTerm * 0.8f + specularTerm * 0.2f, 1.f);
+        const float gr = fminf(color.y * cosTerm * 0.8f + specularTerm * 0.2f, 1.f);
+        const float b = fminf(color.z * cosTerm * 0.8f + specularTerm * 0.2f, 1.f);
+        rgba = pack_u8x4(r * 255.f, gr * 255.f, b * 255.f, 255.f);
+        surf = make_float4(n.x, n.y, n.z, dot(x - camPos, -f3(s.cam.w)));
+    }
+    const size_t offset = (size_t)idy * s.cam.imageW + idx;
+    if (img) img[offset] = rgba;
+    if (surface) surface[offset] = surf;
+    if (label) label[offset] = (uint8_t)lab;
+}
+
+// The slice geometry of svr_render_label_slices, from the host: svr_render_slices' pixel centres and clipped box
+struct LabelSliceScene {
+    svr_volume vol;
+    float3 center, u, v, w, cmin, cmax, dims;
+    uint32_t W, H;
+};
+
+// L of pixel (x, y) of image j: the label of the voxel holding the pixel centre, 0 outside the clipped box
+SVR_DEV uint32_t slice_label(const LabelSliceScene& g, uint32_t x, uint32_t y, uint32_t j)
+{
+    const float fx = __fsub_rn((float)x + 0.5f, 0.5f * (float)g.W), fy = __fsub_rn((float)y + 0.5f, 0.5f * (float)g.H);
+    const float3 c = g.center + fx * g.u + fy * g.v + (float)j * g.w;
+    if (!(c.x >= g.cmin.x && c.y >= g.cmin.y && c.z >= g.cmin.z && c.x <= g.cmax.x && c.y <= g.cmax.y && c.z <= g.cmax.z)) return 0u;
+    const float3 tc = tex_coord(g.vol, c);
+    return label_at(g.vol, (int)floorf(__fmul_rn(tc.x, g.dims.x)), (int)floorf(__fmul_rn(tc.y, g.dims.y)), (int)floorf(__fmul_rn(tc.z, g.dims.z)));
+}
+
+SVR_DEV uint32_t blend_channel(uint32_t in, float a, float c)
+{
+    return (uint32_t)__fadd_rn(__fadd_rn(__fmul_rn(__fsub_rn(1.f, a), (float)in), __fmul_rn(a, __fmul_rn(255.f, c))), 0.5f);
+}
+
+// Label overlays (include/svr_render.h): pixel (x, y) of image blockIdx.z
+__global__ void __launch_bounds__(256) label_slice_kernel(const __grid_constant__ LabelSliceScene g, const __grid_constant__ LabelTable t,
+                                                          uint32_t* __restrict__ img, uint8_t* __restrict__ label, int outline)
+{
+    const uint2 pix = band_pixel(0u, g.H, 0u, 1u);
+    const uint32_t x = pix.x, y = pix.y, j = blockIdx.z;
+    if (x >= g.W || y >= g.H) return;
+    const uint32_t L = slice_label(g, x, y, j);
+    const size_t offset = ((size_t)j * g.H + y) * g.W + x;
+    if (label) label[offset] = (uint8_t)L;
+    if (!img || !label_visible(t, L)) return;
+    bool edge = false;
+    if (outline)
+        edge = (x > 0u && slice_label(g, x - 1u, y, j) != L) || (x + 1u < g.W && slice_label(g, x + 1u, y, j) != L) ||
+               (y > 0u && slice_label(g, x, y - 1u, j) != L) || (y + 1u < g.H && slice_label(g, x, y + 1u, j) != L);
+    const float4 col = t.color[L];
+    const float a = edge ? 1.f : col.w;
+    const uint32_t in = img[offset];
+    img[offset] = blend_channel(in & 255u, a, col.x) | (blend_channel((in >> 8) & 255u, a, col.y) << 8) |
+                  (blend_channel((in >> 16) & 255u, a, col.z) << 16) | (255u << 24);
+}
+
+// The table errors of include/svr_render.h (no CUDA call), and the table the kernels read
+int make_label_table(const char* who, const svr_label_params& p, LabelTable* t)
+{
+    memset(t, 0, sizeof(*t));
+    for (int l = 0; l < 256; ++l) {
+        for (int c = 0; c < 4; ++c)
+            if (!(p.color[l][c] >= 0.f && p.color[l][c] <= 1.f)) {
+                char msg[160];
+                snprintf(msg, sizeof(msg), "%s: table entry color[%d][%d] must be finite and in [0, 1]", who, l, c);
+                return fail_msg(msg);
+            }
+        t->color[l] = make_float4(p.color[l][0], p.color[l][1], p.color[l][2], p.color[l][3]);
+        if (l != 0 && p.color[l][3] > 0.f) t->vis[l >> 5] |= 1u << (l & 31);
+    }
+    return 0;
+}
+
+// A label volume is a point-filtered, unnormalised, element-type 8-bit unsigned 3-D array (svr_labels_create): its array and dims
+int label_volume(const char* who, const svr_volume& v, cudaArray_t* arr, int3* dims)
+{
+    auto err = [&]() { return fail_msg((std::string(who) + ": the volume is not a label volume (svr_labels_create)").c_str()); };
+    if (!v.tex) return err();
+    cudaTextureDesc td;
+    SVR_TRY(cudaGetTextureObjectTextureDesc(&td, v.tex));
+    cudaResourceDesc rd;
+    SVR_TRY(cudaGetTextureObjectResourceDesc(&rd, v.tex));
+    if (rd.resType != cudaResourceTypeArray || td.filterMode != cudaFilterModePoint || td.readMode != cudaReadModeElementType || td.normalizedCoords)
+        return err();
+    cudaChannelFormatDesc ch;
+    cudaExtent ext;
+    unsigned int flags = 0;
+    SVR_TRY(cudaArrayGetInfo(&ch, &ext, &flags, rd.res.array.array));
+    if (ch.x != 8 || ch.y || ch.z || ch.w || ch.f != cudaChannelFormatKindUnsigned || ext.depth == 0) return err();
+    *arr = rd.res.array.array;
+    *dims = make_int3((int)ext.width, (int)ext.height, (int)ext.depth);
+    return 0;
+}
+
+}  // namespace
+}  // namespace svr
+
+extern "C" int svr_render_labels(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrNull, uint8_t* labelOrNull, const svr_volume* labels,
+                                 const svr_camera* camera, const svr_label_params* table, float stepSize, uint32_t phase, uint32_t stride,
+                                 uint32_t* bandRows)
+{
+    HostState& st = state();
+    const char* who = "svr_render_labels";
+    if (!labels || !camera || !table) return fail_msg("svr_render_labels: null labels volume, camera or table");
+    if (!imgOrNull && !surfaceOrNull && !labelOrNull) return fail_msg("svr_render_labels: all three outputs are null");
+    if (!(stepSize > 0.f) || !std::isfinite(stepSize)) return fail_msg("svr_render_labels: stepSize must be positive and finite");
+    LabelTable t;
+    if (int rc = make_label_table(who, *table, &t)) return rc;
+    if (phase >= stride) return fail_msg("svr_render_labels: band phase must be below the band stride");
+    cudaArray_t arr;
+    int3 dims;
+    if (int rc = label_volume(who, *labels, &arr, &dims)) return rc;
+    const int block = st.options[SVR_OPT_RC_BLOCK];
+    const uint32_t tileH = (uint32_t)block / 16u;
+    if (bandRows) *bandRows = tileH;
+
+    LabelScene sc;
+    memset(&sc, 0, sizeof(sc));
+    sc.vol = *labels;
+    sc.cam = *camera;
+    sc.dims = f3((float)dims.x, (float)dims.y, (float)dims.z);
+    const bool skip = st.options[SVR_OPT_RC_SKIP] != 0;
+    const bool count = st.options[SVR_OPT_COUNTERS] != 0;
+    if (skip) {
+        if (int rc = ensure_label_grid(arr, labels->tex, dims, st.options[SVR_OPT_MACROCELL_SIZE])) return rc;
+        const DeviceState& d = st.dev;
+        sc.presence = (const uint4*)d.labelPresence.p;
+        sc.gx = d.labelGridDims.x;
+        sc.gy = d.labelGridDims.y;
+        sc.gz = d.labelGridDims.z;
+        sc.scale = f3((float)dims.x / (float)d.labelCell, (float)dims.y / (float)d.labelCell, (float)dims.z / (float)d.labelCell);
+    }
+    dim3 grid;
+    if (!band_grid(*camera, tileH, phase, stride, &grid)) return 0;
+    Counters* cnt = count ? device_counters() : nullptr;
+    if (count && !cnt) return fail_msg("svr_render_labels: counter allocation failed");
+    const uint32_t H = camera->imageH;
+    uint32_t* img = (uint32_t*)imgOrNull;
+    float4* surface = (float4*)surfaceOrNull;
+    if (skip) {
+        if (count) label_kernel<true, true><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
+        else label_kernel<true, false><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
+    } else {
+        if (count) label_kernel<false, true><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
+        else label_kernel<false, false><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
+    }
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int svr_render_label_slices(svr_u8vec4* imgOrNull, uint8_t* labelOrNull, const svr_volume* labels, const svr_slice_params* params,
+                                       const svr_label_params* table, int outline)
+{
+    HostState& st = state();
+    const char* who = "svr_render_label_slices";
+    if (!labels || !params || !table) return fail_msg("svr_render_label_slices: null labels volume, params or table");
+    if (!imgOrNull && !labelOrNull) return fail_msg("svr_render_label_slices: both outputs are null");
+    const svr_slice_params p = *params;
+    if (int rc = check_slice_params(who, p)) return rc;
+    LabelTable t;
+    if (int rc = make_label_table(who, *table, &t)) return rc;
+    if (outline != 0 && outline != 1) return fail_msg("svr_render_label_slices: outline must be 0 or 1");
+    cudaArray_t arr;
+    int3 dims;
+    if (int rc = label_volume(who, *labels, &arr, &dims)) return rc;
+
+    LabelSliceScene g;
+    memset(&g, 0, sizeof(g));
+    const svr_volume& vo = *labels;
+    g.vol = vo;
+    g.center = f3(p.center[0], p.center[1], p.center[2]);
+    g.u = f3(p.axisU[0], p.axisU[1], p.axisU[2]);
+    g.v = f3(p.axisV[0], p.axisV[1], p.axisV[2]);
+    g.w = p.count > 1u ? f3(p.axisW[0], p.axisW[1], p.axisW[2]) : f3(0.f);
+    g.cmin = f3(vo.bbox.vmin.x * -vo.x_clip.x, vo.bbox.vmin.y * -vo.y_clip.x, vo.bbox.vmin.z * -vo.z_clip.x);
+    g.cmax = f3(vo.bbox.vmax.x * vo.x_clip.y, vo.bbox.vmax.y * vo.y_clip.y, vo.bbox.vmax.z * vo.z_clip.y);
+    g.dims = f3((float)dims.x, (float)dims.y, (float)dims.z);
+    g.W = p.imageW;
+    g.H = p.imageH;
+    const int block = st.options[SVR_OPT_RC_BLOCK];
+    const uint32_t tileH = (uint32_t)block / 16u;
+    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + tileH - 1u) / tileH, p.count);
+    label_slice_kernel<<<grid, block, 0, st.stream>>>(g, t, (uint32_t*)imgOrNull, labelOrNull, outline);
     count_launch();
     SVR_TRY(cudaGetLastError());
     return 0;

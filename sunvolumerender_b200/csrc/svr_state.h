@@ -159,6 +159,15 @@ struct DeviceState {
     size_t curveStageCap = 0;
     cudaEvent_t curveStageEvent = nullptr;
 
+    // Label presence grid (svr_render_labels, svr_macrocell.cu): per cell of labelCell voxels, the 256-bit mask (8 words) of the
+    // labels in the cell and its one-voxel apron, for labelArray; kept apart from the grey range grid above, which a label
+    // render never touches.  labelValid is false until the masks reflect the array's voxels (svr_volume_upload clears it).
+    cudaArray_t labelArray = nullptr;
+    int labelCell = 0;
+    int3 labelGridDims = {0, 0, 0};
+    DevBuf<uint32_t> labelPresence;
+    bool labelValid = false;
+
     DevBuf<Counters> counters;
 
     // Frees every allocation, event, view and the mailbox, and returns every key and flag to its default (svr_api.cu)
@@ -190,6 +199,11 @@ HostState& state();
 
 // drops the macrocell cache (range grid, majorants, distances, point-sampled view)
 void release_grid(HostState& st);
+// drops the label presence grid
+void release_label_grid(HostState& st);
+// The label presence grid of the label volume behind `tex` (array `arr`, dims voxels) for cell edge `cell` (0: 8) into
+// dev.labelPresence / dev.labelGridDims / dev.labelCell, built when the array, the edge or the voxels changed.
+int ensure_label_grid(cudaArray_t arr, cudaTextureObject_t tex, int3 dims, int cell);
 
 // Part-1 error convention, utils/helper_cuda.h:967-981: print, cudaDeviceReset, exit(EXIT_FAILURE)
 inline void check_fatal(cudaError_t e, const char* what, const char* file, int line)

@@ -365,46 +365,121 @@ extern "C" int svr_volume_load_metaimage(const char* path, svr_volume* out, svr_
     }
 }
 
-static int load_metaimage(const char* path, svr_volume* out, svr_volume_stats* stats, uint32_t* histogram, uint32_t histogram_capacity)
+// The data half of a MetaImage load: the element data of the file `path` whose header is `hd`, raw or zlib, into buf (dim[0] *
+// dim[1] * dim[2] elements of hd.element_type, in file byte order); errors are reported as those of `who`.  Host only.
+static int read_metaimage_data(const char* who, const char* path, const svr_metaimage_header& hd, std::vector<unsigned char>* buf)
 {
-    svr_metaimage_header hd;
-    int rc = svr_metaimage_read_header(path, &hd);
-    if (rc) return rc;
-    if (hd.channels != 1) return fail_msg("svr_volume_load_metaimage: only single-channel volumes are renderable");
+    auto err = [&](const std::string& what) { return fail_msg((std::string(who) + ": " + what).c_str()); };
     const size_t n = (size_t)hd.dim[0] * hd.dim[1] * hd.dim[2], bytes = n * met_size(hd.element_type);
     const char* dataPath = hd.data_file[0] ? hd.data_file : path;
     std::ifstream f(dataPath, std::ios::binary | std::ios::ate);
-    if (!f) return fail_msg((std::string("svr_volume_load_metaimage: cannot open ") + dataPath).c_str());
+    if (!f) return err((std::string("cannot open ") + dataPath).c_str());
     const uint64_t fileSize = (uint64_t)f.tellg();
     uint64_t start = hd.data_file[0] ? 0 : hd.data_offset;
     if (hd.data_file[0]) {
         if (hd.header_size > 0) start = (uint64_t)hd.header_size;
         else if (hd.header_size == -1 && !hd.compressed) start = fileSize >= bytes ? fileSize - bytes : 0;
     }
-    std::vector<unsigned char> buf;
-    if (start > fileSize) return fail_msg("svr_volume_load_metaimage: HeaderSize lies beyond the end of the data file");
+    if (start > fileSize) return err("HeaderSize lies beyond the end of the data file");
     if (hd.compressed) {
         uint64_t csize = hd.compressed_size ? hd.compressed_size : fileSize - start;
-        if (csize > fileSize - start) return fail_msg("svr_volume_load_metaimage: compressed data is truncated");
+        if (csize > fileSize - start) return err("compressed data is truncated");
         // zlib's deflate cannot shrink data by more than about 1032 : 1: a header that promises more than the
         // compressed bytes can hold is rejected before anything of that size is allocated
-        if (bytes / 1100 > csize + 64) return fail_msg("svr_volume_load_metaimage: DimSize x ElementType cannot come out of the compressed data");
+        if (bytes / 1100 > csize + 64) return err("DimSize x ElementType cannot come out of the compressed data");
         std::vector<unsigned char> cbuf(csize);
         f.seekg((std::streamoff)start);
         f.read((char*)cbuf.data(), (std::streamsize)csize);
-        buf.resize(bytes);
+        buf->resize(bytes);
         uLongf dlen = (uLongf)bytes;
-        int z = uncompress(buf.data(), &dlen, cbuf.data(), (uLong)csize);
-        if (z != Z_OK || dlen != bytes) return fail_msg("svr_volume_load_metaimage: zlib inflate failed or size mismatch");
+        int z = uncompress(buf->data(), &dlen, cbuf.data(), (uLong)csize);
+        if (z != Z_OK || dlen != bytes) return err("zlib inflate failed or size mismatch");
     } else {
-        if (bytes > fileSize - start) return fail_msg("svr_volume_load_metaimage: data file is shorter than DimSize x ElementType");
-        buf.resize(bytes);
+        if (bytes > fileSize - start) return err("data file is shorter than DimSize x ElementType");
+        buf->resize(bytes);
         f.seekg((std::streamoff)start);
-        f.read((char*)buf.data(), (std::streamsize)bytes);
-        if (!f) return fail_msg("svr_volume_load_metaimage: short read");
+        f.read((char*)buf->data(), (std::streamsize)bytes);
+        if (!f) return err("short read");
     }
+    return 0;
+}
+
+static int load_metaimage(const char* path, svr_volume* out, svr_volume_stats* stats, uint32_t* histogram, uint32_t histogram_capacity)
+{
+    svr_metaimage_header hd;
+    int rc = svr_metaimage_read_header(path, &hd);
+    if (rc) return rc;
+    if (hd.channels != 1) return fail_msg("svr_volume_load_metaimage: only single-channel volumes are renderable");
+    std::vector<unsigned char> buf;
+    rc = read_metaimage_data("svr_volume_load_metaimage", path, hd, &buf);
+    if (rc) return rc;
     return svr_volume_from_raw(buf.data(), hd.element_type, hd.msb, hd.dim[0], hd.dim[1], hd.dim[2], hd.spacing[0], hd.spacing[1],
                                hd.spacing[2], out, stats, histogram, histogram_capacity);
+}
+
+static int load_labels(const char* path, svr_volume* out, uint32_t* maxLabelOrNull);
+
+extern "C" int svr_labels_load_metaimage(const char* path, svr_volume* out, uint32_t* maxLabelOrNull)
+{
+    if (!path || !out) return fail_msg("svr_labels_load_metaimage: null path or out");
+    try {
+        return load_labels(path, out, maxLabelOrNull);
+    } catch (const std::bad_alloc&) {
+        return fail_msg("svr_labels_load_metaimage: out of host memory");
+    } catch (...) {
+        return fail_msg("svr_labels_load_metaimage: unexpected exception");
+    }
+}
+
+// element i of the file's data as an integer, byte-swapped when the file is big-endian
+template <typename T>
+static long long met_int(const unsigned char* data, size_t i, bool swap)
+{
+    unsigned char b[sizeof(T)];
+    memcpy(b, data + i * sizeof(T), sizeof(T));
+    if (swap) std::reverse(b, b + sizeof(T));
+    T v;
+    memcpy(&v, b, sizeof(T));
+    return (long long)v;
+}
+
+static int load_labels(const char* path, svr_volume* out, uint32_t* maxLabelOrNull)
+{
+    svr_metaimage_header hd;
+    int rc = svr_metaimage_read_header(path, &hd);
+    if (rc) return rc;
+    if (hd.channels != 1) return fail_msg("svr_labels_load_metaimage: a label map has one channel");
+    if (hd.element_type == SVR_MET_FLOAT || hd.element_type == SVR_MET_DOUBLE)
+        return fail_msg("svr_labels_load_metaimage: label ids must be integers (ElementType MET_FLOAT / MET_DOUBLE)");
+    std::vector<unsigned char> buf;
+    rc = read_metaimage_data("svr_labels_load_metaimage", path, hd, &buf);
+    if (rc) return rc;
+    const size_t n = (size_t)hd.dim[0] * hd.dim[1] * hd.dim[2];
+    const bool swap = hd.msb != 0;
+    std::vector<uint8_t> lab(n);
+    uint32_t maxLabel = 0;
+    for (size_t i = 0; i < n; ++i) {
+        long long v;
+        switch (hd.element_type) {
+            case SVR_MET_UCHAR: v = buf[i]; break;
+            case SVR_MET_CHAR: v = (signed char)buf[i]; break;
+            case SVR_MET_USHORT: v = met_int<uint16_t>(buf.data(), i, swap); break;
+            case SVR_MET_SHORT: v = met_int<int16_t>(buf.data(), i, swap); break;
+            case SVR_MET_UINT: v = met_int<uint32_t>(buf.data(), i, swap); break;
+            default: v = met_int<int32_t>(buf.data(), i, swap); break;
+        }
+        if (v < 0 || v > 255) {
+            char msg[160];
+            snprintf(msg, sizeof(msg), "svr_labels_load_metaimage: label value %lld at voxel %zu is outside 0..255", v, i);
+            return fail_msg(msg);
+        }
+        lab[i] = (uint8_t)v;
+        maxLabel = std::max(maxLabel, (uint32_t)v);
+    }
+    rc = svr_labels_create(out, lab.data(), 0, hd.dim[0], hd.dim[1], hd.dim[2], hd.spacing[0], hd.spacing[1], hd.spacing[2]);
+    if (rc) return rc;
+    if (maxLabelOrNull) *maxLabelOrNull = maxLabel;
+    return 0;
 }
 
 extern "C" int svr_volume_download(const svr_volume* vol, void* host_out, uint64_t bytes)

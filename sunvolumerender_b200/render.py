@@ -27,6 +27,7 @@ class Renderer:
         L.check(self.lib.svr_set_device(device), "svr_set_device")
         self.sync_stream()
         self.volume = None
+        self.labels = None
         self.tf = None
         self._tf_size = 0
         self.camera = None
@@ -370,6 +371,72 @@ class Renderer:
                 "svr_render_curved")
         return value, img
 
+    # ---- label maps (one label volume per renderer, on the grid of the bound volume when dims and spacing match)
+    def load_labels(self, data, spacing=(1.0, 1.0, 1.0)):
+        """A label volume (svr_labels_create) from u8 label ids shaped (nz, ny, nx): a host numpy array or a device tensor.
+        Replaces the renderer's label volume."""
+        self.free_labels()
+        if isinstance(data, torch.Tensor):
+            if data.dtype != torch.uint8 or data.dim() != 3:
+                raise ValueError("load_labels: a uint8 tensor shaped (nz, ny, nx)")
+            data = data.contiguous()
+            on_device, ptr = (1 if data.is_cuda else 0), _ptr(data)
+        else:
+            data = np.ascontiguousarray(data)
+            if data.dtype != np.uint8 or data.ndim != 3:
+                raise ValueError("load_labels: a uint8 array shaped (nz, ny, nx)")
+            on_device, ptr = 0, C.c_void_p(data.ctypes.data)
+        nz, ny, nx = data.shape
+        vol = L.Volume()
+        L.check(self.lib.svr_labels_create(C.byref(vol), ptr, on_device, nx, ny, nz, spacing[0], spacing[1], spacing[2]), "svr_labels_create")
+        self.labels = vol
+        return vol
+
+    def load_label_metaimage(self, path):
+        """A label volume from a MetaImage file (svr_labels_load_metaimage); returns the largest label id."""
+        self.free_labels()
+        vol, max_label = L.Volume(), C.c_uint32(0)
+        L.check(self.lib.svr_labels_load_metaimage(str(path).encode(), C.byref(vol), C.byref(max_label)), "svr_labels_load_metaimage")
+        self.labels = vol
+        return int(max_label.value)
+
+    def upload_labels(self, data):
+        """New label ids (same dims) into the label volume: a host numpy array or a host or device uint8 tensor."""
+        if isinstance(data, torch.Tensor):
+            data = data.contiguous()
+            on_device, ptr = (1 if data.is_cuda else 0), _ptr(data)
+        else:
+            data = np.ascontiguousarray(data, dtype=np.uint8)
+            on_device, ptr = 0, C.c_void_p(data.ctypes.data)
+        L.check(self.lib.svr_volume_upload(C.byref(self.labels), ptr, on_device), "svr_volume_upload")
+
+    def free_labels(self):
+        if self.labels is not None:
+            L.check(self.lib.svr_volume_destroy(C.byref(self.labels)), "svr_volume_destroy")
+            self.labels = None
+
+    def render_labels(self, table, step_size=None, surface=None, labels=None, img_ptr=None, phase=0, stride=1):
+        """3D label surfaces (svr_render_labels) of the label volume from the bound camera; table: an L.LabelParams
+        (scene.label_table).  surface: optional float tensor, four values per pixel (normal, view-space depth); labels: optional
+        uint8 tensor, the label hit per pixel (0 = none).  The u8 image goes to self.img, or to img_ptr, a raw device pointer.
+        phase / stride: the row bands of render_raycasting_bands.  Returns the band height."""
+        if step_size is None:
+            step_size = S.raycast_step_size(self.labels.spacing.tuple())
+        rows = C.c_uint32(0)
+        L.check(self.lib.svr_render_labels(img_ptr if img_ptr is not None else _ptr(self.img), _ptr(surface), _ptr(labels), C.byref(self.labels),
+                                           C.byref(self.camera), C.byref(table), step_size, phase, stride, C.byref(rows)), "svr_render_labels")
+        return int(rows.value)
+
+    def render_label_slices(self, params, table, img=None, labels=None, outline=False):
+        """Label overlays (svr_render_label_slices) on the slices of params (an L.SliceParams, as given to render_slices):
+        img, a uint8 (count, H, W, 4) device tensor holding the grey slices, is composited in place where given; labels, uint8
+        (count, H, W), receives the label per pixel and is allocated when not given.  Returns (labels, img)."""
+        if labels is None:
+            labels = torch.empty((params.count, params.imageH, params.imageW), dtype=torch.uint8, device=self.device)
+        L.check(self.lib.svr_render_label_slices(_ptr(img), _ptr(labels), C.byref(self.labels), C.byref(params), C.byref(table),
+                                                 1 if outline else 0), "svr_render_label_slices")
+        return labels, img
+
     # ---- results
     def hdr_image(self):
         return self.hdr.view(self.camera.imageH, self.camera.imageW, 3)
@@ -379,6 +446,7 @@ class Renderer:
 
     def close(self):
         self.free_volume()
+        self.free_labels()
         if self.tf is not None:
             self.lib.svr_tf_destroy(C.byref(self.tf))
             self.tf = None

@@ -301,6 +301,45 @@ def curve_frames(points, up, station_spacing, n):
     return out
 
 
+# label maps (svr_render_labels, svr_render_label_slices): the levels of the generated CT's skin, soft tissue and bone, on its
+# normalised values (svr_generate_volume writes shells at 0.25, 0.45 and 0.85)
+CT_LABEL_LEVELS = (0.15, 0.35, 0.7)
+
+
+def label_table(colors):
+    """svr_label_params from {label id: (r, g, b, a)}; every other id is hidden (all zero).  a = 0 hides a label; in 2D
+    overlays a is the fill opacity."""
+    p = L.LabelParams()
+    for lab, rgba in colors.items():
+        if not 0 <= int(lab) <= 255:
+            raise ValueError(f"label_table: label id {lab} is outside 0..255")
+        p.color[int(lab)][:] = [float(np.float32(c)) for c in rgba]
+    return p
+
+
+def label_palette(n, alpha=1.0):
+    """A deterministic colour per label id 1..n, {id: (r, g, b, alpha)}, distinct for every id (the red byte (73 id + 91) mod 256
+    alone differs between any two ids).  Each channel is byte / 255 in float32, as tools/svr_headless.cpp computes it."""
+    out = {}
+    for lab in range(1, int(n) + 1):
+        rgb = ((73 * lab + 91) & 255, (151 * lab + 17) & 255, (29 * lab + 193) & 255)
+        out[lab] = tuple(float(np.float32(c) / np.float32(255)) for c in rgb) + (float(alpha),)
+    return out
+
+
+def labels_from_thresholds(volume, levels):
+    """u8 labels of a grey volume: the number of `levels` (increasing) at or below each voxel's value, so that
+    levels = CT_LABEL_LEVELS gives 1 skin, 2 soft tissue and 3 bone on the generated CT.  Values are compared as the volume
+    texture returns them: unsigned integer voxels over their type's maximum (normalised reads), floats as stored."""
+    v = np.asarray(volume)
+    if np.issubdtype(v.dtype, np.unsignedinteger):
+        v = v.astype(np.float32) / np.float32(np.iinfo(v.dtype).max)
+    out = np.zeros(v.shape, np.uint8)
+    for level in levels:
+        out += (v >= np.float32(level)).astype(np.uint8)
+    return out
+
+
 @dataclass
 class Config:
     """One BASELINE.json configuration."""

@@ -4,8 +4,8 @@
 // render_raycasting -- on the synthetic configurations of SURVEY.md section 8d, times the loop with
 // CUDA events and writes the image as PPM (tone-mapped u8) and PFM (float accumulator).
 //
-//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip|iso|slice|cpr] [--window C,W] [--iso V] [--axis x|y|z --index I --slab N]
-//                [--curve FILE] [--up x,y,z]
+//   svr_headless [--config C1|C2|C3|C4] [--mode pt|rc|mip|minip|aip|iso|slice|cpr|labels] [--window C,W] [--iso V]
+//                [--axis x|y|z --index I --slab N] [--curve FILE] [--up x,y,z] [--labels FILE [--outline]]
 //                [--spp N] [--depth D] [--batched 0|1]
 //                [--pt-mode 0|1|2] [--n N --w W --h H] [--out prefix] [--reps R] [--volume file.mhd|.mha] [--tf file.tf|app]
 //                [--interact script.txt]
@@ -26,6 +26,10 @@
 // --mode cpr renders the --w x --h straightened curved planar reformation (svr_render_curved) along the polyline of --curve FILE
 // (whitespace-separated world xyz triples), the frame's roll fixed by --up (default 0,0,1), pixel and station spacing the
 // smallest voxel spacing; --slab N and --window as for slices.
+// --labels FILE loads a MetaImage label map (svr_labels_load_metaimage); it lines up with the volume when dims and spacing match.
+// --mode labels renders its label surfaces (svr_render_labels) with the ray caster's step size, every label 1..max drawn in
+// label_palette's colour (below; scene.label_palette in Python).  --mode slice with --labels overlays the labels on the grey slice
+// (svr_render_label_slices) at half opacity, --outline drawing the outline pixels opaque.
 // --volume loads a MetaImage file the way Canvas::LoadVolume does (core/VolumeReader.cpp:13-94) instead of
 // generating the configuration's synthetic volume; camera and light are framed on its extent.
 // --tf loads a transfer function saved by the application (gui/transferfunction.cpp:55-88); `app` is the
@@ -165,8 +169,18 @@ int main(int argc, char** argv)
     int sliceAxis = 2, sliceIndex = -1, slab = 0;
     std::string curvePath;
     float up[3] = {0.f, 0.f, 1.f};
-    for (int i = 1; i + 1 < argc; i += 2) {
-        std::string k = argv[i], v = argv[i + 1];
+    std::string labelsPath;
+    int outline = 0;
+    for (int i = 1; i < argc;) {
+        std::string k = argv[i];
+        if (k == "--outline") {  // the one option without a value
+            outline = 1;
+            ++i;
+            continue;
+        }
+        if (i + 1 >= argc) break;
+        std::string v = argv[i + 1];
+        i += 2;
         if (k == "--config") {
             bool ok = false;
             for (const Config& c : kConfigs)
@@ -195,6 +209,7 @@ int main(int argc, char** argv)
         } else if (k == "--index") sliceIndex = atoi(v.c_str());
         else if (k == "--slab") slab = atoi(v.c_str());
         else if (k == "--curve") curvePath = v;
+        else if (k == "--labels") labelsPath = v;
         else if (k == "--up") {
             if (sscanf(v.c_str(), "%f,%f,%f", &up[0], &up[1], &up[2]) != 3) { fprintf(stderr, "--up wants x,y,z\n"); return 2; }
         }
@@ -248,6 +263,20 @@ int main(int argc, char** argv)
         CK(cudaFree(dVox));
     }
     setup_volume(&vol);
+    svr_volume labels;
+    memset(&labels, 0, sizeof(labels));
+    uint32_t maxLabel = 0;
+    if (!labelsPath.empty()) SVR(svr_labels_load_metaimage(labelsPath.c_str(), &labels, &maxLabel));
+    if (mode == "labels" && labelsPath.empty()) { fprintf(stderr, "--mode labels wants --labels FILE\n"); return 2; }
+    // label_palette (scene.py): label l in ((73 l + 91) mod 256, (151 l + 17) mod 256, (29 l + 193) mod 256) / 255
+    svr_label_params palette;
+    memset(&palette, 0, sizeof(palette));
+    for (uint32_t l = 1; l <= maxLabel; ++l) {
+        palette.color[l][0] = (float)((73u * l + 91u) & 255u) / 255.f;
+        palette.color[l][1] = (float)((151u * l + 17u) & 255u) / 255.f;
+        palette.color[l][2] = (float)((29u * l + 193u) & 255u) / 255.f;
+        palette.color[l][3] = mode == "labels" ? 1.f : 0.5f;
+    }
 
     std::vector<float> table;
     tf_table(cfg.tf, table);
@@ -393,8 +422,11 @@ int main(int argc, char** argv)
             SVR(svr_render_projection(dImg, dValue, &vol, &cam, &proj, 0, 1, nullptr));
         } else if (mode == "iso") {
             SVR(svr_render_isosurface(dImg, nullptr, &vol, &cam, &iso, 0, 1, nullptr));
+        } else if (mode == "labels") {
+            SVR(svr_render_labels(dImg, nullptr, nullptr, &labels, &cam, &palette, stepSize, 0, 1, nullptr));
         } else if (mode == "slice") {
             SVR(svr_render_slices(dImg, dValue, &vol, &slice));
+            if (labels.tex) SVR(svr_render_label_slices(dImg, nullptr, &labels, &slice, &palette, outline));
         } else if (mode == "cpr") {
             SVR(svr_render_curved(dImg, dValue, &vol, &cpr, curve.data(), (uint32_t)(curve.size() / 3)));
         } else if (batched) {
@@ -412,7 +444,7 @@ int main(int argc, char** argv)
         CK(cudaEventElapsedTime(&ms, e0, e1));
         if (rep > 0 && ms < best) best = ms;
     }
-    if (mode == "rc" || mode == "iso" || mode == "slice" || mode == "cpr" || projMode >= 0)
+    if (mode == "rc" || mode == "iso" || mode == "labels" || mode == "slice" || mode == "cpr" || projMode >= 0)
         printf("{\"config\": \"%s\", \"mode\": \"%s\", \"ms\": %.4f, \"mrays_per_s\": %.2f, \"launches\": %llu}\n", cfg.name, mode.c_str(),
                best, npix / (best * 1e-3) / 1e6, (unsigned long long)svr_launch_count());
     else
@@ -442,7 +474,7 @@ int main(int argc, char** argv)
             fwrite(value.data(), sizeof(float), value.size(), f);
             fclose(f);
         }
-    } else if (mode != "rc" && mode != "iso" && mode != "slice" && mode != "cpr") {
+    } else if (mode != "rc" && mode != "iso" && mode != "labels" && mode != "slice" && mode != "cpr") {
         std::vector<float> hdr(npix * 3);
         CK(cudaMemcpy(hdr.data(), rp.hdrBuffer, npix * 12, cudaMemcpyDeviceToHost));
         FILE* f = fopen((out + ".pfm").c_str(), "wb");
@@ -453,6 +485,7 @@ int main(int argc, char** argv)
         }
     }
     svr_volume_destroy(&vol);
+    svr_volume_destroy(&labels);
     svr_tf_destroy(&tf);
     cudaFree(rp.hdrBuffer);
     cudaFree(dImg);
