@@ -23,6 +23,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <type_traits>
 #include <vector>
 
 #include "svr_state.h"
@@ -151,6 +152,27 @@ SVR_DEV float fold_samples(const ProjScene& s, const Ray& ray, float t0, float h
     return acc;
 }
 
+// The samples of a camera ray through the volume on [tNear, tFar] (include/svr_render.h): K, with *t0 = max(tNear, 0) and
+// *h = stepSize / 2.  K uses the fast-math division (2 ulp), as grey_rgba does: the correctly rounded one is a subroutine
+// call, around which the counting variants spill.  K can then differ by one from the exact formula where
+// (tFar - t0) / h + 1/2 is within 2 ulp of an integer; it is the same with skipping on and off.
+SVR_DEV uint32_t sample_count(float stepSize, float tNear, float tFar, float* t0, float* h)
+{
+    *h = stepSize * 0.5f;
+    *t0 = fmaxf(tNear, 0.f);
+    const float span = tFar > *t0 ? floorf(__fadd_rn(__fsub_rn(tFar, *t0) / *h, 0.5f)) : 0.f;
+    return (uint32_t)span;
+}
+
+// The grey image of a projected value P in the display window: (trunc(255 g), trunc(255 g), trunc(255 g), 255),
+// g = clamp((P - (windowCenter - windowWidth / 2)) / windowWidth, 0, 1)
+SVR_DEV uint32_t grey_rgba(float P, float windowCenter, float windowWidth)
+{
+    const float g = fminf(fmaxf((P - (windowCenter - 0.5f * windowWidth)) / windowWidth, 0.f), 1.f);
+    const float q = 255.f * g;
+    return pack_u8x4(q, q, q, 255.f);
+}
+
 template <int OP, bool SKIP, bool COUNT>
 __global__ void __launch_bounds__(256) project_kernel(const __grid_constant__ ProjScene s, float stepSize, float windowCenter, float windowWidth,
                                                       uint32_t* __restrict__ img, float* __restrict__ value, uint32_t y0, uint32_t y1,
@@ -165,24 +187,15 @@ __global__ void __launch_bounds__(256) project_kernel(const __grid_constant__ Pr
         float P = 0.f;
         float tNear, tFar;
         if (intersect_volume(s.vol, ray, &tNear, &tFar)) {
-            const float h = stepSize * 0.5f;
-            const float t0 = fmaxf(tNear, 0.f);
-            // K and the window use the fast-math division (2 ulp): the correctly rounded one is a subroutine call, around which
-            // the counting variants spill.  K can then differ by one from the exact formula where (tFar - t0) / h + 1/2 is
-            // within 2 ulp of an integer; it is the same with skipping on and off.
-            const float span = tFar > t0 ? floorf(__fadd_rn(__fsub_rn(tFar, t0) / h, 0.5f)) : 0.f;
-            const uint32_t K = (uint32_t)span;
+            float t0, h;
+            const uint32_t K = sample_count(stepSize, tNear, tFar, &t0, &h);
             lc.add(SVR_CNT_STEPS, K);
             const float acc = fold_samples<OP, SKIP>(s, ray, t0, h, 0u, K, lc);
             if (K > 0u) P = OP == SVR_PROJECT_MEAN ? __fdiv_rn(acc, (float)K) : acc;
         }
         const size_t offset = (size_t)idy * s.cam.imageW + idx;
         if (value) value[offset] = P;
-        if (img) {
-            const float g = fminf(fmaxf((P - (windowCenter - 0.5f * windowWidth)) / windowWidth, 0.f), 1.f);
-            const float q = 255.f * g;
-            img[offset] = pack_u8x4(q, q, q, 255.f);
-        }
+        if (img) img[offset] = grey_rgba(P, windowCenter, windowWidth);
     }
     lc.flush(cnt);
 }
@@ -207,9 +220,75 @@ SVR_DEV float2 refine_crossing(const V& value, float iso, float lo, float hi, fl
     return make_float2(lo + (hi - lo) * (iso - vLo) / (vHi - vLo), hi);
 }
 
+// The first hit of iso_kernel and label_kernel (include/svr_render.h, svr_render_isosurface): the first of the K samples of the
+// ray, sample k at t0 + (k + 1/2) h, whose value(t) reaches iso, with UNROLL fetches in flight per lane; with SKIP through the
+// grid of S, dropping the samples of every cell for which mayHit(cell) is false.  A hit is refined by refine_crossing from the
+// sample before it, recomputed from its index: *hit = (t_hit, the final bisection upper bound), both t_0 for a hit at k = 0.
+// Counts steps, shade_taps, skipped and cells (the refinement's taps are not counted).
+template <bool SKIP, int UNROLL, bool COUNT, class S, class V, class M>
+SVR_DEV bool first_hit(const S& s, const Ray& ray, float t0, float h, uint32_t K, const V& value, float iso, const M& mayHit,
+                       LocalCounters<COUNT>& lc, float2* hit)
+{
+    auto t_of = [&](uint32_t k) { return __fadd_rn(t0, __fmul_rn((float)k + 0.5f, h)); };
+    // the first index in [k, kEnd) whose value reaches iso (its value in vHit), else kEnd
+    float vHit = 0.f;
+    auto find = [&](uint32_t k, uint32_t kEnd) {
+        if constexpr (UNROLL > 1) {
+            for (; k + (uint32_t)UNROLL <= kEnd; k += (uint32_t)UNROLL) {
+                float v[UNROLL];
+#pragma unroll
+                for (int u = 0; u < UNROLL; ++u) v[u] = value(t_of(k + u));
+                int first = UNROLL;
+#pragma unroll
+                for (int u = UNROLL - 1; u >= 0; --u)
+                    if (v[u] >= iso) first = u, vHit = v[u];
+                if (first < UNROLL) return k + (uint32_t)first;
+            }
+        }
+        for (; k < kEnd; ++k) {
+            const float v = value(t_of(k));
+            if (v >= iso) {
+                vHit = v;
+                return k;
+            }
+        }
+        return kEnd;
+    };
+    uint32_t kHit = K;
+    if constexpr (!SKIP) {
+        kHit = find(0u, K);
+        lc.add(SVR_CNT_SHADE_TAPS, kHit < K ? kHit + 1u : K);
+    } else {
+        const CellWalk walk(s, ray);
+        for (uint32_t k = 0; k < K;) {
+            const CellVisit c = walk.visit(s, ray, t0, h, k, K);
+            lc.add(SVR_CNT_CELLS, 1);
+            if (!mayHit(c.cell)) {
+                lc.add(SVR_CNT_SKIPPED, c.kEnd - k);
+            } else {
+                const uint32_t f = find(k, c.kEnd);
+                lc.add(SVR_CNT_SHADE_TAPS, (f < c.kEnd ? f + 1u : c.kEnd) - k);
+                if (f < c.kEnd) {
+                    kHit = f;
+                    break;
+                }
+            }
+            k = c.kEnd;
+        }
+    }
+    lc.add(SVR_CNT_STEPS, kHit < K ? kHit + 1u : K);
+    if (kHit >= K) return false;
+    hit->x = hit->y = t_of(kHit);
+    if (kHit > 0u) {
+        const float lo = t_of(kHit - 1u);
+        *hit = refine_crossing(value, iso, lo, hit->x, value(lo), vHit);
+    }
+    return true;
+}
+
 // Isosurface (include/svr_render.h): the first sample at or above iso along the projection's samples, refined by 4 bisection
 // steps and a linear interpolation, shaded with the ray caster's headlight.  Skipping drops the samples of cells whose maximum is
-// below iso: none of them can be the first hit, and the refinement recomputes the sample before the hit from its index.
+// below iso: none of them can be the first hit.
 template <bool SKIP, bool COUNT>
 __global__ void __launch_bounds__(256) iso_kernel(const __grid_constant__ ProjScene s, float stepSize, float iso, float3 color,
                                                   uint32_t* __restrict__ img, float4* __restrict__ surface, uint32_t y1,
@@ -221,77 +300,26 @@ __global__ void __launch_bounds__(256) iso_kernel(const __grid_constant__ ProjSc
     LocalCounters<COUNT> lc;
     Ray ray;
     bool found = false;
-    float tHit = 0.f;
+    float2 hit = make_float2(0.f, 0.f);
     if (inside) {
         ray = camera_ray_center(s.cam, idx, idy);
         lc.add(SVR_CNT_PATHS, 1);
         float tNear, tFar;
         if (intersect_volume(s.vol, ray, &tNear, &tFar)) {
-            const float h = stepSize * 0.5f;
-            const float t0 = fmaxf(tNear, 0.f);
-            const float span = tFar > t0 ? floorf(__fadd_rn(__fsub_rn(tFar, t0) / h, 0.5f)) : 0.f;
-            const uint32_t K = (uint32_t)span;
+            float t0, h;
+            const uint32_t K = sample_count(stepSize, tNear, tFar, &t0, &h);
             const float ds = s.vol.densityScale;
-            auto t_of = [&](uint32_t k) { return __fadd_rn(t0, __fmul_rn((float)k + 0.5f, h)); };
             auto value = [&](float t) {
                 const float3 tc = tex_coord(s.vol, ray.orig + t * ray.dir);
                 return tex3D<float>(s.vol.tex, tc.x, tc.y, tc.z) * ds;
             };
-            // the first index in [k, kEnd) whose value reaches iso (its value in vHit), else kEnd: four fetches in flight per lane
-            float vHit = 0.f;
-            auto find = [&](uint32_t k, uint32_t kEnd) {
-                for (; k + 4u <= kEnd; k += 4u) {
-                    float v[4];
-#pragma unroll
-                    for (int u = 0; u < 4; ++u) v[u] = value(t_of(k + u));
-                    int first = 4;
-#pragma unroll
-                    for (int u = 3; u >= 0; --u)
-                        if (v[u] >= iso) first = u, vHit = v[u];
-                    if (first < 4) return k + (uint32_t)first;
-                }
-                for (; k < kEnd; ++k) {
-                    const float v = value(t_of(k));
-                    if (v >= iso) {
-                        vHit = v;
-                        return k;
-                    }
-                }
-                return kEnd;
+            // a cell may hold a hit unless its widened maximum is below iso
+            auto mayHit = [&](size_t cell) {
+                const float2 range = __ldg(s.range + cell);
+                const float top = fmaxf(range.x * ds, range.y * ds);
+                return !(top + fabsf(top) * RANGE_MARGIN < iso);
             };
-            uint32_t hit = K;
-            if constexpr (!SKIP) {
-                hit = find(0u, K);
-                lc.add(SVR_CNT_SHADE_TAPS, hit < K ? hit + 1u : K);
-            } else {
-                const CellWalk walk(s, ray);
-                for (uint32_t k = 0; k < K;) {
-                    const CellVisit c = walk.visit(s, ray, t0, h, k, K);
-                    lc.add(SVR_CNT_CELLS, 1);
-                    const float2 range = __ldg(s.range + c.cell);
-                    const float top = fmaxf(range.x * ds, range.y * ds);
-                    if (top + fabsf(top) * RANGE_MARGIN < iso) {
-                        lc.add(SVR_CNT_SKIPPED, c.kEnd - k);
-                    } else {
-                        const uint32_t f = find(k, c.kEnd);
-                        lc.add(SVR_CNT_SHADE_TAPS, (f < c.kEnd ? f + 1u : c.kEnd) - k);
-                        if (f < c.kEnd) {
-                            hit = f;
-                            break;
-                        }
-                    }
-                    k = c.kEnd;
-                }
-            }
-            lc.add(SVR_CNT_STEPS, hit < K ? hit + 1u : K);
-            if (hit < K) {
-                found = true;
-                tHit = t_of(hit);
-                if (hit > 0u) {
-                    const float lo = t_of(hit - 1u);
-                    tHit = refine_crossing(value, iso, lo, tHit, value(lo), vHit).x;
-                }
-            }
+            found = first_hit<SKIP, 4>(s, ray, t0, h, K, value, iso, mayHit, lc, &hit);
         }
     }
     // the counts are complete (the refinement and gradient taps are not counted): flushed before the shading, which then needs
@@ -301,7 +329,7 @@ __global__ void __launch_bounds__(256) iso_kernel(const __grid_constant__ ProjSc
     uint32_t rgba = 0u;
     float4 surf = make_float4(0.f, 0.f, 0.f, INFINITY);
     if (found) {
-        const float3 x = ray.orig + tHit * ray.dir;
+        const float3 x = ray.orig + hit.x * ray.dir;
         const float3 camPos = f3(s.cam.pos);
         const float3 g = gradient_at(s.vol, x);
         const float gm = sqrtf(dot(g, g));
@@ -345,8 +373,9 @@ SVR_HD TurnedBox turn_box(float3 dir, float3 cmin, float3 cmax)
 // at orig + (t0 + (k + 1/2) h) dir, against the box turned for dir.  Each component of x_k is monotone in k (s_k and the
 // rounded products and sums are), so the lower bounds of the turned box hold from kLo on and its upper bounds below kHi; two
 // binary searches find both.  A component with dir = 0 is constant: its two conditions hold for every k or for none.
-SVR_DEV uint2 included_range(const Ray& ray, float t0, float h, uint32_t K, const float3& sg, const float3& bLo, const float3& bHi)
+SVR_DEV uint2 included_range(const Ray& ray, float t0, float h, uint32_t K, const TurnedBox& box)
 {
+    const float3 &sg = box.sg, &bLo = box.lo, &bHi = box.hi;
     // sg * x_k is non-decreasing in k on every component: "sg x_k >= lo" holds from some k on, "sg x_k <= hi" up to some k
     auto at = [&](uint32_t k) { return sg * (ray.orig + __fadd_rn(t0, __fmul_rn((float)k + 0.5f, h)) * ray.dir); };
     auto rises = [&](uint32_t k) {
@@ -374,11 +403,22 @@ SVR_DEV uint2 included_range(const Ray& ray, float t0, float h, uint32_t K, cons
     return make_uint2(kLo, lo);
 }
 
+// P and its grey image at pixel (x, y) of image blockIdx.z of a W x H stack, (0, 0, 0, 0) where no sample was taken.  The
+// pixel's place comes from the launch geometry again: nothing but P and the count stays live across the MEAN division, which is
+// a subroutine call (else the MEAN variants spill the pixel around it).
+SVR_DEV void write_slab(float P, uint32_t taken, uint32_t W, uint32_t H, float windowCenter, float windowWidth, uint32_t* img, float* value)
+{
+    const uint2 q = band_pixel(0u, H, 0u, 1u);
+    const size_t offset = ((size_t)blockIdx.z * H + q.y) * W + q.x;
+    if (value) value[offset] = P;
+    if (img) img[offset] = taken > 0u ? grey_rgba(P, windowCenter, windowWidth) : 0u;
+}
+
 // The plane geometry of svr_render_slices (include/svr_render.h), from the host: n, K, t0 and h of the slab rule, and the
 // clipped box turned for n (TurnedBox).
 struct SliceGeom {
     float3 center, u, v, w, n;
-    float3 sg, lo, hi;
+    TurnedBox box;
     uint32_t W, H, K;
     float t0, h;
 };
@@ -398,29 +438,15 @@ __global__ void __launch_bounds__(256) slice_kernel(const __grid_constant__ Proj
         Ray ray;
         ray.orig = g.center + fx * g.u + fy * g.v + (float)j * g.w;
         ray.dir = g.n;
-        const uint2 kr = included_range(ray, g.t0, g.h, g.K, g.sg, g.lo, g.hi);
-        const uint32_t kLo = kr.x, kHi = kr.y;
-        const uint32_t taken = kHi > kLo ? kHi - kLo : 0u;
+        const uint2 kr = included_range(ray, g.t0, g.h, g.K, g.box);
+        const uint32_t taken = kr.y > kr.x ? kr.y - kr.x : 0u;
         float P = 0.f;
         if (taken > 0u) {
             lc.add(SVR_CNT_STEPS, taken);
-            const float acc = fold_samples<OP, SKIP>(s, ray, g.t0, g.h, kLo, kHi, lc);
+            const float acc = fold_samples<OP, SKIP>(s, ray, g.t0, g.h, kr.x, kr.y, lc);
             P = OP == SVR_PROJECT_MEAN ? __fdiv_rn(acc, (float)taken) : acc;
         }
-        // the pixel's place from the launch geometry again: nothing but P and the count stays live across the division, which
-        // is a subroutine call (else the MEAN variant spills the pixel around it)
-        const uint2 q = band_pixel(0u, g.H, 0u, 1u);
-        const size_t offset = ((size_t)blockIdx.z * g.H + q.y) * g.W + q.x;
-        if (value) value[offset] = P;
-        if (img) {
-            uint32_t rgba = 0u;
-            if (taken > 0u) {
-                const float gr = fminf(fmaxf((P - (windowCenter - 0.5f * windowWidth)) / windowWidth, 0.f), 1.f);
-                const float grey = 255.f * gr;
-                rgba = pack_u8x4(grey, grey, grey, 255.f);
-            }
-            img[offset] = rgba;
-        }
+        write_slab(P, taken, g.W, g.H, windowCenter, windowWidth, img, value);
     }
     lc.flush(cnt);
 }
@@ -469,7 +495,7 @@ __global__ void __launch_bounds__(256) curved_kernel(const __grid_constant__ Pro
                 ray.dir = e;
             }
             const TurnedBox box = turn_box(ray.dir, g.cmin, g.cmax);
-            const uint2 kr = included_range(ray, g.t0, g.h, g.K, box.sg, box.lo, box.hi);
+            const uint2 kr = included_range(ray, g.t0, g.h, g.K, box);
             taken = kr.y > kr.x ? kr.y - kr.x : 0u;
             if (taken > 0u) {
                 lc.add(SVR_CNT_STEPS, taken);
@@ -477,39 +503,9 @@ __global__ void __launch_bounds__(256) curved_kernel(const __grid_constant__ Pro
                 P = OP == SVR_PROJECT_MEAN ? __fdiv_rn(acc, (float)taken) : acc;
             }
         }
-        // as slice_kernel: the pixel's place from the launch geometry again, after the division
-        const uint2 q = band_pixel(0u, g.H, 0u, 1u);
-        const size_t offset = ((size_t)blockIdx.z * g.H + q.y) * g.W + q.x;
-        if (value) value[offset] = P;
-        if (img) {
-            uint32_t rgba = 0u;
-            if (taken > 0u) {
-                const float gr = fminf(fmaxf((P - (windowCenter - 0.5f * windowWidth)) / windowWidth, 0.f), 1.f);
-                const float grey = 255.f * gr;
-                rgba = pack_u8x4(grey, grey, grey, 255.f);
-            }
-            img[offset] = rgba;
-        }
+        write_slab(P, taken, g.W, g.H, windowCenter, windowWidth, img, value);
     }
     lc.flush(cnt);
-}
-
-template <int OP, bool SKIP>
-void launch_op(bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const svr_projection_params& p, uint32_t* img,
-               float* value, uint32_t y1, uint32_t phase, uint32_t stride, Counters* cnt)
-{
-    if (count)
-        project_kernel<OP, SKIP, true><<<grid, block, 0, stream>>>(sc, p.stepSize, p.windowCenter, p.windowWidth, img, value, 0u, y1, phase, stride, cnt);
-    else
-        project_kernel<OP, SKIP, false><<<grid, block, 0, stream>>>(sc, p.stepSize, p.windowCenter, p.windowWidth, img, value, 0u, y1, phase, stride, cnt);
-}
-
-template <int OP>
-void launch_mode(bool skip, bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const svr_projection_params& p,
-                 uint32_t* img, float* value, uint32_t y1, uint32_t phase, uint32_t stride, Counters* cnt)
-{
-    if (skip) launch_op<OP, true>(count, grid, block, stream, sc, p, img, value, y1, phase, stride, cnt);
-    else launch_op<OP, false>(count, grid, block, stream, sc, p, img, value, y1, phase, stride, cnt);
 }
 
 // The scene of a projection, isosurface or slice call (a slice has no camera: cameraOrNull null leaves cam zero); with
@@ -545,6 +541,75 @@ bool band_grid(const svr_camera& camera, uint32_t tileH, uint32_t phase, uint32_
     return true;
 }
 
+// f(op, skip, count) with the kernel variant of a call as compile-time constants: op std::integral_constant<int, mode>, skip
+// and count std::bool_constant.  The isosurface and label kernels take no mode: f(skip, count).
+template <class F>
+void with_variant(bool skip, bool count, F&& f)
+{
+    if (skip) {
+        if (count) f(std::true_type(), std::true_type());
+        else f(std::true_type(), std::false_type());
+    } else {
+        if (count) f(std::false_type(), std::true_type());
+        else f(std::false_type(), std::false_type());
+    }
+}
+
+template <class F>
+void with_variant(int mode, bool skip, bool count, F&& f)
+{
+    auto with_op = [&](auto op) { with_variant(skip, count, [&](auto sk, auto ct) { f(op, sk, ct); }); };
+    if (mode == SVR_PROJECT_MAX) with_op(std::integral_constant<int, SVR_PROJECT_MAX>());
+    else if (mode == SVR_PROJECT_MIN) with_op(std::integral_constant<int, SVR_PROJECT_MIN>());
+    else with_op(std::integral_constant<int, SVR_PROJECT_MEAN>());
+}
+
+// What every launch of this file takes from the options: the threads per block (SVR_OPT_RC_BLOCK) in band_pixel's blocks of
+// 16 columns and tileH rows, skipping (SVR_OPT_RC_SKIP) and counting (SVR_OPT_COUNTERS)
+struct LaunchOptions {
+    int block;
+    uint32_t tileH;
+    bool skip, count;
+};
+
+LaunchOptions launch_options()
+{
+    const int* o = state().options;
+    return {o[SVR_OPT_RC_BLOCK], (uint32_t)o[SVR_OPT_RC_BLOCK] / 16u, o[SVR_OPT_RC_SKIP] != 0, o[SVR_OPT_COUNTERS] != 0};
+}
+
+// "<who>: <what>" as the call's error
+int fail_in(const char* who, const char* what) { return fail_msg((std::string(who) + ": " + what).c_str()); }
+
+// The device counters into *cnt when counting, else null; the error of `who` when they cannot be allocated
+int launch_counters(const char* who, bool count, Counters** cnt)
+{
+    *cnt = count ? device_counters() : nullptr;
+    return count && !*cnt ? fail_in(who, "counter allocation failed") : 0;
+}
+
+// After a kernel launch: counts it and returns its error
+int launched()
+{
+    count_launch();
+    SVR_TRY(cudaGetLastError());
+    return 0;
+}
+
+// The parameter errors of a projection mode and of a display window, reported as those of `who`
+int check_mode(const char* who, int mode)
+{
+    if (mode < SVR_PROJECT_MAX || mode > SVR_PROJECT_MEAN) return fail_in(who, "mode must be 0 (max), 1 (min) or 2 (mean)");
+    return 0;
+}
+
+int check_window(const char* who, float windowCenter, float windowWidth)
+{
+    if (!(windowWidth > 0.f) || !std::isfinite(windowWidth) || !std::isfinite(windowCenter))
+        return fail_in(who, "windowWidth must be positive and finite, windowCenter finite");
+    return 0;
+}
+
 }  // namespace
 }  // namespace svr
 
@@ -554,34 +619,29 @@ extern "C" int svr_render_projection(svr_u8vec4* imgOrNull, float* valueOrNull, 
                                      const svr_projection_params* params, uint32_t phase, uint32_t stride, uint32_t* bandRows)
 {
     HostState& st = state();
+    const char* who = "svr_render_projection";
     if (!volume || !camera || !params) return fail_msg("svr_render_projection: null volume, camera or params");
     if (!imgOrNull && !valueOrNull) return fail_msg("svr_render_projection: both outputs are null");
     const svr_projection_params p = *params;
-    if (p.mode < SVR_PROJECT_MAX || p.mode > SVR_PROJECT_MEAN) return fail_msg("svr_render_projection: mode must be 0 (max), 1 (min) or 2 (mean)");
+    if (int rc = check_mode(who, p.mode)) return rc;
     if (!(p.stepSize > 0.f) || !std::isfinite(p.stepSize)) return fail_msg("svr_render_projection: stepSize must be positive and finite");
-    if (!(p.windowWidth > 0.f) || !std::isfinite(p.windowWidth) || !std::isfinite(p.windowCenter))
-        return fail_msg("svr_render_projection: windowWidth must be positive and finite, windowCenter finite");
+    if (int rc = check_window(who, p.windowCenter, p.windowWidth)) return rc;
     if (phase >= stride) return fail_msg("svr_render_projection: band phase must be below the band stride");
-    const int block = st.options[SVR_OPT_RC_BLOCK];
-    const uint32_t tileH = (uint32_t)block / 16u;
-    if (bandRows) *bandRows = tileH;
+    const LaunchOptions o = launch_options();
+    if (bandRows) *bandRows = o.tileH;
 
     ProjScene sc;
-    const bool skip = st.options[SVR_OPT_RC_SKIP] != 0;
-    const bool count = st.options[SVR_OPT_COUNTERS] != 0;
-    if (int rc = make_scene(&sc, *volume, camera, skip)) return rc;
+    if (int rc = make_scene(&sc, *volume, camera, o.skip)) return rc;
     dim3 grid;
-    if (!band_grid(*camera, tileH, phase, stride, &grid)) return 0;
-    Counters* cnt = count ? device_counters() : nullptr;
-    if (count && !cnt) return fail_msg("svr_render_projection: counter allocation failed");
+    if (!band_grid(*camera, o.tileH, phase, stride, &grid)) return 0;
+    Counters* cnt;
+    if (int rc = launch_counters(who, o.count, &cnt)) return rc;
     const uint32_t H = camera->imageH;
-    uint32_t* img = (uint32_t*)imgOrNull;
-    if (p.mode == SVR_PROJECT_MAX) launch_mode<SVR_PROJECT_MAX>(skip, count, grid, block, st.stream, sc, p, img, valueOrNull, H, phase, stride, cnt);
-    else if (p.mode == SVR_PROJECT_MIN) launch_mode<SVR_PROJECT_MIN>(skip, count, grid, block, st.stream, sc, p, img, valueOrNull, H, phase, stride, cnt);
-    else launch_mode<SVR_PROJECT_MEAN>(skip, count, grid, block, st.stream, sc, p, img, valueOrNull, H, phase, stride, cnt);
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    return 0;
+    with_variant(p.mode, o.skip, o.count, [&](auto op, auto sk, auto ct) {
+        project_kernel<op, sk, ct><<<grid, o.block, 0, st.stream>>>(sc, p.stepSize, p.windowCenter, p.windowWidth, (uint32_t*)imgOrNull,
+                                                                    valueOrNull, 0u, H, phase, stride, cnt);
+    });
+    return launched();
 }
 
 extern "C" int svr_render_isosurface(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrNull, const svr_volume* volume, const svr_camera* camera,
@@ -596,76 +656,74 @@ extern "C" int svr_render_isosurface(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrN
     for (float c : p.color)
         if (!(c >= 0.f && c <= 1.f)) return fail_msg("svr_render_isosurface: each colour component must be in [0, 1]");
     if (phase >= stride) return fail_msg("svr_render_isosurface: band phase must be below the band stride");
-    const int block = st.options[SVR_OPT_RC_BLOCK];
-    const uint32_t tileH = (uint32_t)block / 16u;
-    if (bandRows) *bandRows = tileH;
+    const LaunchOptions o = launch_options();
+    if (bandRows) *bandRows = o.tileH;
 
     ProjScene sc;
-    const bool skip = st.options[SVR_OPT_RC_SKIP] != 0;
-    const bool count = st.options[SVR_OPT_COUNTERS] != 0;
-    if (int rc = make_scene(&sc, *volume, camera, skip)) return rc;
+    if (int rc = make_scene(&sc, *volume, camera, o.skip)) return rc;
     dim3 grid;
-    if (!band_grid(*camera, tileH, phase, stride, &grid)) return 0;
-    Counters* cnt = count ? device_counters() : nullptr;
-    if (count && !cnt) return fail_msg("svr_render_isosurface: counter allocation failed");
+    if (!band_grid(*camera, o.tileH, phase, stride, &grid)) return 0;
+    Counters* cnt;
+    if (int rc = launch_counters("svr_render_isosurface", o.count, &cnt)) return rc;
     const uint32_t H = camera->imageH;
     const float3 color = f3(p.color[0], p.color[1], p.color[2]);
-    uint32_t* img = (uint32_t*)imgOrNull;
-    float4* surface = (float4*)surfaceOrNull;
-    if (skip) {
-        if (count) iso_kernel<true, true><<<grid, block, 0, st.stream>>>(sc, p.stepSize, p.isoValue, color, img, surface, H, phase, stride, cnt);
-        else iso_kernel<true, false><<<grid, block, 0, st.stream>>>(sc, p.stepSize, p.isoValue, color, img, surface, H, phase, stride, cnt);
-    } else {
-        if (count) iso_kernel<false, true><<<grid, block, 0, st.stream>>>(sc, p.stepSize, p.isoValue, color, img, surface, H, phase, stride, cnt);
-        else iso_kernel<false, false><<<grid, block, 0, st.stream>>>(sc, p.stepSize, p.isoValue, color, img, surface, H, phase, stride, cnt);
-    }
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    return 0;
+    with_variant(o.skip, o.count, [&](auto sk, auto ct) {
+        iso_kernel<sk, ct><<<grid, o.block, 0, st.stream>>>(sc, p.stepSize, p.isoValue, color, (uint32_t*)imgOrNull, (float4*)surfaceOrNull, H,
+                                                            phase, stride, cnt);
+    });
+    return launched();
 }
 
 namespace {
 
-template <int OP, bool SKIP>
-void launch_slices(bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const SliceGeom& g, const svr_slice_params& p,
-                   uint32_t* img, float* value, Counters* cnt)
-{
-    if (count) slice_kernel<OP, SKIP, true><<<grid, block, 0, stream>>>(sc, g, p.windowCenter, p.windowWidth, img, value, cnt);
-    else slice_kernel<OP, SKIP, false><<<grid, block, 0, stream>>>(sc, g, p.windowCenter, p.windowWidth, img, value, cnt);
-}
-
-template <int OP>
-void launch_slice_mode(bool skip, bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const SliceGeom& g,
-                       const svr_slice_params& p, uint32_t* img, float* value, Counters* cnt)
-{
-    if (skip) launch_slices<OP, true>(count, grid, block, stream, sc, g, p, img, value, cnt);
-    else launch_slices<OP, false>(count, grid, block, stream, sc, g, p, img, value, cnt);
-}
-
 bool finite3(const float* a) { return std::isfinite(a[0]) && std::isfinite(a[1]) && std::isfinite(a[2]); }
+
+// The parameter errors svr_render_slices and svr_render_curved share (include/svr_render.h), reported as those of `who`: image
+// size and count, mode, slab and window; no CUDA call
+template <class P>
+int check_stack_params(const char* who, const P& p)
+{
+    if (p.imageW == 0u || p.imageW > 16384u || p.imageH == 0u || p.imageH > 16384u) return fail_in(who, "imageW and imageH must be in 1..16384");
+    if (p.count == 0u || p.count > 65535u) return fail_in(who, "count must be in 1..65535");
+    if (int rc = check_mode(who, p.mode)) return rc;
+    if (!(p.thickness >= 0.f) || !std::isfinite(p.thickness)) return fail_in(who, "thickness must be finite and not negative");
+    if (p.thickness > 0.f) {
+        if (!(p.sampleSpacing > 0.f) || !std::isfinite(p.sampleSpacing)) return fail_in(who, "sampleSpacing must be positive and finite for a slab");
+        if (!(p.thickness / p.sampleSpacing <= 65536.f)) return fail_in(who, "thickness / sampleSpacing must be at most 65536");
+    }
+    return check_window(who, p.windowCenter, p.windowWidth);
+}
 
 // svr_render_slices' parameter errors (include/svr_render.h), reported as those of `who`; no CUDA call
 int check_slice_params(const char* who, const svr_slice_params& p)
 {
-    auto err = [&](const char* what) { return fail_msg((std::string(who) + ": " + what).c_str()); };
-    if (!finite3(p.axisU) || !finite3(p.axisV)) return err("axisU and axisV must be finite");
+    if (!finite3(p.axisU) || !finite3(p.axisV)) return fail_in(who, "axisU and axisV must be finite");
     const float3 nc = cross(f3(p.axisU[0], p.axisU[1], p.axisU[2]), f3(p.axisV[0], p.axisV[1], p.axisV[2]));
     const float nn = dot(nc, nc);
-    if (!(nn > 0.f) || !std::isfinite(nn)) return err("cross(axisU, axisV) must be nonzero and finite");
-    if (p.count > 1u && !finite3(p.axisW)) return err("axisW must be finite when count > 1");
-    if (p.imageW == 0u || p.imageW > 16384u || p.imageH == 0u || p.imageH > 16384u)
-        return err("imageW and imageH must be in 1..16384");
-    if (p.count == 0u || p.count > 65535u) return err("count must be in 1..65535");
-    if (p.mode < SVR_PROJECT_MAX || p.mode > SVR_PROJECT_MEAN) return err("mode must be 0 (max), 1 (min) or 2 (mean)");
-    if (!(p.thickness >= 0.f) || !std::isfinite(p.thickness)) return err("thickness must be finite and not negative");
-    if (p.thickness > 0.f) {
-        if (!(p.sampleSpacing > 0.f) || !std::isfinite(p.sampleSpacing))
-            return err("sampleSpacing must be positive and finite for a slab");
-        if (!(p.thickness / p.sampleSpacing <= 65536.f)) return err("thickness / sampleSpacing must be at most 65536");
-    }
-    if (!(p.windowWidth > 0.f) || !std::isfinite(p.windowWidth) || !std::isfinite(p.windowCenter))
-        return err("windowWidth must be positive and finite, windowCenter finite");
-    return 0;
+    if (!(nn > 0.f) || !std::isfinite(nn)) return fail_in(who, "cross(axisU, axisV) must be nonzero and finite");
+    if (p.count > 1u && !finite3(p.axisW)) return fail_in(who, "axisW must be finite when count > 1");
+    return check_stack_params(who, p);
+}
+
+// The slab rule of include/svr_render.h (svr_render_slices, svr_render_curved): K samples h apart, the first at t0 + h / 2; a
+// thin image (thickness 0) is one sample at 0
+struct Slab {
+    uint32_t K;
+    float t0, h;
+};
+
+Slab slab_rule(float thickness, float sampleSpacing)
+{
+    const float h = thickness > 0.f ? sampleSpacing : 0.f;
+    const uint32_t K = thickness > 0.f ? (uint32_t)std::max(1.f, std::floor(thickness / h + 0.5f)) : 1u;
+    return {K, -((float)K * h) * 0.5f, h};
+}
+
+// The volume's box clipped by its clip planes, [cmin, cmax] (include/svr_render.h, svr_render_slices)
+void clipped_box(const svr_volume& v, float3* cmin, float3* cmax)
+{
+    *cmin = f3(v.bbox.vmin.x * -v.x_clip.x, v.bbox.vmin.y * -v.y_clip.x, v.bbox.vmin.z * -v.z_clip.x);
+    *cmax = f3(v.bbox.vmax.x * v.x_clip.y, v.bbox.vmax.y * v.y_clip.y, v.bbox.vmax.z * v.z_clip.y);
 }
 
 }  // namespace
@@ -673,10 +731,11 @@ int check_slice_params(const char* who, const svr_slice_params& p)
 extern "C" int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, const svr_volume* volume, const svr_slice_params* params)
 {
     HostState& st = state();
+    const char* who = "svr_render_slices";
     if (!volume || !params) return fail_msg("svr_render_slices: null volume or params");
     if (!imgOrNull && !valueOrNull) return fail_msg("svr_render_slices: both outputs are null");
     const svr_slice_params p = *params;
-    if (int rc = check_slice_params("svr_render_slices", p)) return rc;
+    if (int rc = check_slice_params(who, p)) return rc;
     const float3 u = f3(p.axisU[0], p.axisU[1], p.axisU[2]), v = f3(p.axisV[0], p.axisV[1], p.axisV[2]);
     const float3 nc = cross(u, v);
     const float nn = dot(nc, nc);
@@ -689,33 +748,25 @@ extern "C" int svr_render_slices(svr_u8vec4* imgOrNull, float* valueOrNull, cons
     g.n = nc / std::sqrt(nn);
     g.W = p.imageW;
     g.H = p.imageH;
-    g.h = p.thickness > 0.f ? p.sampleSpacing : 0.f;
-    g.K = p.thickness > 0.f ? (uint32_t)std::max(1.f, std::floor(p.thickness / g.h + 0.5f)) : 1u;
-    g.t0 = -((float)g.K * g.h) * 0.5f;
-    const svr_volume& vo = *volume;
-    const float cmin[3] = {vo.bbox.vmin.x * -vo.x_clip.x, vo.bbox.vmin.y * -vo.y_clip.x, vo.bbox.vmin.z * -vo.z_clip.x};
-    const float cmax[3] = {vo.bbox.vmax.x * vo.x_clip.y, vo.bbox.vmax.y * vo.y_clip.y, vo.bbox.vmax.z * vo.z_clip.y};
-    const TurnedBox box = turn_box(g.n, f3(cmin[0], cmin[1], cmin[2]), f3(cmax[0], cmax[1], cmax[2]));
-    g.sg = box.sg;
-    g.lo = box.lo;
-    g.hi = box.hi;
+    const Slab slab = slab_rule(p.thickness, p.sampleSpacing);
+    g.K = slab.K;
+    g.t0 = slab.t0;
+    g.h = slab.h;
+    float3 cmin, cmax;
+    clipped_box(*volume, &cmin, &cmax);
+    g.box = turn_box(g.n, cmin, cmax);
 
-    const int block = st.options[SVR_OPT_RC_BLOCK];
-    const uint32_t tileH = (uint32_t)block / 16u;
+    const LaunchOptions o = launch_options();
     ProjScene sc;
-    const bool skip = st.options[SVR_OPT_RC_SKIP] != 0 && g.K > 1u;  // a thin slice takes its one fetch and never walks
-    const bool count = st.options[SVR_OPT_COUNTERS] != 0;
+    const bool skip = o.skip && g.K > 1u;  // a thin slice takes its one fetch and never walks
     if (int rc = make_scene(&sc, *volume, nullptr, skip)) return rc;
-    Counters* cnt = count ? device_counters() : nullptr;
-    if (count && !cnt) return fail_msg("svr_render_slices: counter allocation failed");
-    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + tileH - 1u) / tileH, p.count);
-    uint32_t* img = (uint32_t*)imgOrNull;
-    if (p.mode == SVR_PROJECT_MAX) launch_slice_mode<SVR_PROJECT_MAX>(skip, count, grid, block, st.stream, sc, g, p, img, valueOrNull, cnt);
-    else if (p.mode == SVR_PROJECT_MIN) launch_slice_mode<SVR_PROJECT_MIN>(skip, count, grid, block, st.stream, sc, g, p, img, valueOrNull, cnt);
-    else launch_slice_mode<SVR_PROJECT_MEAN>(skip, count, grid, block, st.stream, sc, g, p, img, valueOrNull, cnt);
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    return 0;
+    Counters* cnt;
+    if (int rc = launch_counters(who, o.count, &cnt)) return rc;
+    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + o.tileH - 1u) / o.tileH, p.count);
+    with_variant(p.mode, skip, o.count, [&](auto op, auto sk, auto ct) {
+        slice_kernel<op, sk, ct><<<grid, o.block, 0, st.stream>>>(sc, g, p.windowCenter, p.windowWidth, (uint32_t*)imgOrNull, valueOrNull, cnt);
+    });
+    return launched();
 }
 
 namespace {
@@ -841,22 +892,6 @@ int stage_curve_table(HostState& st, const std::vector<svr_vec4>& table)
     return 0;
 }
 
-template <int OP, bool SKIP>
-void launch_curved(bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const CurveGeom& g, const float4* frames,
-                   const svr_curved_params& p, uint32_t* img, float* value, Counters* cnt)
-{
-    if (count) curved_kernel<OP, SKIP, true><<<grid, block, 0, stream>>>(sc, g, frames, p.windowCenter, p.windowWidth, img, value, cnt);
-    else curved_kernel<OP, SKIP, false><<<grid, block, 0, stream>>>(sc, g, frames, p.windowCenter, p.windowWidth, img, value, cnt);
-}
-
-template <int OP>
-void launch_curved_mode(bool skip, bool count, dim3 grid, int block, cudaStream_t stream, const ProjScene& sc, const CurveGeom& g,
-                        const float4* frames, const svr_curved_params& p, uint32_t* img, float* value, Counters* cnt)
-{
-    if (skip) launch_curved<OP, true>(count, grid, block, stream, sc, g, frames, p, img, value, cnt);
-    else launch_curved<OP, false>(count, grid, block, stream, sc, g, frames, p, img, value, cnt);
-}
-
 }  // namespace
 
 extern "C" int svr_curve_frames(const float* points, uint32_t nPoints, const float up[3], float stationSpacing, uint32_t nStations,
@@ -870,67 +905,52 @@ extern "C" int svr_render_curved(svr_u8vec4* imgOrNull, float* valueOrNull, cons
                                  const float* points, uint32_t nPoints)
 {
     HostState& st = state();
+    const char* who = "svr_render_curved";
     if (!volume || !params || !points) return fail_msg("svr_render_curved: null volume, params or points");
     if (!imgOrNull && !valueOrNull) return fail_msg("svr_render_curved: both outputs are null");
     const svr_curved_params p = *params;
     if (p.layout != SVR_CURVED_STRAIGHTENED && p.layout != SVR_CURVED_CROSS)
         return fail_msg("svr_render_curved: layout must be 0 (straightened) or 1 (cross-sections)");
-    if (p.imageW == 0u || p.imageW > 16384u || p.imageH == 0u || p.imageH > 16384u)
-        return fail_msg("svr_render_curved: imageW and imageH must be in 1..16384");
-    if (p.count == 0u || p.count > 65535u) return fail_msg("svr_render_curved: count must be in 1..65535");
-    if (p.mode < SVR_PROJECT_MAX || p.mode > SVR_PROJECT_MEAN) return fail_msg("svr_render_curved: mode must be 0 (max), 1 (min) or 2 (mean)");
+    if (int rc = check_stack_params(who, p)) return rc;
     if (!(p.pixelSpacing > 0.f) || !std::isfinite(p.pixelSpacing)) return fail_msg("svr_render_curved: pixelSpacing must be positive and finite");
     if (!std::isfinite(p.angle0) || !std::isfinite(p.angleStep)) return fail_msg("svr_render_curved: angle0 and angleStep must be finite");
-    if (!(p.thickness >= 0.f) || !std::isfinite(p.thickness)) return fail_msg("svr_render_curved: thickness must be finite and not negative");
-    if (p.thickness > 0.f) {
-        if (!(p.sampleSpacing > 0.f) || !std::isfinite(p.sampleSpacing))
-            return fail_msg("svr_render_curved: sampleSpacing must be positive and finite for a slab");
-        if (!(p.thickness / p.sampleSpacing <= 65536.f)) return fail_msg("svr_render_curved: thickness / sampleSpacing must be at most 65536");
-    }
-    if (!(p.windowWidth > 0.f) || !std::isfinite(p.windowWidth) || !std::isfinite(p.windowCenter))
-        return fail_msg("svr_render_curved: windowWidth must be positive and finite, windowCenter finite");
     const bool cross = p.layout == SVR_CURVED_CROSS;
     const uint32_t nStations = cross ? p.count : p.imageH, nTrig = cross ? 1u : p.count;
     std::vector<svr_vec4> table(4 * (size_t)nStations + nTrig);
-    if (int rc = curve_frames("svr_render_curved", points, nPoints, p.up, p.stationSpacing, nStations, table.data())) return rc;
+    if (int rc = curve_frames(who, points, nPoints, p.up, p.stationSpacing, nStations, table.data())) return rc;
     for (uint32_t j = 0; j < nTrig; ++j) {
         const double theta = (double)p.angle0 + (double)j * (double)p.angleStep;
         table[4 * (size_t)nStations + j] = svr_vec4{(float)std::cos(theta), (float)std::sin(theta), 0.f, 0.f};
     }
 
     CurveGeom g;
-    const svr_volume& vo = *volume;
-    g.cmin = f3(vo.bbox.vmin.x * -vo.x_clip.x, vo.bbox.vmin.y * -vo.y_clip.x, vo.bbox.vmin.z * -vo.z_clip.x);
-    g.cmax = f3(vo.bbox.vmax.x * vo.x_clip.y, vo.bbox.vmax.y * vo.y_clip.y, vo.bbox.vmax.z * vo.z_clip.y);
+    clipped_box(*volume, &g.cmin, &g.cmax);
     g.W = p.imageW;
     g.H = p.imageH;
-    g.h = p.thickness > 0.f ? p.sampleSpacing : 0.f;
-    g.K = p.thickness > 0.f ? (uint32_t)std::max(1.f, std::floor(p.thickness / g.h + 0.5f)) : 1u;
-    g.t0 = -((float)g.K * g.h) * 0.5f;
+    const Slab slab = slab_rule(p.thickness, p.sampleSpacing);
+    g.K = slab.K;
+    g.t0 = slab.t0;
+    g.h = slab.h;
     g.ps = p.pixelSpacing;
     g.trig = 4u * nStations;
     g.cross = cross ? 1 : 0;
 
-    const int block = st.options[SVR_OPT_RC_BLOCK];
-    const uint32_t tileH = (uint32_t)block / 16u;
+    const LaunchOptions o = launch_options();
     ProjScene sc;
     // slabs of fewer than CURVED_WALK_MIN_K samples, and thin images, do not walk: 16-sample slabs measured slower with the walk,
     // 64-sample ones faster (DESIGN.md section 7k)
-    const bool skip = st.options[SVR_OPT_RC_SKIP] != 0 && g.K >= CURVED_WALK_MIN_K;
-    const bool count = st.options[SVR_OPT_COUNTERS] != 0;
+    const bool skip = o.skip && g.K >= CURVED_WALK_MIN_K;
     if (int rc = make_scene(&sc, *volume, nullptr, skip)) return rc;
-    Counters* cnt = count ? device_counters() : nullptr;
-    if (count && !cnt) return fail_msg("svr_render_curved: counter allocation failed");
+    Counters* cnt;
+    if (int rc = launch_counters(who, o.count, &cnt)) return rc;
     if (int rc = stage_curve_table(st, table)) return rc;
     const float4* frames = st.dev.curveFrames.p;
-    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + tileH - 1u) / tileH, p.count);
-    uint32_t* img = (uint32_t*)imgOrNull;
-    if (p.mode == SVR_PROJECT_MAX) launch_curved_mode<SVR_PROJECT_MAX>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
-    else if (p.mode == SVR_PROJECT_MIN) launch_curved_mode<SVR_PROJECT_MIN>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
-    else launch_curved_mode<SVR_PROJECT_MEAN>(skip, count, grid, block, st.stream, sc, g, frames, p, img, valueOrNull, cnt);
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    return 0;
+    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + o.tileH - 1u) / o.tileH, p.count);
+    with_variant(p.mode, skip, o.count, [&](auto op, auto sk, auto ct) {
+        curved_kernel<op, sk, ct><<<grid, o.block, 0, st.stream>>>(sc, g, frames, p.windowCenter, p.windowWidth, (uint32_t*)imgOrNull,
+                                                                   valueOrNull, cnt);
+    });
+    return launched();
 }
 
 namespace svr {
@@ -1049,65 +1069,22 @@ __global__ void __launch_bounds__(256) label_kernel(const __grid_constant__ Labe
     LocalCounters<COUNT> lc;
     Ray ray;
     bool found = false;
-    float tHit = 0.f, tHi = 0.f;
+    float2 hit = make_float2(0.f, 0.f);
     if (inside) {
         ray = camera_ray_center(s.cam, idx, idy);
         lc.add(SVR_CNT_PATHS, 1);
         float tNear, tFar;
         if (intersect_volume(s.vol, ray, &tNear, &tFar)) {
-            const float h = stepSize * 0.5f;
-            const float t0 = fmaxf(tNear, 0.f);
-            const float span = tFar > t0 ? floorf(__fadd_rn(__fsub_rn(tFar, t0) / h, 0.5f)) : 0.f;
-            const uint32_t K = (uint32_t)span;
-            auto t_of = [&](uint32_t k) { return __fadd_rn(t0, __fmul_rn((float)k + 0.5f, h)); };
+            float t0, h;
+            const uint32_t K = sample_count(stepSize, tNear, tFar, &t0, &h);
             auto value = [&](float tt) { return label_indicator(s, t, ray.orig + tt * ray.dir); };
-            float vHit = 0.f;
-            auto find = [&](uint32_t k, uint32_t kEnd) {
-                for (; k < kEnd; ++k) {
-                    const float v = value(t_of(k));
-                    if (v >= 0.5f) {
-                        vHit = v;
-                        return k;
-                    }
-                }
-                return kEnd;
+            // a cell may hold a hit if its presence mask holds a visible label
+            auto mayHit = [&](size_t cell) {
+                const uint4 p0 = __ldg(s.presence + 2 * cell), p1 = __ldg(s.presence + 2 * cell + 1);
+                return ((p0.x & t.vis[0]) | (p0.y & t.vis[1]) | (p0.z & t.vis[2]) | (p0.w & t.vis[3]) | (p1.x & t.vis[4]) |
+                        (p1.y & t.vis[5]) | (p1.z & t.vis[6]) | (p1.w & t.vis[7])) != 0u;
             };
-            uint32_t hit = K;
-            if constexpr (!SKIP) {
-                hit = find(0u, K);
-                lc.add(SVR_CNT_SHADE_TAPS, hit < K ? hit + 1u : K);
-            } else {
-                const CellWalk walk(s, ray);
-                for (uint32_t k = 0; k < K;) {
-                    const CellVisit c = walk.visit(s, ray, t0, h, k, K);
-                    lc.add(SVR_CNT_CELLS, 1);
-                    const uint4 p0 = __ldg(s.presence + 2 * c.cell), p1 = __ldg(s.presence + 2 * c.cell + 1);
-                    const uint32_t any = (p0.x & t.vis[0]) | (p0.y & t.vis[1]) | (p0.z & t.vis[2]) | (p0.w & t.vis[3]) | (p1.x & t.vis[4]) |
-                                         (p1.y & t.vis[5]) | (p1.z & t.vis[6]) | (p1.w & t.vis[7]);
-                    if (any == 0u) {
-                        lc.add(SVR_CNT_SKIPPED, c.kEnd - k);
-                    } else {
-                        const uint32_t f = find(k, c.kEnd);
-                        lc.add(SVR_CNT_SHADE_TAPS, (f < c.kEnd ? f + 1u : c.kEnd) - k);
-                        if (f < c.kEnd) {
-                            hit = f;
-                            break;
-                        }
-                    }
-                    k = c.kEnd;
-                }
-            }
-            lc.add(SVR_CNT_STEPS, hit < K ? hit + 1u : K);
-            if (hit < K) {
-                found = true;
-                tHit = tHi = t_of(hit);
-                if (hit > 0u) {
-                    const float lo = t_of(hit - 1u);
-                    const float2 r = refine_crossing(value, 0.5f, lo, tHit, value(lo), vHit);
-                    tHit = r.x;
-                    tHi = r.y;
-                }
-            }
+            found = first_hit<SKIP, 1>(s, ray, t0, h, K, value, 0.5f, mayHit, lc, &hit);
         }
     }
     // as iso_kernel: the counts are complete, flushed before the shading
@@ -1116,8 +1093,8 @@ __global__ void __launch_bounds__(256) label_kernel(const __grid_constant__ Labe
     uint32_t rgba = 0u, lab = 0u;
     float4 surf = make_float4(0.f, 0.f, 0.f, INFINITY);
     if (found) {
-        lab = label_pick(s, t, ray.orig + tHi * ray.dir);
-        const float3 x = ray.orig + tHit * ray.dir;
+        lab = label_pick(s, t, ray.orig + hit.y * ray.dir);
+        const float3 x = ray.orig + hit.x * ray.dir;
         const float3 camPos = f3(s.cam.pos);
         const float3 g = label_gradient(s, t, x);
         float3 n = f3(0.f);
@@ -1241,18 +1218,15 @@ extern "C" int svr_render_labels(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrNull,
     cudaArray_t arr;
     int3 dims;
     if (int rc = label_volume(who, *labels, &arr, &dims)) return rc;
-    const int block = st.options[SVR_OPT_RC_BLOCK];
-    const uint32_t tileH = (uint32_t)block / 16u;
-    if (bandRows) *bandRows = tileH;
+    const LaunchOptions o = launch_options();
+    if (bandRows) *bandRows = o.tileH;
 
     LabelScene sc;
     memset(&sc, 0, sizeof(sc));
     sc.vol = *labels;
     sc.cam = *camera;
     sc.dims = f3((float)dims.x, (float)dims.y, (float)dims.z);
-    const bool skip = st.options[SVR_OPT_RC_SKIP] != 0;
-    const bool count = st.options[SVR_OPT_COUNTERS] != 0;
-    if (skip) {
+    if (o.skip) {
         if (int rc = ensure_label_grid(arr, labels->tex, dims, st.options[SVR_OPT_MACROCELL_SIZE])) return rc;
         const DeviceState& d = st.dev;
         sc.presence = (const uint4*)d.labelPresence.p;
@@ -1262,22 +1236,15 @@ extern "C" int svr_render_labels(svr_u8vec4* imgOrNull, svr_vec4* surfaceOrNull,
         sc.scale = f3((float)dims.x / (float)d.labelCell, (float)dims.y / (float)d.labelCell, (float)dims.z / (float)d.labelCell);
     }
     dim3 grid;
-    if (!band_grid(*camera, tileH, phase, stride, &grid)) return 0;
-    Counters* cnt = count ? device_counters() : nullptr;
-    if (count && !cnt) return fail_msg("svr_render_labels: counter allocation failed");
+    if (!band_grid(*camera, o.tileH, phase, stride, &grid)) return 0;
+    Counters* cnt;
+    if (int rc = launch_counters(who, o.count, &cnt)) return rc;
     const uint32_t H = camera->imageH;
-    uint32_t* img = (uint32_t*)imgOrNull;
-    float4* surface = (float4*)surfaceOrNull;
-    if (skip) {
-        if (count) label_kernel<true, true><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
-        else label_kernel<true, false><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
-    } else {
-        if (count) label_kernel<false, true><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
-        else label_kernel<false, false><<<grid, block, 0, st.stream>>>(sc, t, stepSize, img, surface, labelOrNull, H, phase, stride, cnt);
-    }
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    return 0;
+    with_variant(o.skip, o.count, [&](auto sk, auto ct) {
+        label_kernel<sk, ct><<<grid, o.block, 0, st.stream>>>(sc, t, stepSize, (uint32_t*)imgOrNull, (float4*)surfaceOrNull, labelOrNull, H,
+                                                              phase, stride, cnt);
+    });
+    return launched();
 }
 
 extern "C" int svr_render_label_slices(svr_u8vec4* imgOrNull, uint8_t* labelOrNull, const svr_volume* labels, const svr_slice_params* params,
@@ -1298,22 +1265,17 @@ extern "C" int svr_render_label_slices(svr_u8vec4* imgOrNull, uint8_t* labelOrNu
 
     LabelSliceScene g;
     memset(&g, 0, sizeof(g));
-    const svr_volume& vo = *labels;
-    g.vol = vo;
+    g.vol = *labels;
     g.center = f3(p.center[0], p.center[1], p.center[2]);
     g.u = f3(p.axisU[0], p.axisU[1], p.axisU[2]);
     g.v = f3(p.axisV[0], p.axisV[1], p.axisV[2]);
     g.w = p.count > 1u ? f3(p.axisW[0], p.axisW[1], p.axisW[2]) : f3(0.f);
-    g.cmin = f3(vo.bbox.vmin.x * -vo.x_clip.x, vo.bbox.vmin.y * -vo.y_clip.x, vo.bbox.vmin.z * -vo.z_clip.x);
-    g.cmax = f3(vo.bbox.vmax.x * vo.x_clip.y, vo.bbox.vmax.y * vo.y_clip.y, vo.bbox.vmax.z * vo.z_clip.y);
+    clipped_box(*labels, &g.cmin, &g.cmax);
     g.dims = f3((float)dims.x, (float)dims.y, (float)dims.z);
     g.W = p.imageW;
     g.H = p.imageH;
-    const int block = st.options[SVR_OPT_RC_BLOCK];
-    const uint32_t tileH = (uint32_t)block / 16u;
-    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + tileH - 1u) / tileH, p.count);
-    label_slice_kernel<<<grid, block, 0, st.stream>>>(g, t, (uint32_t*)imgOrNull, labelOrNull, outline);
-    count_launch();
-    SVR_TRY(cudaGetLastError());
-    return 0;
+    const LaunchOptions o = launch_options();
+    const dim3 grid((p.imageW + 15u) / 16u, (p.imageH + o.tileH - 1u) / o.tileH, p.count);
+    label_slice_kernel<<<grid, o.block, 0, st.stream>>>(g, t, (uint32_t*)imgOrNull, labelOrNull, outline);
+    return launched();
 }

@@ -1,28 +1,21 @@
 """TEST INFRASTRUCTURE -- the CPU restatement of svr_render_isosurface (tests/isosurface_oracle.cpp, on the CPU oracle's ray
-generation, texture filter and gradient), compiled on first use into a temporary directory."""
+generation, texture filter and gradient), compiled on first use (tests/_cpp_oracle.py)."""
 import ctypes as C
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 from oracle import binding as B
 
-SRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "isosurface_oracle.cpp")
+import _cpp_oracle as O
+
 _lib = None
 
 
 def lib():
     global _lib
     if _lib is None:
-        out = os.path.join(tempfile.mkdtemp(prefix="svr_isosurface_oracle_"), "libsvr_isosurface_oracle.so")
-        # the flags of oracle/Makefile's cpu target (the distro compiler: it has libgomp)
-        subprocess.check_call(["/usr/bin/g++", "-O3", "-fopenmp", "-fno-fast-math", "-shared", "-fPIC", "-o", out, SRC])
-        lib_ = C.CDLL(out)
-        lib_.svr_oracle_isosurface.argtypes = [C.POINTER(B.OracleScene), C.c_float, C.c_float, C.POINTER(C.c_float), C.c_uint32, C.c_uint32,
-                                               C.c_uint32, C.c_void_p, C.c_void_p]
-        _lib = lib_
+        _lib = O.load("isosurface_oracle", {"svr_oracle_isosurface": [C.POINTER(B.OracleScene), C.c_float, C.c_float, C.POINTER(C.c_float),
+                                                                      C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]})
     return _lib
 
 

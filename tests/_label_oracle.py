@@ -1,30 +1,25 @@
 """TEST INFRASTRUCTURE -- the CPU restatement of svr_render_labels and svr_render_label_slices (tests/label_oracle.cpp, on the
-CPU oracle's rays), compiled on first use into a temporary directory."""
+CPU oracle's rays), compiled on first use (tests/_cpp_oracle.py)."""
 import ctypes as C
 import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 from oracle import binding as B
 from sunvolumerender_b200 import _lib as L
 
-SRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "label_oracle.cpp")
+import _cpp_oracle as O
+
 _lib = None
 
 
 def lib():
     global _lib
     if _lib is None:
-        out = os.path.join(tempfile.mkdtemp(prefix="svr_label_oracle_"), "libsvr_label_oracle.so")
-        # the flags of oracle/Makefile's cpu target (the distro compiler: it has libgomp)
-        subprocess.check_call(["/usr/bin/g++", "-O3", "-fopenmp", "-fno-fast-math", "-shared", "-fPIC", "-o", out, SRC])
-        lib_ = C.CDLL(out)
-        lib_.svr_oracle_labels.argtypes = [C.POINTER(B.OracleScene), C.c_void_p, C.c_float, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
-                                           C.c_void_p, C.c_void_p]
-        lib_.svr_oracle_label_slices.argtypes = [C.POINTER(B.OracleScene), C.POINTER(L.SliceParams), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
-        _lib = lib_
+        _lib = O.load("label_oracle", {
+            "svr_oracle_labels": [C.POINTER(B.OracleScene), C.c_void_p, C.c_float, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
+                                  C.c_void_p],
+            "svr_oracle_label_slices": [C.POINTER(B.OracleScene), C.POINTER(L.SliceParams), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]})
     return _lib
 
 

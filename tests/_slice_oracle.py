@@ -1,9 +1,6 @@
 """TEST INFRASTRUCTURE -- the CPU restatement of svr_render_slices (tests/slice_oracle.cpp, on the CPU oracle's texture
-filter), compiled on first use into a temporary directory."""
+filter), compiled on first use (tests/_cpp_oracle.py)."""
 import ctypes as C
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
@@ -11,19 +8,15 @@ from oracle import binding as B
 from sunvolumerender_b200 import _lib as L
 from sunvolumerender_b200 import scene as S
 
-SRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "slice_oracle.cpp")
+import _cpp_oracle as O
+
 _lib = None
 
 
 def lib():
     global _lib
     if _lib is None:
-        out = os.path.join(tempfile.mkdtemp(prefix="svr_slice_oracle_"), "libsvr_slice_oracle.so")
-        # the flags of oracle/Makefile's cpu target (the distro compiler: it has libgomp)
-        subprocess.check_call(["/usr/bin/g++", "-O3", "-fopenmp", "-fno-fast-math", "-shared", "-fPIC", "-o", out, SRC])
-        lib_ = C.CDLL(out)
-        lib_.svr_oracle_slices.argtypes = [C.POINTER(B.OracleScene), C.POINTER(L.SliceParams), C.c_void_p, C.c_void_p]
-        _lib = lib_
+        _lib = O.load("slice_oracle", {"svr_oracle_slices": [C.POINTER(B.OracleScene), C.POINTER(L.SliceParams), C.c_void_p, C.c_void_p]})
     return _lib
 
 

@@ -12,7 +12,6 @@ table; --json PATH also writes the results."""
 import argparse
 import json
 import os
-import subprocess
 import sys
 
 import torch
@@ -22,41 +21,9 @@ from sunvolumerender_b200 import _lib as L  # noqa: E402
 from sunvolumerender_b200 import scene as S  # noqa: E402
 from sunvolumerender_b200.render import Renderer, setup_config  # noqa: E402
 
+from gpu_projection import card, counted, events  # noqa: E402
+
 THRESHOLDS = (0.15, 0.7)
-
-
-def card():
-    name = torch.cuda.get_device_name(0)
-    try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"], capture_output=True, text=True, timeout=30)
-        return name, q.stdout.strip().splitlines()[0]
-    except Exception as e:  # the numbers below still stand; the power limit is then unknown
-        return name, f"power limit unavailable ({e})"
-
-
-def events(fn, frames=10, windows=5):
-    fn()
-    torch.cuda.synchronize()
-    best = float("inf")
-    for _ in range(windows):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(frames):
-            fn()
-        e1.record()
-        e1.synchronize()
-        best = min(best, e0.elapsed_time(e1) / frames)
-    return best
-
-
-def counted(r, fn):
-    r.set_option(L.OPT_COUNTERS, 1)
-    r.reset_counters()
-    fn()
-    torch.cuda.synchronize()
-    c = r.counters()
-    r.set_option(L.OPT_COUNTERS, 0)
-    return c
 
 
 def main():

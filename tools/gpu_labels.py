@@ -23,7 +23,7 @@ from sunvolumerender_b200 import scene as S  # noqa: E402
 from sunvolumerender_b200.render import Renderer, setup_config  # noqa: E402
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-from gpu_isosurface import card, counted, events  # noqa: E402
+from gpu_projection import card, counted, events  # noqa: E402
 
 TABLES = {"all": S.label_table(S.label_palette(3)), "bone": S.label_table({3: (1.0, 1.0, 0.9, 1.0)})}
 
