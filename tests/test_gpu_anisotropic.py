@@ -25,9 +25,9 @@ class _Cfg:  # what reference() and the helpers read from a Config
     width, height, name, fmt, dims = W, H, "aniso", L.VOXEL_U16, DIMS
 
 
-def _voxels():
+def _voxels(dims=DIMS):
     """Two overlapping ellipsoids with a dense core, u16, indexed (z, y, x); air is exactly 0."""
-    nx, ny, nz = DIMS
+    nx, ny, nz = dims
     z, y, x = np.meshgrid(np.arange(nz), np.arange(ny), np.arange(nx), indexing="ij")
     fx, fy, fz = (x + 0.5) / nx - 0.5, (y + 0.5) / ny - 0.5, (z + 0.5) / nz - 0.5
     body = 1.0 - np.sqrt((fx / 0.42) ** 2 + (fy / 0.36) ** 2 + (fz / 0.40) ** 2)

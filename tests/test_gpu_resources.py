@@ -202,13 +202,17 @@ def test_range_grid_follows_uploads_from_host_and_device(renderer, fmt, cell, di
     assert renderer.lib.svr_fused_upload_count() == fused0 + 2
     renderer.set_option(L.OPT_FUSED_UPLOAD, 1)
     assert ra_lin[..., 0].min() == 0.0 and ra_lin[..., 1].max() > 0.9
-    # against numpy on the same voxels: min / max over texels cC-1 .. (c+1)C with a zero border
+    # against numpy on the same voxels, every cell (the last one of each axis partial): min / max over texels cC-1 .. (c+1)C with
+    # a zero border
     norm = {L.VOXEL_U8: 255.0, L.VOXEL_U16: 65535.0}.get(fmt, 1.0)
-    pad = np.zeros((dims[2] + 2 * cell + 2, dims[1] + 2 * cell + 2, dims[0] + 2 * cell + 2), np.float64)
-    pad[1:1 + dims[2], 1:1 + dims[1], 1:1 + dims[0]] = a.astype(np.float64) / norm
-    for (gz, gy, gx) in ((0, 0, 0), (ra_lin.shape[0] - 1, ra_lin.shape[1] - 1, ra_lin.shape[2] - 1), (1, 1, 2)):
-        blk = pad[gz * cell:gz * cell + cell + 2, gy * cell:gy * cell + cell + 2, gx * cell:gx * cell + cell + 2]
-        assert ra_lin[gz, gy, gx, 0] == np.float32(blk.min()) and ra_lin[gz, gy, gx, 1] == np.float32(blk.max())
+    for vox, got in ((a, ra_lin), (b, rb_lin)):
+        assert got.shape[:3] == tuple(-(-d // cell) for d in dims[::-1])
+        pad = np.zeros((dims[2] + 2 * cell + 2, dims[1] + 2 * cell + 2, dims[0] + 2 * cell + 2), np.float64)
+        pad[1:1 + dims[2], 1:1 + dims[1], 1:1 + dims[0]] = vox.astype(np.float64) / norm
+        win = np.lib.stride_tricks.sliding_window_view(pad, (cell + 2,) * 3)[::cell, ::cell, ::cell]
+        win = win[:got.shape[0], :got.shape[1], :got.shape[2]]
+        assert np.array_equal(got[..., 0], win.min(axis=(3, 4, 5)).astype(np.float32))
+        assert np.array_equal(got[..., 1], win.max(axis=(3, 4, 5)).astype(np.float32))
 
 
 def test_volume_stream_equals_direct_uploads(renderer):
